@@ -238,6 +238,24 @@ def per_bounce_table(ctx, kind=0, limit=20):
     return rows
 
 
+DUMP_BYTES = 63 << 20          # the dump stays under 64 MB, .npy headers included
+
+
+def dump_outputs(dirname, film):
+    """The float4 film [H, W, 4] the timed steps summed into, as the caller reads it back, as accum.npy.  A film larger
+    than DUMP_BYTES (cfg 4 at 4K) is cut to a fixed, seeded sample of its pixels: accum.npy [n, 4] holds them in
+    ascending order and accum_pixel_index.npy [n] their row-major indices into the film (float64, exact)."""
+    import numpy as np
+    os.makedirs(dirname, exist_ok=True)
+    if film.nbytes > DUMP_BYTES:
+        flat = film.reshape(-1, 4)
+        n = DUMP_BYTES // (flat[0].nbytes + 8)
+        keep = np.sort(np.random.default_rng(0).choice(len(flat), n, replace=False))
+        film = flat[keep]
+        np.save(os.path.join(dirname, "accum_pixel_index.npy"), keep.astype(np.float64))
+    np.save(os.path.join(dirname, "accum.npy"), np.ascontiguousarray(film, np.float32))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -256,6 +274,8 @@ def main():
     ap.add_argument("--cpu-threads", type=int, default=0)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-other-configs", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the film they accumulated (rank 0, after the exchange) as DIR/accum.npy")
     args = ap.parse_args()
 
     # stdout carries exactly one JSON line: park fd 1 on stderr until then (NCCL / libraries may print)
@@ -415,6 +435,8 @@ def main():
     ms_max, ms_exchange = [float(v) for v in t.tolist()]
     rays, paths, launches, rays_ref_eq, r_closest, r_shadow, r_mis, r_mis_culled, r_tail_culled = [float(v) for v in tot.tolist()]
     value = rays / ms_max / 1e3
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, ctx.read_accum())
 
     # ---- N > 1: is the N-GPU frame the 1-GPU frame?  (outside the timed region; SURVEY 8e: max rel diff <= 1e-5)
     multi_gpu_check = None

@@ -1029,8 +1029,11 @@ long long agpt_oracle_render(void* h, int W, int H, int x0, int y0, int x1, int 
 	return (long long)(x1 - x0) * (y1 - y0) * ns;
 }
 
-long long agpt_oracle_primary_hits(void* h, int W, int H, int sample, int threads, agpt_hit* out) {
+// counters_out (optional, 3): interior visits, box tests, triangle tests of the whole table.
+long long agpt_oracle_primary_hits(void* h, int W, int H, int sample, int threads, agpt_hit* out, unsigned long long* counters_out) {
 	const OScene& sc = *(OScene*)h;
+	Counters total;
+	std::atomic<int> lock(0);
 	ParallelRows(0, H, threads, [&](int y) {
 		Counters c;
 		Rng rng;
@@ -1045,7 +1048,11 @@ long long agpt_oracle_primary_hits(void* h, int W, int H, int sample, int thread
 			o.tri = (found && hit.slot >= 0) ? MeshOfPrim(sc, sc.prims[hit.prim]).ids[hit.slot] : -1;
 			o.t = found ? hit.t : 0.f;
 		}
+		while (lock.exchange(1)) {}
+		total.Add(c);
+		lock.store(0);
 	});
+	if (counters_out) { counters_out[0] = total.interior; counters_out[1] = total.boxes; counters_out[2] = total.tris; }
 	return 0;
 }
 

@@ -103,10 +103,11 @@ class PortScene:
         names = ["rays_closest", "rays_any", "interior", "boxes", "tris", "analytic"]
         return out, dict(zip(names, list(cnt)), paths=n)
 
-    def primary_hits(self, W, H, sample, threads=0):
+    def primary_hits(self, W, H, sample, threads=0, want_counts=False):
         hits = np.zeros(W * H, HIT_DTYPE)
-        lib().agpt_oracle_primary_hits(self._h, c_int(W), c_int(H), c_int(sample), c_int(threads or os.cpu_count() or 1), hits.ctypes.data_as(c_void_p))
-        return hits
+        st = (c_ulonglong * 3)()
+        lib().agpt_oracle_primary_hits(self._h, c_int(W), c_int(H), c_int(sample), c_int(threads or os.cpu_count() or 1), hits.ctypes.data_as(c_void_p), st)
+        return (hits, dict(interior=st[0], boxes=st[1], tris=st[2])) if want_counts else hits
 
     def li_pixels(self, W, H, xs, ys, ss, max_depth, depth_arg=0):
         xs = np.ascontiguousarray(xs, np.int32); ys = np.ascontiguousarray(ys, np.int32); ss = np.ascontiguousarray(ss, np.int32)

@@ -8,6 +8,7 @@ import importlib.util
 import os
 import sys
 
+import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -43,6 +44,23 @@ def ref():
     if not ref_binding.available():
         pytest.skip("oracle/_ref/libagpt_ref.so not built (needs /root/reference at build time)")
     return ref_binding
+
+
+@pytest.fixture(scope="session")
+def ref_live():
+    """The reference's own code where oracle/_ref is built, else None: the test then compares with what
+    tests/golden/make_golden_fullsize.py stored (ref_golden)."""
+    from oracle import ref_binding
+    return ref_binding if ref_binding.available() else None
+
+
+@pytest.fixture(scope="session")
+def ref_golden():
+    def load(name):
+        g = np.load(os.path.join(ROOT, "tests", "golden", name))
+        print(f"compared with tests/golden/{name} (source: {g['source']})")
+        return g
+    return load
 
 
 @pytest.fixture(scope="session")

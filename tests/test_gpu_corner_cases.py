@@ -64,14 +64,17 @@ def test_cfg8_against_golden(agpt, gpu_ctx):
     assert same_floats(li, want).all(axis=1).mean() >= 0.97
 
 
-def test_cfg8_live_against_reference(agpt, ref, gpu_ctx):
+def test_cfg8_live_against_reference(agpt, ref_live, ref_golden, gpu_ctx):
     W, H, spp, level = 320, 180, 8, 3
     d = agpt.config_defaults(8)
-    hs = agpt.HostScene(8, level); rs = ref.RefScene(8, level)
+    hs = agpt.HostScene(8, level)
     hs.upload(gpu_ctx); gpu_ctx.set_film(W, H); gpu_ctx.clear()
     gpu_ctx.render(0, spp, d["max_depth"], d["depth_arg"])
     got = gpu_ctx.read_accum()
-    want, _ = rs.render(W, H, 0, spp, d["max_depth"], d["depth_arg"])
+    if ref_live:
+        want, _ = ref_live.RefScene(8, level).render(W, H, 0, spp, d["max_depth"], d["depth_arg"])
+    else:
+        want = ref_golden("ref_cfg8_live.npz")["rgb"]
     exact = same_floats(got[..., :3], want[..., :3]).all(axis=-1).mean()
     print(f"cfg8 live: bit-identical pixels {exact:.5f}")
     assert exact >= 0.999

@@ -32,10 +32,11 @@ def test_port_matches_golden(agpt, port, cfg):
     _, level, W, H, spp, md, da = [int(v) for v in g["case"]]
     hs = agpt.HostScene(cfg, level)
     ps = port.PortScene(hs)
-    hits = ps.primary_hits(W, H, 0)
+    hits, walk = ps.primary_hits(W, H, 0, want_counts=True)
     for f in ("found", "prim", "tri"):
         assert np.array_equal(hits[f], g["hits"][f]), f
     assert np.array_equal(bits(hits["t"]), bits(g["hits"]["t"]))
+    assert (walk["interior"], walk["boxes"], walk["tris"]) == tuple(int(v) for v in g["walk_stats"]), "walk counts differ from the reference's"
     acc, cnt = ps.render(W, H, 0, spp, md, da)
     assert np.array_equal(bits(acc), bits(g["accum"])), "accumulator differs from the reference's"
     li, draws = ps.li_pixels(W, H, g["li_xs"], g["li_ys"], g["li_ss"], md, da)
