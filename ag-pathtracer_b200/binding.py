@@ -50,10 +50,13 @@ class MeshDesc(ctypes.Structure):  # agpt_mesh_desc
 PRIM_DTYPE = np.dtype([("type", np.int32), ("payload", np.int32), ("material", np.int32), ("area_light", np.int32)])        # agpt_prim
 SPHERE_DTYPE = np.dtype([("center", np.float32, 3), ("r", np.float32), ("r2", np.float32), ("pad", np.float32, 3)])        # agpt_sphere
 PLANE_DTYPE = np.dtype([("o", np.float32, 3), ("half_x", np.float32), ("half_z", np.float32), ("pad", np.float32, 3)])     # agpt_plane
-LIGHT_DTYPE = np.dtype([("type", np.int32), ("prim", np.int32), ("pad", np.float32, 2), ("lemit", np.float32, 3), ("pad2", np.float32)])   # agpt_light
+# agpt_light; flags and pad share one sub-record so that rows written as (type, prim, (0, 0), lemit, 0) keep working
+LIGHT_DTYPE = np.dtype([("type", np.int32), ("prim", np.int32), ("ext", [("flags", np.uint32), ("pad", np.float32)]), ("lemit", np.float32, 3),
+                        ("pad2", np.float32)])
 NODE_DTYPE = np.dtype([("bmin", np.float32, 3), ("bmax", np.float32, 3), ("first", np.int32), ("count", np.int32)])        # agpt_bvh_node
 PRIM_SPHERE, PRIM_PLANE, PRIM_BVH_MESH, PRIM_MESH, PRIM_INSTANCE = 0, 1, 2, 3, 4
 LIGHT_AREA, LIGHT_UNIFORM_INFINITE, LIGHT_INFINITE_AREA = 0, 1, 2
+LIGHT_SAMPLE_SHAPE = 1     # agpt_light.flags (extension): next-event estimation samples the area light's plane or mesh
 
 
 class RawMesh:
@@ -355,6 +358,14 @@ class Context:
         in9 = np.ascontiguousarray(in9, np.float32).reshape(-1, 9)
         out = np.empty((len(in9), 8), np.float32)
         _check(core().agpt_probe_sphere_sample(self._h, c_int(len(in9)), _fptr(in9), _fptr(out)))
+        return out
+
+    def probe_light_sample(self, light, in8):
+        """Extension: Sample_Li / Pdf_Li of resident light `light` (an area light with LIGHT_SAMPLE_SHAPE on a plane or mesh).
+        in8 rows: ref point, u (2), query direction; out rows: sampled point, its pdf, Pdf_Li(query direction), light normal."""
+        in8 = np.ascontiguousarray(in8, np.float32).reshape(-1, 8)
+        out = np.empty((len(in8), 8), np.float32)
+        _check(core().agpt_probe_light_sample(self._h, c_int(light), c_int(len(in8)), _fptr(in8), _fptr(out)))
         return out
 
     def probe_stream(self, pixel_index, sample, k):

@@ -12,6 +12,9 @@
 
 #include "agpt_kernels.cuh"
 #include "agpt_multigpu.cuh"
+#include "../host/sampling.h"
+
+static inline int Blocks(size_t n, int threads) { return (int)((n + threads - 1) / threads); }
 
 // ---- error plumbing ----------------------------------------------------------------------
 static thread_local std::string g_error;
@@ -79,6 +82,11 @@ struct agpt_ctx {
 	std::vector<agpt_instance> hostInstances;
 	int nInstances = 0;
 	bool hasGlass = false;        // some material is a rough dielectric (extension): shade runs the GLASS instantiation
+	bool hasShapeLights = false;  // some area light samples its plane or mesh (extension): shade runs a SHAPES instantiation
+	bool shapesDirty = true;      // the sampling tables below follow the mesh, plane, primitive and light tables
+	DevBuf<DShapeLight> shapeLights;
+	DevBuf<float> shapeCdf;
+	std::vector<agpt_plane> hostPlanes;
 	DevBuf<int> sphereRun;
 	DevBuf<float4> sphereRunBox;
 	DevBuf<float4> keyBoxes;         // root boxes of the meshes that do not cover the scene (ray-bucket key)
@@ -202,6 +210,55 @@ static int BuildSphereRuns(agpt_ctx* c) {
 	return AGPT_OK;
 }
 
+// EXTENSION (agpt.h AGPT_LIGHT_SAMPLE_SHAPE): per light, the total area of a sampled plane or mesh and, for a mesh, the
+// Distribution1D over its triangle areas in slot order.  The areas come from the device (k_triangle_areas, the degenerate
+// flags of the upload), the sums are host/sampling.h's sequential ones.
+static int BuildShapeLights(agpt_ctx* c) {
+	const int nl = (int)c->hostLights.size();
+	std::vector<DShapeLight> table((size_t)nl);
+	std::vector<float> cdf;
+	c->hasShapeLights = false;
+	for (int i = 0; i < nl; i++) {
+		DShapeLight& e = table[i];
+		e.cdfOff = 0; e.n = 0; e.area = 0.f; e.pad = 0.f;
+		const agpt_light& l = c->hostLights[i];
+		if (l.type != AGPT_LIGHT_AREA || !(l.flags & AGPT_LIGHT_SAMPLE_SHAPE)) continue;
+		const agpt_prim& pr = c->hostPrims[l.prim];
+		if (pr.type == AGPT_PRIM_PLANE) {
+			e.area = 4.f * c->hostPlanes[pr.payload].half_x * c->hostPlanes[pr.payload].half_z;
+			c->hasShapeLights = true;
+			continue;
+		}
+		if (pr.type != AGPT_PRIM_MESH && pr.type != AGPT_PRIM_BVH_MESH) continue;      // a sphere is sampled as a sphere anyway
+		c->hasShapeLights = true;
+		const int n = (int)(c->meshStore[pr.payload].tris.n / 3);
+		if (n == 0) continue;
+		DevBuf<float> dev;
+		std::vector<float> area((size_t)n);
+		CU(dev.Alloc((size_t)n));
+		k_triangle_areas<<<Blocks(n, 256), 256, 0, c->stream>>>(c->meshStore[pr.payload].tris.p, n, dev.p);
+		CU(cudaGetLastError());
+		c->stats.kernel_launches++;
+		CU(cudaMemcpyAsync(area.data(), dev.p, (size_t)n * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
+		CU(cudaStreamSynchronize(c->stream));
+		dev.Free();
+		Distribution1D d(area.data(), n);
+		if (d.funcInt == 0) continue;                       // nothing to sample (Distribution1D's uniform fallback is not used)
+		float total = 0;
+		for (float a : area) total += a;
+		e.cdfOff = (int)cdf.size(); e.n = n; e.area = total;
+		cdf.insert(cdf.end(), d.cdf.begin(), d.cdf.end());
+	}
+	c->shapeLights.Free(); c->shapeCdf.Free();
+	if (c->hasShapeLights) {
+		CU(c->shapeLights.Upload(table.data(), table.size(), c->stream));
+		CU(c->shapeCdf.Upload(cdf.data(), cdf.size(), c->stream));
+		CU(cudaStreamSynchronize(c->stream));
+	}
+	c->shapesDirty = false;
+	return AGPT_OK;
+}
+
 static void SetBucketGrid(DScene& s, const float* lo, const float* hi) {
 	for (int a = 0; a < 3; a++) { s.cellLo[a] = lo[a]; float e = hi[a] - lo[a]; s.cellScale[a] = e > 0 ? (float)(1 << AGPT_CELL_BITS) / e : 0.f; }
 }
@@ -248,6 +305,13 @@ static int EnsureCapacity(agpt_ctx* c, size_t paths) {
 
 static int BuildSphereRuns(agpt_ctx* c);
 
+// agpt_light.flags (extension): only AGPT_LIGHT_SAMPLE_SHAPE, and only on area lights
+static int CheckLightFlags(const agpt_light& l) {
+	NEED((l.flags & ~(uint32_t)AGPT_LIGHT_SAMPLE_SHAPE) == 0, AGPT_ERR_INVALID, "unknown agpt_light.flags bits");
+	NEED(l.flags == 0 || l.type == AGPT_LIGHT_AREA, AGPT_ERR_INVALID, "AGPT_LIGHT_SAMPLE_SHAPE on a light that is not an area light");
+	return AGPT_OK;
+}
+
 static int CheckReady(agpt_ctx* c, bool needFilm) {
 	NEED(c != nullptr, AGPT_ERR_INVALID, "null context");
 	NEED(c->prims.n > 0, AGPT_ERR_STATE, "no primitives uploaded (agpt_upload_primitives)");
@@ -269,6 +333,12 @@ static int CheckReady(agpt_ctx* c, bool needFilm) {
 		NEED(l.type != AGPT_LIGHT_INFINITE_AREA || c->envW > 0, AGPT_ERR_STATE, "InfiniteAreaLight without an environment map (agpt_upload_envmap)");
 	for (auto& l : c->hostLights)
 		NEED(l.type != AGPT_LIGHT_AREA || (l.prim >= 0 && l.prim < (int)c->hostPrims.size()), AGPT_ERR_INVALID, "area light without a primitive");
+	for (auto& l : c->hostLights) {
+		int rcode = CheckLightFlags(l);
+		if (rcode != AGPT_OK) return rcode;
+		NEED(!(l.flags & AGPT_LIGHT_SAMPLE_SHAPE) || c->hostPrims[l.prim].type != AGPT_PRIM_INSTANCE, AGPT_ERR_INVALID,
+			"AGPT_LIGHT_SAMPLE_SHAPE on an instanced shape (instanced emitters are not sampled)");
+	}
 	// An AreaLight wraps exactly one shape upstream (scene.h addAreaLight; lights.h:70-86), and the exact
 	// MIS-ray cull relies on it: the primitive a light names must be the only one that names the light.
 	for (size_t i = 0; i < c->hostPrims.size(); i++) {
@@ -289,10 +359,14 @@ static int CheckReady(agpt_ctx* c, bool needFilm) {
 		int rcode = BuildSphereRuns(c);
 		if (rcode != AGPT_OK) return rcode;
 	}
+	if (c->shapesDirty) {
+		CU(cudaSetDevice(c->device));
+		int rcode = BuildShapeLights(c);
+		if (rcode != AGPT_OK) return rcode;
+	}
 	return AGPT_OK;
 }
 
-static inline int Blocks(size_t n, int threads) { return (int)((n + threads - 1) / threads); }
 
 // A film upload started by agpt_write_accum_begin may still be in flight: whatever touches the film next waits for it.
 static int JoinUpload(agpt_ctx* c) {
@@ -392,7 +466,7 @@ int agpt_destroy(agpt_ctx* c) {
 	cudaStreamSynchronize(c->stream);
 	for (int r = 0; r < c->peerWorld; r++) if (r != c->peerRank && c->peerAccum[r]) cudaIpcCloseMemHandle(c->peerAccum[r]);
 	for (auto& m : c->meshStore) m.Free();
-	c->meshes.Free(); c->instances.Free(); c->spheres.Free(); c->planes.Free(); c->prims.Free(); c->sphereRun.Free(); c->sphereRunBox.Free(); c->keyBoxes.Free(); c->mats.Free(); c->lights.Free();
+	c->meshes.Free(); c->shapeLights.Free(); c->shapeCdf.Free(); c->instances.Free(); c->spheres.Free(); c->planes.Free(); c->prims.Free(); c->sphereRun.Free(); c->sphereRunBox.Free(); c->keyBoxes.Free(); c->mats.Free(); c->lights.Free();
 	c->accumOwn.Free(); c->resolved.Free();
 	c->envRgb.Free(); c->envFunc.Free(); c->envCdf.Free();
 	for (auto& b : c->f4) b.Free();
@@ -511,6 +585,7 @@ int agpt_upload_meshes(agpt_ctx* c, const agpt_mesh_desc* meshes, int n) {
 	c->hostRoots.assign((size_t)n, agpt_bvh_node());
 	for (int i = 0; i < n; i++) { if (meshes[i].n_nodes > 0) c->hostRoots[i] = meshes[i].nodes[0]; else c->hostRoots[i].count = -1; }
 	c->runsDirty = true;
+	c->shapesDirty = true;
 	bool any = false;
 	for (int i = 0; i < n; i++) {
 		if (meshes[i].n_nodes == 0) continue;
@@ -535,9 +610,18 @@ int agpt_upload_meshes(agpt_ctx* c, const agpt_mesh_desc* meshes, int n) {
 		return AGPT_OK; \
 	}
 SIMPLE_UPLOAD(agpt_upload_spheres, agpt_sphere, spheres, c->nSpheres = n; c->hostSpheres.assign(rows, rows + n); c->runsDirty = true)
-SIMPLE_UPLOAD(agpt_upload_planes, agpt_plane, planes, c->nPlanes = n)
+SIMPLE_UPLOAD(agpt_upload_planes, agpt_plane, planes, c->nPlanes = n; c->hostPlanes.assign(rows, rows + n); c->shapesDirty = true)
 SIMPLE_UPLOAD(agpt_upload_materials, agpt_material, mats, c->nMats = n; c->hasGlass = false; for (int i = 0; i < n; i++) if (rows[i].lobes & (AGPT_LOBE_GLASS_REFLECT | AGPT_LOBE_GLASS_TRANSMIT)) c->hasGlass = true)
-SIMPLE_UPLOAD(agpt_upload_lights, agpt_light, lights, c->hostLights.assign(rows, rows + n))
+static int UploadLights(agpt_ctx* c, const agpt_light* rows, int n);
+SIMPLE_UPLOAD(UploadLights, agpt_light, lights, c->hostLights.assign(rows, rows + n); c->shapesDirty = true)
+int agpt_upload_lights(agpt_ctx* c, const agpt_light* rows, int n) {
+	// refused flags leave the resident scene as it was
+	for (int i = 0; rows != nullptr && i < n; i++) {
+		int rcode = CheckLightFlags(rows[i]);
+		if (rcode != AGPT_OK) return rcode;
+	}
+	return UploadLights(c, rows, n);
+}
 int agpt_upload_primitives(agpt_ctx* c, const agpt_prim* rows, int n) {
 	NEED(c != nullptr && n >= 0 && (n == 0 || rows != nullptr), AGPT_ERR_INVALID, "bad table");
 	CU(cudaSetDevice(c->device));
@@ -545,6 +629,7 @@ int agpt_upload_primitives(agpt_ctx* c, const agpt_prim* rows, int n) {
 	CU(c->prims.Upload(rows, (size_t)n, c->stream));
 	c->hostPrims.assign(rows, rows + n);
 	c->runsDirty = true;
+	c->shapesDirty = true;
 	CU(cudaStreamSynchronize(c->stream));
 	return AGPT_OK;
 }
@@ -594,7 +679,8 @@ int agpt_set_film(agpt_ctx* c, int width, int height) {
 
 int agpt_scene_bytes(agpt_ctx* c, uint64_t* out) {
 	NEED(c != nullptr && out != nullptr, AGPT_ERR_INVALID, "null argument");
-	uint64_t b = c->envRgb.Bytes() + c->envFunc.Bytes() + c->envCdf.Bytes() + c->meshes.Bytes() + c->spheres.Bytes() + c->planes.Bytes() + c->prims.Bytes() + c->instances.Bytes() + c->mats.Bytes() + c->lights.Bytes();
+	uint64_t b = c->envRgb.Bytes() + c->envFunc.Bytes() + c->envCdf.Bytes() + c->meshes.Bytes() + c->spheres.Bytes() + c->planes.Bytes() + c->prims.Bytes() + c->instances.Bytes() + c->mats.Bytes() + c->lights.Bytes()
+		+ c->shapeLights.Bytes() + c->shapeCdf.Bytes();
 	for (auto& m : c->meshStore) b += m.nodes.Bytes() + m.tris.Bytes() + m.normals.Bytes() + m.uvs.Bytes() + m.ids.Bytes();
 	*out = b;
 	return AGPT_OK;
@@ -807,10 +893,14 @@ static int RunWaves(agpt_ctx* c, const DScene& scIn, PathState& ps, int n, int m
 		const int shadeBlocks = Blocks(ubActive, AGPT_SHADE_THREADS);      // upper bound: blocks past the survivor count return at once
 		if (c->envW > 0) k_shade_a<true><<<Blocks(ubActive, 256), 256, 0, c->stream>>>(sc, ps, qin.active, q[cur].counts + 2, c->survivors.p, c->survivorCount.p, max_depth);
 		else k_shade_a<false><<<Blocks(ubActive, 256), 256, 0, c->stream>>>(sc, ps, qin.active, q[cur].counts + 2, c->survivors.p, c->survivorCount.p, max_depth);
-		// (ENV: the scene has an InfiniteAreaLight, GLASS: a rough-dielectric material -- each instantiation carries only what it needs)
-#define SHADE_B(E, G) k_shade_b<E, G><<<shadeBlocks, AGPT_SHADE_THREADS, 0, c->stream>>>(sc, ps, c->survivors.p, q[cur ^ 1], sp, c->rayCounters.p)
-		if (c->envW > 0) { if (c->hasGlass) SHADE_B(true, true); else SHADE_B(true, false); }
-		else { if (c->hasGlass) SHADE_B(false, true); else SHADE_B(false, false); }
+		// (ENV: the scene has an InfiniteAreaLight, GLASS: a rough-dielectric material -- each instantiation carries only what it needs;
+		// SHAPES, an area light that samples its plane or mesh: the lean one, or the one that carries everything)
+		DShapeTables st;
+		st.lights = c->shapeLights.p; st.cdf = c->shapeCdf.p;
+#define SHADE_B(E, G, S) k_shade_b<E, G, S><<<shadeBlocks, AGPT_SHADE_THREADS, 0, c->stream>>>(sc, st, ps, c->survivors.p, q[cur ^ 1], sp, c->rayCounters.p)
+		if (c->hasShapeLights) { if (c->envW > 0 || c->hasGlass) SHADE_B(true, true, true); else SHADE_B(false, false, true); }
+		else if (c->envW > 0) { if (c->hasGlass) SHADE_B(true, true, false); else SHADE_B(true, false, false); }
+		else { if (c->hasGlass) SHADE_B(false, true, false); else SHADE_B(false, false, false); }
 #undef SHADE_B
 		c->stats.kernel_launches++;
 		c->stats.kernel_launches++; c->stats.launches_shade++;
@@ -1464,6 +1554,24 @@ __global__ void k_probe_sphere_sample(int n, const float* in9, float* out8) {
 	o[7] = SpherePdfFrom(s, f3(a[4], a[5], a[6]));
 }
 
+// EXTENSION: Sample_Li / Pdf_Li of one sampled plane / mesh light through the same functions k_shade_b runs.  No early
+// return: the mesh walk of Pdf_Li votes with the whole warp.
+__global__ void __launch_bounds__(128) k_probe_light_sample(DScene sc, DShapeTables st, int light, int n, const float* in8, float* out8) {
+	__shared__ unsigned stack[AGPT_SHADE_STACK_SMEM * 128];
+	const int i = blockIdx.x * blockDim.x + threadIdx.x;
+	const bool lane = i < n;
+	const float* a = in8 + 8 * (lane ? i : 0);
+	const float3 refP = f3(a[0], a[1], a[2]);
+	float3 p = f3(0.f), nn = f3(0.f);
+	float pdf = 0.f;
+	if (lane) ShapeSampleFrom(sc, st, light, sc.prims[sc.lights[light].prim], refP, make_float2(a[3], a[4]), &p, &nn, &pdf);
+	const float pdfLi = ShapePdfLi<AGPT_SHADE_STACK_SMEM>(sc, st, light, refP, f3(a[5], a[6], a[7]), stack + threadIdx.x, 128, lane);
+	if (lane) {
+		float* o = out8 + 8 * i;
+		o[0] = p.x; o[1] = p.y; o[2] = p.z; o[3] = pdf; o[4] = pdfLi; o[5] = nn.x; o[6] = nn.y; o[7] = nn.z;
+	}
+}
+
 __global__ void k_probe_stream(uint32_t pixel, uint32_t sample, int k, float* out) {
 	uint32_t s = StreamSeed(pixel, sample);
 	for (int i = 0; i < k; i++) out[i] = RandomFloat(s);
@@ -1517,6 +1625,23 @@ int agpt_probe_sphere_sample(agpt_ctx* c, int n, const float* in9, float* out8) 
 	CU(cudaSetDevice(c->device));
 	return ProbeRun(c, in9, 9 * (size_t)n, out8, 8 * (size_t)n, [&](const float* din, float* dout) {
 		k_probe_sphere_sample<<<Blocks(n, 128), 128, 0, c->stream>>>(n, din, dout);
+	});
+}
+
+int agpt_probe_light_sample(agpt_ctx* c, int light, int n, const float* in8, float* out8) {
+	NEED(c != nullptr && n > 0 && in8 && out8, AGPT_ERR_INVALID, "bad probe arguments");
+	int rcode = CheckReady(c, false);
+	if (rcode != AGPT_OK) return rcode;
+	NEED(light >= 0 && light < (int)c->hostLights.size(), AGPT_ERR_INVALID, "light index out of range");
+	const agpt_light& l = c->hostLights[light];
+	NEED(l.type == AGPT_LIGHT_AREA && (l.flags & AGPT_LIGHT_SAMPLE_SHAPE) && c->hostPrims[l.prim].type != AGPT_PRIM_SPHERE, AGPT_ERR_INVALID,
+		"not an area light that samples its plane or mesh (AGPT_LIGHT_SAMPLE_SHAPE)");
+	CU(cudaSetDevice(c->device));
+	const DScene sc = MakeScene(c);
+	DShapeTables st;
+	st.lights = c->shapeLights.p; st.cdf = c->shapeCdf.p;
+	return ProbeRun(c, in8, 8 * (size_t)n, out8, 8 * (size_t)n, [&](const float* din, float* dout) {
+		k_probe_light_sample<<<Blocks(n, 128), 128, 0, c->stream>>>(sc, st, light, n, din, dout);
 	});
 }
 

@@ -43,6 +43,18 @@ struct DMesh {
 	int n_nodes, n_tris;
 };
 
+// EXTENSION: sampling table of a plane or mesh area light with AGPT_LIGHT_SAMPLE_SHAPE (agpt.h), one per light.
+struct DShapeLight {
+	int cdfOff;              // meshes: Distribution1D::cdf over the triangle areas in slot order at shapeCdf[cdfOff .. cdfOff + n]
+	int n;                   // triangles
+	float area;              // total area; 0: never sampled (not a sampled shape light, or nothing to sample)
+	float pad;
+};
+struct DShapeTables {        // passed beside DScene, to the kernels that sample shapes only
+	const DShapeLight* lights;       // n_lights entries, or nullptr when no light samples its shape
+	const float* cdf;
+};
+
 struct DScene {
 	const agpt_prim* prims;
 	const int* sphereRun;            // per primitive: length of the run of sphere primitives with consecutive payloads starting here (0: not a sphere)
@@ -521,4 +533,59 @@ __device__ __forceinline__ bool PlaneTest(const agpt_plane& p, float3 O, float3 
 	float v = (P.z - p.o[2]) / p.half_z;
 	if (fabsf(u) <= 1 && fabsf(v) <= 1) { tOut = t; return true; }
 	return false;
+}
+
+// ---------------------------------------------------------------------------------------
+// EXTENSION: Sample_Li of a plane or mesh area light with AGPT_LIGHT_SAMPLE_SHAPE (agpt.h; CPU statement:
+// oracle/agpt_shape_oracle.cpp ShapeSample).  PBRT-v3's Shape::Sample(ref, u) in solid angle: SampleDiscrete over the area cdf
+// (FindInterval as sampling.h:4-18), UniformSampleTriangle on the remapped u.x and u.y; a plane samples its rectangle.
+// ---------------------------------------------------------------------------------------
+__device__ __forceinline__ float ShapeSolidAnglePdf(float d2, float3 n, float3 wi, float area) {
+	float c = absdot(n, wi);
+	if (c == 0) return 0.f;
+	float pdf = d2 / (c * area);
+	return isinf(pdf) ? 0.f : pdf;
+}
+__device__ __forceinline__ float3 TriangleGeomNormal(const float4* tri) {
+	float4 a = tri[0], b = tri[1], c = tri[2];
+	float3 v0 = f3(a.x, a.y, a.z);
+	return normalize(cross(f3(b.x, b.y, b.z) - v0, f3(c.x, c.y, c.z) - v0));
+}
+__device__ __forceinline__ void ShapeSampleFrom(const DScene& sc, const DShapeTables& st, int light, const agpt_prim& pr, float3 refP, float2 u, float3* pOut, float3* nOut, float* pdf) {
+	const DShapeLight sl = st.lights[light];
+	*pdf = 0.f; *pOut = f3(0.f); *nOut = f3(0.f);
+	if (!(sl.area > 0)) return;
+	float3 p, n;
+	if (pr.type == AGPT_PRIM_PLANE) {
+		const agpt_plane& pl = sc.planes[pr.payload];
+		p = f3(pl.o[0] + (2 * u.x - 1) * pl.half_x, pl.o[1], pl.o[2] + (2 * u.y - 1) * pl.half_z);
+		n = f3(0.f, 1.f, 0.f);
+	}
+	else {
+		const float* cdf = st.cdf + sl.cdfOff;
+		const int size = sl.n + 1;
+		int first = 0, len = size;
+		while (len > 0) {
+			int half = len >> 1, middle = first + half;
+			if (cdf[middle] <= u.x) { first = middle + 1; len -= half + 1; }
+			else len = half;
+		}
+		const int offset = min(max(first - 1, 0), size - 2);
+		const float width = cdf[offset + 1] - cdf[offset];
+		if (!(width > 0)) return;                          // a zero-area triangle (u.x == 1 can land on one at the end)
+		const float ur = (u.x - cdf[offset]) / width;
+		const float4* tri = sc.meshes[pr.payload].tris + 3 * offset;
+		float4 a = tri[0], b = tri[1], c = tri[2];
+		float3 v0 = f3(a.x, a.y, a.z), v1 = f3(b.x, b.y, b.z), v2 = f3(c.x, c.y, c.z);
+		float su0 = sqrtf(ur);
+		float b0 = 1 - su0, b1 = u.y * su0;
+		p = b0 * v0 + b1 * v1 + (1 - b0 - b1) * v2;
+		n = normalize(cross(v1 - v0, v2 - v0));
+	}
+	*pOut = p; *nOut = n;
+	float3 wi = p - refP;
+	float d2 = sqrLength(wi);
+	if (d2 == 0) return;
+	wi /= sqrtf(d2);
+	*pdf = ShapeSolidAnglePdf(d2, n, wi, sl.area);
 }

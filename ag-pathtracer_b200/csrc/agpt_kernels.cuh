@@ -486,9 +486,16 @@ __global__ void __launch_bounds__(256) k_shade_a(DScene sc, PathState ps, const 
 #ifndef AGPT_SHADE_MIN_BLOCKS
 #define AGPT_SHADE_MIN_BLOCKS 1
 #endif
+// SHAPES instantiation: traversal-stack entries per thread in shared memory for the light-only walk of a mesh light (the
+// rest in local memory, as in the trace kernels).  8 x 768 threads = 24 KB: emissive meshes are small, their trees shallow.
+#define AGPT_SHADE_STACK_SMEM 8
 
-template <bool ENV, bool GLASS>
-__global__ void __launch_bounds__(AGPT_SHADE_THREADS, AGPT_SHADE_MIN_BLOCKS) k_shade_b(DScene sc, PathState ps, const int* __restrict__ survivors, WaveQueues qout, ShadeParams sp, RayCounters* rc) {
+// SHAPES (extension): some area light samples its plane or mesh (AGPT_LIGHT_SAMPLE_SHAPE); other scenes run the
+// instantiations without that code.
+template <bool ENV, bool GLASS, bool SHAPES>
+__global__ void __launch_bounds__(AGPT_SHADE_THREADS, AGPT_SHADE_MIN_BLOCKS) k_shade_b(DScene sc, DShapeTables st, PathState ps, const int* __restrict__ survivors, WaveQueues qout, ShadeParams sp,
+		RayCounters* rc) {
+	__shared__ unsigned shapeStack[SHAPES ? AGPT_SHADE_STACK_SMEM * AGPT_SHADE_THREADS : 1];
 	const int lane = threadIdx.x & 31;
 	const int count = *sp.count;
 	// one block-sized piece of the list per block, no loop: warps that start together stay together
@@ -556,6 +563,7 @@ __global__ void __launch_bounds__(AGPT_SHADE_THREADS, AGPT_SHADE_MIN_BLOCKS) k_s
 		DRay vis;
 		vis.O = f3(0.f); vis.D = f3(0.f); vis.t = 0.f;
 		int lightType = -1, lightPrimType = -1, lightPayload = 0;
+		bool lightShape = false;          // SHAPES: the chosen light samples its plane or mesh
 		VertexBsdfInit<GLASS>(vb, si, mat, wo);       // cheap enough to run unconditionally (keeps vb defined for idle threads)
 		if (full) {
 			doNee = !BSDF_IsPerfectlySpecular(vb.b) && sc.n_lights > 0;
@@ -572,12 +580,14 @@ __global__ void __launch_bounds__(AGPT_SHADE_THREADS, AGPT_SHADE_MIN_BLOCKS) k_s
 				lemit = f3(light.lemit);
 				lightType = light.type;
 				if (lightType == AGPT_LIGHT_AREA) {
-					// AreaLight::Sample_Li (lights.cpp:115-126); only spheres can be sampled
+					// AreaLight::Sample_Li (lights.cpp:115-126); upstream can sample spheres only, the extension planes and meshes
 					const agpt_prim& lp = sc.prims[light.prim];
 					lightPrimType = lp.type; lightPayload = lp.payload;
-					if (lp.type == AGPT_PRIM_SPHERE) {
+					lightShape = SHAPES && lp.type != AGPT_PRIM_SPHERE && (light.flags & AGPT_LIGHT_SAMPLE_SHAPE);
+					if (lp.type == AGPT_PRIM_SPHERE || lightShape) {
 						float3 pS, nS;
-						SphereSampleFrom(sc.spheres[lp.payload], si.p, uLight, &pS, &nS, &lightPdf);
+						if (lp.type == AGPT_PRIM_SPHERE) SphereSampleFrom(sc.spheres[lp.payload], si.p, uLight, &pS, &nS, &lightPdf);
+						else ShapeSampleFrom(sc, st, numLight, lp, si.p, uLight, &pS, &nS, &lightPdf);
 						if (lightPdf == 0 || sqrLength(pS - si.p) == 0) lightPdf = 0;
 						else {
 							wiL = pS - si.p;
@@ -641,6 +651,14 @@ __global__ void __launch_bounds__(AGPT_SHADE_THREADS, AGPT_SHADE_MIN_BLOCKS) k_s
 		// largest possible ray.t), a uniform sky needs Pdf_Li != 0 (lights.cpp:26-28).  Where it cannot, the BSDF value at
 		// that direction -- one of this vertex's three evaluations -- is never used, and is not computed.  (With
 		// AGPT_FLAG_COUNTERS it is: whether the reference would have traced the ray depends on that value being non-black.)
+		// A sampled plane / mesh light's Pdf_Li is exact for the same reason the sky's is: it depends on the direction only.  It is
+		// the light-only intersection phase E needs as the MIS pdf, taken here by the whole warp (the mesh walk votes).
+		float shapeLp = 0.f;
+		if (SHAPES) {
+			const bool q = full && doNee && smpMis.ok && lightShape;
+			shapeLp = ShapePdfLi<AGPT_SHADE_STACK_SMEM>(sc, st, numLight, si.p, q ? LocalToWorld(vb.b, smpMis.wi) : f3(0.f, 1.f, 0.f), shapeStack + threadIdx.x,
+				AGPT_SHADE_THREADS, q);
+		}
 		bool misUseful = true;
 		if (full && doNee && smpMis.ok && !sp.exact_counts) {
 			const float3 wim = LocalToWorld(vb.b, smpMis.wi);
@@ -651,6 +669,7 @@ __global__ void __launch_bounds__(AGPT_SHADE_THREADS, AGPT_SHADE_MIN_BLOCKS) k_s
 					float tLight;
 					misUseful = SphereTest(sc.spheres[lightPayload], mr.O, mr.D, mr.t, tLight);
 				}
+				else if (SHAPES && lightShape) misUseful = shapeLp != 0;
 			}
 			else if (!(ENV && lightType == AGPT_LIGHT_INFINITE_AREA)) misUseful = dot(si.n, wim) > 0;
 		}
@@ -710,7 +729,7 @@ __global__ void __launch_bounds__(AGPT_SHADE_THREADS, AGPT_SHADE_MIN_BLOCKS) k_s
 					f *= absdot(wim, si.sn);
 					if (!IsBlack(f) && scatteringPdf > 0) {
 						float lp;
-						if (lightType == AGPT_LIGHT_AREA) lp = lightPrimType == AGPT_PRIM_SPHERE ? SpherePdfFrom(sc.spheres[lightPayload], si.p) : 0.f;
+						if (lightType == AGPT_LIGHT_AREA) lp = lightPrimType == AGPT_PRIM_SPHERE ? SpherePdfFrom(sc.spheres[lightPayload], si.p) : (SHAPES && lightShape) ? shapeLp : 0.f;
 						else if (ENV && lightType == AGPT_LIGHT_INFINITE_AREA) lp = EnvPdfLi(sc, wim);
 						else lp = dot(si.n, wim) > 0 ? AGPT_INV2PI : 0.f;       // lights.cpp:26-28 (geometric n)
 						if (lp != 0) {
@@ -724,9 +743,10 @@ __global__ void __launch_bounds__(AGPT_SHADE_THREADS, AGPT_SHADE_MIN_BLOCKS) k_s
 							// Sphere::Intersect test Scene::Intersect would run, with the largest possible
 							// ray.t -- nothing it could hit matters, so it is not traced.  Same result, far
 							// fewer closest-hit rays for small or distant lights (Sphere::Pdf never checks
-							// that wi points at the sphere, intersectable.h:306-317, so upstream traces them all).
+							// that wi points at the sphere, intersectable.h:306-317, so upstream traces them all).  A sampled plane / mesh
+							// light's ray met the shape already (lp != 0).
 							float tLight;
-							bool canReachLight = lightType != AGPT_LIGHT_AREA || SphereTest(sc.spheres[lightPayload], mr.O, mr.D, mr.t, tLight);
+							bool canReachLight = lightType != AGPT_LIGHT_AREA || (SHAPES && lightShape) || SphereTest(sc.spheres[lightPayload], mr.O, mr.D, mr.t, tLight);
 							misCulled = !canReachLight;
 							ps.neeMis[path] = make_float4(term.x, term.y, term.z, __int_as_float(numLight));
 							ps.misO[path] = make_float4(mr.O.x, mr.O.y, mr.O.z, mr.t);
@@ -902,4 +922,14 @@ __global__ void k_flag_degenerate(float4* tris, const float2* uvs, int n) {
 	float3 dpdu, dpdv;
 	bool ok = TriangleDerivatives(f3(a.x, a.y, a.z), f3(b.x, b.y, b.z), f3(c.x, c.y, c.z), uv0, uv1, uv2, dpdu, dpdv);
 	tris[3 * j].w = ok ? 0.f : 1.f;
+}
+
+// ---- EXTENSION: sampling tables of the plane / mesh area lights (AGPT_LIGHT_SAMPLE_SHAPE): triangle areas in slot order,
+// 0 for a triangle k_flag_degenerate marked (CPU statement: oracle/agpt_shape_oracle.cpp BuildShapeLights)
+__global__ void k_triangle_areas(const float4* __restrict__ tris, int n, float* area) {
+	int j = blockIdx.x * blockDim.x + threadIdx.x;
+	if (j >= n) return;
+	float4 a = tris[3 * j], b = tris[3 * j + 1], c = tris[3 * j + 2];
+	float3 v0 = f3(a.x, a.y, a.z);
+	area[j] = a.w != 0.f ? 0.f : 0.5f * length(cross(f3(b.x, b.y, b.z) - v0, f3(c.x, c.y, c.z) - v0));
 }

@@ -129,11 +129,12 @@ __device__ __forceinline__ const DMesh& MeshOfPrim(const DScene& sc, const agpt_
 // tests is the reference's; the root tests just happen in lockstep instead of one loop step
 // each (a typical ray hits 1-2 of 5 roots).
 // `lane` is false for threads without a ray; they must still call (full-mask votes).
-template <bool ANY, bool COUNT, bool FAST, bool INST>
+// SMEM: stack entries per thread in shared memory (the rest of the AGPT_STACK_SMEM + AGPT_STACK_LOCAL levels in local memory).
+template <bool ANY, bool COUNT, bool FAST, bool INST, int SMEM = AGPT_STACK_SMEM>
 __device__ __forceinline__ bool TraceMeshRun(const DScene& sc, int p0, int p1, float3 O, float3 D, float3 rD, bool filterOk, float& rayT, HitRecord& hit,
 		unsigned* stack, int stackStride, TraceCounters& cnt, bool lane) {
 	bool found = false;
-	unsigned local[AGPT_STACK_LOCAL];
+	unsigned local[AGPT_STACK_SMEM + AGPT_STACK_LOCAL - SMEM];
 	unsigned cand = 0;               // meshes of the run this lane still has to enter (bit m - p0)
 	unsigned bvhMask = 0;            // meshes of the run that have a root box
 	const float rayT0 = rayT;
@@ -241,7 +242,7 @@ __device__ __forceinline__ bool TraceMeshRun(const DScene& sc, int p0, int p1, f
 					if (hl && hr) {
 						unsigned farE = swapKids ? el : er;
 						AGPT_CHECK(sp < AGPT_STACK_SMEM + AGPT_STACK_LOCAL, AGPT_DBG_STACK, sp);
-						if (sp < AGPT_STACK_SMEM) stack[sp * stackStride] = farE; else local[sp - AGPT_STACK_SMEM] = farE;
+						if (sp < SMEM) stack[sp * stackStride] = farE; else local[sp - SMEM] = farE;
 						sp++;
 						cur = swapKids ? er : el;
 						pop = false;
@@ -271,7 +272,7 @@ __device__ __forceinline__ bool TraceMeshRun(const DScene& sc, int p0, int p1, f
 					if (sp == 0) inside = false;
 					else {
 						sp--;
-						cur = (sp < AGPT_STACK_SMEM) ? stack[sp * stackStride] : local[sp - AGPT_STACK_SMEM];
+						cur = (sp < SMEM) ? stack[sp * stackStride] : local[sp - SMEM];
 					}
 				}
 			}
@@ -356,6 +357,43 @@ __device__ __forceinline__ bool TraceScene(const DScene& sc, float3 O, float3 D,
 		}
 	}
 	return found;
+}
+
+// EXTENSION: Pdf_Li of a plane or mesh area light with AGPT_LIGHT_SAMPLE_SHAPE (agpt.h; CPU statement: oracle/agpt_shape_oracle.cpp
+// ShapePdf) -- PBRT-v3's Shape::Pdf(ref, wi): the ray MakeRay(refP + EPSILON wi, wi) against the light's shape ALONE
+// (Plane::Intersect, or the mesh's own closest-hit walk, TraceMeshRun over the one-primitive run), 0 without a hit, else
+// dist^2 / (|cos| * area) at the hit.  Every lane of the warp must call (lane = false: no query): the walk votes with full masks.
+template <int SMEM>
+__device__ __forceinline__ float ShapePdfLi(const DScene& sc, const DShapeTables& st, int light, float3 refP, float3 wi, unsigned* stack, int stackStride, bool lane) {
+	DShapeLight sl;
+	sl.area = 0.f;
+	if (lane) sl = st.lights[light];
+	lane = lane && sl.area > 0;
+	const int primIdx = lane ? sc.lights[light].prim : 0;
+	const agpt_prim pr = sc.prims[primIdx];
+	DRay r;
+	r.O = refP; r.D = f3(1.f, 0.f, 0.f); r.t = FLT_MAX;
+	if (lane) r = MakeRay(refP + AGPT_EPSILON * wi, wi);
+	bool found = false;
+	float t = 0.f;
+	float3 n = f3(0.f, 1.f, 0.f);
+	if (lane && pr.type == AGPT_PRIM_PLANE) found = PlaneTest(sc.planes[pr.payload], r.O, r.D, r.t, t);
+	const bool mesh = lane && pr.type != AGPT_PRIM_PLANE;
+	if (__any_sync(0xffffffffu, mesh)) {
+		HitRecord hit;
+		hit.prim = -1; hit.slot = -1; hit.t = 0.f; hit.b1 = 0.f; hit.b2 = 0.f;
+		TraceCounters cnt = { 0, 0, 0, 0, 0, 0 };
+		float rayT = r.t;
+		const float3 rD = f3(1.0f / r.D.x, 1.0f / r.D.y, 1.0f / r.D.z);
+		if (TraceMeshRun<false, false, true, false, SMEM>(sc, primIdx, primIdx + 1, r.O, r.D, rD, FilterOk<true>(r.O, r.D), rayT, hit, stack, stackStride, cnt, mesh)) {
+			found = true;
+			t = hit.t;
+			n = TriangleGeomNormal(sc.meshes[pr.payload].tris + 3 * hit.slot);
+		}
+	}
+	if (!found) return 0.f;
+	float3 p = r.O + t * r.D;
+	return ShapeSolidAnglePdf(sqrLength(p - refP), n, wi, sl.area);
 }
 
 // Warp-aggregated flush of per-thread counters: one atomic per counter per warp.  `totals` = 8 counters of

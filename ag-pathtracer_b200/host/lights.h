@@ -19,6 +19,7 @@ public:
 	virtual bool IsInfinite() const { return false; }
 	virtual int Kind() const = 0;      // AGPT_LIGHT_*
 	virtual float3 Emission() const = 0;
+	virtual uint32_t Flags() const { return 0; }   // agpt_light.flags
 };
 
 class UniformInfiniteLight : public Light {
@@ -41,6 +42,16 @@ public:
 	shared_ptr<Intersectable> Shape;
 protected:
 	const float3 Lemit;
+};
+
+// EXTENSION (not a reference class; agpt.h AGPT_LIGHT_SAMPLE_SHAPE): an AreaLight whose Plane, TriangleMesh or BVHTriMesh
+// next-event estimation samples (PBRT-v3's Shape::Sample / Pdf, one light for the whole mesh).  Emission stays two-sided.
+// Scene::addSampledAreaLight makes one; a plain AreaLight keeps the reference's behaviour.
+#define AGPT_HAS_SAMPLED_AREA_LIGHTS 1
+class SampledAreaLight : public AreaLight {
+public:
+	SampledAreaLight(shared_ptr<Intersectable> shape, const float3& l) : AreaLight(shape, l) {}
+	uint32_t Flags() const override { return AGPT_LIGHT_SAMPLE_SHAPE; }
 };
 
 // Environment light over a lat-long HDR map with importance sampling (upstream builds with ILS

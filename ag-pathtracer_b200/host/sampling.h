@@ -4,7 +4,7 @@
 // total); sampling it (SampleContinuous, :38-53) is device code.
 #pragma once
 
-#include "precomp.h"
+#include <vector>        // (no precomp.h: the library's CUDA translation unit builds its light tables with this too)
 
 struct Distribution1D {
 	Distribution1D(const float* f, int n) : func(f, f + n), cdf(n + 1) {

@@ -80,6 +80,11 @@ public:
 		primitives.push_back(shape);
 		lights.push_back(make_shared<AreaLight>(shape, L));
 	}
+	// EXTENSION: the same, with the shape sampled for next-event estimation (host/lights.h SampledAreaLight)
+	void addSampledAreaLight(std::shared_ptr<Intersectable> shape, const float3& L) {
+		primitives.push_back(shape);
+		lights.push_back(make_shared<SampledAreaLight>(shape, L));
+	}
 
 	// Object graph -> device tables.  Materials are de-duplicated by pointer.
 	std::shared_ptr<FlatScene> Flatten() const {
@@ -159,6 +164,7 @@ public:
 			agpt_light rec;
 			memset(&rec, 0, sizeof(rec));
 			rec.type = l->Kind();
+			rec.flags = l->Flags();
 			rec.prim = -1;
 			if (rec.type == AGPT_LIGHT_AREA) {
 				auto it = primIndex.find(static_cast<const AreaLight*>(l.get())->Shape.get());

@@ -43,6 +43,7 @@ inline ConfigDefaults Defaults(int config) {
 	case 8: return { 640, 360, 16, 6, 4, "cfg8_test_degenerate_triangles_deep_tree_overflowing_light" };
 	case 9: return { 3840, 2160, 1024, 8, 0, "cfg9_ext_cfg4_with_true_instances_one_mesh_8_placements" };
 	case 10: return { 1920, 1080, 64, 16, 0, "cfg10_ext_cfg5_rough_glass_rr_by_bounce" };
+	case 11: return { 1920, 1080, 64, 16, 4, "cfg11_ext_cfg5_sampled_panel_plane_and_mesh_lights" };
 	default: return { 0, 0, 0, 0, 0, "unknown" };
 	}
 }
@@ -524,6 +525,41 @@ inline void BuildConfig10(Scene* scene, int level) {
 }
 #endif
 
+#ifdef AGPT_HAS_SAMPLED_AREA_LIGHTS
+// cfg 11 (EXTENSION, host mirror only -- the reference cannot sample a plane or a mesh): cfg 5's room and objects lit by
+// three SAMPLED area lights (Scene::addSampledAreaLight) instead of the sphere: a two-triangle TriangleMesh panel just below
+// the ceiling, a Plane panel a little lower (no coplanar ties with the ceiling or with the other panel) and a small
+// emissive BVHTriMesh icosphere (level 2).  Without the flag the walls would be lit only through specular chains.
+inline void BuildConfig11(Scene* scene, int level) {
+	auto wall = DisneyMaterial::Make(float3(.73f, .73f, .73f), 1.f, 0.f);
+	auto room = MakeRoom(float3(-4, -1, -9), float3(4, 5, 4), wall);
+	scene->primitives.push_back(std::make_shared<BVHTriMesh>(room, wall, 1));
+	auto roughMetal = DisneyMaterial::Make(float3(0.912f, 0.914f, 0.920f), .6f, 1.f);
+	auto diffuse = DisneyMaterial::Make(float3(.2f, .45f, .7f), 1.f, 0.f);
+	auto a = MakeIcosphere(level, float3(-1.4f, .2f, .5f), 1.2f, roughMetal);
+	auto b = MakeIcosphere(level, float3(1.4f, .2f, -.5f), 1.2f, diffuse);
+	scene->primitives.push_back(std::make_shared<BVHTriMesh>(a, roughMetal, 1));
+	scene->primitives.push_back(std::make_shared<BVHTriMesh>(b, diffuse, 1));
+	{
+		// 1.6 x 1.2 panel at y = 4.97, facing down
+		std::vector<float3> vertices = { float3(-.8f, 4.97f, -2.2f), float3(.8f, 4.97f, -2.2f), float3(.8f, 4.97f, -1.f), float3(-.8f, 4.97f, -1.f) };
+		std::vector<float3> normals(4, float3(0, -1, 0));
+		std::vector<float2> texcoords;
+		std::vector<index_type> indices;
+		for (int v : { 0, 2, 1, 0, 3, 2 }) indices.push_back(index_type(v));
+		scene->addSampledAreaLight(std::make_shared<TriangleMesh>(indices, vertices, normals, texcoords, nullptr), WarmWhite(6));
+	}
+	scene->addSampledAreaLight(std::make_shared<Plane>(float3(-2.2f, 4.93f, -5.f), float2(1.f, 1.f), nullptr), WarmWhite(8));
+	scene->addSampledAreaLight(std::make_shared<BVHTriMesh>(MakeIcosphere(2, float3(2.3f, 2.2f, -3.5f), .3f, nullptr), nullptr, 1), WarmWhite(10));
+	scene->camera.lookfrom = float3(0, 1.8f, -8.5f);
+	scene->camera.lookat = float3(0, .6f, 0);
+	scene->camera.vup = float3(0, 1, 0);
+	scene->camera.aspect_ratio = 16.f / 9.f;
+	scene->camera.vfov = 40;
+	scene->camera.aperture = 0;
+}
+#endif
+
 // level <= 0 selects the BASELINE.json size of each configuration.
 inline bool BuildConfig(Scene* scene, int config, int level) {
 	switch (config) {
@@ -540,6 +576,9 @@ inline bool BuildConfig(Scene* scene, int config, int level) {
 #endif
 #ifdef AGPT_HAS_GLASS
 	case 10: BuildConfig10(scene, level > 0 ? level : 7); return true;
+#endif
+#ifdef AGPT_HAS_SAMPLED_AREA_LIGHTS
+	case 11: BuildConfig11(scene, level > 0 ? level : 7); return true;
 #endif
 	default: return false;
 	}

@@ -3,7 +3,7 @@
 // headless on one or several GPUs and writing the displayed frame (Accumulator::CopyToSurface
 // semantics) as a PPM.
 //
-//   make -C ag-pathtracer_b200 example && build/render_ppm out.ppm <config 1..8> <spp> [gpus]
+//   make -C ag-pathtracer_b200 example && build/render_ppm out.ppm <config 1..11> <spp> [gpus]
 //
 // With gpus > 1 the samples are split by index over the GPUs (SURVEY 8e) and the accumulators are
 // summed and resolved by one fused kernel per GPU over NVLink peer memory (agpt_reduce_resolve).

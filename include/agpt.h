@@ -133,11 +133,32 @@ typedef struct agpt_material {
 
 enum { AGPT_LIGHT_AREA = 0, AGPT_LIGHT_UNIFORM_INFINITE = 1, AGPT_LIGHT_INFINITE_AREA = 2 };
 
+/* agpt_light.flags */
+enum {
+	/* EXTENSION (not reference behaviour: upstream's Plane and TriangleMesh inherit Sample / Pdf stubs that return pdf 0,
+	 * so an emissive quad or mesh lights only what sees it directly or through a mirror).  On an AGPT_LIGHT_AREA light
+	 * whose shape is an AGPT_PRIM_PLANE, AGPT_PRIM_MESH or AGPT_PRIM_BVH_MESH, next-event estimation samples the shape,
+	 * as PBRT-v3's Shape::Sample / Shape::Pdf do, stated on the CPU in oracle/agpt_shape_oracle.cpp:
+	 *   - the whole mesh is one light: a triangle is picked by Distribution1D::SampleDiscrete(uLight.x) over the triangle
+	 *     areas 0.5 * |cross(v1 - v0, v2 - v0)| in slot (leaf) order, and the remapped uLight.x with uLight.y picks a point
+	 *     by UniformSampleTriangle; degenerate triangles (the ones a hit would reject) have area 0 and are never picked;
+	 *     a plane picks a uniform point of its rectangle, o + ((2 u.x - 1) half_x, 0, (2 u.y - 1) half_z);
+	 *   - the light normal is the geometric one (plane: +y), emission stays two-sided, the solid-angle pdf is
+	 *     dist^2 / (|cos| * total area) and 0 where the cosine is 0 or the total area is 0;
+	 *   - the MIS pdf (Pdf_Li) intersects the MIS ray with the light's shape ALONE and is 0 when it misses;
+	 *   - only the two uLight numbers the vertex draws anyway are used: every later draw of a path stays where it was.
+	 * Without the flag a scene renders exactly as the reference does; on a sphere the flag changes nothing (spheres are
+	 * sampled already).  The flag on a non-area light, on an instanced shape (AGPT_PRIM_INSTANCE) or any other bit set
+	 * is refused with AGPT_ERR_INVALID. */
+	AGPT_LIGHT_SAMPLE_SHAPE = 1u
+};
+
 /* Scene::lights in list order (lights.h:37-51,72-87). */
 typedef struct agpt_light {
 	int32_t type;        /* AGPT_LIGHT_* */
 	int32_t prim;        /* AREA: scene primitive index of the emitting shape; else -1 */
-	float pad[2];
+	uint32_t flags;      /* AGPT_LIGHT_SAMPLE_SHAPE or 0 */
+	float pad;
 	float lemit[3];
 	float pad2;
 } agpt_light;
@@ -234,7 +255,7 @@ int agpt_upload_planes(agpt_ctx* ctx, const agpt_plane* planes, int n);
 int agpt_upload_primitives(agpt_ctx* ctx, const agpt_prim* prims, int n);
 int agpt_upload_instances(agpt_ctx* ctx, const agpt_instance* instances, int n);  /* EXTENSION; rows of AGPT_PRIM_INSTANCE point here */
 int agpt_upload_materials(agpt_ctx* ctx, const agpt_material* materials, int n);
-int agpt_upload_lights(agpt_ctx* ctx, const agpt_light* lights, int n);
+int agpt_upload_lights(agpt_ctx* ctx, const agpt_light* lights, int n);   /* refuses bad flags (see agpt_light.flags), scene unchanged */
 int agpt_upload_envmap(agpt_ctx* ctx, const agpt_envmap* env);          /* NULL clears it */
 int agpt_set_camera(agpt_ctx* ctx, const agpt_camera* camera);          /* Camera, camera.h:38-56 */
 int agpt_set_film(agpt_ctx* ctx, int width, int height);                /* Accumulator(w,h), myapp.h:10-13 */
@@ -349,6 +370,10 @@ int agpt_probe_bsdf(agpt_ctx* ctx, int n, const agpt_material* mat, const float*
 /* Sphere::Sample(ref,u) / Sphere::Pdf (intersectable.h:239-317): in9 = center3 r refp3 u2;
  * out8 = p3 n3 pdf pdf_only. */
 int agpt_probe_sphere_sample(agpt_ctx* ctx, int n, const float* in9, float* out8);
+/* EXTENSION: Sample_Li / Pdf_Li of resident light `light`, which must be an area light with AGPT_LIGHT_SAMPLE_SHAPE on a
+ * plane or mesh (agpt_light.flags): in8 = ref point3 u2 query direction3; out8 = sampled point3, its solid-angle pdf,
+ * Pdf_Li(ref, query direction), light normal3 at the sampled point. */
+int agpt_probe_light_sample(agpt_ctx* ctx, int light, int n, const float* in8, float* out8);
 /* First k floats of the RNG stream of (pixel_index, sample) (SURVEY 8a row 3). */
 int agpt_probe_stream(agpt_ctx* ctx, uint32_t pixel_index, uint32_t sample, int k, float* out);
 
