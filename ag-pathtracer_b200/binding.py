@@ -77,6 +77,15 @@ class RawMesh:
                         ptr(self.normals), ptr(self.uvs))
 
 
+class Adaptive(ctypes.Structure):  # agpt_adaptive (extension: adaptive sampling)
+    _fields_ = [("min_samples", c_int32), ("max_samples", c_int32), ("step", c_int32), ("tolerance", c_float), ("floor", c_float)]
+
+
+def adaptive(min_samples, max_samples, step, tolerance, floor=0.0):
+    """agpt_adaptive record; the convergence test it parameterises is stated in include/agpt.h and oracle/adaptive.py."""
+    return Adaptive(int(min_samples), int(max_samples), int(step), float(tolerance), float(floor))
+
+
 class Stats(ctypes.Structure):  # agpt_stats
     _fields_ = [(n, c_uint64) for n in ("paths", "rays_closest", "rays_shadow", "rays_mis", "rays_skip", "rays_mis_culled", "rays_tail_culled")] + \
                [(n, c_uint64 * 2) for n in ("node_visits", "box_tests", "tri_tests", "analytic_tests", "warp_steps", "lane_steps")] + \
@@ -256,6 +265,37 @@ class Context:
     def resolve(self, samples):
         out = np.empty((self.height, self.width), np.uint32)
         _check(core().agpt_resolve(self._h, c_int(samples), out.ctypes.data_as(POINTER(c_uint32))))
+        return out
+
+    # ---- adaptive sampling (extension) -------------------------------------------------------------
+    def set_moments(self, enable=True):
+        """Per-pixel moments (sum of squares per channel, sample count) beside the film; off by default."""
+        _check(core().agpt_set_moments(self._h, c_int(1 if enable else 0)))
+
+    def read_moments(self, out=None):
+        """float32 [H, W, 4] in the film's row order: .xyz = sum of c*c, .w = samples added."""
+        if out is None:
+            out = np.empty((self.height, self.width, 4), np.float32)
+        _check(core().agpt_read_moments(self._h, _fptr(out)))
+        return out
+
+    def adaptive_select(self, params, want_pixels=True):
+        """The convergence test over the film: (count, film pixel indices y*W + x of the selected pixels, or None)."""
+        n = c_int(0)
+        buf = np.empty(self.width * self.height, np.int32) if want_pixels else None
+        _check(core().agpt_adaptive_select(self._h, byref(params), None if buf is None else buf.ctypes.data_as(POINTER(c_int32)), byref(n)))
+        return n.value, (None if buf is None else buf[:n.value].copy())
+
+    def render_adaptive(self, params, max_depth, depth_arg=0, flags=0):
+        """A frame from scratch, adaptively: returns (rounds, camera paths)."""
+        rounds = c_int(0); paths = c_int64(0)
+        _check(core().agpt_render_adaptive(self._h, byref(params), c_int(max_depth), c_int(depth_arg), c_uint32(flags), byref(rounds), byref(paths)))
+        return rounds.value, paths.value
+
+    def resolve_counts(self):
+        """agpt_resolve with each pixel's own sample count (moments .w)."""
+        out = np.empty((self.height, self.width), np.uint32)
+        _check(core().agpt_resolve_counts(self._h, out.ctypes.data_as(POINTER(c_uint32))))
         return out
 
     def trace_primary(self, sample, flags=0):
@@ -559,6 +599,14 @@ class HostTracer:
                                                       c_int(first_sample), c_int(num_samples), c_int(depth_arg), c_uint32(flags),
                                                       out.ctypes.data_as(POINTER(c_uint32))), host_side=True)
         return out
+
+    def render_adaptive(self, scene, width, height, accum, params, depth_arg=0, flags=0):
+        """CudaPathTracer::RenderAdaptive: the film replaces `accum`; returns the per-pixel sample counts [H, W] (row 0 = top)."""
+        assert accum.dtype == np.float32 and accum.shape == (height, width, 4) and accum.flags.c_contiguous
+        counts = np.empty((height, width), np.int32)
+        _check(host().agpt_host_tracer_render_adaptive(self._h, scene.handle, c_int(width), c_int(height), _fptr(accum), byref(params),
+                                                       c_int(depth_arg), c_uint32(flags), counts.ctypes.data_as(POINTER(c_int32))), host_side=True)
+        return counts
 
     def li(self, scene, origin, direction, depth_arg=0):
         o = (c_float * 3)(*origin); d = (c_float * 3)(*direction); out = (c_float * 3)()

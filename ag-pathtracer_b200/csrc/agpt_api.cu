@@ -2,6 +2,7 @@
 // wavefront kernels.  Host code here only moves tables into HBM, sizes launches and drives
 // the wave loop; every ray is traced and shaded on the device.  There is no CPU path: if no
 // CUDA device can be opened agpt_create() fails and the caller gets the CUDA error text.
+#include <cmath>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -115,6 +116,11 @@ struct agpt_ctx {
 	DevBuf<float4> accumOwn;
 	DevBuf<uint32_t> resolved;    // agpt_resolve's packed output, kept between calls
 	float4* accum = nullptr;      // accumOwn.p or caller-owned
+	// adaptive sampling (agpt_set_moments): per-pixel sum of squares and sample count, always context-owned
+	bool momentsOn = false;
+	DevBuf<float4> moments;
+	DevBuf<int> adaptiveList;     // agpt_adaptive_select's compacted pixel list (W*H) and its length
+	DevBuf<int> adaptiveCount;
 
 	// wavefront state
 	size_t capacity = 0;          // path slots allocated
@@ -468,6 +474,7 @@ int agpt_destroy(agpt_ctx* c) {
 	for (auto& m : c->meshStore) m.Free();
 	c->meshes.Free(); c->shapeLights.Free(); c->shapeCdf.Free(); c->instances.Free(); c->spheres.Free(); c->planes.Free(); c->prims.Free(); c->sphereRun.Free(); c->sphereRunBox.Free(); c->keyBoxes.Free(); c->mats.Free(); c->lights.Free();
 	c->accumOwn.Free(); c->resolved.Free();
+	c->moments.Free(); c->adaptiveList.Free(); c->adaptiveCount.Free();
 	c->envRgb.Free(); c->envFunc.Free(); c->envCdf.Free();
 	for (auto& b : c->f4) b.Free();
 	for (auto& b : c->i32) b.Free();
@@ -661,6 +668,16 @@ int agpt_set_camera(agpt_ctx* c, const agpt_camera* cam) {
 	return AGPT_OK;
 }
 
+// moments, pixel list and count for the current film, zeroed
+static int AllocMoments(agpt_ctx* c) {
+	const size_t wh = (size_t)c->width * c->height;
+	CU(c->moments.Alloc(wh));
+	CU(c->adaptiveList.Alloc(wh));
+	if (!c->adaptiveCount.p) CU(c->adaptiveCount.Alloc(1));
+	CU(cudaMemsetAsync(c->moments.p, 0, c->moments.Bytes(), c->stream));
+	return AGPT_OK;
+}
+
 int agpt_set_film(agpt_ctx* c, int width, int height) {
 	JOIN(c);
 	NEED(c != nullptr && width > 0 && height > 0 && (long long)width * height < (1ll << 30), AGPT_ERR_INVALID, "bad film size");
@@ -673,6 +690,10 @@ int agpt_set_film(agpt_ctx* c, int width, int height) {
 		CU(c->accumOwn.Alloc((size_t)width * height));
 		c->accum = c->accumOwn.p;
 		CU(cudaMemsetAsync(c->accum, 0, c->accumOwn.Bytes(), c->stream));
+	}
+	if (c->momentsOn) {
+		int rcode = AllocMoments(c);
+		if (rcode != AGPT_OK) return rcode;
 	}
 	return AGPT_OK;
 }
@@ -692,6 +713,7 @@ int agpt_clear(agpt_ctx* c) {
 	NEED(c != nullptr && c->accum != nullptr, AGPT_ERR_STATE, "film not set");
 	CU(cudaSetDevice(c->device));
 	CU(cudaMemsetAsync(c->accum, 0, (size_t)c->width * c->height * sizeof(float4), c->stream));
+	if (c->momentsOn) CU(cudaMemsetAsync(c->moments.p, 0, c->moments.Bytes(), c->stream));
 	return AGPT_OK;
 }
 int agpt_accum_ptr_dev(agpt_ctx* c, void** p) {
@@ -977,7 +999,7 @@ int agpt_render(agpt_ctx* c, int first_sample, int num_samples, int sample_strid
 		GenParams g;
 		memset(&g, 0, sizeof(g));
 		g.n = n; g.first_sample = first_sample + done * sample_stride; g.sample_stride = sample_stride; g.tiled = 1; g.samples = ns;
-		k_generate<<<Blocks(n, 256), 256, 0, c->stream>>>(sc, ps, q0, g);
+		k_generate<false><<<Blocks(n, 256), 256, 0, c->stream>>>(sc, ps, q0, g);
 		CU(cudaGetLastError());
 		c->stats.kernel_launches++;
 		c->stats.paths += (uint64_t)n;
@@ -985,7 +1007,8 @@ int agpt_render(agpt_ctx* c, int first_sample, int num_samples, int sample_strid
 		rcode = RunWaves(c, sc, ps, n, max_depth, rr_depth_arg, flags);
 		if (rcode != AGPT_OK) return rcode;
 		if (c->uploadPending) CU(cudaStreamWaitEvent(c->stream, c->evUpload, 0));      // the film this batch adds to may still be on its way (agpt_write_accum_begin)
-		k_accumulate<<<Blocks(wh, 256), 256, 0, c->stream>>>(ps.Lout, c->accum, c->width, c->height, ns);
+		if (c->momentsOn) k_accumulate<true, false><<<Blocks(wh, 256), 256, 0, c->stream>>>(ps.Lout, c->accum, c->width, c->height, ns, c->moments.p);
+		else k_accumulate<false, false><<<Blocks(wh, 256), 256, 0, c->stream>>>(ps.Lout, c->accum, c->width, c->height, ns);
 		CU(cudaGetLastError());
 		c->stats.kernel_launches++;
 	}
@@ -995,6 +1018,161 @@ int agpt_render(agpt_ctx* c, int first_sample, int num_samples, int sample_strid
 	float ms = 0;
 	cudaEventElapsedTime(&ms, r0, r1);
 	c->stats.ms_render += ms;
+	return AGPT_OK;
+}
+
+// ---- adaptive sampling (EXTENSION, agpt.h agpt_adaptive) ----------------------------------------------------------------
+int agpt_set_moments(agpt_ctx* c, int enable) {
+	JOIN(c);
+	NEED(c != nullptr, AGPT_ERR_INVALID, "null context");
+	CU(cudaSetDevice(c->device));
+	CU(cudaStreamSynchronize(c->stream));
+	if (!enable) {
+		c->momentsOn = false;
+		c->moments.Free(); c->adaptiveList.Free(); c->adaptiveCount.Free();
+		return AGPT_OK;
+	}
+	if (c->momentsOn) return AGPT_OK;
+	if (c->width > 0) {                      // (else agpt_set_film allocates them)
+		int rcode = AllocMoments(c);
+		if (rcode != AGPT_OK) { c->moments.Free(); c->adaptiveList.Free(); c->adaptiveCount.Free(); return rcode; }
+	}
+	c->momentsOn = true;
+	return AGPT_OK;
+}
+
+int agpt_read_moments(agpt_ctx* c, float* host) {
+	JOIN(c);
+	NEED(c != nullptr && host != nullptr, AGPT_ERR_INVALID, "null argument");
+	NEED(c->momentsOn && c->moments.p != nullptr, AGPT_ERR_STATE, "moments are off (agpt_set_moments) or film not set");
+	CU(cudaSetDevice(c->device));
+	CU(cudaMemcpyAsync(host, c->moments.p, c->moments.Bytes(), cudaMemcpyDeviceToHost, c->stream));
+	CU(cudaStreamSynchronize(c->stream));
+	return AGPT_OK;
+}
+
+static int CheckAdaptive(const agpt_adaptive* p) {
+	NEED(p != nullptr, AGPT_ERR_INVALID, "null agpt_adaptive");
+	NEED(p->min_samples >= 2 && p->min_samples <= p->max_samples && p->max_samples <= (1 << 24), AGPT_ERR_INVALID,
+		"agpt_adaptive: need 2 <= min_samples <= max_samples <= 1<<24");
+	NEED(p->step >= 1, AGPT_ERR_INVALID, "agpt_adaptive: step < 1");
+	NEED(std::isfinite(p->tolerance) && p->tolerance >= 0.f && std::isfinite(p->floor) && p->floor >= 0.f, AGPT_ERR_INVALID,
+		"agpt_adaptive: tolerance and floor must be finite and >= 0");
+	return AGPT_OK;
+}
+
+// The convergence test over the film -> c->adaptiveList[0, *count) on the device, *count on the host.
+static int SelectPixels(agpt_ctx* c, const agpt_adaptive& a, int* count) {
+	const int wh = c->width * c->height;
+	CU(cudaMemsetAsync(c->adaptiveCount.p, 0, sizeof(int), c->stream));
+	k_adaptive_select<<<Blocks(wh, 256), 256, 0, c->stream>>>(c->accum, c->moments.p, c->width, c->height, a.max_samples, a.step, a.tolerance, a.floor,
+		c->adaptiveList.p, c->adaptiveCount.p);
+	CU(cudaGetLastError());
+	c->stats.kernel_launches++;
+	CU(cudaMemcpyAsync(count, c->adaptiveCount.p, sizeof(int), cudaMemcpyDeviceToHost, c->stream));
+	CU(cudaStreamSynchronize(c->stream));
+	return AGPT_OK;
+}
+
+int agpt_adaptive_select(agpt_ctx* c, const agpt_adaptive* params, int32_t* pixels_out, int* n_out) {
+	JOIN(c);
+	NEED(c != nullptr && n_out != nullptr, AGPT_ERR_INVALID, "null argument");
+	int rcode = CheckAdaptive(params);
+	if (rcode != AGPT_OK) return rcode;
+	NEED(c->momentsOn && c->moments.p != nullptr && c->accum != nullptr, AGPT_ERR_STATE, "moments are off (agpt_set_moments) or film not set");
+	CU(cudaSetDevice(c->device));
+	int n = 0;
+	rcode = SelectPixels(c, *params, &n);
+	if (rcode != AGPT_OK) return rcode;
+	if (pixels_out && n > 0) {
+		CU(cudaMemcpyAsync(pixels_out, c->adaptiveList.p, (size_t)n * sizeof(int), cudaMemcpyDeviceToHost, c->stream));
+		CU(cudaStreamSynchronize(c->stream));
+	}
+	*n_out = n;
+	return AGPT_OK;
+}
+
+// One adaptive round: samples [n_p, n_p + step) of the `count` pixels of c->adaptiveList, through the wave loop of agpt_render.
+// A batch holds whole pixels (at most maxPathsPerBatch / step of them, at least one).
+static int RenderListed(agpt_ctx* c, int count, int step, int maxSamples, int max_depth, int rr_depth_arg, uint32_t flags) {
+	size_t perBatch = c->maxPathsPerBatch / (size_t)step;
+	if (perBatch < 1) perBatch = 1;
+	if (perBatch > (size_t)count) perBatch = (size_t)count;
+	int rcode = EnsureCapacity(c, perBatch * step);
+	if (rcode != AGPT_OK) return rcode;
+	DScene sc = MakeScene(c);
+	PathState ps = MakePathState(c);
+	WaveQueues q0;
+	q0.closest = c->queues[0].p; q0.shadow = c->queues[2].p; q0.active = c->queues[4].p; q0.counts = c->counts.p; q0.keys = nullptr; q0.shadowKeys = nullptr;
+	CU(cudaEventRecord(c->evRender0, c->stream));
+	for (int done = 0; done < count; done += (int)perBatch) {
+		const int np = count - done < (int)perBatch ? count - done : (int)perBatch;
+		const int n = np * step;
+		GenParams g;
+		memset(&g, 0, sizeof(g));
+		g.n = n; g.samples = step; g.list = c->adaptiveList.p; g.listBase = done; g.listCount = count; g.moments = c->moments.p; g.maxSamples = maxSamples;
+		k_generate<true><<<Blocks(n, 256), 256, 0, c->stream>>>(sc, ps, q0, g);
+		CU(cudaGetLastError());
+		c->stats.kernel_launches++;
+		c->stats.paths += (uint64_t)n;
+		c->stats.rays_closest += (uint64_t)n;
+		rcode = RunWaves(c, sc, ps, n, max_depth, rr_depth_arg, flags);
+		if (rcode != AGPT_OK) return rcode;
+		k_accumulate<true, true><<<Blocks(np, 256), 256, 0, c->stream>>>(ps.Lout, c->accum, c->width, c->height, step, c->moments.p, c->adaptiveList.p + done, np, maxSamples);
+		CU(cudaGetLastError());
+		c->stats.kernel_launches++;
+	}
+	CU(cudaEventRecord(c->evRender1, c->stream));
+	CU(cudaStreamSynchronize(c->stream));
+	float ms = 0;
+	cudaEventElapsedTime(&ms, c->evRender0, c->evRender1);
+	c->stats.ms_render += ms;
+	return AGPT_OK;
+}
+
+int agpt_render_adaptive(agpt_ctx* c, const agpt_adaptive* params, int max_depth, int rr_depth_arg, uint32_t flags, int* rounds_out, int64_t* paths_out) {
+	NEED(c != nullptr, AGPT_ERR_INVALID, "null context");
+	int rcode = CheckAdaptive(params);
+	if (rcode != AGPT_OK) return rcode;
+	NEED(max_depth >= 0, AGPT_ERR_INVALID, "bad depth");
+	NEED(c->momentsOn, AGPT_ERR_STATE, "moments are off (agpt_set_moments)");
+	rcode = CheckReady(c, true);
+	if (rcode != AGPT_OK) return rcode;
+	NEED(c->accum != nullptr && c->moments.p != nullptr, AGPT_ERR_STATE, "no accumulator");
+	const agpt_adaptive a = *params;
+	rcode = agpt_clear(c);                                  // film and moments
+	if (rcode != AGPT_OK) return rcode;
+	rcode = agpt_render(c, 0, a.min_samples, 1, max_depth, rr_depth_arg, flags);
+	if (rcode != AGPT_OK) return rcode;
+	int64_t paths = (int64_t)c->width * c->height * a.min_samples;
+	int rounds = 0;
+	while (true) {
+		int n = 0;
+		rcode = SelectPixels(c, a, &n);
+		if (rcode != AGPT_OK) return rcode;
+		if (n == 0) break;
+		rcode = RenderListed(c, n, a.step, a.max_samples, max_depth, rr_depth_arg, flags);
+		if (rcode != AGPT_OK) return rcode;
+		rounds++;
+		paths += (int64_t)n * a.step;
+	}
+	if (rounds_out) *rounds_out = rounds;
+	if (paths_out) *paths_out = paths;
+	return AGPT_OK;
+}
+
+int agpt_resolve_counts(agpt_ctx* c, uint32_t* host) {
+	JOIN(c);
+	NEED(c != nullptr && host != nullptr && c->accum != nullptr, AGPT_ERR_STATE, "film not set");
+	NEED(c->momentsOn && c->moments.p != nullptr, AGPT_ERR_STATE, "moments are off (agpt_set_moments)");
+	CU(cudaSetDevice(c->device));
+	int n = c->width * c->height;
+	if (c->resolved.n != (size_t)n) CU(c->resolved.Alloc(n));
+	k_resolve_counts<<<Blocks(n, 256), 256, 0, c->stream>>>(c->accum, c->moments.p, c->resolved.p, n);
+	CU(cudaGetLastError());
+	c->stats.kernel_launches++;
+	CU(cudaMemcpyAsync(host, c->resolved.p, n * sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream));
+	CU(cudaStreamSynchronize(c->stream));
 	return AGPT_OK;
 }
 
@@ -1028,7 +1206,7 @@ int agpt_trace_primary(agpt_ctx* c, int sample, uint32_t flags, agpt_hit* out_ho
 	GenParams g;
 	memset(&g, 0, sizeof(g));
 	g.n = (int)wh; g.first_sample = sample; g.sample_stride = 1;
-	k_generate<<<Blocks(wh, 256), 256, 0, c->stream>>>(sc, ps, q0, g);
+	k_generate<false><<<Blocks(wh, 256), 256, 0, c->stream>>>(sc, ps, q0, g);
 	CU(cudaGetLastError());
 	c->stats.kernel_launches++;
 	return TraceTable(c, sc, ps.rayO, ps.rayD, (int)wh, 0, flags, out_host);
@@ -1055,7 +1233,7 @@ int agpt_trace_rays(agpt_ctx* c, int64_t n, const float* rays7, int any_hit, uin
 	GenParams g;
 	memset(&g, 0, sizeof(g));
 	g.n = (int)n; g.rays7 = rays.p; g.seeds = seeds.p; g.raysFinal = (flags & AGPT_FLAG_RAYS_FINAL) ? 1 : 0;
-	k_generate<<<Blocks(n, 256), 256, 0, c->stream>>>(sc, ps, q0, g);
+	k_generate<false><<<Blocks(n, 256), 256, 0, c->stream>>>(sc, ps, q0, g);
 	CU(cudaGetLastError());
 	c->stats.kernel_launches++;
 	rcode = TraceTable(c, sc, ps.rayO, ps.rayD, (int)n, any_hit, flags, out_host);
@@ -1071,7 +1249,7 @@ static int LiGeneric(agpt_ctx* c, GenParams g, int max_depth, int rr_depth_arg, 
 	PathState ps = MakePathState(c);
 	WaveQueues q0;
 	q0.closest = c->queues[0].p; q0.shadow = c->queues[2].p; q0.active = c->queues[4].p; q0.counts = c->counts.p; q0.keys = nullptr; q0.shadowKeys = nullptr;
-	k_generate<<<Blocks(n, 256), 256, 0, c->stream>>>(sc, ps, q0, g);
+	k_generate<false><<<Blocks(n, 256), 256, 0, c->stream>>>(sc, ps, q0, g);
 	CU(cudaGetLastError());
 	c->stats.kernel_launches++;
 	c->stats.paths += (uint64_t)n;

@@ -227,6 +227,12 @@ struct GenParams {
 	int raysFinal;         // rays7 directions are unit length already (a host Ray object): use as given
 	int tiled;             // whole-film mode of agpt_render: slot = tile-order pixel slot * samples + sample (else sample-major rows)
 	int samples;           // samples per pixel in this batch (tiled mode)
+	// list mode (k_generate<true>, adaptive rounds): slot = (list entry - listBase) * samples + j renders sample n_p + j of
+	// pixel list[entry], n_p = the pixel's moments .w (the samples it has so far)
+	const int* list;       // film pixel indices y * W + x
+	int listBase, listCount;
+	const float4* moments; // per pixel, film row order (H-1-y)
+	int maxSamples;        // (debug checks) no pixel may pass it
 };
 
 // Path slot <-> pixel.  Rendering keeps the samples of a pixel in neighbouring slots and orders
@@ -248,13 +254,26 @@ __device__ __forceinline__ int PixelToSlot(int x, int y, int width, int height, 
 	return y * width + x;
 }
 
+template <bool LIST>
 __global__ void __launch_bounds__(256) k_generate(DScene sc, PathState ps, WaveQueues q, GenParams g) {
 	int i = blockIdx.x * blockDim.x + threadIdx.x;
 	if (i == 0 && q.counts) { q.counts[0] = g.n; q.counts[1] = 0; q.counts[2] = g.n; }   // wave 0: n camera rays, n paths to shade
 	if (i >= g.n) return;
 	DRay ray;
 	uint32_t rng;
-	if (g.rays7) {
+	if constexpr (LIST) {
+		// the step samples of a listed pixel sit next to each other, like the samples of a pixel in the tiled mode
+		const int entry = g.listBase + i / g.samples, j = i % g.samples;
+		AGPT_CHECK(entry >= 0 && entry < g.listCount, AGPT_DBG_LIST, entry);
+		const int pixel = g.list[entry];
+		AGPT_CHECK(pixel >= 0 && pixel < sc.width * sc.height, AGPT_DBG_LIST, pixel);
+		const int x = pixel % sc.width, y = pixel / sc.width;
+		const int have = (int)g.moments[(size_t)(sc.height - 1 - y) * sc.width + x].w;
+		AGPT_CHECK(have >= 0 && have + g.samples <= g.maxSamples, AGPT_DBG_SAMPLE, have);
+		rng = StreamSeed((uint32_t)pixel, (uint32_t)(have + j));
+		ray = CameraRay(sc, x, y, rng);
+	}
+	else if (g.rays7) {
 		const float* r = g.rays7 + 7 * (size_t)i;
 		if (g.raysFinal) { ray.O = f3(r[0], r[1], r[2]); ray.D = f3(r[3], r[4], r[5]); ray.t = r[6]; }
 		else ray = MakeRay(f3(r[0], r[1], r[2]), f3(r[3], r[4], r[5]), r[6]);
@@ -863,21 +882,91 @@ __global__ void __launch_bounds__(AGPT_SHADE_THREADS, AGPT_SHADE_MIN_BLOCKS) k_s
 // ---- accumulate: myapp.cpp:169-173 + Accumulator::AddSample (myapp.h:17-19) --------------
 // One thread per pixel adds its samples of this batch in ascending sample order, the order
 // the reference's successive Ticks add them in.
-__global__ void __launch_bounds__(256) k_accumulate(const float4* __restrict__ Lout, float4* accum, int width, int height, int samplesInBatch) {
+// MOMENTS (agpt_set_moments): the same filtered sample c also adds c * c per channel to moments.xyz and 1 to moments.w, in the
+// same order.  LIST (adaptive rounds): one thread per entry of list[0, listCount), whose samplesInBatch samples sit at
+// Lout[entry * samplesInBatch ..] (k_generate<true>); film and moments of pixel list[entry].  <false, false> is agpt_render's.
+template <bool MOMENTS, bool LIST>
+__global__ void __launch_bounds__(256) k_accumulate(const float4* __restrict__ Lout, float4* accum, int width, int height, int samplesInBatch,
+		float4* moments = nullptr, const int* __restrict__ list = nullptr, int listCount = 0, int maxSamples = 0) {
 	int pixel = blockIdx.x * blockDim.x + threadIdx.x;
 	int wh = width * height;
-	if (pixel >= wh) return;
+	size_t slot;
+	if constexpr (LIST) {
+		if (pixel >= listCount) return;
+		slot = (size_t)pixel * samplesInBatch;
+		pixel = list[pixel];
+		AGPT_CHECK(pixel >= 0 && pixel < wh, AGPT_DBG_LIST, pixel);
+	}
+	else if (pixel >= wh) return;
 	int x = pixel % width, y = pixel / width;
-	const size_t slot = (size_t)PixelToSlot(x, y, width, height, true) * samplesInBatch;       // agpt_render generates tiled
+	if constexpr (!LIST) slot = (size_t)PixelToSlot(x, y, width, height, true) * samplesInBatch;       // agpt_render generates tiled
 	float4* dst = accum + (size_t)(height - 1 - y) * width + x;
 	float4 a = *dst;
+	float4 m;
+	if constexpr (MOMENTS) {
+		m = moments[dst - accum];
+		AGPT_CHECK(!LIST || (int)m.w + samplesInBatch <= maxSamples, AGPT_DBG_SAMPLE, (int)m.w);
+	}
 	for (int s = 0; s < samplesInBatch; s++) {
 		float4 c = Lout[slot + s];
 		float lum = 0.212671f * c.x + 0.715160f * c.y + 0.072169f * c.z;     // Luminance (precomp.h:717)
 		if (isnan(c.x) || isnan(c.y) || isnan(c.z) || isinf(lum)) c = make_float4(0.f, 0.f, 0.f, 0.f);
 		a.x += c.x; a.y += c.y; a.z += c.z;
+		if constexpr (MOMENTS) { m.x += c.x * c.x; m.y += c.y * c.y; m.z += c.z * c.z; m.w += 1.f; }
 	}
 	*dst = a;
+	if constexpr (MOMENTS) moments[dst - accum] = m;
+}
+
+// ---- adaptive sampling: the convergence test of agpt_adaptive_select (agpt.h), per pixel ------------------------------
+// Film sum a, moments q and count n of one channel; every operation rounded on its own (--fmad=false, IEEE / and sqrt).
+// True: the channel's standard error is not (yet) within tolerance, or not finite.
+__device__ __forceinline__ bool ChannelUnconverged(float a, float q, float n, float tolerance, float floor_) {
+	float mu = a / n;
+	float d = q - a * mu;
+	float v = d / (n - 1.f);
+	v = v < 0.f ? 0.f : v;                      // (a NaN stays NaN)
+	float se = sqrtf(v / n);
+	float thr = tolerance * (mu > floor_ ? mu : floor_);
+	return !(se <= thr);
+}
+__device__ __forceinline__ bool PixelSelected(float4 a, float4 q, int maxSamples, int step, float tolerance, float floor_) {
+	if (!((long long)q.w + step <= maxSamples)) return false;
+	return ChannelUnconverged(a.x, q.x, q.w, tolerance, floor_) || ChannelUnconverged(a.y, q.y, q.w, tolerance, floor_) ||
+		ChannelUnconverged(a.z, q.z, q.w, tolerance, floor_);
+}
+// One thread per pixel, pixels in the tiled slot order of agpt_render (8x4 tiles), so neighbouring list entries are
+// neighbouring pixels and a round's warps cover compact patches.  The selected pixels of a block are compacted with
+// warp ballots and a shared-memory prefix over the warps, one global atomic per block, as the queue appends of k_shade_b.
+__global__ void __launch_bounds__(256) k_adaptive_select(const float4* __restrict__ accum, const float4* __restrict__ moments, int width, int height,
+		int maxSamples, int step, float tolerance, float floor_, int* __restrict__ list, int* count) {
+	__shared__ int warpCount[8];
+	__shared__ int blockBase;
+	const int i = blockIdx.x * blockDim.x + threadIdx.x;
+	const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+	bool sel = false;
+	int pixel = 0;
+	if (i < width * height) {
+		int x, y;
+		SlotToPixel(i, width, height, true, x, y);
+		pixel = y * width + x;
+		const size_t f = (size_t)(height - 1 - y) * width + x;
+		sel = PixelSelected(accum[f], moments[f], maxSamples, step, tolerance, floor_);
+	}
+	const unsigned m = __ballot_sync(0xffffffffu, sel);
+	if (lane == 0) warpCount[warp] = __popc(m);
+	__syncthreads();
+	if (threadIdx.x == 0) {
+		int total = 0;
+		for (int w = 0; w < 8; w++) { int c = warpCount[w]; warpCount[w] = total; total += c; }
+		blockBase = total ? atomicAdd(count, total) : 0;
+	}
+	__syncthreads();
+	if (sel) {
+		const int at = blockBase + warpCount[warp] + __popc(m & ((1u << lane) - 1u));
+		AGPT_CHECK(at >= 0 && at < width * height, AGPT_DBG_LIST, at);
+		list[at] = pixel;
+	}
 }
 
 // ---- resolve: Accumulator::CopyToSurface (myapp.h:34-41) + lin2rgb / rgb2uint (common.h:41-51)
@@ -895,6 +984,13 @@ __global__ void __launch_bounds__(256) k_resolve(const float4* __restrict__ accu
 	int i = blockIdx.x * blockDim.x + threadIdx.x;
 	if (i >= n) return;
 	out[i] = ResolvePixel(accum[i], samples);
+}
+// agpt_resolve_counts: each pixel divided by its own sample count (moments .w); a pixel without samples resolves to 0
+__global__ void __launch_bounds__(256) k_resolve_counts(const float4* __restrict__ accum, const float4* __restrict__ moments, uint32_t* out, int n) {
+	int i = blockIdx.x * blockDim.x + threadIdx.x;
+	if (i >= n) return;
+	const float s = moments[i].w;
+	out[i] = s > 0.f ? ResolvePixel(accum[i], s) : 0u;
 }
 
 // ---- bandwidth probe: what a plain streaming read of this library's own making reaches on this GPU ----

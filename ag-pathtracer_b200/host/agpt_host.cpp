@@ -245,6 +245,19 @@ int agpt_host_tracer_render_resolve(agpt_host_tracer* t, agpt_host_scene* s, int
 	return AGPT_OK;
 }
 
+int agpt_host_tracer_render_adaptive(agpt_host_tracer* t, agpt_host_scene* s, int width, int height, float* host_rgba,
+		const agpt_adaptive* params, int depth_arg, uint32_t flags, int32_t* host_counts) {
+	if (!t || !s || !host_rgba || !params || !host_counts) return HostFail("null argument");
+	g_hostError.clear();
+	HOST_TRY(
+		Accumulator acc(width, height, reinterpret_cast<float3*>(host_rgba));
+		std::vector<int> counts;
+		t->tracer->RenderAdaptive(s->scene, *s->camera, acc, *params, depth_arg, counts, flags);
+		std::copy(counts.begin(), counts.end(), host_counts);
+	)
+	return AGPT_OK;
+}
+
 int agpt_host_tracer_li(agpt_host_tracer* t, agpt_host_scene* s, const float* o, const float* d, int depth_arg, float* out3) {
 	if (!t || !s || !o || !d || !out3) return HostFail("null argument");
 	g_hostError.clear();

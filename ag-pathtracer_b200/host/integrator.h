@@ -15,6 +15,8 @@
 #pragma once
 
 #include <stdexcept>
+#include <string>
+#include <vector>
 
 #include "precomp.h"
 #include "scene.h"
@@ -78,6 +80,33 @@ public:
 		acc.SetNumSamples(acc.NumSamples() + numSamples);
 		Check(agpt_reduce_resolve(ctxs.data(), (int)ctxs.size(), acc.NumSamples(), 1, rgb8));
 		Check(agpt_read_accum(ctxs[0], &acc.Pixels()->x));
+	}
+
+	// EXTENSION (agpt.h agpt_adaptive): a frame rendered adaptively on the tracer's one GPU -- every pixel gets min_samples,
+	// then `step` more per round while its standard error is above tolerance, up to max_samples.  The film replaces acc's
+	// contents (acc.NumSamples() is set to 0: pixels differ in their sample counts) and counts[y*W + x] receives each
+	// pixel's number of samples; film pixel (H-1-y)*W + x divided by it is the pixel's mean.  Throws for a device list (the
+	// moments would have to be reduced with the film every round).
+	void RenderAdaptive(const Scene& scene, const Camera& camera, Accumulator& acc, const agpt_adaptive& params, int depth,
+			std::vector<int>& counts, uint32_t flags = 0) const {
+		if (ctxs.size() != 1) throw std::runtime_error("CudaPathTracer::RenderAdaptive: renders on one device only");
+		if (uploaded != scene.Fingerprint()) Upload(scene);
+		agpt_camera cam = camera.Export();
+		agpt_ctx* c = ctxs[0];
+		Check(agpt_set_camera(c, &cam));
+		Check(agpt_set_film(c, acc.width, acc.height));
+		Check(agpt_set_moments(c, 1));
+		int rc = agpt_render_adaptive(c, &params, MaxDepth, depth, flags, nullptr, nullptr);
+		std::vector<float> m(rc == AGPT_OK ? 4 * (size_t)acc.width * acc.height : 0);
+		if (rc == AGPT_OK) rc = agpt_read_accum(c, &acc.Pixels()->x);
+		if (rc == AGPT_OK) rc = agpt_read_moments(c, m.data());
+		std::string err = rc == AGPT_OK ? "" : agpt_last_error();
+		agpt_set_moments(c, 0);             // plain Render calls stay as they were
+		if (rc != AGPT_OK) throw std::runtime_error("agpt: " + err);
+		counts.resize((size_t)acc.width * acc.height);
+		for (int y = 0; y < acc.height; y++)
+			for (int x = 0; x < acc.width; x++) counts[(size_t)y * acc.width + x] = (int)m[4 * ((size_t)(acc.height - 1 - y) * acc.width + x) + 3];
+		acc.SetNumSamples(0);
 	}
 
 	// Single-ray entry point.  The reference's Li draws from the global generator; here the

@@ -303,6 +303,45 @@ int agpt_write_accum_begin(agpt_ctx* ctx, const float* host_rgba);
 /* Accumulator::CopyToSurface (myapp.h:34-41): /samples, pow(1/2.2), 8-bit pack 0x00RRGGBB. */
 int agpt_resolve(agpt_ctx* ctx, int samples, uint32_t* host_rgb8);
 
+/* ---- adaptive sampling (EXTENSION: the reference gives every pixel the same number of samples) ----------------------
+ * Per-pixel moments: a second float4[W*H] owned by the context, in the film's row order (row H-1-y).  .xyz = sum of c*c per
+ * channel and .w = n, the number of samples added (a float: exact up to 2^24), where c is each sample after the film's filter
+ * (a sample with a NaN channel or an infinite luminance adds 0, and still counts in n), added in ascending sample order like
+ * the film.  Off by default; while off, nothing about the film or the kernels that run changes.  On: the buffer is allocated
+ * and zeroed, re-allocated (zeroed) by agpt_set_film and zeroed by agpt_clear, and agpt_render (any stride) adds the samples
+ * it renders.  agpt_write_accum*, agpt_set_accum_dev and the multi-GPU reduce calls leave it alone: after them the caller
+ * owns the consistency between film and moments. */
+int agpt_set_moments(agpt_ctx* ctx, int enable);
+int agpt_read_moments(agpt_ctx* ctx, float* host_rgba);            /* D2H of float4[W*H]; AGPT_ERR_STATE while moments are off */
+
+/* Convergence test.  Valid: 2 <= min_samples <= max_samples <= 1<<24, step >= 1, tolerance and floor finite and >= 0
+ * (else AGPT_ERR_INVALID).  Pixel p, with film sum a, moments q and count n, is SELECTED (needs `step` more samples) iff
+ * n + step <= max_samples and, for at least one channel, in float32 with every operation rounded on its own:
+ *     mu = a / n;  d = q - a * mu;  v = d / (n - 1);  v = v < 0 ? 0 : v;  se = sqrt(v / n);
+ *     thr = tolerance * (mu > floor ? mu : floor);  !(se <= thr)
+ * (a NaN v stays NaN: a pixel whose se is not finite keeps sampling until max_samples).  oracle/adaptive.py states the same
+ * rule element for element. */
+typedef struct agpt_adaptive {
+	int32_t min_samples, max_samples, step;
+	float tolerance;   /* relative standard error of the pixel mean that is good enough */
+	float floor;       /* darker pixels are held to tolerance * floor instead of tolerance * mean */
+} agpt_adaptive;
+/* Runs the test over the film on the device and leaves the compacted list of selected pixels there; *n_out = its length,
+ * pixels_out (NULL, or W*H entries) receives the film pixel indices y*W + x.  The order of the list is unspecified (8x4 tiles
+ * stay together) and never affects results. */
+int agpt_adaptive_select(agpt_ctx* ctx, const agpt_adaptive* params, int32_t* pixels_out, int* n_out);
+/* A frame from scratch: clears film and moments, renders samples [0, min_samples) of every pixel (agpt_render), then
+ * repeats { agpt_adaptive_select; samples [n_p, n_p + step) of every selected pixel } until nothing is selected, at most
+ * (max - min) / step rounds.  Each pixel of the result equals, bit for bit, the same pixel of agpt_render(0, n_p) on a cleared
+ * film, n_p being its final count (moments .w): every draw of a path depends only on its pixel and sample index, and the film
+ * adds a pixel's samples in ascending order whatever the batches.  *rounds_out (may be NULL) = selection rounds that rendered
+ * something, *paths_out (may be NULL) = camera paths of the whole frame.  AGPT_ERR_STATE with moments off or without film,
+ * scene or camera; a refused call leaves film and moments as they were. */
+int agpt_render_adaptive(agpt_ctx* ctx, const agpt_adaptive* params, int max_depth, int rr_depth_arg, uint32_t flags,
+		int* rounds_out, int64_t* paths_out);
+/* agpt_resolve with each pixel's own sample count: ResolvePixel(film[i], moments[i].w); a pixel with n = 0 resolves to 0. */
+int agpt_resolve_counts(agpt_ctx* ctx, uint32_t* host_rgb8);
+
 /* ---- multi-GPU: sample-index sharding (SURVEY 8e; north star "NCCL reduces the accumulators over NVLink") ----
  * One context per GPU of ONE process, each holding the whole scene and a film of the same size.  GPU g of G
  * renders the samples s = first + g (mod G) into its own accumulator (agpt_render with sample_stride = G, or

@@ -84,6 +84,10 @@ int agpt_host_tracer_render(agpt_host_tracer* tracer, agpt_host_scene* scene, in
  * GPUs and the display transform fused in one kernel per GPU. */
 int agpt_host_tracer_render_resolve(agpt_host_tracer* tracer, agpt_host_scene* scene, int width, int height, float* host_rgba,
 		int samples_so_far, int first_sample, int num_samples, int depth_arg, uint32_t flags, uint32_t* host_rgb8);
+/* EXTENSION: CudaPathTracer::RenderAdaptive (agpt.h agpt_adaptive) on a one-device tracer: the film replaces host_rgba,
+ * host_counts[y*W + x] (W*H ints) receives each pixel's sample count. */
+int agpt_host_tracer_render_adaptive(agpt_host_tracer* tracer, agpt_host_scene* scene, int width, int height, float* host_rgba,
+		const agpt_adaptive* params, int depth_arg, uint32_t flags, int32_t* host_counts);
 /* CudaPathTracer::Li(Ray(o, d), scene, depth_arg) */
 int agpt_host_tracer_li(agpt_host_tracer* tracer, agpt_host_scene* scene, const float* o3, const float* d3, int depth_arg, float* out3);
 
