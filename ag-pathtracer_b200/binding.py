@@ -86,6 +86,17 @@ def adaptive(min_samples, max_samples, step, tolerance, floor=0.0):
     return Adaptive(int(min_samples), int(max_samples), int(step), float(tolerance), float(floor))
 
 
+class DenoiseParams(ctypes.Structure):  # struct agpt_denoise (extension: the a-trous denoiser)
+    _fields_ = [("iterations", c_int32), ("sigma_luminance", c_float), ("sigma_depth", c_float), ("normal_power_log2", c_int32)]
+
+
+def denoise_params(iterations=5, sigma_luminance=8.0, sigma_depth=0.1, normal_power_log2=7):
+    """struct agpt_denoise record; the filter it parameterises is stated in include/agpt.h and oracle/denoise.py.  The defaults
+    are the best of tests/perf_denoise.py's sweep on cfg 3 at 16 spp and within 3 % of the best on cfg 5 (DESIGN.md section 10
+    has the measurements)."""
+    return DenoiseParams(int(iterations), float(sigma_luminance), float(sigma_depth), int(normal_power_log2))
+
+
 class Stats(ctypes.Structure):  # agpt_stats
     _fields_ = [(n, c_uint64) for n in ("paths", "rays_closest", "rays_shadow", "rays_mis", "rays_skip", "rays_mis_culled", "rays_tail_culled")] + \
                [(n, c_uint64 * 2) for n in ("node_visits", "box_tests", "tri_tests", "analytic_tests", "warp_steps", "lane_steps")] + \
@@ -297,6 +308,26 @@ class Context:
         out = np.empty((self.height, self.width), np.uint32)
         _check(core().agpt_resolve_counts(self._h, out.ctypes.data_as(POINTER(c_uint32))))
         return out
+
+    # ---- denoising (extension) ---------------------------------------------------------------------
+    def render_guides(self, num_samples, flags=0):
+        """First hits of the camera rays of samples [0, num_samples) of every pixel -> the context's guide buffers."""
+        _check(core().agpt_render_guides(self._h, c_int(num_samples), c_uint32(flags)))
+
+    def read_guides(self):
+        """(albedo, normal_depth): float32 [H, W, 4] each, in the film's row order."""
+        alb = np.empty((self.height, self.width, 4), np.float32)
+        nd = np.empty((self.height, self.width, 4), np.float32)
+        _check(core().agpt_read_guides(self._h, _fptr(alb), _fptr(nd)))
+        return alb, nd
+
+    def denoise(self, params):
+        """The a-trous filter over the resident film, moments and guides: (float32 [H, W, 4] mean radiance, uint32 [H, W] packed
+        pixels), both in the film's row order."""
+        out = np.empty((self.height, self.width, 4), np.float32)
+        rgb8 = np.empty((self.height, self.width), np.uint32)
+        _check(core().agpt_denoise(self._h, byref(params), _fptr(out), rgb8.ctypes.data_as(POINTER(c_uint32))))
+        return out, rgb8
 
     def trace_primary(self, sample, flags=0):
         out = np.empty(self.width * self.height, HIT_DTYPE)
@@ -607,6 +638,19 @@ class HostTracer:
         _check(host().agpt_host_tracer_render_adaptive(self._h, scene.handle, c_int(width), c_int(height), _fptr(accum), byref(params),
                                                        c_int(depth_arg), c_uint32(flags), counts.ctypes.data_as(POINTER(c_int32))), host_side=True)
         return counts
+
+    def render_adaptive_denoised(self, scene, width, height, accum, params, denoise, guide_samples, depth_arg=0, flags=0):
+        """CudaPathTracer::RenderAdaptiveDenoised: the film replaces `accum`; returns (counts [H, W] with row 0 = top, denoised
+        float32 [H, W, 4] and packed uint32 [H, W], both in the film's row order)."""
+        assert accum.dtype == np.float32 and accum.shape == (height, width, 4) and accum.flags.c_contiguous
+        counts = np.empty((height, width), np.int32)
+        out = np.empty((height, width, 4), np.float32)
+        rgb8 = np.empty((height, width), np.uint32)
+        _check(host().agpt_host_tracer_render_adaptive_denoised(self._h, scene.handle, c_int(width), c_int(height), _fptr(accum), byref(params),
+                                                                byref(denoise), c_int(guide_samples), c_int(depth_arg), c_uint32(flags),
+                                                                counts.ctypes.data_as(POINTER(c_int32)), _fptr(out),
+                                                                rgb8.ctypes.data_as(POINTER(c_uint32))), host_side=True)
+        return counts, out, rgb8
 
     def li(self, scene, origin, direction, depth_arg=0):
         o = (c_float * 3)(*origin); d = (c_float * 3)(*direction); out = (c_float * 3)()

@@ -121,6 +121,11 @@ struct agpt_ctx {
 	DevBuf<float4> moments;
 	DevBuf<int> adaptiveList;     // agpt_adaptive_select's compacted pixel list (W*H) and its length
 	DevBuf<int> adaptiveCount;
+	// denoising (agpt_render_guides, agpt_denoise): guides traced for the scene, camera and film of generation guidesGen
+	uint64_t stateGen = 1;        // bumped by agpt_set_film, agpt_set_camera and every agpt_upload_* past its argument checks
+	uint64_t guidesGen = 0;       // 0: no guides
+	DevBuf<float4> guideAlbedo, guideNormal;
+	DevBuf<float4> denoiseE[2], denoiseG, denoiseOut;   // ping-pong (e, v_l), the filter's guide, the result
 
 	// wavefront state
 	size_t capacity = 0;          // path slots allocated
@@ -475,6 +480,7 @@ int agpt_destroy(agpt_ctx* c) {
 	c->meshes.Free(); c->shapeLights.Free(); c->shapeCdf.Free(); c->instances.Free(); c->spheres.Free(); c->planes.Free(); c->prims.Free(); c->sphereRun.Free(); c->sphereRunBox.Free(); c->keyBoxes.Free(); c->mats.Free(); c->lights.Free();
 	c->accumOwn.Free(); c->resolved.Free();
 	c->moments.Free(); c->adaptiveList.Free(); c->adaptiveCount.Free();
+	c->guideAlbedo.Free(); c->guideNormal.Free(); c->denoiseE[0].Free(); c->denoiseE[1].Free(); c->denoiseG.Free(); c->denoiseOut.Free();
 	c->envRgb.Free(); c->envFunc.Free(); c->envCdf.Free();
 	for (auto& b : c->f4) b.Free();
 	for (auto& b : c->i32) b.Free();
@@ -561,6 +567,7 @@ int agpt_upload_meshes(agpt_ctx* c, const agpt_mesh_desc* meshes, int n) {
 	CU(cudaSetDevice(c->device));
 	CU(cudaStreamSynchronize(c->stream));
 	c->gridCalibrated = false;
+	c->stateGen++;
 	// from here on a failure must not leave the device table pointing at freed buffers
 	for (auto& m : c->meshStore) m.Free();
 	c->meshStore.assign(n, MeshStore());
@@ -611,6 +618,7 @@ int agpt_upload_meshes(agpt_ctx* c, const agpt_mesh_desc* meshes, int n) {
 		NEED(c != nullptr && n >= 0 && (n == 0 || rows != nullptr), AGPT_ERR_INVALID, "bad table"); \
 		CU(cudaSetDevice(c->device)); \
 		CU(cudaStreamSynchronize(c->stream)); \
+		c->stateGen++; \
 		CU(c->member.Upload(rows, (size_t)n, c->stream)); \
 		CU(cudaStreamSynchronize(c->stream)); \
 		counter; \
@@ -633,6 +641,7 @@ int agpt_upload_primitives(agpt_ctx* c, const agpt_prim* rows, int n) {
 	NEED(c != nullptr && n >= 0 && (n == 0 || rows != nullptr), AGPT_ERR_INVALID, "bad table");
 	CU(cudaSetDevice(c->device));
 	CU(cudaStreamSynchronize(c->stream));
+	c->stateGen++;
 	CU(c->prims.Upload(rows, (size_t)n, c->stream));
 	c->hostPrims.assign(rows, rows + n);
 	c->runsDirty = true;
@@ -649,6 +658,7 @@ int agpt_upload_envmap(agpt_ctx* c, const agpt_envmap* env) {
 	CU(cudaStreamSynchronize(c->stream));
 	c->envRgb.Free(); c->envFunc.Free(); c->envCdf.Free();
 	c->envW = c->envH = 0; c->envFuncInt = 0;
+	c->stateGen++;
 	if (!env || env->width == 0) return AGPT_OK;
 	NEED(env->width > 0 && env->height > 0 && env->rgb && env->func && env->cdf, AGPT_ERR_INVALID, "bad environment map");
 	size_t n = (size_t)env->width * env->height;
@@ -664,6 +674,7 @@ int agpt_set_camera(agpt_ctx* c, const agpt_camera* cam) {
 	NEED(c != nullptr && cam != nullptr, AGPT_ERR_INVALID, "null camera");
 	c->cam = *cam;
 	c->haveCam = true;
+	c->stateGen++;
 	c->gridCalibrated = false;
 	return AGPT_OK;
 }
@@ -682,6 +693,7 @@ int agpt_set_film(agpt_ctx* c, int width, int height) {
 	JOIN(c);
 	NEED(c != nullptr && width > 0 && height > 0 && (long long)width * height < (1ll << 30), AGPT_ERR_INVALID, "bad film size");
 	CU(cudaSetDevice(c->device));
+	c->stateGen++;
 	if (width == c->width && height == c->height) return AGPT_OK;
 	CU(cudaStreamSynchronize(c->stream));
 	bool own = c->accum == c->accumOwn.p;
@@ -1172,6 +1184,104 @@ int agpt_resolve_counts(agpt_ctx* c, uint32_t* host) {
 	CU(cudaGetLastError());
 	c->stats.kernel_launches++;
 	CU(cudaMemcpyAsync(host, c->resolved.p, n * sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream));
+	CU(cudaStreamSynchronize(c->stream));
+	return AGPT_OK;
+}
+
+// ---- denoising (EXTENSION, agpt.h agpt_render_guides / agpt_denoise) ------------------------------------------------------
+// The camera rays of samples [0, num_samples) as agpt_render generates them (k_generate<false>, tiled), batch by batch through
+// the closest-hit trace alone; k_guides folds each batch into the guide sums.
+int agpt_render_guides(agpt_ctx* c, int num_samples, uint32_t flags) {
+	int rcode = CheckReady(c, true);
+	if (rcode != AGPT_OK) return rcode;
+	NEED(num_samples >= 1 && num_samples <= (1 << 24), AGPT_ERR_INVALID, "agpt_render_guides: need 1 <= num_samples <= 1<<24");
+	CU(cudaSetDevice(c->device));
+	const size_t wh = (size_t)c->width * c->height;
+	int perBatch = (int)(c->maxPathsPerBatch / wh);
+	if (perBatch < 1) perBatch = 1;
+	if (perBatch > num_samples) perBatch = num_samples;
+	rcode = EnsureCapacity(c, wh * perBatch);
+	if (rcode != AGPT_OK) return rcode;
+	c->guidesGen = 0;                                    // valid again only once this call has completed
+	if (c->guideAlbedo.n != wh) { CU(c->guideAlbedo.Alloc(wh)); CU(c->guideNormal.Alloc(wh)); }
+	DScene sc = MakeScene(c);
+	PathState ps = MakePathState(c);
+	WaveQueues q0;
+	q0.closest = c->queues[0].p; q0.shadow = c->queues[2].p; q0.active = c->queues[4].p; q0.counts = c->counts.p; q0.keys = nullptr; q0.shadowKeys = nullptr;
+	const bool count = flags & AGPT_FLAG_COUNTERS, strictBoxes = flags & AGPT_FLAG_STRICT_BOXES;
+	for (int done = 0; done < num_samples; done += perBatch) {
+		const int ns = num_samples - done < perBatch ? num_samples - done : perBatch;
+		const int n = (int)(wh * ns);
+		GenParams g;
+		memset(&g, 0, sizeof(g));
+		g.n = n; g.first_sample = done; g.sample_stride = 1; g.tiled = 1; g.samples = ns;
+		k_generate<false><<<Blocks(n, 256), 256, 0, c->stream>>>(sc, ps, q0, g);
+		LaunchClosest(count, strictBoxes, c->nInstances > 0, Blocks(n, AGPT_TRACE_THREADS), c->stream, sc, ps, q0.closest, q0.counts + 0, c->traceCounters.p, nullptr);
+		k_guides<<<Blocks(wh, 256), 256, 0, c->stream>>>(sc, ps, ns, done == 0, done + ns == num_samples ? num_samples : 0, c->guideAlbedo.p, c->guideNormal.p);
+		CU(cudaGetLastError());
+		c->stats.kernel_launches += 3; c->stats.launches_closest++;
+	}
+	CU(cudaStreamSynchronize(c->stream));
+	c->guidesGen = c->stateGen;
+	return AGPT_OK;
+}
+
+static bool GuidesFresh(const agpt_ctx* c) {
+	return c->guidesGen != 0 && c->guidesGen == c->stateGen && c->guideAlbedo.n == (size_t)c->width * c->height;
+}
+
+int agpt_read_guides(agpt_ctx* c, float* albedo_rgba, float* normal_depth_rgba) {
+	NEED(c != nullptr, AGPT_ERR_INVALID, "null context");
+	NEED(GuidesFresh(c), AGPT_ERR_STATE, "no guides for the current scene, camera and film (agpt_render_guides)");
+	CU(cudaSetDevice(c->device));
+	if (albedo_rgba) CU(cudaMemcpyAsync(albedo_rgba, c->guideAlbedo.p, c->guideAlbedo.Bytes(), cudaMemcpyDeviceToHost, c->stream));
+	if (normal_depth_rgba) CU(cudaMemcpyAsync(normal_depth_rgba, c->guideNormal.p, c->guideNormal.Bytes(), cudaMemcpyDeviceToHost, c->stream));
+	CU(cudaStreamSynchronize(c->stream));
+	return AGPT_OK;
+}
+
+static int CheckDenoise(const agpt_denoise_params* p) {
+	NEED(p != nullptr, AGPT_ERR_INVALID, "null agpt_denoise");
+	NEED(p->iterations >= 0 && p->iterations <= 10, AGPT_ERR_INVALID, "agpt_denoise: need 0 <= iterations <= 10");
+	NEED(std::isfinite(p->sigma_luminance) && p->sigma_luminance >= 0.f && std::isfinite(p->sigma_depth) && p->sigma_depth >= 0.f, AGPT_ERR_INVALID,
+		"agpt_denoise: sigmas must be finite and >= 0");
+	NEED(p->normal_power_log2 >= 0 && p->normal_power_log2 <= 10, AGPT_ERR_INVALID, "agpt_denoise: need 0 <= normal_power_log2 <= 10");
+	return AGPT_OK;
+}
+
+// k_denoise_prepare, then one k_denoise_atrous per iteration ping-ponging between denoiseE[0] and [1]; the last writes the
+// remodulated floats and the packed pixels.
+int agpt_denoise(agpt_ctx* c, const agpt_denoise_params* params, float* out_rgba, uint32_t* out_rgb8) {
+	JOIN(c);
+	NEED(c != nullptr, AGPT_ERR_INVALID, "null context");
+	int rcode = CheckDenoise(params);
+	if (rcode != AGPT_OK) return rcode;
+	NEED(c->momentsOn && c->moments.p != nullptr && c->accum != nullptr, AGPT_ERR_STATE, "moments are off (agpt_set_moments) or film not set");
+	NEED(GuidesFresh(c), AGPT_ERR_STATE, "guides missing or stale: agpt_render_guides after the last agpt_set_film / agpt_set_camera / agpt_upload_*");
+	const agpt_denoise_params p = *params;
+	CU(cudaSetDevice(c->device));
+	const int W = c->width, H = c->height, n = W * H;
+	if (c->denoiseOut.n != (size_t)n) CU(c->denoiseOut.Alloc(n));
+	if (c->resolved.n != (size_t)n) CU(c->resolved.Alloc(n));
+	if (p.iterations > 0 && c->denoiseG.n != (size_t)n) { CU(c->denoiseE[0].Alloc(n)); CU(c->denoiseE[1].Alloc(n)); CU(c->denoiseG.Alloc(n)); }
+	k_denoise_prepare<<<Blocks(n, 256), 256, 0, c->stream>>>(c->accum, c->moments.p, c->guideAlbedo.p, c->guideNormal.p, n, c->denoiseE[0].p, c->denoiseG.p,
+		p.iterations == 0 ? c->denoiseOut.p : nullptr, c->resolved.p);
+	CU(cudaGetLastError());
+	c->stats.kernel_launches++;
+	const dim3 block(32, 8), grid(Blocks(W, 32), Blocks(H, 8));
+	for (int i = 0; i < p.iterations; i++) {
+		const float4* in = c->denoiseE[i & 1].p;
+		if (i == p.iterations - 1)
+			k_denoise_atrous<true><<<grid, block, 0, c->stream>>>(in, c->denoiseG.p, c->guideAlbedo.p, W, H, 1 << i, p.sigma_luminance, p.sigma_depth, p.normal_power_log2,
+				c->denoiseOut.p, c->resolved.p);
+		else
+			k_denoise_atrous<false><<<grid, block, 0, c->stream>>>(in, c->denoiseG.p, c->guideAlbedo.p, W, H, 1 << i, p.sigma_luminance, p.sigma_depth, p.normal_power_log2,
+				c->denoiseE[(i + 1) & 1].p, nullptr);
+		CU(cudaGetLastError());
+		c->stats.kernel_launches++;
+	}
+	if (out_rgba) CU(cudaMemcpyAsync(out_rgba, c->denoiseOut.p, (size_t)n * sizeof(float4), cudaMemcpyDeviceToHost, c->stream));
+	if (out_rgb8) CU(cudaMemcpyAsync(out_rgb8, c->resolved.p, (size_t)n * sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream));
 	CU(cudaStreamSynchronize(c->stream));
 	return AGPT_OK;
 }

@@ -920,13 +920,18 @@ __global__ void __launch_bounds__(256) k_accumulate(const float4* __restrict__ L
 
 // ---- adaptive sampling: the convergence test of agpt_adaptive_select (agpt.h), per pixel ------------------------------
 // Film sum a, moments q and count n of one channel; every operation rounded on its own (--fmad=false, IEEE / and sqrt).
-// True: the channel's standard error is not (yet) within tolerance, or not finite.
-__device__ __forceinline__ bool ChannelUnconverged(float a, float q, float n, float tolerance, float floor_) {
-	float mu = a / n;
+// The variance of the channel's mean, v / n (and the mean mu), as the convergence test and the denoiser both estimate it.
+__device__ __forceinline__ float ChannelVarianceOfMean(float a, float q, float n, float& mu) {
+	mu = a / n;
 	float d = q - a * mu;
 	float v = d / (n - 1.f);
 	v = v < 0.f ? 0.f : v;                      // (a NaN stays NaN)
-	float se = sqrtf(v / n);
+	return v / n;
+}
+// True: the channel's standard error is not (yet) within tolerance, or not finite.
+__device__ __forceinline__ bool ChannelUnconverged(float a, float q, float n, float tolerance, float floor_) {
+	float mu;
+	float se = sqrtf(ChannelVarianceOfMean(a, q, n, mu));
 	float thr = tolerance * (mu > floor_ ? mu : floor_);
 	return !(se <= thr);
 }
@@ -991,6 +996,161 @@ __global__ void __launch_bounds__(256) k_resolve_counts(const float4* __restrict
 	if (i >= n) return;
 	const float s = moments[i].w;
 	out[i] = s > 0.f ? ResolvePixel(accum[i], s) : 0u;
+}
+
+// ---- EXTENSION: denoising (agpt.h agpt_render_guides / agpt_denoise; CPU statements oracle/agpt_guides_oracle.cpp and
+// oracle/denoise.py) --------------------------------------------------------------------------------------------------------
+// k_guides: one thread per pixel after k_generate<false> (tiled) and k_trace_closest have run the batch's camera rays.  It walks
+// the pixel's slots in sample order and adds each sample's first hit to the running sums in albedo (.xyz, .w = hits) and
+// normalDepth (.xyz, .w = t sum).  `total` > 0 on the last batch: the sums become the means of all `total` samples.
+__global__ void __launch_bounds__(256) k_guides(DScene sc, PathState ps, int samplesInBatch, bool firstBatch, int total, float4* albedo, float4* normalDepth) {
+	const int pixel = blockIdx.x * blockDim.x + threadIdx.x;
+	const int width = sc.width, height = sc.height;
+	if (pixel >= width * height) return;
+	const int x = pixel % width, y = pixel / width;
+	const size_t f = (size_t)(height - 1 - y) * width + x;
+	float4 a = make_float4(0.f, 0.f, 0.f, 0.f), nd = a;
+	if (!firstBatch) { a = albedo[f]; nd = normalDepth[f]; }
+	const size_t base = (size_t)PixelToSlot(x, y, width, height, true) * samplesInBatch;     // k_generate's tiled slots
+	for (int s = 0; s < samplesInBatch; s++) {
+		const size_t slot = base + s;
+		AGPT_CHECK(slot < (size_t)ps.slots, AGPT_DBG_GUIDE, slot);
+		const float4 h = ps.hitA[slot];
+		const int hitPrim = __float_as_int(h.w);
+		AGPT_CHECK(hitPrim < sc.n_prims, AGPT_DBG_PRIM, hitPrim);
+		float3 alb = f3(1.f), n = f3(0.f);
+		if (hitPrim >= 0) {
+			const float4 o4 = ps.rayO[slot], d4 = ps.rayD[slot];
+			const float3 O = f3(o4.x, o4.y, o4.z), D = f3(d4.x, d4.y, d4.z);
+			const agpt_prim prim = sc.prims[hitPrim];
+			DSurface si;
+			// the surface of the closest hit as k_shade_b rebuilds it
+			if (prim.type == AGPT_PRIM_SPHERE) SphereSurface(sc.spheres[prim.payload], O, D, h.x, si);
+			else if (prim.type == AGPT_PRIM_PLANE) PlaneSurface(O, D, h.x, si);
+			else if (prim.type == AGPT_PRIM_INSTANCE) {
+				const agpt_instance& in = sc.instances[prim.payload];
+				TriangleSurface(sc.meshes[in.mesh], ps.hitSlot[slot], O, D, h.x, h.y, h.z, si, &in);
+			}
+			else TriangleSurface(sc.meshes[prim.payload], ps.hitSlot[slot], O, D, h.x, h.y, h.z, si, nullptr);
+			n = dot(si.sn, D) > 0.f ? -si.sn : si.sn;
+			if (prim.material >= 0) {
+				const agpt_material& m = sc.mats[prim.material];
+				if (m.type == AGPT_MAT_MIRROR) alb = f3(m.mirror_r);
+				else if (m.type == AGPT_MAT_GLASS) alb = f3(m.mirror_r) + f3(m.diffuse_r);
+				else alb = f3(m.diffuse_r) + f3(m.spec_r0);
+				alb = f3(alb.x < 1.f ? alb.x : 1.f, alb.y < 1.f ? alb.y : 1.f, alb.z < 1.f ? alb.z : 1.f);
+			}
+			a.w += 1.f;
+			nd.w += h.x;
+		}
+		a.x += alb.x; a.y += alb.y; a.z += alb.z;
+		nd.x += n.x; nd.y += n.y; nd.z += n.z;
+	}
+	if (total > 0) {
+		const float t = (float)total;
+		nd.w = a.w > 0.f ? nd.w / a.w : 0.f;
+		a = make_float4(a.x / t, a.y / t, a.z / t, a.w / t);
+		nd.x /= t; nd.y /= t; nd.z /= t;
+	}
+	albedo[f] = a;
+	normalDepth[f] = nd;
+}
+
+#define AGPT_DENOISE_ALBEDO_EPS 0.01f
+#define AGPT_DENOISE_LUM_EPS 1e-4f
+__device__ __forceinline__ float DenoiseLum(float4 e) { return 0.212671f * e.x + 0.715160f * e.y + 0.072169f * e.z; }
+__device__ __forceinline__ float3 DenoiseAlbedo(float4 a) {
+	return f3(a.x > AGPT_DENOISE_ALBEDO_EPS ? a.x : AGPT_DENOISE_ALBEDO_EPS, a.y > AGPT_DENOISE_ALBEDO_EPS ? a.y : AGPT_DENOISE_ALBEDO_EPS,
+		a.z > AGPT_DENOISE_ALBEDO_EPS ? a.z : AGPT_DENOISE_ALBEDO_EPS);
+}
+__device__ __forceinline__ bool Finite4(float4 v) { return isfinite(v.x) && isfinite(v.y) && isfinite(v.z) && isfinite(v.w); }
+
+// k_denoise_prepare: one thread per film pixel.  iterations > 0: the demodulated mean and its luminance variance into E, the
+// filter's guide (normal, depth or -1 for a pixel that missed) into G.  iterations == 0 (out != nullptr): the means themselves
+// into out and their packed pixels into rgb8.
+__global__ void __launch_bounds__(256) k_denoise_prepare(const float4* __restrict__ accum, const float4* __restrict__ moments, const float4* __restrict__ albedo,
+		const float4* __restrict__ normalDepth, int n, float4* __restrict__ E, float4* __restrict__ G, float4* __restrict__ out, uint32_t* __restrict__ rgb8) {
+	const int i = blockIdx.x * blockDim.x + threadIdx.x;
+	if (i >= n) return;
+	const float4 a = accum[i], q = moments[i];
+	float3 mu = f3(0.f), var = f3(0.f);
+	if (q.w > 0.f) { mu = f3(a.x / q.w, a.y / q.w, a.z / q.w); }
+	if (out) {
+		const float4 o = make_float4(mu.x, mu.y, mu.z, 0.f);
+		out[i] = o;
+		rgb8[i] = ResolvePixel(o, 1.f);
+		return;
+	}
+	if (q.w >= 2.f) {
+		float m;
+		var = f3(ChannelVarianceOfMean(a.x, q.x, q.w, m), ChannelVarianceOfMean(a.y, q.y, q.w, m), ChannelVarianceOfMean(a.z, q.z, q.w, m));
+	}
+	const float4 alb = albedo[i], nd = normalDepth[i];
+	const float3 al = DenoiseAlbedo(alb);
+	const float wr = 0.212671f * 0.212671f, wg = 0.715160f * 0.715160f, wb = 0.072169f * 0.072169f;
+	const float vl = ((wr * var.x) / (al.x * al.x) + (wg * var.y) / (al.y * al.y)) + (wb * var.z) / (al.z * al.z);
+	E[i] = make_float4(mu.x / al.x, mu.y / al.y, mu.z / al.z, vl);
+	G[i] = make_float4(nd.x, nd.y, nd.z, alb.w == 0.f ? -1.f : nd.w);
+}
+
+// k_denoise_atrous: one a-trous pass at tap spacing `step`, one thread per pixel (a 32 x 8 block covers a film patch).  The 25
+// taps are plain loads: neighbouring threads share most of them through L1.  LAST: remodulated by the albedo into out, packed
+// into rgb8.
+template <bool LAST>
+__global__ void __launch_bounds__(256) k_denoise_atrous(const float4* __restrict__ Ein, const float4* __restrict__ G, const float4* __restrict__ albedo, int width, int height,
+		int step, float sigmaL, float sigmaZ, int normalPow, float4* __restrict__ Eout, uint32_t* __restrict__ rgb8) {
+	const int x = blockIdx.x * blockDim.x + threadIdx.x, r = blockIdx.y * blockDim.y + threadIdx.y;
+	if (x >= width || r >= height) return;
+	const int p = r * width + x;
+	const float h[5] = { 1.f / 16, 1.f / 4, 3.f / 8, 1.f / 4, 1.f / 16 };
+	const float4 ep = Ein[p];
+	float4 res = ep;
+	if (Finite4(ep)) {
+		const float4 gp = G[p];
+		const bool missP = gp.w < 0.f;
+		const float lp = DenoiseLum(ep);
+		const float den = (sigmaL * sigmaL) * ep.w + AGPT_DENOISE_LUM_EPS;
+		float sw = 0.f, sv = 0.f;
+		float3 se = f3(0.f);
+#pragma unroll
+		for (int dy = -2; dy <= 2; dy++) {
+			const int rq = r + dy * step;
+			if (rq < 0 || rq >= height) continue;
+#pragma unroll
+			for (int dx = -2; dx <= 2; dx++) {
+				const int xq = x + dx * step;
+				if (xq < 0 || xq >= width) continue;
+				const int q = rq * width + xq;
+				AGPT_CHECK(q >= 0 && q < width * height, AGPT_DBG_TAP, q);
+				const float4 eq = Ein[q];
+				if (!Finite4(eq)) continue;
+				const float4 gq = G[q];
+				const float dl = lp - DenoiseLum(eq);
+				const float wl = 1.f / (1.f + (dl * dl) / den);
+				float m = gp.x * gq.x + gp.y * gq.y + gp.z * gq.z;
+				m = m > 0.f ? m : 0.f;
+				for (int k = 0; k < normalPow; k++) m = m * m;
+				const bool missQ = gq.w < 0.f;
+				const float wz = (missP && missQ) ? 1.f : (missP != missQ) ? 0.f : 1.f / (1.f + fabsf(gp.w - gq.w) / (sigmaZ * gp.w));
+				const float w = (((h[dx + 2] * h[dy + 2]) * wl) * m) * wz;
+				if (!isfinite(w)) continue;
+				sw += w;
+				se.x += w * eq.x; se.y += w * eq.y; se.z += w * eq.z;
+				sv += (w * w) * eq.w;
+			}
+		}
+		if (sw > 0.f) {
+			const float4 e2 = make_float4(se.x / sw, se.y / sw, se.z / sw, sv / (sw * sw));
+			if (Finite4(e2)) res = e2;
+		}
+	}
+	if (LAST) {
+		const float3 al = DenoiseAlbedo(albedo[p]);
+		const float4 o = make_float4(res.x * al.x, res.y * al.y, res.z * al.z, 0.f);
+		Eout[p] = o;
+		rgb8[p] = ResolvePixel(o, 1.f);
+	}
+	else Eout[p] = res;
 }
 
 // ---- bandwidth probe: what a plain streaming read of this library's own making reaches on this GPU ----

@@ -258,6 +258,21 @@ int agpt_host_tracer_render_adaptive(agpt_host_tracer* t, agpt_host_scene* s, in
 	return AGPT_OK;
 }
 
+int agpt_host_tracer_render_adaptive_denoised(agpt_host_tracer* t, agpt_host_scene* s, int width, int height, float* host_rgba,
+		const agpt_adaptive* params, const agpt_denoise_params* denoise, int guide_samples, int depth_arg, uint32_t flags, int32_t* host_counts,
+		float* out_rgba, uint32_t* out_rgb8) {
+	if (!t || !s || !host_rgba || !params || !denoise || !host_counts) return HostFail("null argument");
+	g_hostError.clear();
+	HOST_TRY(
+		Accumulator acc(width, height, reinterpret_cast<float3*>(host_rgba));
+		std::vector<int> counts;
+		t->tracer->RenderAdaptiveDenoised(s->scene, *s->camera, acc, *params, *denoise, guide_samples, depth_arg, counts,
+			reinterpret_cast<float3*>(out_rgba), out_rgb8, flags);
+		std::copy(counts.begin(), counts.end(), host_counts);
+	)
+	return AGPT_OK;
+}
+
 int agpt_host_tracer_li(agpt_host_tracer* t, agpt_host_scene* s, const float* o, const float* d, int depth_arg, float* out3) {
 	if (!t || !s || !o || !d || !out3) return HostFail("null argument");
 	g_hostError.clear();

@@ -89,24 +89,15 @@ public:
 	// moments would have to be reduced with the film every round).
 	void RenderAdaptive(const Scene& scene, const Camera& camera, Accumulator& acc, const agpt_adaptive& params, int depth,
 			std::vector<int>& counts, uint32_t flags = 0) const {
-		if (ctxs.size() != 1) throw std::runtime_error("CudaPathTracer::RenderAdaptive: renders on one device only");
-		if (uploaded != scene.Fingerprint()) Upload(scene);
-		agpt_camera cam = camera.Export();
-		agpt_ctx* c = ctxs[0];
-		Check(agpt_set_camera(c, &cam));
-		Check(agpt_set_film(c, acc.width, acc.height));
-		Check(agpt_set_moments(c, 1));
-		int rc = agpt_render_adaptive(c, &params, MaxDepth, depth, flags, nullptr, nullptr);
-		std::vector<float> m(rc == AGPT_OK ? 4 * (size_t)acc.width * acc.height : 0);
-		if (rc == AGPT_OK) rc = agpt_read_accum(c, &acc.Pixels()->x);
-		if (rc == AGPT_OK) rc = agpt_read_moments(c, m.data());
-		std::string err = rc == AGPT_OK ? "" : agpt_last_error();
-		agpt_set_moments(c, 0);             // plain Render calls stay as they were
-		if (rc != AGPT_OK) throw std::runtime_error("agpt: " + err);
-		counts.resize((size_t)acc.width * acc.height);
-		for (int y = 0; y < acc.height; y++)
-			for (int x = 0; x < acc.width; x++) counts[(size_t)y * acc.width + x] = (int)m[4 * ((size_t)(acc.height - 1 - y) * acc.width + x) + 3];
-		acc.SetNumSamples(0);
+		AdaptiveFrame(scene, camera, acc, params, nullptr, 0, depth, counts, nullptr, nullptr, flags);
+	}
+
+	// EXTENSION (agpt.h agpt_render_guides / agpt_denoise): RenderAdaptive, then the guides of samples [0, guideSamples) and the
+	// denoiser over the film, before the moments are switched off again.  min == max gives a uniform frame.  out (W*H, film row
+	// order like acc) and rgb8 (W*H packed pixels, film row order) receive the denoised image; either may be null.
+	void RenderAdaptiveDenoised(const Scene& scene, const Camera& camera, Accumulator& acc, const agpt_adaptive& params, const agpt_denoise_params& denoise,
+			int guideSamples, int depth, std::vector<int>& counts, float3* out, uint32_t* rgb8, uint32_t flags = 0) const {
+		AdaptiveFrame(scene, camera, acc, params, &denoise, guideSamples, depth, counts, out, rgb8, flags);
 	}
 
 	// Single-ray entry point.  The reference's Li draws from the global generator; here the
@@ -122,6 +113,30 @@ protected:
 		if (status != AGPT_OK) throw std::runtime_error(std::string("agpt: ") + agpt_last_error());
 	}
 	void Destroy() { for (agpt_ctx* c : ctxs) agpt_destroy(c); ctxs.clear(); }
+	// RenderAdaptive, and with `denoise` the guides and the denoiser, all while the moments are on
+	void AdaptiveFrame(const Scene& scene, const Camera& camera, Accumulator& acc, const agpt_adaptive& params, const agpt_denoise_params* denoise,
+			int guideSamples, int depth, std::vector<int>& counts, float3* out, uint32_t* rgb8, uint32_t flags) const {
+		if (ctxs.size() != 1) throw std::runtime_error("CudaPathTracer: adaptive frames render on one device only");
+		if (uploaded != scene.Fingerprint()) Upload(scene);
+		agpt_camera cam = camera.Export();
+		agpt_ctx* c = ctxs[0];
+		Check(agpt_set_camera(c, &cam));
+		Check(agpt_set_film(c, acc.width, acc.height));
+		Check(agpt_set_moments(c, 1));
+		int rc = agpt_render_adaptive(c, &params, MaxDepth, depth, flags, nullptr, nullptr);
+		std::vector<float> m(rc == AGPT_OK ? 4 * (size_t)acc.width * acc.height : 0);
+		if (rc == AGPT_OK) rc = agpt_read_accum(c, &acc.Pixels()->x);
+		if (rc == AGPT_OK) rc = agpt_read_moments(c, m.data());
+		if (rc == AGPT_OK && denoise) rc = agpt_render_guides(c, guideSamples, flags & (AGPT_FLAG_COUNTERS | AGPT_FLAG_STRICT_BOXES));
+		if (rc == AGPT_OK && denoise) rc = agpt_denoise(c, denoise, out ? &out->x : nullptr, rgb8);
+		std::string err = rc == AGPT_OK ? "" : agpt_last_error();
+		agpt_set_moments(c, 0);             // plain Render calls stay as they were
+		if (rc != AGPT_OK) throw std::runtime_error("agpt: " + err);
+		counts.resize((size_t)acc.width * acc.height);
+		for (int y = 0; y < acc.height; y++)
+			for (int x = 0; x < acc.width; x++) counts[(size_t)y * acc.width + x] = (int)m[4 * ((size_t)(acc.height - 1 - y) * acc.width + x) + 3];
+		acc.SetNumSamples(0);
+	}
 	// every GPU's share of the samples into its own accumulator; GPU 0's starts from the caller's film
 	void RenderShards(const Scene& scene, const Camera& camera, Accumulator& acc, int firstSample, int numSamples, int depth, uint32_t flags) const {
 		if (uploaded != scene.Fingerprint()) Upload(scene);

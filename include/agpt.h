@@ -342,6 +342,68 @@ int agpt_render_adaptive(agpt_ctx* ctx, const agpt_adaptive* params, int max_dep
 /* agpt_resolve with each pixel's own sample count: ResolvePixel(film[i], moments[i].w); a pixel with n = 0 resolves to 0. */
 int agpt_resolve_counts(agpt_ctx* ctx, uint32_t* host_rgb8);
 
+/* ---- denoising (EXTENSION: the reference only divides the film by the sample count) ----------------------------------
+ * Guide buffers: what the camera rays of samples [0, num_samples) of every pixel hit first -- the rays agpt_render starts
+ * those samples with (same StreamSeed, CameraRay, jitter and lens draws), traced by the closest-hit kernels (flags:
+ * AGPT_FLAG_COUNTERS, AGPT_FLAG_STRICT_BOXES).  Two context-owned float4[W*H] in the film's row order (row H-1-y):
+ *   albedo:       .xyz = mean albedo, .w = fraction of the samples that hit something;
+ *   normal/depth: .xyz = mean normal (not renormalised: shorter than 1 where the samples disagree), .w = mean hit distance t
+ *                 over the samples that hit, 0 if none hit.
+ * One sample: the FIRST hit of its camera ray, no skip-through.
+ *   - a miss: albedo (1,1,1), normal 0, no depth (adds nothing to the hit count or the t sum);
+ *   - a hit: normal = the shading normal sn of the surface rebuilt as shade rebuilds it (instances included), flipped to face
+ *     the ray: dot(sn, D) > 0 ? -sn : sn; albedo by material, each channel then clamped as a < 1 ? a : 1:
+ *     null material (an emitter) (1,1,1); AGPT_MAT_MIRROR mirror_r; AGPT_MAT_GLASS mirror_r + diffuse_r;
+ *     otherwise (Disney) diffuse_r + spec_r0.
+ * Per pixel, float32 sums in ascending sample order; then albedo.xyz = sum / num_samples, albedo.w = hits / num_samples,
+ * normal.xyz = sum / num_samples, depth = hits > 0 ? t_sum / hits : 0.  Batched like agpt_render (whole samples per batch);
+ * the film and moments are not touched.  The guides belong to the scene, camera and film they were traced with:
+ * agpt_set_film, agpt_set_camera and every agpt_upload_* that passes its argument checks (a later failure too) make them stale (agpt_clear and agpt_render* do not).
+ * oracle/agpt_guides_oracle.cpp states the same on the CPU. */
+int agpt_render_guides(agpt_ctx* ctx, int num_samples, uint32_t flags);   /* 1 <= num_samples <= 1<<24 */
+int agpt_read_guides(agpt_ctx* ctx, float* albedo_rgba, float* normal_depth_rgba);   /* either may be NULL; AGPT_ERR_STATE if none */
+
+/* The spatial part of SVGF (Schied et al. 2017): the edge-avoiding a-trous wavelet filter of Dammertz et al. 2010 driven by
+ * per-pixel variance, without temporal reprojection, over the resident film, moments and (fresh) guides.  float32, every
+ * operation rounded on its own (+ - * / sqrt, compares, selects), stated element for element in oracle/denoise.py:
+ *   per pixel (a = film, q = moments.xyz, n = moments.w, per channel c):
+ *     mu_c  = n > 0 ? a_c / n : 0;
+ *     var_c = n < 2 ? 0 : v / n with mu = a / n; d = q - a * mu; v = d / (n - 1); v = v < 0 ? 0 : v   (the arithmetic of the
+ *             convergence test of agpt_adaptive, shared with it);
+ *     al_c  = albedo_c > EPS_A ? albedo_c : EPS_A,  EPS_A = 0.01;   e_c = mu_c / al_c;
+ *     lum(x) = (0.212671 * x.r + 0.715160 * x.g) + 0.072169 * x.b;
+ *     v_l   = (t_r + t_g) + t_b,  t_c = ((W_c * W_c) * var_c) / (al_c * al_c),  W = the luminance weights above;
+ *     missed: none of the pixel's guide samples hit (albedo.w == 0).  Its guide normal is then 0, so its w_n is 0 for every
+ *     tap: a pixel that saw only sky is never filtered (w_z's miss cases decide only for guides whose normal is not 0).
+ *   iteration i = 0 .. iterations-1, every pixel p from the previous iteration's (e, v_l), step = 2^i:
+ *     for dy = -2..2 (outer), dx = -2..2 (inner): q = (film row of p + dy * step, column of p + dx * step); a tap outside the
+ *     film is skipped;
+ *       w_l = 1 / (1 + (dl * dl) / ((s_l * s_l) * v_p + EPS_L)),  dl = lum(e_p) - lum(e_q),  EPS_L = 1e-4,  s_l = sigma_luminance;
+ *       w_n = m squared normal_power_log2 times (m = m * m), m = dot(n_p, n_q) (= (x*x' + y*y') + z*z'), m = m > 0 ? m : 0;
+ *       w_z = 1 if both missed, 0 if exactly one missed, else 1 / (1 + |z_p - z_q| / (sigma_depth * z_p));
+ *       w   = (((h[dx] * h[dy]) * w_l) * w_n) * w_z,  h = (1/16, 1/4, 3/8, 1/4, 1/16);
+ *       W += w;  S_c += w * e_q,c;  V += (w * w) * v_q   (sums from 0, in tap order);
+ *     e'_c = S_c / W,  v' = V / (W * W).
+ *   end: out_c = e_c * al_c (out.w = 0); packed = ResolvePixel(out, 1) (agpt_resolve's lin2rgb / rgb2uint of the floats).
+ *   iterations == 0: out = (mu, 0), no demodulation: the per-pixel means, and the packed pixels equal agpt_resolve_counts.
+ * Non-finite values (cfg 8: sums of squares that overflow to inf): a pixel is INVALID when one of its e_c or its v_l is not
+ * finite.  An invalid pixel keeps its (e, v_l) through every iteration and is skipped as a tap.  A tap whose w is not finite
+ * (NaN: inf / inf, 0 / 0) is skipped.  A pixel whose W is not > 0 (sky pixels: normal 0), or whose e' or v' is not finite,
+ * keeps its (e, v_l) in that iteration.  sigma_depth = 0 therefore turns the filter off: every hit pixel's centre tap is
+ * 0 / 0 and every other tap that hit has w_z = 0.
+ * Refused with AGPT_ERR_INVALID (params NULL, iterations outside [0, 10], a sigma not finite or < 0, normal_power_log2
+ * outside [0, 10]) and AGPT_ERR_STATE (moments off, no film, guides missing or stale); a refused call writes nothing and
+ * leaves film, moments and guides as they were.  out_rgba: float4[W*H] in film row order like agpt_read_accum; out_rgb8:
+ * W*H packed pixels in agpt_resolve_counts' layout; either may be NULL. */
+struct agpt_denoise {
+	int32_t iterations;        /* a-trous passes, 0 .. 10 */
+	float sigma_luminance;     /* luminance edge stop, in standard deviations of the pixel's luminance */
+	float sigma_depth;         /* depth edge stop, relative to the pixel's depth */
+	int32_t normal_power_log2; /* w_n = max(0, dot(n_p, n_q)) ^ (2 ^ normal_power_log2) */
+};
+typedef struct agpt_denoise agpt_denoise_params;
+int agpt_denoise(agpt_ctx* ctx, const agpt_denoise_params* params, float* out_rgba, uint32_t* out_rgb8);
+
 /* ---- multi-GPU: sample-index sharding (SURVEY 8e; north star "NCCL reduces the accumulators over NVLink") ----
  * One context per GPU of ONE process, each holding the whole scene and a film of the same size.  GPU g of G
  * renders the samples s = first + g (mod G) into its own accumulator (agpt_render with sample_stride = G, or

@@ -88,6 +88,12 @@ int agpt_host_tracer_render_resolve(agpt_host_tracer* tracer, agpt_host_scene* s
  * host_counts[y*W + x] (W*H ints) receives each pixel's sample count. */
 int agpt_host_tracer_render_adaptive(agpt_host_tracer* tracer, agpt_host_scene* scene, int width, int height, float* host_rgba,
 		const agpt_adaptive* params, int depth_arg, uint32_t flags, int32_t* host_counts);
+/* EXTENSION: CudaPathTracer::RenderAdaptiveDenoised (agpt.h agpt_render_guides / agpt_denoise): the adaptive frame as above,
+ * then the guides of samples [0, guide_samples) and the denoiser; out_rgba (W*H float4) and out_rgb8 (W*H) receive the denoised
+ * image in film row order, either may be NULL. */
+int agpt_host_tracer_render_adaptive_denoised(agpt_host_tracer* tracer, agpt_host_scene* scene, int width, int height, float* host_rgba,
+		const agpt_adaptive* params, const agpt_denoise_params* denoise, int guide_samples, int depth_arg, uint32_t flags, int32_t* host_counts,
+		float* out_rgba, uint32_t* out_rgb8);
 /* CudaPathTracer::Li(Ray(o, d), scene, depth_arg) */
 int agpt_host_tracer_li(agpt_host_tracer* tracer, agpt_host_scene* scene, const float* o3, const float* d3, int depth_arg, float* out3);
 
