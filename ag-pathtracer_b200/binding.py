@@ -290,6 +290,12 @@ class Context:
         _check(core().agpt_read_moments(self._h, _fptr(out)))
         return out
 
+    def write_moments(self, arr):
+        """Moments in read_moments' layout back to the device (resume an adaptive render along with write_accum)."""
+        arr = np.ascontiguousarray(arr, np.float32)
+        assert arr.shape == (self.height, self.width, 4)
+        _check(core().agpt_write_moments(self._h, _fptr(arr)))
+
     def adaptive_select(self, params, want_pixels=True):
         """The convergence test over the film: (count, film pixel indices y*W + x of the selected pixels, or None)."""
         n = c_int(0)

@@ -1063,6 +1063,21 @@ int agpt_read_moments(agpt_ctx* c, float* host) {
 	return AGPT_OK;
 }
 
+int agpt_write_moments(agpt_ctx* c, const float* host) {
+	JOIN(c);
+	NEED(c != nullptr && host != nullptr, AGPT_ERR_INVALID, "null argument");
+	NEED(c->momentsOn && c->moments.p != nullptr, AGPT_ERR_STATE, "moments are off (agpt_set_moments) or film not set");
+	// k_generate<true> seeds a listed pixel's paths from (int)moments.w: every count must be one it can hold
+	for (size_t i = 0; i < c->moments.n; i++) {
+		const float w = host[4 * i + 3];
+		NEED(w >= 0.f && w <= 16777216.f && w == std::floor(w), AGPT_ERR_INVALID, "agpt_write_moments: every .w must be an integer in [0, 2^24]");
+	}
+	CU(cudaSetDevice(c->device));
+	CU(cudaMemcpyAsync(c->moments.p, host, c->moments.Bytes(), cudaMemcpyHostToDevice, c->stream));
+	CU(cudaStreamSynchronize(c->stream));
+	return AGPT_OK;
+}
+
 static int CheckAdaptive(const agpt_adaptive* p) {
 	NEED(p != nullptr, AGPT_ERR_INVALID, "null agpt_adaptive");
 	NEED(p->min_samples >= 2 && p->min_samples <= p->max_samples && p->max_samples <= (1 << 24), AGPT_ERR_INVALID,

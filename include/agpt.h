@@ -313,6 +313,10 @@ int agpt_resolve(agpt_ctx* ctx, int samples, uint32_t* host_rgb8);
  * owns the consistency between film and moments. */
 int agpt_set_moments(agpt_ctx* ctx, int enable);
 int agpt_read_moments(agpt_ctx* ctx, float* host_rgba);            /* D2H of float4[W*H]; AGPT_ERR_STATE while moments are off */
+/* H2D of float4[W*H] (resume, with agpt_write_accum).  Every .w must be an integer in [0, 2^24] (NaN and inf are not), else
+ * AGPT_ERR_INVALID and the moments stay as they were; AGPT_ERR_STATE while moments are off.  Like agpt_write_accum, it leaves
+ * fresh guides fresh. */
+int agpt_write_moments(agpt_ctx* ctx, const float* host_rgba);
 
 /* Convergence test.  Valid: 2 <= min_samples <= max_samples <= 1<<24, step >= 1, tolerance and floor finite and >= 0
  * (else AGPT_ERR_INVALID).  Pixel p, with film sum a, moments q and count n, is SELECTED (needs `step` more samples) iff

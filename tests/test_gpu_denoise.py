@@ -48,19 +48,25 @@ def setup(agpt, ctx, cfg, w=W, h=H):
     return d, hs
 
 
-@pytest.mark.parametrize("cfg,h", [(c, H) for c in LEVELS] + [(5, 56)])
-def test_guides_equal_the_statement(agpt, dctx, cfg, h):
+# 1x1, one row, one column, one 8x4 tile, partial tiles in both axes, tiled films
+GUIDE_SHAPES = [pytest.param(c, W, H, id=f"{c}-{H}") for c in LEVELS] + [pytest.param(5, W, 56, id="5-56")] + \
+    [pytest.param(c, w, h, id=f"{c}-{w}x{h}") for c, w, h in [(1, 1, 1), (1, 1, 37), (1, 37, 1), (1, 8, 4), (1, 9, 5), (1, 33, 9),
+                                                              (1, 97, 55), (1, 104, 60), (5, 33, 9)]]
+
+
+@pytest.mark.parametrize("cfg,w,h", GUIDE_SHAPES)
+def test_guides_equal_the_statement(agpt, dctx, cfg, w, h):
     """At 96x54 the film takes the row-major slot order, at 96x56 (a multiple of the 8x4 tile) the tiled one."""
     from oracle import guides_binding
-    d, hs = setup(agpt, dctx, cfg, W, h)
+    d, hs = setup(agpt, dctx, cfg, w, h)
     dctx.render_guides(4)
     alb, nd = dctx.read_guides()
-    _, want_alb, want_nd = guides_binding.GuideScene(hs).guides(W, h, 4)
+    _, want_alb, want_nd = guides_binding.GuideScene(hs).guides(w, h, 4)
     assert same_floats(alb, want_alb) and same_floats(nd, want_nd)
     # one sample: hit or miss and t are trace_primary(0)'s
     dctx.render_guides(1)
     alb, nd = dctx.read_guides()
-    hits = dctx.trace_primary(0).reshape(h, W)[::-1]
+    hits = dctx.trace_primary(0).reshape(h, w)[::-1]
     assert np.array_equal(alb[..., 3], hits["found"].astype(np.float32))
     assert np.array_equal(bits(nd[..., 3]), bits(hits["t"]))
 
@@ -95,7 +101,7 @@ def test_denoise_equals_the_statement(agpt, dctx, cfg, mode):
     if cfg == 8:
         assert not np.isfinite(mom).all()          # sums of squares that overflowed: the non-finite rule is exercised
     counts = dctx.resolve_counts()
-    for it in (0, 1, 5):
+    for it in (0, 1, 5, 10):
         p = agpt.denoise_params(iterations=it)
         out, rgb8 = dctx.denoise(p)
         want = dn.denoise(film, mom, alb, nd, it, p.sigma_luminance, p.sigma_depth, p.normal_power_log2)
