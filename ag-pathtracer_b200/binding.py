@@ -97,6 +97,17 @@ def denoise_params(iterations=5, sigma_luminance=8.0, sigma_depth=0.1, normal_po
     return DenoiseParams(int(iterations), float(sigma_luminance), float(sigma_depth), int(normal_power_log2))
 
 
+class ReprojectParams(ctypes.Structure):  # agpt_reproject (extension: reprojection across camera moves)
+    _fields_ = [("max_history", c_float), ("sigma_depth", c_float), ("min_normal_dot", c_float)]
+
+
+def reproject_params(max_history=8.0, sigma_depth=0.05, min_normal_dot=0.5):
+    """agpt_reproject record; the reprojection it parameterises is stated in include/agpt.h and oracle/reproject.py.  The defaults
+    are the best of tests/perf_temporal.py's sweep on cfg 3 along a 16-frame orbit at 4 spp per frame and within 3 % of the best on
+    cfg 5 (DESIGN.md section 10 has the measurements)."""
+    return ReprojectParams(float(max_history), float(sigma_depth), float(min_normal_dot))
+
+
 class Stats(ctypes.Structure):  # agpt_stats
     _fields_ = [(n, c_uint64) for n in ("paths", "rays_closest", "rays_shadow", "rays_mis", "rays_skip", "rays_mis_culled", "rays_tail_culled")] + \
                [(n, c_uint64 * 2) for n in ("node_visits", "box_tests", "tri_tests", "analytic_tests", "warp_steps", "lane_steps")] + \
@@ -334,6 +345,11 @@ class Context:
         rgb8 = np.empty((self.height, self.width), np.uint32)
         _check(core().agpt_denoise(self._h, byref(params), _fptr(out), rgb8.ctypes.data_as(POINTER(c_uint32))))
         return out, rgb8
+
+    # ---- reprojection (extension) ------------------------------------------------------------------
+    def reproject_film(self, params):
+        """Carry the film and moments from the saved view into the current camera's (needs fresh guides), then save this view."""
+        _check(core().agpt_reproject_film(self._h, byref(params)))
 
     def trace_primary(self, sample, flags=0):
         out = np.empty(self.width * self.height, HIT_DTYPE)
@@ -657,6 +673,21 @@ class HostTracer:
                                                                 counts.ctypes.data_as(POINTER(c_int32)), _fptr(out),
                                                                 rgb8.ctypes.data_as(POINTER(c_uint32))), host_side=True)
         return counts, out, rgb8
+
+    def render_temporal(self, scene, width, height, accum, first_sample, num_samples, reproject, denoise, guide_samples, camera=None,
+                        depth_arg=0, flags=0):
+        """CudaPathTracer::RenderTemporal with `camera` (19 floats of agpt_camera, None: the scene's): the film replaces `accum`;
+        returns (denoised float32 [H, W, 4], packed uint32 [H, W]), both in the film's row order."""
+        assert accum.dtype == np.float32 and accum.shape == (height, width, 4) and accum.flags.c_contiguous
+        out = np.empty((height, width, 4), np.float32)
+        rgb8 = np.empty((height, width), np.uint32)
+        cam = None if camera is None else np.ascontiguousarray(camera, np.float32)
+        assert cam is None or cam.size == 19
+        _check(host().agpt_host_tracer_render_temporal(self._h, scene.handle, None if cam is None else cam.ctypes.data_as(c_void_p), c_int(width),
+                                                       c_int(height), _fptr(accum), c_int(first_sample), c_int(num_samples), byref(reproject),
+                                                       byref(denoise), c_int(guide_samples), c_int(depth_arg), c_uint32(flags), _fptr(out),
+                                                       rgb8.ctypes.data_as(POINTER(c_uint32))), host_side=True)
+        return out, rgb8
 
     def li(self, scene, origin, direction, depth_arg=0):
         o = (c_float * 3)(*origin); d = (c_float * 3)(*direction); out = (c_float * 3)()

@@ -126,6 +126,14 @@ struct agpt_ctx {
 	uint64_t guidesGen = 0;       // 0: no guides
 	DevBuf<float4> guideAlbedo, guideNormal;
 	DevBuf<float4> denoiseE[2], denoiseG, denoiseOut;   // ping-pong (e, v_l), the filter's guide, the result
+	// reprojection (agpt_reproject_film): the saved view is viewCam and the guide G per pixel in viewG[viewCur]
+	uint64_t historyGen = 1;      // bumped by what makes a saved view wrong: agpt_set_film to a new size, every agpt_upload_* past
+	                              // its argument checks, agpt_set_moments(0).  Not by agpt_set_camera: carrying across it is the point
+	uint64_t viewGen = 0;         // the historyGen the saved view was taken in; 0: none
+	agpt_camera viewCam;
+	DevBuf<float4> viewG[2];      // ping-pong: a call reads its saved G from one and saves the current G into the other
+	int viewCur = 0;
+	DevBuf<float4> reprojFilm, reprojMoments;   // the gathered film and moments (the gathers read the old ones)
 
 	// wavefront state
 	size_t capacity = 0;          // path slots allocated
@@ -481,6 +489,7 @@ int agpt_destroy(agpt_ctx* c) {
 	c->accumOwn.Free(); c->resolved.Free();
 	c->moments.Free(); c->adaptiveList.Free(); c->adaptiveCount.Free();
 	c->guideAlbedo.Free(); c->guideNormal.Free(); c->denoiseE[0].Free(); c->denoiseE[1].Free(); c->denoiseG.Free(); c->denoiseOut.Free();
+	c->viewG[0].Free(); c->viewG[1].Free(); c->reprojFilm.Free(); c->reprojMoments.Free();
 	c->envRgb.Free(); c->envFunc.Free(); c->envCdf.Free();
 	for (auto& b : c->f4) b.Free();
 	for (auto& b : c->i32) b.Free();
@@ -568,6 +577,7 @@ int agpt_upload_meshes(agpt_ctx* c, const agpt_mesh_desc* meshes, int n) {
 	CU(cudaStreamSynchronize(c->stream));
 	c->gridCalibrated = false;
 	c->stateGen++;
+	c->historyGen++;
 	// from here on a failure must not leave the device table pointing at freed buffers
 	for (auto& m : c->meshStore) m.Free();
 	c->meshStore.assign(n, MeshStore());
@@ -619,6 +629,7 @@ int agpt_upload_meshes(agpt_ctx* c, const agpt_mesh_desc* meshes, int n) {
 		CU(cudaSetDevice(c->device)); \
 		CU(cudaStreamSynchronize(c->stream)); \
 		c->stateGen++; \
+		c->historyGen++; \
 		CU(c->member.Upload(rows, (size_t)n, c->stream)); \
 		CU(cudaStreamSynchronize(c->stream)); \
 		counter; \
@@ -642,6 +653,7 @@ int agpt_upload_primitives(agpt_ctx* c, const agpt_prim* rows, int n) {
 	CU(cudaSetDevice(c->device));
 	CU(cudaStreamSynchronize(c->stream));
 	c->stateGen++;
+	c->historyGen++;
 	CU(c->prims.Upload(rows, (size_t)n, c->stream));
 	c->hostPrims.assign(rows, rows + n);
 	c->runsDirty = true;
@@ -659,6 +671,7 @@ int agpt_upload_envmap(agpt_ctx* c, const agpt_envmap* env) {
 	c->envRgb.Free(); c->envFunc.Free(); c->envCdf.Free();
 	c->envW = c->envH = 0; c->envFuncInt = 0;
 	c->stateGen++;
+	c->historyGen++;
 	if (!env || env->width == 0) return AGPT_OK;
 	NEED(env->width > 0 && env->height > 0 && env->rgb && env->func && env->cdf, AGPT_ERR_INVALID, "bad environment map");
 	size_t n = (size_t)env->width * env->height;
@@ -695,6 +708,7 @@ int agpt_set_film(agpt_ctx* c, int width, int height) {
 	CU(cudaSetDevice(c->device));
 	c->stateGen++;
 	if (width == c->width && height == c->height) return AGPT_OK;
+	c->historyGen++;
 	CU(cudaStreamSynchronize(c->stream));
 	bool own = c->accum == c->accumOwn.p;
 	c->width = width; c->height = height;
@@ -1041,7 +1055,8 @@ int agpt_set_moments(agpt_ctx* c, int enable) {
 	CU(cudaStreamSynchronize(c->stream));
 	if (!enable) {
 		c->momentsOn = false;
-		c->moments.Free(); c->adaptiveList.Free(); c->adaptiveCount.Free();
+		c->historyGen++;
+		c->moments.Free(); c->adaptiveList.Free(); c->adaptiveCount.Free(); c->reprojMoments.Free();
 		return AGPT_OK;
 	}
 	if (c->momentsOn) return AGPT_OK;
@@ -1298,6 +1313,58 @@ int agpt_denoise(agpt_ctx* c, const agpt_denoise_params* params, float* out_rgba
 	if (out_rgba) CU(cudaMemcpyAsync(out_rgba, c->denoiseOut.p, (size_t)n * sizeof(float4), cudaMemcpyDeviceToHost, c->stream));
 	if (out_rgb8) CU(cudaMemcpyAsync(out_rgb8, c->resolved.p, (size_t)n * sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream));
 	CU(cudaStreamSynchronize(c->stream));
+	return AGPT_OK;
+}
+
+// ---- reprojection (EXTENSION, agpt.h agpt_reproject_film) -----------------------------------------------------------------------
+static int CheckReproject(const agpt_reproject* p) {
+	NEED(p != nullptr, AGPT_ERR_INVALID, "null agpt_reproject");
+	NEED(p->max_history >= 1.f && p->max_history <= 16777216.f, AGPT_ERR_INVALID, "agpt_reproject: need 1 <= max_history <= 2^24");
+	NEED(std::isfinite(p->sigma_depth) && p->sigma_depth > 0.f, AGPT_ERR_INVALID, "agpt_reproject: sigma_depth must be finite and > 0");
+	NEED(p->min_normal_dot >= -1.f && p->min_normal_dot <= 1.f, AGPT_ERR_INVALID, "agpt_reproject: need -1 <= min_normal_dot <= 1");
+	return AGPT_OK;
+}
+
+// One k_reproject_film: CARRY gathers film and moments from the saved view into reprojFilm / reprojMoments, which then replace
+// them (the film by a copy, so that a caller-owned or exported film keeps its address); either way the current G goes into the
+// other viewG buffer, which becomes the saved view.
+int agpt_reproject_film(agpt_ctx* c, const agpt_reproject* params) {
+	JOIN(c);
+	NEED(c != nullptr, AGPT_ERR_INVALID, "null context");
+	int rcode = CheckReproject(params);
+	if (rcode != AGPT_OK) return rcode;
+	NEED(c->momentsOn && c->moments.p != nullptr && c->accum != nullptr, AGPT_ERR_STATE, "moments are off (agpt_set_moments) or film not set");
+	NEED(GuidesFresh(c), AGPT_ERR_STATE, "guides missing or stale: agpt_render_guides after the last agpt_set_film / agpt_set_camera / agpt_upload_*");
+	const agpt_reproject p = *params;
+	CU(cudaSetDevice(c->device));
+	const int W = c->width, H = c->height;
+	const size_t n = (size_t)W * H;
+	const bool saved = c->viewGen != 0 && c->viewGen == c->historyGen && c->viewG[c->viewCur].n == n;
+	// A static camera keeps film and moments as they are.  Recomputing the identity map in float rounds some pixel centres to
+	// within an ulp of a pixel edge, and their bilinear weights would leak a tiny share of a neighbour into every static frame;
+	// with this rule a static camera accumulates exactly as without reprojection.
+	const bool carry = saved && memcmp(&c->viewCam, &c->cam, sizeof(agpt_camera)) != 0;
+	const int next = c->viewCur ^ 1;
+	if (c->viewG[next].n != n) CU(c->viewG[next].Alloc(n));
+	if (carry && c->reprojFilm.n != n) CU(c->reprojFilm.Alloc(n));
+	if (carry && c->reprojMoments.n != n) CU(c->reprojMoments.Alloc(n));     // (agpt_set_moments(0) frees it)
+	const dim3 block(32, 8), grid(Blocks(W, 32), Blocks(H, 8));
+	if (carry)
+		k_reproject_film<true><<<grid, block, 0, c->stream>>>(c->accum, c->moments.p, c->viewG[c->viewCur].p, c->guideAlbedo.p, c->guideNormal.p, W, H,
+			c->cam, c->viewCam, p.max_history, p.sigma_depth, p.min_normal_dot, c->reprojFilm.p, c->reprojMoments.p, c->viewG[next].p);
+	else
+		k_reproject_film<false><<<grid, block, 0, c->stream>>>(nullptr, nullptr, nullptr, c->guideAlbedo.p, c->guideNormal.p, W, H,
+			c->cam, c->cam, p.max_history, p.sigma_depth, p.min_normal_dot, nullptr, nullptr, c->viewG[next].p);
+	CU(cudaGetLastError());
+	c->stats.kernel_launches++;
+	if (carry) {
+		CU(cudaMemcpyAsync(c->accum, c->reprojFilm.p, n * sizeof(float4), cudaMemcpyDeviceToDevice, c->stream));
+		std::swap(c->moments, c->reprojMoments);
+	}
+	CU(cudaStreamSynchronize(c->stream));
+	c->viewCur = next;
+	c->viewCam = c->cam;
+	c->viewGen = c->historyGen;
 	return AGPT_OK;
 }
 

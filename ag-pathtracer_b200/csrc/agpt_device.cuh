@@ -27,7 +27,7 @@
 // pool this was developed on, so the small GPU tests are run once per round against this build.
 enum { AGPT_DBG_STACK = 1, AGPT_DBG_NODE = 2, AGPT_DBG_TRI = 3, AGPT_DBG_QUEUE = 4, AGPT_DBG_PATH = 5, AGPT_DBG_PRIM = 6, AGPT_DBG_MATERIAL = 7,
        AGPT_DBG_LIST = 8 /* adaptive pixel list entry or pixel index */, AGPT_DBG_SAMPLE = 9 /* a pixel's samples past max_samples */,
-       AGPT_DBG_GUIDE = 10 /* k_guides: path slot */, AGPT_DBG_TAP = 11 /* denoise: filter tap outside the film */ };
+       AGPT_DBG_GUIDE = 10 /* k_guides: path slot */, AGPT_DBG_TAP = 11 /* denoise, reprojection: filter or history tap outside the film */ };
 #ifdef AGPT_DEBUG
 __device__ unsigned long long g_agptDebug[4];     // [0] failures, [1] first code, [2] first value, [3] checks executed
 #define AGPT_CHECK(cond, code, value) do { atomicAdd(&g_agptDebug[3], 1ull); if (!(cond)) { \

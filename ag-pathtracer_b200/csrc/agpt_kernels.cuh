@@ -1153,6 +1153,81 @@ __global__ void __launch_bounds__(256) k_denoise_atrous(const float4* __restrict
 	else Eout[p] = res;
 }
 
+// ---- EXTENSION: reprojection of the film and its moments across a camera move (agpt.h agpt_reproject_film; CPU statement
+// oracle/reproject.py) -------------------------------------------------------------------------------------------------------
+// k_reproject_film: one thread per film pixel (a 32 x 8 block covers a film patch).  Every pixel writes its guide G (normal,
+// depth or -1 for a pixel whose guide samples all missed, as k_denoise_prepare builds it) into Gout, the view the next call
+// reprojects from.  CARRY: the pixel's centre ray is projected into the saved camera `prev` and the film and moments are
+// gathered from the accepted bilinear taps of the old film (accumIn, momentsIn, Gin) into accumOut and momentsOut.
+template <bool CARRY>
+__global__ void __launch_bounds__(256) k_reproject_film(const float4* __restrict__ accumIn, const float4* __restrict__ momentsIn, const float4* __restrict__ Gin,
+		const float4* __restrict__ albedo, const float4* __restrict__ normalDepth, int width, int height, agpt_camera cur, agpt_camera prev,
+		float maxHistory, float sigmaDepth, float minNormalDot, float4* __restrict__ accumOut, float4* __restrict__ momentsOut, float4* __restrict__ Gout) {
+	const int x = blockIdx.x * blockDim.x + threadIdx.x, r = blockIdx.y * blockDim.y + threadIdx.y;
+	if (x >= width || r >= height) return;
+	const int p = r * width + x, y = height - 1 - r;
+	const float4 nd = normalDepth[p];
+	const float4 gp = make_float4(nd.x, nd.y, nd.z, albedo[p].w == 0.f ? -1.f : nd.w);
+	const bool hitP = gp.w >= 0.f;
+	Gout[p] = gp;
+	if (!CARRY) return;
+	const float W = (float)width, Hf = (float)height;
+	const float s = (x + 0.5f) / W, t = (y + 0.5f) / Hf;
+	const float3 O = f3(cur.origin), O1 = f3(prev.origin), H1 = f3(prev.horizontal), V1 = f3(prev.vertical);
+	const float3 D = normalize(((f3(cur.lower_left_corner) + s * f3(cur.horizontal)) + t * f3(cur.vertical)) - O);
+	float3 d = D;
+	float z = 0.f;
+	if (hitP) {
+		d = (O + gp.w * D) - O1;
+		z = length(d);
+	}
+	float4 A = make_float4(0.f, 0.f, 0.f, 0.f), Q = A;
+	float sw = 0.f;
+	const float3 f = ((f3(prev.lower_left_corner) + 0.5f * H1) + 0.5f * V1) - O1;
+	const float den = dot(d, f);
+	if (den > 0.f) {
+		const float lam = dot(f, f) / den;
+		const float u = 0.5f + (lam * dot(d, H1)) / dot(H1, H1);
+		const float v = 0.5f + (lam * dot(d, V1)) / dot(V1, V1);
+		const float px = u * W - 0.5f, py = v * Hf - 0.5f;
+		const float x0 = floorf(px), y0 = floorf(py);
+		// (a NaN or infinite px / py fails these compares too; within them the tap indices fit an int)
+		if (x0 >= -1.f && x0 <= W - 1.f && y0 >= -1.f && y0 <= Hf - 1.f) {
+			const float fx = px - x0, fy = py - y0;
+			const float wx[2] = { 1.f - fx, fx }, wy[2] = { 1.f - fy, fy };
+			const int ix = (int)x0, iy = (int)y0;
+#pragma unroll
+			for (int k = 0; k < 4; k++) {
+				const int tx = ix + (k & 1), ty = iy + (k >> 1);
+				const float w = wx[k & 1] * wy[k >> 1];
+				if (tx < 0 || tx >= width || ty < 0 || ty >= height || !(w > 0.f)) continue;
+				const int q = (height - 1 - ty) * width + tx;
+				AGPT_CHECK(q >= 0 && q < width * height, AGPT_DBG_TAP, q);
+				const float4 a = accumIn[q], m = momentsIn[q], g = Gin[q];
+				if (!Finite4(a) || !Finite4(m)) continue;
+				const bool hitQ = g.w >= 0.f;
+				if (hitQ != hitP) continue;
+				if (hitP && !(fabsf(g.w - z) <= sigmaDepth * z && (gp.x * g.x + gp.y * g.y) + gp.z * g.z >= minNormalDot)) continue;
+				sw += w;
+				A.x += w * a.x; A.y += w * a.y; A.z += w * a.z; A.w += w * a.w;
+				Q.x += w * m.x; Q.y += w * m.y; Q.z += w * m.z; Q.w += w * m.w;
+			}
+		}
+	}
+	if (sw > 0.f) {
+		A = make_float4(A.x / sw, A.y / sw, A.z / sw, A.w / sw);
+		Q = make_float4(Q.x / sw, Q.y / sw, Q.z / sw, Q.w / sw);
+		if (Q.w > maxHistory) {
+			const float k = maxHistory / Q.w;
+			A = make_float4(A.x * k, A.y * k, A.z * k, A.w * k);
+			Q = make_float4(Q.x * k, Q.y * k, Q.z * k, maxHistory);
+		}
+	}
+	else { A = make_float4(0.f, 0.f, 0.f, 0.f); Q = A; }
+	accumOut[p] = A;
+	momentsOut[p] = Q;
+}
+
 // ---- bandwidth probe: what a plain streaming read of this library's own making reaches on this GPU ----
 // `n16` 16-byte words read `iters` times by a persistent grid with 128-bit loads.  A buffer that fits in L2
 // measures L2 bandwidth (the roofline denominator for the trace kernels' L2 traffic), one far larger than L2

@@ -273,6 +273,33 @@ int agpt_host_tracer_render_adaptive_denoised(agpt_host_tracer* t, agpt_host_sce
 	return AGPT_OK;
 }
 
+// A Camera whose derived vectors are given (a viewer moved it): Export() returns them as they are.
+struct GivenCamera : Camera {
+	GivenCamera(const CameraDesc& d, const agpt_camera& k) : Camera(d) {
+		origin = float3(k.origin[0], k.origin[1], k.origin[2]);
+		lower_left_corner = float3(k.lower_left_corner[0], k.lower_left_corner[1], k.lower_left_corner[2]);
+		horizontal = float3(k.horizontal[0], k.horizontal[1], k.horizontal[2]);
+		vertical = float3(k.vertical[0], k.vertical[1], k.vertical[2]);
+		u = float3(k.u[0], k.u[1], k.u[2]);
+		v = float3(k.v[0], k.v[1], k.v[2]);
+		lens_radius = k.lens_radius;
+	}
+};
+
+int agpt_host_tracer_render_temporal(agpt_host_tracer* t, agpt_host_scene* s, const agpt_camera* camera, int width, int height, float* host_rgba,
+		int first_sample, int num_samples, const agpt_reproject* reproject, const agpt_denoise_params* denoise, int guide_samples, int depth_arg,
+		uint32_t flags, float* out_rgba, uint32_t* out_rgb8) {
+	if (!t || !s || !host_rgba || !reproject || !denoise) return HostFail("null argument");
+	g_hostError.clear();
+	HOST_TRY(
+		Accumulator acc(width, height, reinterpret_cast<float3*>(host_rgba));
+		GivenCamera cam(s->scene.camera, camera ? *camera : s->camera->Export());
+		t->tracer->RenderTemporal(s->scene, cam, acc, first_sample, num_samples, *reproject, *denoise, guide_samples, depth_arg,
+			reinterpret_cast<float3*>(out_rgba), out_rgb8, flags);
+	)
+	return AGPT_OK;
+}
+
 int agpt_host_tracer_li(agpt_host_tracer* t, agpt_host_scene* s, const float* o, const float* d, int depth_arg, float* out3) {
 	if (!t || !s || !o || !d || !out3) return HostFail("null argument");
 	g_hostError.clear();

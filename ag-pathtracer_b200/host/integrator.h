@@ -47,6 +47,7 @@ public:
 	// the scene's fingerprint differs from the resident one (another Scene object, or primitives /
 	// lights added since).
 	void Upload(const Scene& scene) const {
+		temporalW = temporalH = 0;
 		auto flat = scene.Flatten();
 		for (agpt_ctx* ctx : ctxs) {
 			Check(agpt_upload_meshes(ctx, flat->meshes.data(), (int)flat->meshes.size()));
@@ -100,6 +101,33 @@ public:
 		AdaptiveFrame(scene, camera, acc, params, &denoise, guideSamples, depth, counts, out, rgb8, flags);
 	}
 
+	// EXTENSION (agpt.h agpt_reproject_film): one frame of a viewer whose camera may have moved since the last frame, on a
+	// one-GPU tracer: the guides of samples [0, guideSamples) of this camera, the film and moments carried over from the last
+	// RenderTemporal frame into this view, samples [firstSample, firstSample + numSamples) added, and the denoiser.  Film,
+	// moments and the saved view stay on the device between the calls; the first frame, a new film size or a new scene start
+	// from a cleared film.  firstSample must keep advancing from frame to frame (agpt.h says why).  acc receives the film
+	// (acc.NumSamples() is set to 0: the counts are per pixel and fractional); out and rgb8 (film row order) the denoised image,
+	// either may be null.  Throws for a device list.
+	void RenderTemporal(const Scene& scene, const Camera& camera, Accumulator& acc, int firstSample, int numSamples, const agpt_reproject& reproject,
+			const agpt_denoise_params& denoise, int guideSamples, int depth, float3* out, uint32_t* rgb8, uint32_t flags = 0) const {
+		if (ctxs.size() != 1) throw std::runtime_error("CudaPathTracer: temporal frames render on one device only");
+		if (uploaded != scene.Fingerprint()) Upload(scene);
+		agpt_camera cam = camera.Export();
+		agpt_ctx* c = ctxs[0];
+		Check(agpt_set_camera(c, &cam));
+		Check(agpt_set_film(c, acc.width, acc.height));
+		Check(agpt_set_moments(c, 1));
+		if (temporalW != acc.width || temporalH != acc.height) Check(agpt_clear(c));
+		temporalW = temporalH = 0;
+		Check(agpt_render_guides(c, guideSamples, flags & (AGPT_FLAG_COUNTERS | AGPT_FLAG_STRICT_BOXES)));
+		Check(agpt_reproject_film(c, &reproject));
+		Check(agpt_render(c, firstSample, numSamples, 1, MaxDepth, depth, flags));
+		Check(agpt_read_accum(c, &acc.Pixels()->x));
+		Check(agpt_denoise(c, &denoise, out ? &out->x : nullptr, rgb8));
+		temporalW = acc.width; temporalH = acc.height;
+		acc.SetNumSamples(0);
+	}
+
 	// Single-ray entry point.  The reference's Li draws from the global generator; here the
 	// ray gets the RNG stream of (pixel 0, sample liCalls++), film/camera are not involved.
 	float3 Li(const Ray& ray, const Scene& scene, int depth = 0) const override;
@@ -118,6 +146,7 @@ protected:
 			int guideSamples, int depth, std::vector<int>& counts, float3* out, uint32_t* rgb8, uint32_t flags) const {
 		if (ctxs.size() != 1) throw std::runtime_error("CudaPathTracer: adaptive frames render on one device only");
 		if (uploaded != scene.Fingerprint()) Upload(scene);
+		temporalW = temporalH = 0;
 		agpt_camera cam = camera.Export();
 		agpt_ctx* c = ctxs[0];
 		Check(agpt_set_camera(c, &cam));
@@ -140,6 +169,7 @@ protected:
 	// every GPU's share of the samples into its own accumulator; GPU 0's starts from the caller's film
 	void RenderShards(const Scene& scene, const Camera& camera, Accumulator& acc, int firstSample, int numSamples, int depth, uint32_t flags) const {
 		if (uploaded != scene.Fingerprint()) Upload(scene);
+		temporalW = temporalH = 0;
 		agpt_camera cam = camera.Export();
 		for (size_t g = 0; g < ctxs.size(); g++) {
 			Check(agpt_set_camera(ctxs[g], &cam));
@@ -154,6 +184,7 @@ protected:
 	mutable std::vector<agpt_ctx*> ctxs;
 	mutable uint64_t uploaded = 0;     // Scene::Fingerprint() of the resident tables (0: none)
 	mutable unsigned liCalls = 0;
+	mutable int temporalW = 0, temporalH = 0;   // film size of the last RenderTemporal frame, whose film and view are resident (0: none)
 };
 
 // (defined here so that the mirror stays header-only; libagpt.so is the only link dependency)

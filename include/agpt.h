@@ -408,6 +408,57 @@ struct agpt_denoise {
 typedef struct agpt_denoise agpt_denoise_params;
 int agpt_denoise(agpt_ctx* ctx, const agpt_denoise_params* params, float* out_rgba, uint32_t* out_rgb8);
 
+/* ---- reprojection across camera moves (EXTENSION: the reference clears the film whenever the camera moves) ---------------
+ * The temporal half of SVGF for the sample statistics: the film and its moments are carried into the current camera's view, so
+ * a frame after a camera move starts from the samples of the frames before it instead of from none.  What is carried is
+ * "per-pixel sums + counts" as before, so agpt_denoise, agpt_resolve_counts and the convergence test apply unchanged.
+ *
+ * A viewer's frame, one per camera:  agpt_set_camera;  agpt_render_guides(ctx, g, 0);  agpt_reproject_film;
+ * agpt_render(ctx, first, k, ...) with first = the number of sample indices used by all frames so far;  agpt_denoise or
+ * agpt_resolve_counts.  The sample indices must keep advancing from frame to frame: a path's random numbers depend only on its
+ * (pixel, sample index), so a frame that reuses sample indices repeats the random numbers of the history it lands on and its
+ * samples are not independent of that history.
+ *
+ * The context keeps a SAVED VIEW: the camera and, per pixel in film row order, G = (mean guide normal, mean hit depth, or -1 for
+ * a pixel whose guide samples all missed) -- the G of k_denoise_prepare.  agpt_reproject_film (moments on, a film, fresh guides):
+ *   - no saved view: film and moments are left as they are; the view is saved;
+ *   - the saved camera is bitwise equal to the current one: film and moments are left as they are (recomputing the identity
+ *     map in float32 would put some pixel centres an ulp from a pixel edge and leak a tiny share of a neighbour into every
+ *     static frame: with this rule a static camera accumulates exactly as without reprojection); the view is saved again;
+ *   - otherwise, per current pixel (x, y) (film row H-1-y), float32, every operation rounded on its own:
+ *     1. centre ray: s = (x + 0.5) / W, t = (y + 0.5) / H, D = normalize(((L + s*Hz) + t*Vt) - O) with normalize(v) =
+ *        v * (1 / sqrt(dot(v, v))) and dot(a, b) = (a.x*b.x + a.y*b.y) + a.z*b.z (O, L, Hz, Vt: the current camera's origin,
+ *        lower-left corner, horizontal, vertical: CameraRay without jitter and lens offset);
+ *     2. a hit pixel (guide hit fraction > 0): X = O + depth * D, d = X - O', z = length(d) = sqrt(dot(d, d)) (primes: the
+ *        saved camera); a sky pixel: d = D (a point at infinity);
+ *     3. f = ((L' + 0.5*Hz') + 0.5*Vt') - O', den = dot(d, f); !(den > 0): no history.  lam = dot(f, f) / den,
+ *        u = 0.5 + (lam * dot(d, Hz')) / dot(Hz', Hz'), v = 0.5 + (lam * dot(d, Vt')) / dot(Vt', Vt'), px = u * W - 0.5,
+ *        py = v * H - 0.5;
+ *     4. x0 = floor(px), y0 = floor(py); unless -1 <= x0 <= W - 1 and -1 <= y0 <= H - 1 (false for a px or py that is not
+ *        finite) no history.  fx = px - x0, fy = py - y0, wx = (1 - fx, fx), wy = (1 - fy, fy); taps k = 0..3 in this order:
+ *        (x0 + (k & 1), y0 + (k >> 1)) with w = wx[k & 1] * wy[k >> 1], read at film row H-1-(y0 + (k >> 1)).  A tap is
+ *        ACCEPTED when it is inside the film, w > 0, its film and moments values are finite (all four channels each), its saved
+ *        G is a hit (G'.w >= 0) exactly when the current pixel's is, and for hits |G'.w - z| <= sigma_depth * z and
+ *        dot(n, n') >= min_normal_dot (n, n': current and saved guide normals);
+ *     5. over the accepted taps in tap order, from 0: Wt += w; S += w * a (film, four channels); Q += w * q (moments, four
+ *        channels).  Wt > 0: a' = S / Wt, q' = Q / Wt per channel, and if q'.w > max_history: k = max_history / q'.w,
+ *        a' = a' * k (four channels), q'.xyz = q'.xyz * k, q'.w = max_history.  Otherwise (a disocclusion) a' = q' = 0;
+ *   and the current camera and the current guides' G become the saved view.  oracle/reproject.py states the same.
+ * The saved view is dropped by agpt_set_film to a new size, by every agpt_upload_* past its argument checks (the scene changed)
+ * and by agpt_set_moments(0); agpt_set_camera keeps it.
+ * Consequences: counts become fractional, so agpt_resolve(samples) no longer describes the film (use agpt_resolve_counts or
+ * agpt_denoise), and agpt_write_moments still refuses fractional counts; agpt_render_adaptive still starts from a cleared film;
+ * one GPU only (like adaptive sampling); view-dependent radiance (mirror, glass, glossy lobes) ghosts, by up to max_history
+ * samples' worth.  Refused with AGPT_ERR_INVALID (params NULL, max_history outside [1, 2^24], sigma_depth not finite or <= 0,
+ * min_normal_dot outside [-1, 1]) and AGPT_ERR_STATE (moments off, no film, guides missing or stale); a refused call leaves
+ * film, moments and the saved view as they were.  The film keeps its address (agpt_set_accum_dev films too). */
+typedef struct agpt_reproject {
+	float max_history;     /* most samples a pixel may carry into the new view, 1 .. 2^24 */
+	float sigma_depth;     /* relative depth tolerance of a history tap, finite, > 0 */
+	float min_normal_dot;  /* least dot(normal, history normal) of a history tap, in [-1, 1] */
+} agpt_reproject;
+int agpt_reproject_film(agpt_ctx* ctx, const agpt_reproject* params);
+
 /* ---- multi-GPU: sample-index sharding (SURVEY 8e; north star "NCCL reduces the accumulators over NVLink") ----
  * One context per GPU of ONE process, each holding the whole scene and a film of the same size.  GPU g of G
  * renders the samples s = first + g (mod G) into its own accumulator (agpt_render with sample_stride = G, or

@@ -94,6 +94,13 @@ int agpt_host_tracer_render_adaptive(agpt_host_tracer* tracer, agpt_host_scene* 
 int agpt_host_tracer_render_adaptive_denoised(agpt_host_tracer* tracer, agpt_host_scene* scene, int width, int height, float* host_rgba,
 		const agpt_adaptive* params, const agpt_denoise_params* denoise, int guide_samples, int depth_arg, uint32_t flags, int32_t* host_counts,
 		float* out_rgba, uint32_t* out_rgb8);
+/* EXTENSION: CudaPathTracer::RenderTemporal (agpt.h agpt_reproject_film) on a one-device tracer: one viewer frame with the
+ * camera `camera` (NULL: the scene's own) -- guides, the film and moments of the last such frame carried into this view, samples
+ * [first_sample, first_sample + num_samples) added, denoised.  The film replaces host_rgba; out_rgba (W*H float4) and out_rgb8
+ * (W*H) receive the denoised image in film row order, either may be NULL. */
+int agpt_host_tracer_render_temporal(agpt_host_tracer* tracer, agpt_host_scene* scene, const agpt_camera* camera, int width, int height,
+		float* host_rgba, int first_sample, int num_samples, const agpt_reproject* reproject, const agpt_denoise_params* denoise,
+		int guide_samples, int depth_arg, uint32_t flags, float* out_rgba, uint32_t* out_rgb8);
 /* CudaPathTracer::Li(Ray(o, d), scene, depth_arg) */
 int agpt_host_tracer_li(agpt_host_tracer* tracer, agpt_host_scene* scene, const float* o3, const float* d3, int depth_arg, float* out3);
 
