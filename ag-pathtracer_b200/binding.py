@@ -139,6 +139,10 @@ class Stats(ctypes.Structure):  # agpt_stats
         return 64 * self.node_visits[k] + 48 * self.tri_tests[k] + 32 * self.analytic_tests[k] + 64 * rays
 
 
+class Texture(ctypes.Structure):      # agpt_texture
+    _fields_ = [("width", c_int), ("height", c_int), ("rgb", POINTER(c_float))]
+
+
 HIT_DTYPE = np.dtype([("found", np.uint32), ("prim", np.int32), ("tri", np.int32), ("t", np.float32)])
 
 _core = None
@@ -242,6 +246,18 @@ class Context:
         rows = np.ascontiguousarray(rows)
         assert rows.dtype.itemsize == 112
         _check(core().agpt_upload_instances(self._h, rows.ctypes.data_as(c_void_p), c_int(len(rows))))
+
+    def upload_textures(self, images, material_texture):
+        """EXTENSION (agpt.h agpt_upload_textures): images = base-colour textures, each a numpy (H, W, 3) float32 array of linear
+        RGB, row 0 at v in [0, 1/H); material_texture[i] = index into images of material i's texture, or -1.  ([], []) clears."""
+        imgs = [np.ascontiguousarray(a, np.float32) for a in images]
+        for a in imgs:
+            if a.ndim != 3 or a.shape[2] != 3:
+                raise AgptError("upload_textures: every image must be an (H, W, 3) array")
+        rows = (Texture * max(len(imgs), 1))(*[Texture(a.shape[1], a.shape[0], _fptr(a)) for a in imgs])
+        mt = np.ascontiguousarray(material_texture, np.int32)
+        _check(core().agpt_upload_textures(self._h, rows if imgs else None, c_int(len(imgs)),
+                                           mt.ctypes.data_as(POINTER(c_int)) if mt.size else None, c_int(mt.size)))
 
     def set_camera(self, cam19):
         cam19 = np.ascontiguousarray(cam19, np.float32)
@@ -577,7 +593,7 @@ class HostScene:
 
     def tables(self):
         """agpt_scene_tables view (opaque bytes) of the flattened scene, valid while the scene lives."""
-        buf = ctypes.create_string_buffer(256)       # sizeof(agpt_scene_tables) = 232
+        buf = ctypes.create_string_buffer(512)       # sizeof(agpt_scene_tables) = 248
         _check(host().agpt_host_scene_tables(self._h, buf), host_side=True)
         return buf
 

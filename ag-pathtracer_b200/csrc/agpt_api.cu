@@ -96,6 +96,13 @@ struct agpt_ctx {
 	bool runsDirty = true;
 	int maxSphereRun = 1 << 20;   // AGPT_MAX_SPHERE_RUN
 	DevBuf<agpt_material> mats;
+	std::vector<int32_t> hostMatTypes;
+	// image textures on the base colour of Disney materials (extension, agpt_upload_textures)
+	DevBuf<float4> texels;
+	DevBuf<DTexture> textures;
+	DevBuf<int> matTex;
+	std::vector<int32_t> hostMatTex;
+	bool hasTextures = false;     // some material has a texture: shade and guides run the textured instantiations
 	DevBuf<agpt_light> lights;
 	DevBuf<float> envRgb, envFunc, envCdf;
 	float envFuncInt = 0;
@@ -365,6 +372,12 @@ static int CheckReady(agpt_ctx* c, bool needFilm) {
 		NEED(al < 0 || (c->hostLights[al].type == AGPT_LIGHT_AREA && c->hostLights[al].prim == (int)i), AGPT_ERR_INVALID,
 			"primitive and area light do not name each other (one shape per AreaLight)");
 	}
+	if (c->hasTextures) {
+		// textures (extension): the binding table belongs to the resident material table, and binds Disney materials only
+		NEED(c->hostMatTex.size() == (size_t)c->nMats, AGPT_ERR_INVALID, "texture bindings were uploaded for a different number of materials");
+		for (size_t i = 0; i < c->hostMatTex.size(); i++)
+			NEED(c->hostMatTex[i] < 0 || c->hostMatTypes[i] == AGPT_MAT_DISNEY, AGPT_ERR_INVALID, "a texture is bound to a material that is not AGPT_MAT_DISNEY");
+	}
 	if (c->mats.p == nullptr) {
 		// a scene of null-material (emissive) shapes only is legal upstream; shade still needs a record to point idle lanes at
 		CU(cudaSetDevice(c->device));
@@ -485,7 +498,7 @@ int agpt_destroy(agpt_ctx* c) {
 	cudaStreamSynchronize(c->stream);
 	for (int r = 0; r < c->peerWorld; r++) if (r != c->peerRank && c->peerAccum[r]) cudaIpcCloseMemHandle(c->peerAccum[r]);
 	for (auto& m : c->meshStore) m.Free();
-	c->meshes.Free(); c->shapeLights.Free(); c->shapeCdf.Free(); c->instances.Free(); c->spheres.Free(); c->planes.Free(); c->prims.Free(); c->sphereRun.Free(); c->sphereRunBox.Free(); c->keyBoxes.Free(); c->mats.Free(); c->lights.Free();
+	c->meshes.Free(); c->shapeLights.Free(); c->shapeCdf.Free(); c->instances.Free(); c->spheres.Free(); c->planes.Free(); c->prims.Free(); c->sphereRun.Free(); c->sphereRunBox.Free(); c->keyBoxes.Free(); c->mats.Free(); c->lights.Free(); c->texels.Free(); c->textures.Free(); c->matTex.Free();
 	c->accumOwn.Free(); c->resolved.Free();
 	c->moments.Free(); c->adaptiveList.Free(); c->adaptiveCount.Free();
 	c->guideAlbedo.Free(); c->guideNormal.Free(); c->denoiseE[0].Free(); c->denoiseE[1].Free(); c->denoiseG.Free(); c->denoiseOut.Free();
@@ -637,7 +650,8 @@ int agpt_upload_meshes(agpt_ctx* c, const agpt_mesh_desc* meshes, int n) {
 	}
 SIMPLE_UPLOAD(agpt_upload_spheres, agpt_sphere, spheres, c->nSpheres = n; c->hostSpheres.assign(rows, rows + n); c->runsDirty = true)
 SIMPLE_UPLOAD(agpt_upload_planes, agpt_plane, planes, c->nPlanes = n; c->hostPlanes.assign(rows, rows + n); c->shapesDirty = true)
-SIMPLE_UPLOAD(agpt_upload_materials, agpt_material, mats, c->nMats = n; c->hasGlass = false; for (int i = 0; i < n; i++) if (rows[i].lobes & (AGPT_LOBE_GLASS_REFLECT | AGPT_LOBE_GLASS_TRANSMIT)) c->hasGlass = true)
+SIMPLE_UPLOAD(agpt_upload_materials, agpt_material, mats, c->nMats = n; c->hasGlass = false; for (int i = 0; i < n; i++) if (rows[i].lobes & (AGPT_LOBE_GLASS_REFLECT | AGPT_LOBE_GLASS_TRANSMIT)) c->hasGlass = true;
+	c->hostMatTypes.resize((size_t)n); for (int i = 0; i < n; i++) c->hostMatTypes[i] = rows[i].type)
 static int UploadLights(agpt_ctx* c, const agpt_light* rows, int n);
 SIMPLE_UPLOAD(UploadLights, agpt_light, lights, c->hostLights.assign(rows, rows + n); c->shapesDirty = true)
 int agpt_upload_lights(agpt_ctx* c, const agpt_light* rows, int n) {
@@ -681,6 +695,52 @@ int agpt_upload_envmap(agpt_ctx* c, const agpt_envmap* env) {
 	CU(cudaStreamSynchronize(c->stream));
 	c->envW = env->width; c->envH = env->height; c->envFuncInt = env->func_int;
 	return AGPT_OK;
+}
+
+// EXTENSION (agpt.h agpt_upload_textures): every argument is checked before anything resident changes.
+int agpt_upload_textures(agpt_ctx* c, const agpt_texture* textures, int n_textures, const int32_t* material_texture, int n_materials) {
+	NEED(c != nullptr && n_textures >= 0 && n_materials >= 0 && (n_textures == 0 || textures != nullptr) && (n_materials == 0 || material_texture != nullptr),
+		AGPT_ERR_INVALID, "agpt_upload_textures: bad table");
+	size_t total = 0;
+	for (int i = 0; i < n_textures; i++) {
+		const agpt_texture& t = textures[i];
+		NEED(t.width >= 1 && t.height >= 1 && (long long)t.width * t.height <= (1ll << 28), AGPT_ERR_INVALID, "agpt_upload_textures: need 1 <= width, height and width * height <= 2^28");
+		NEED(t.rgb != nullptr, AGPT_ERR_INVALID, "agpt_upload_textures: texture without texels");
+		const size_t n = 3 * (size_t)t.width * t.height;
+		for (size_t k = 0; k < n; k++) NEED(std::isfinite(t.rgb[k]), AGPT_ERR_INVALID, "agpt_upload_textures: texel not finite");
+		total += (size_t)t.width * t.height;
+	}
+	for (int i = 0; i < n_materials; i++)
+		NEED(material_texture[i] >= -1 && material_texture[i] < n_textures, AGPT_ERR_INVALID, "agpt_upload_textures: material points outside the texture table");
+	CU(cudaSetDevice(c->device));
+	CU(cudaStreamSynchronize(c->stream));
+	c->stateGen++;
+	c->historyGen++;
+	std::vector<float4> texels(total);
+	std::vector<DTexture> desc((size_t)n_textures);
+	size_t off = 0;
+	for (int i = 0; i < n_textures; i++) {
+		const agpt_texture& t = textures[i];
+		desc[i].width = t.width; desc[i].height = t.height; desc[i].off = (long long)off;
+		const size_t n = (size_t)t.width * t.height;
+		for (size_t k = 0; k < n; k++) texels[off + k] = make_float4(t.rgb[3 * k], t.rgb[3 * k + 1], t.rgb[3 * k + 2], 0.f);
+		off += n;
+	}
+	c->hasTextures = false;
+	c->hostMatTex.assign(material_texture, material_texture + n_materials);
+	for (int32_t t : c->hostMatTex) if (t >= 0) c->hasTextures = true;
+	CU(c->texels.Upload(texels.data(), texels.size(), c->stream));
+	CU(c->textures.Upload(desc.data(), desc.size(), c->stream));
+	CU(c->matTex.Upload(c->hostMatTex.data(), c->hostMatTex.size(), c->stream));
+	CU(cudaStreamSynchronize(c->stream));
+	return AGPT_OK;
+}
+
+static DTexTables MakeTexTables(const agpt_ctx* c) {
+	DTexTables t;
+	t.texels = c->texels.p; t.textures = c->textures.p; t.matTex = c->matTex.p;
+	t.nTextures = (int)c->textures.n; t.nTexels = (long long)c->texels.n;
+	return t;
 }
 
 int agpt_set_camera(agpt_ctx* c, const agpt_camera* cam) {
@@ -727,7 +787,7 @@ int agpt_set_film(agpt_ctx* c, int width, int height) {
 int agpt_scene_bytes(agpt_ctx* c, uint64_t* out) {
 	NEED(c != nullptr && out != nullptr, AGPT_ERR_INVALID, "null argument");
 	uint64_t b = c->envRgb.Bytes() + c->envFunc.Bytes() + c->envCdf.Bytes() + c->meshes.Bytes() + c->spheres.Bytes() + c->planes.Bytes() + c->prims.Bytes() + c->instances.Bytes() + c->mats.Bytes() + c->lights.Bytes()
-		+ c->shapeLights.Bytes() + c->shapeCdf.Bytes();
+		+ c->shapeLights.Bytes() + c->shapeCdf.Bytes() + c->texels.Bytes() + c->textures.Bytes() + c->matTex.Bytes();
 	for (auto& m : c->meshStore) b += m.nodes.Bytes() + m.tris.Bytes() + m.normals.Bytes() + m.uvs.Bytes() + m.ids.Bytes();
 	*out = b;
 	return AGPT_OK;
@@ -945,11 +1005,16 @@ static int RunWaves(agpt_ctx* c, const DScene& scIn, PathState& ps, int n, int m
 		// SHAPES, an area light that samples its plane or mesh: the lean one, or the one that carries everything)
 		DShapeTables st;
 		st.lights = c->shapeLights.p; st.cdf = c->shapeCdf.p;
-#define SHADE_B(E, G, S) k_shade_b<E, G, S><<<shadeBlocks, AGPT_SHADE_THREADS, 0, c->stream>>>(sc, st, ps, c->survivors.p, q[cur ^ 1], sp, c->rayCounters.p)
-		if (c->hasShapeLights) { if (c->envW > 0 || c->hasGlass) SHADE_B(true, true, true); else SHADE_B(false, false, true); }
+		const DTexTables tt = MakeTexTables(c);
+#define SHADE_B(E, G, S) k_shade_b<E, G, S, false><<<shadeBlocks, AGPT_SHADE_THREADS, 0, c->stream>>>(sc, st, ps, c->survivors.p, q[cur ^ 1], sp, c->rayCounters.p, tt)
+#define SHADE_B_TEX(E, G, S) k_shade_b<E, G, S, true><<<shadeBlocks, AGPT_SHADE_THREADS, 0, c->stream>>>(sc, st, ps, c->survivors.p, q[cur ^ 1], sp, c->rayCounters.p, tt)
+		// (TEX, some material is textured: the lean textured instantiation, or the one that carries everything)
+		if (c->hasTextures) { if (c->hasShapeLights || c->envW > 0 || c->hasGlass) SHADE_B_TEX(true, true, true); else SHADE_B_TEX(false, false, false); }
+		else if (c->hasShapeLights) { if (c->envW > 0 || c->hasGlass) SHADE_B(true, true, true); else SHADE_B(false, false, true); }
 		else if (c->envW > 0) { if (c->hasGlass) SHADE_B(true, true, false); else SHADE_B(true, false, false); }
 		else { if (c->hasGlass) SHADE_B(false, true, false); else SHADE_B(false, false, false); }
 #undef SHADE_B
+#undef SHADE_B_TEX
 		c->stats.kernel_launches++;
 		c->stats.kernel_launches++; c->stats.launches_shade++;
 		CU(cudaGetLastError());
@@ -1247,7 +1312,8 @@ int agpt_render_guides(agpt_ctx* c, int num_samples, uint32_t flags) {
 		g.n = n; g.first_sample = done; g.sample_stride = 1; g.tiled = 1; g.samples = ns;
 		k_generate<false><<<Blocks(n, 256), 256, 0, c->stream>>>(sc, ps, q0, g);
 		LaunchClosest(count, strictBoxes, c->nInstances > 0, Blocks(n, AGPT_TRACE_THREADS), c->stream, sc, ps, q0.closest, q0.counts + 0, c->traceCounters.p, nullptr);
-		k_guides<<<Blocks(wh, 256), 256, 0, c->stream>>>(sc, ps, ns, done == 0, done + ns == num_samples ? num_samples : 0, c->guideAlbedo.p, c->guideNormal.p);
+		if (c->hasTextures) k_guides_tex<<<Blocks(wh, 256), 256, 0, c->stream>>>(sc, MakeTexTables(c), ps, ns, done == 0, done + ns == num_samples ? num_samples : 0, c->guideAlbedo.p, c->guideNormal.p);
+		else k_guides<<<Blocks(wh, 256), 256, 0, c->stream>>>(sc, ps, ns, done == 0, done + ns == num_samples ? num_samples : 0, c->guideAlbedo.p, c->guideNormal.p);
 		CU(cudaGetLastError());
 		c->stats.kernel_launches += 3; c->stats.launches_closest++;
 	}

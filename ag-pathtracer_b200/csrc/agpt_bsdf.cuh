@@ -78,6 +78,10 @@ __device__ __forceinline__ float3 FrSchlick(float3 R0, float cosTheta) { return 
 __device__ __forceinline__ float3 DisneyFresnel(const agpt_material& m, float cosI) {
 	return Lerp(m.metallic, f3(FrDielectric(cosI, 1, m.eta)), FrSchlick(f3(m.spec_r0), cosI));
 }
+// the same with a per-hit R0 (extension: textured base colour)
+__device__ __forceinline__ float3 DisneyFresnel(const agpt_material& m, float3 R0, float cosI) {
+	return Lerp(m.metallic, f3(FrDielectric(cosI, 1, m.eta)), FrSchlick(R0, cosI));
+}
 
 // ---------------------------------------------------------------------------------------
 // Trowbridge-Reitz distribution (microfacet.h:34-153) with Disney's separable G (disney.h:73-82)
@@ -239,7 +243,8 @@ __device__ __forceinline__ DBSDF MakeBSDF(const DSurface& s, const agpt_material
 }
 
 // Sphere hit -> interaction (intersectable.h:183-204); dpdu/dpdv are passed swapped upstream.
-__device__ __forceinline__ void SphereSurface(const agpt_sphere& sp, float3 O, float3 D, float root, DSurface& s) {
+// uv (extension, textured instantiations only; agpt.h agpt_upload_textures): the sphere's surface uv, or nullptr.
+__device__ __forceinline__ void SphereSurface(const agpt_sphere& sp, float3 O, float3 D, float root, DSurface& s, float2* uv = nullptr) {
 	float3 p = O + root * D;
 	float3 pHit = p - f3(sp.center);
 	if (pHit.x == 0 && pHit.y == 0) pHit.x = AGPT_EPSILON * sp.r;
@@ -251,20 +256,28 @@ __device__ __forceinline__ void SphereSurface(const agpt_sphere& sp, float3 O, f
 	float3 dpdu = f3(-AGPT_TWOPI * pHit.y, AGPT_TWOPI * pHit.x, 0);
 	float3 dpdv = AGPT_PI * f3(pHit.z * cosPhi, pHit.z * sinPhi, -sp.r * rsin(theta));
 	SurfaceInit(s, p, dpdv, dpdu);
+	if (uv) {
+		float phi = ratan2T<1>(pHit.y, pHit.x);
+		if (phi < 0) phi = phi + AGPT_TWOPI;
+		*uv = make_float2(phi / AGPT_TWOPI, theta / AGPT_PI);
+	}
 }
 __device__ __forceinline__ void PlaneSurface(float3 O, float3 D, float t, DSurface& s) {   // intersectable.h:128-133
 	SurfaceInit(s, O + t * D, f3(0, 0, 1), f3(1, 0, 0));
 }
 // Triangle hit -> interaction + shading frame (trianglemesh.cpp:45-113, intersectable.h:80-89)
 // `in` (extension, agpt.h agpt_instance): the mesh is a placed one -- vertices go to world space first, the shading
-// normal through transpose(W2O); nullptr for the reference's own meshes.
-__device__ __forceinline__ void TriangleSurface(const DMesh& mesh, int slot, float3 O, float3 D, float t, float b1, float b2, DSurface& s, const agpt_instance* in) {
+// normal through transpose(W2O); nullptr for the reference's own meshes.  uvOut (extension, textured instantiations only): the
+// interpolated uv, or nullptr.
+__device__ __forceinline__ void TriangleSurface(const DMesh& mesh, int slot, float3 O, float3 D, float t, float b1, float b2, DSurface& s, const agpt_instance* in,
+		float2* uvOut = nullptr) {
 	float4 a = __ldg(mesh.tris + 3 * slot), b = __ldg(mesh.tris + 3 * slot + 1), c = __ldg(mesh.tris + 3 * slot + 2);
 	float3 v0 = f3(a.x, a.y, a.z), v1 = f3(b.x, b.y, b.z), v2 = f3(c.x, c.y, c.z);
 	if (in) { v0 = XformPoint(in->object_to_world, v0); v1 = XformPoint(in->object_to_world, v1); v2 = XformPoint(in->object_to_world, v2); }
 	float b0 = 1.f - b1 - b2;
 	float2 uv0 = make_float2(0, 0), uv1 = make_float2(1, 0), uv2 = make_float2(1, 1);
 	if (mesh.uvs) { uv0 = __ldg(mesh.uvs + 3 * slot); uv1 = __ldg(mesh.uvs + 3 * slot + 1); uv2 = __ldg(mesh.uvs + 3 * slot + 2); }
+	if (uvOut) *uvOut = make_float2((b0 * uv0.x + b1 * uv1.x) + b2 * uv2.x, (b0 * uv0.y + b1 * uv1.y) + b2 * uv2.y);
 	float3 dpdu, dpdv;
 	TriangleDerivatives(v0, v1, v2, uv0, uv1, uv2, dpdu, dpdv);
 	SurfaceInit(s, O + t * D, dpdu, dpdv);
@@ -283,6 +296,51 @@ __device__ __forceinline__ void TriangleSurface(const DMesh& mesh, int slot, flo
 		s.sn = normalize(cross(ss, ts));
 		s.n = Faceforward(s.n, s.sn);
 	}
+}
+
+// ---------------------------------------------------------------------------------------
+// EXTENSION: image textures on the base colour of Disney materials, stated in agpt.h (agpt_upload_textures) and on the
+// CPU in statements/agpt_texture_oracle.cpp.  Plain loads: the texture unit's filtering weights are 8-bit fractions.
+// ---------------------------------------------------------------------------------------
+__device__ __forceinline__ float2 PlaneUV(const agpt_plane& pl, float3 p) {
+	return make_float2(((p.x - pl.o[0]) / pl.half_x + 1) * 0.5f, ((p.z - pl.o[2]) / pl.half_z + 1) * 0.5f);
+}
+__device__ __forceinline__ int TexWrap(int x, int n) { return x < 0 ? x + n : x >= n ? x - n : x; }
+__device__ __forceinline__ float3 TexelAt(const DTexTables& tt, const DTexture& d, int x, int y) {
+	const long long i = d.off + (long long)y * d.width + x;
+	AGPT_CHECK(i >= d.off && i < d.off + (long long)d.width * d.height && i < tt.nTexels, AGPT_DBG_TEXEL, i);
+	const float4 t = __ldg(tt.texels + i);
+	return f3(t.x, t.y, t.z);
+}
+// bilinear, repeat-wrapped, texel centres at (i + 0.5) / W
+__device__ __forceinline__ float3 TexLookup(const DTexTables& tt, int tex, float2 uv) {
+	AGPT_CHECK(tex >= 0 && tex < tt.nTextures, AGPT_DBG_TEXTURE, tex);
+	const DTexture d = tt.textures[tex];
+	const float u = isfinite(uv.x) ? uv.x - floorf(uv.x) : 0.f, v = isfinite(uv.y) ? uv.y - floorf(uv.y) : 0.f;
+	const float s = u * (float)d.width - 0.5f, t = v * (float)d.height - 0.5f;
+	const float fs = floorf(s), ft = floorf(t);
+	const int x0 = TexWrap((int)fs, d.width), x1 = TexWrap((int)fs + 1, d.width);
+	const int y0 = TexWrap((int)ft, d.height), y1 = TexWrap((int)ft + 1, d.height);
+	const float fx = s - fs, fy = t - ft;
+	const float3 t00 = TexelAt(tt, d, x0, y0), t10 = TexelAt(tt, d, x1, y0), t01 = TexelAt(tt, d, x0, y1), t11 = TexelAt(tt, d, x1, y1);
+	const float3 a = t00 + fx * (t10 - t00), b = t01 + fx * (t11 - t01);
+	return a + fy * (b - a);
+}
+// The two colours a Disney material derives from its base colour (host/material.h DisneyMaterial), for one hit.
+struct TexColors {
+	float3 diffuse;   // agpt_material.diffuse_r
+	float3 spec0;     // agpt_material.spec_r0
+};
+__device__ __forceinline__ TexColors HitColors(const DTexTables& tt, int material, const agpt_material& m, float2 uv) {
+	TexColors tc;
+	const int tex = tt.matTex[material];
+	if (tex < 0) { tc.diffuse = f3(m.diffuse_r); tc.spec0 = f3(m.spec_r0); return tc; }
+	const float3 c = TexLookup(tt, tex, uv);
+	const float dw = (1 - m.metallic) * (1 - 0.f);
+	tc.diffuse = dw > 0 ? dw * c : f3(0.f);
+	const float r0 = ((m.eta - 1) * (m.eta - 1)) / ((m.eta + 1) * (m.eta + 1));
+	tc.spec0 = Lerp(m.metallic, f3(r0), c);
+	return tc;
 }
 
 // ---------------------------------------------------------------------------------------
@@ -452,8 +510,9 @@ struct LobeEval {
 	float3 fT;         // GLASS: f of the transmission lobe (contributes when wi, wo lie on opposite sides of the geometric normal)
 	float pdfT;        // GLASS: MicrofacetTransmission::Pdf
 };
-template <bool GLASS>
-__device__ __forceinline__ void EvalLobes(const VertexBsdf& v, float3 wi, LobeEval& out) {
+// TEX (extension): the diffuse reflectance and Schlick R0 come from tc (the hit's textured colours), not from the record.
+template <bool GLASS, bool TEX = false>
+__device__ __forceinline__ void EvalLobes(const VertexBsdf& v, float3 wi, LobeEval& out, TexColors tc = TexColors()) {
 	const agpt_material& m = *v.b.mat;
 	const float absCosI = AbsCosTheta(wi);
 	const bool same = SameHemisphere(v.wo, wi);
@@ -464,7 +523,7 @@ __device__ __forceinline__ void EvalLobes(const VertexBsdf& v, float3 wi, LobeEv
 	const bool whZero = wh.x == 0 && wh.y == 0 && wh.z == 0;
 	wh = normalize(wh);
 	const float Fi = SchlickWeight(absCosI);
-	const float3 R = f3(m.diffuse_r);
+	const float3 R = TEX ? tc.diffuse : f3(m.diffuse_r);
 	if (m.lobes & AGPT_LOBE_DIFFUSE) f += R * AGPT_INVPI * (1 - v.Fo / 2) * (1 - Fi / 2);                 // disney.h:27-34
 	if (m.lobes & AGPT_LOBE_RETRO) {                                                                    // disney.h:42-54
 		float3 fr = f3(0.f);
@@ -478,7 +537,7 @@ __device__ __forceinline__ void EvalLobes(const VertexBsdf& v, float3 wi, LobeEv
 	if (m.lobes & AGPT_LOBE_MICROFACET) {                                                               // reflection.h:42-54,67-71
 		float3 fm = f3(0.f);
 		if (!(absCosI == 0 || v.absCosO == 0) && !whZero) {
-			float3 F = DisneyFresnel(m, dot(wi, Faceforward(wh, f3(0, 0, 1))));
+			float3 F = TEX ? DisneyFresnel(m, tc.spec0, dot(wi, Faceforward(wh, f3(0, 0, 1)))) : DisneyFresnel(m, dot(wi, Faceforward(wh, f3(0, 0, 1))));
 			float D = TR_D(m.alpha_x, m.alpha_y, wh);
 			float G = v.G1o * TR_G1(m.alpha_x, m.alpha_y, wi);
 			fm = f3(1.f) * D * G * F / (4 * absCosI * v.absCosO);

@@ -27,7 +27,8 @@
 // pool this was developed on, so the small GPU tests are run once per round against this build.
 enum { AGPT_DBG_STACK = 1, AGPT_DBG_NODE = 2, AGPT_DBG_TRI = 3, AGPT_DBG_QUEUE = 4, AGPT_DBG_PATH = 5, AGPT_DBG_PRIM = 6, AGPT_DBG_MATERIAL = 7,
        AGPT_DBG_LIST = 8 /* adaptive pixel list entry or pixel index */, AGPT_DBG_SAMPLE = 9 /* a pixel's samples past max_samples */,
-       AGPT_DBG_GUIDE = 10 /* k_guides: path slot */, AGPT_DBG_TAP = 11 /* denoise, reprojection: filter or history tap outside the film */ };
+       AGPT_DBG_GUIDE = 10 /* k_guides: path slot */, AGPT_DBG_TAP = 11 /* denoise, reprojection: filter or history tap outside the film */,
+       AGPT_DBG_TEXTURE = 12 /* texture index of a material */, AGPT_DBG_TEXEL = 13 /* texel index of a lookup */ };
 #ifdef AGPT_DEBUG
 __device__ unsigned long long g_agptDebug[4];     // [0] failures, [1] first code, [2] first value, [3] checks executed
 #define AGPT_CHECK(cond, code, value) do { atomicAdd(&g_agptDebug[3], 1ull); if (!(cond)) { \
@@ -55,6 +56,20 @@ struct DShapeLight {
 struct DShapeTables {        // passed beside DScene, to the kernels that sample shapes only
 	const DShapeLight* lights;       // n_lights entries, or nullptr when no light samples its shape
 	const float* cdf;
+};
+
+// EXTENSION: image textures on the base colour of Disney materials (agpt.h agpt_upload_textures), passed beside DScene to the
+// textured instantiations only.
+struct DTexture {
+	int width, height;
+	long long off;               // first texel in DTexTables::texels
+};
+struct DTexTables {
+	const float4* texels;        // every texture's texels, row-major, .w unused: one bilinear lookup = four 128-bit loads
+	const DTexture* textures;
+	const int* matTex;           // per material: its base-colour texture, or -1
+	int nTextures;
+	long long nTexels;
 };
 
 struct DScene {
@@ -221,8 +236,11 @@ __device__ __noinline__ float racos(float x) {
 // atan2f: Sun fdlibm e_atan2f.c / s_atanf.c in float (the lineage of glibc's).  On this path it
 // only feeds SphericalPhi -> a texel column of the environment map (lights.cpp:84-90,100-111),
 // a discrete index, so the last ulp is immaterial; measured against glibc 2.39 on the host it
-// differs in 31 of 3e7 arguments, all with |y/x| > 2^24.
-__device__ __noinline__ float ratanf(float x) {
+// differs in 31 of 3e7 arguments, all with |y/x| > 2^24.  The sphere uv of textured materials (extension) states this
+// algorithm, not glibc's (statements/agpt_texture_oracle.cpp ports it).  COPY: the textured kernels call copy 1, so the call
+// graph of the kernels that ran before textures existed, and with it their code, stays as it was.
+template <int COPY>
+__device__ __noinline__ float ratanfT(float x) {
 	const float atanhi[4] = { 4.6364760399e-01f, 7.8539812565e-01f, 9.8279368877e-01f, 1.5707962513e+00f };
 	const float atanlo[4] = { 5.0121582440e-09f, 3.7748947079e-08f, 3.4473217170e-08f, 7.5497894159e-08f };
 	const float aT[11] = { 3.3333334327e-01f, -2.0000000298e-01f, 1.4285714924e-01f, -1.1111110449e-01f, 9.0908870101e-02f,
@@ -254,11 +272,12 @@ __device__ __noinline__ float ratanf(float x) {
 	z = atanhi[id] - ((x * (s1 + s2) - atanlo[id]) - x);
 	return hx < 0 ? -z : z;
 }
-__device__ __noinline__ float ratan2(float y, float x) {
+template <int COPY>
+__device__ __noinline__ float ratan2T(float y, float x) {
 	const float tiny = 1.0e-30f, pi_o_4 = 7.8539818525e-01f, pi_o_2 = 1.5707963705e+00f, pi = 3.1415927410e+00f, pi_lo = -8.7422776573e-08f;
 	int hx = __float_as_int(x), ix = hx & 0x7fffffff, hy = __float_as_int(y), iy = hy & 0x7fffffff;
 	if (ix > 0x7f800000 || iy > 0x7f800000) return x + y;
-	if (hx == 0x3f800000) return ratanf(y);
+	if (hx == 0x3f800000) return ratanfT<COPY>(y);
 	int m = ((hy >> 31) & 1) | ((hx >> 30) & 2);
 	if (iy == 0) return m < 2 ? y : (m == 2 ? pi + tiny : -pi - tiny);
 	if (ix == 0) return hy < 0 ? -pi_o_2 - tiny : pi_o_2 + tiny;
@@ -271,7 +290,7 @@ __device__ __noinline__ float ratan2(float y, float x) {
 	float z;
 	if (k > 24) z = pi_o_2 + 0.5f * pi_lo;
 	else if (hx < 0 && k < -24) z = 0.0f;
-	else z = ratanf(fabsf(y / x));
+	else z = ratanfT<COPY>(fabsf(y / x));
 	switch (m) {
 	case 0: return z;
 	case 1: return -z;
@@ -279,6 +298,7 @@ __device__ __noinline__ float ratan2(float y, float x) {
 	default: return (z - pi_lo) - pi;
 	}
 }
+__device__ __forceinline__ float ratan2(float y, float x) { return ratan2T<0>(y, x); }
 
 // powf with the oracle's bits, for Accumulator::CopyToSurface's gamma (common.h:41-44: pow(c, 1/2.2f)
 // on floats = powf).  glibc 2.39's powf is the ARM optimized-routines algorithm

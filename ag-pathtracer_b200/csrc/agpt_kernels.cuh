@@ -510,10 +510,12 @@ __global__ void __launch_bounds__(256) k_shade_a(DScene sc, PathState ps, const 
 #define AGPT_SHADE_STACK_SMEM 8
 
 // SHAPES (extension): some area light samples its plane or mesh (AGPT_LIGHT_SAMPLE_SHAPE); other scenes run the
-// instantiations without that code.
-template <bool ENV, bool GLASS, bool SHAPES>
+// instantiations without that code.  TEX (extension): some Disney material has an image texture on its base colour
+// (agpt_upload_textures): two instantiations run, <false, false, false, true> and <true, true, true, true>; `tt` is read only by
+// them (the others take it last, after every parameter they had before, and their code is what it was).
+template <bool ENV, bool GLASS, bool SHAPES, bool TEX>
 __global__ void __launch_bounds__(AGPT_SHADE_THREADS, AGPT_SHADE_MIN_BLOCKS) k_shade_b(DScene sc, DShapeTables st, PathState ps, const int* __restrict__ survivors, WaveQueues qout, ShadeParams sp,
-		RayCounters* rc) {
+		RayCounters* rc, DTexTables tt) {
 	__shared__ unsigned shapeStack[SHAPES ? AGPT_SHADE_STACK_SMEM * AGPT_SHADE_THREADS : 1];
 	const int lane = threadIdx.x & 31;
 	const int count = *sp.count;
@@ -546,19 +548,23 @@ __global__ void __launch_bounds__(AGPT_SHADE_THREADS, AGPT_SHADE_MIN_BLOCKS) k_s
 		DSurface si;
 		si.p = f3(0.f); si.n = f3(0.f); si.sn = f3(0.f); si.sdpdu = f3(0.f);
 		const agpt_material* mat = sc.mats;      // (never null: agpt keeps one dummy record resident when the scene has no materials)
+		float2 uv = make_float2(0.f, 0.f);       // TEX: surface uv of the hit
+		TexColors tc;                            // TEX: the hit's diffuse reflectance and Schlick R0
+		tc.diffuse = f3(0.f); tc.spec0 = f3(0.f);
 
 		// the surface at the hit (a survivor has one); null materials pass straight through
 		if (valid) {
 			AGPT_CHECK(__float_as_int(h.w) >= 0 && __float_as_int(h.w) < sc.n_prims, AGPT_DBG_PRIM, __float_as_int(h.w));
 			agpt_prim prim = sc.prims[__float_as_int(h.w)];
 			// SurfaceInteraction of the closest hit
-			if (prim.type == AGPT_PRIM_SPHERE) SphereSurface(sc.spheres[prim.payload], O, D, h.x, si);
+			if (prim.type == AGPT_PRIM_SPHERE) SphereSurface(sc.spheres[prim.payload], O, D, h.x, si, TEX ? &uv : nullptr);
 			else if (prim.type == AGPT_PRIM_PLANE) PlaneSurface(O, D, h.x, si);
 			else if (prim.type == AGPT_PRIM_INSTANCE) {          // extension: a placed mesh
 				const agpt_instance& in = sc.instances[prim.payload];
-				TriangleSurface(sc.meshes[in.mesh], hitSlot, O, D, h.x, h.y, h.z, si, &in);
+				TriangleSurface(sc.meshes[in.mesh], hitSlot, O, D, h.x, h.y, h.z, si, &in, TEX ? &uv : nullptr);
 			}
-			else TriangleSurface(sc.meshes[prim.payload], hitSlot, O, D, h.x, h.y, h.z, si, nullptr);
+			else TriangleSurface(sc.meshes[prim.payload], hitSlot, O, D, h.x, h.y, h.z, si, nullptr, TEX ? &uv : nullptr);
+			if (TEX && prim.type == AGPT_PRIM_PLANE) uv = PlaneUV(sc.planes[prim.payload], si.p);
 
 			if (prim.material < 0) {
 				// null material: pass straight through, bounce count unchanged (integrator.h:152-161)
@@ -568,7 +574,10 @@ __global__ void __launch_bounds__(AGPT_SHADE_THREADS, AGPT_SHADE_MIN_BLOCKS) k_s
 				emitExtend = true; skipRay = true; stayActive = true;
 				keyExtend = RayBucket(sc, nr.O, nr.D, -1, true);
 			}
-			else { full = true; mat = sc.mats + prim.material; }
+			else {
+				full = true; mat = sc.mats + prim.material;
+				if (TEX) tc = HitColors(tt, prim.material, *mat, uv);     // the one lookup of this vertex
+			}
 		}
 
 		// ================= phase B: BSDF frame, random numbers, light sample =================
@@ -708,7 +717,7 @@ __global__ void __launch_bounds__(AGPT_SHADE_THREADS, AGPT_SHADE_MIN_BLOCKS) k_s
 			float3 wiLoc = k == 0 ? WorldToLocal(vb.b, wiL) : sampledWi;
 			LobeEval ev;
 			ev.f = f3(0.f); ev.pdfCos = 0.f; ev.pdfMicro = 0.f; ev.fT = f3(0.f); ev.pdfT = 0.f;
-			if (need) EvalLobes<GLASS>(vb, wiLoc, ev);
+			if (need) EvalLobes<GLASS, TEX>(vb, wiLoc, ev, tc);
 			if (k == 0) {
 				if (need) fLight = FinishEval<GLASS>(vb, ev, wiL, &pdfLight);     // BSDF::f and BSDF::Pdf at the light direction
 			}
@@ -1003,7 +1012,9 @@ __global__ void __launch_bounds__(256) k_resolve_counts(const float4* __restrict
 // k_guides: one thread per pixel after k_generate<false> (tiled) and k_trace_closest have run the batch's camera rays.  It walks
 // the pixel's slots in sample order and adds each sample's first hit to the running sums in albedo (.xyz, .w = hits) and
 // normalDepth (.xyz, .w = t sum).  `total` > 0 on the last batch: the sums become the means of all `total` samples.
-__global__ void __launch_bounds__(256) k_guides(DScene sc, PathState ps, int samplesInBatch, bool firstBatch, int total, float4* albedo, float4* normalDepth) {
+// TEX (extension): a textured Disney material's albedo is the hit's textured diffuse_r + spec_r0 (k_guides_tex).
+template <bool TEX>
+__device__ __forceinline__ void Guides(DScene sc, DTexTables tt, PathState ps, int samplesInBatch, bool firstBatch, int total, float4* albedo, float4* normalDepth) {
 	const int pixel = blockIdx.x * blockDim.x + threadIdx.x;
 	const int width = sc.width, height = sc.height;
 	if (pixel >= width * height) return;
@@ -1024,19 +1035,22 @@ __global__ void __launch_bounds__(256) k_guides(DScene sc, PathState ps, int sam
 			const float3 O = f3(o4.x, o4.y, o4.z), D = f3(d4.x, d4.y, d4.z);
 			const agpt_prim prim = sc.prims[hitPrim];
 			DSurface si;
+			float2 uv = make_float2(0.f, 0.f);
 			// the surface of the closest hit as k_shade_b rebuilds it
-			if (prim.type == AGPT_PRIM_SPHERE) SphereSurface(sc.spheres[prim.payload], O, D, h.x, si);
+			if (prim.type == AGPT_PRIM_SPHERE) SphereSurface(sc.spheres[prim.payload], O, D, h.x, si, TEX ? &uv : nullptr);
 			else if (prim.type == AGPT_PRIM_PLANE) PlaneSurface(O, D, h.x, si);
 			else if (prim.type == AGPT_PRIM_INSTANCE) {
 				const agpt_instance& in = sc.instances[prim.payload];
-				TriangleSurface(sc.meshes[in.mesh], ps.hitSlot[slot], O, D, h.x, h.y, h.z, si, &in);
+				TriangleSurface(sc.meshes[in.mesh], ps.hitSlot[slot], O, D, h.x, h.y, h.z, si, &in, TEX ? &uv : nullptr);
 			}
-			else TriangleSurface(sc.meshes[prim.payload], ps.hitSlot[slot], O, D, h.x, h.y, h.z, si, nullptr);
+			else TriangleSurface(sc.meshes[prim.payload], ps.hitSlot[slot], O, D, h.x, h.y, h.z, si, nullptr, TEX ? &uv : nullptr);
+			if (TEX && prim.type == AGPT_PRIM_PLANE) uv = PlaneUV(sc.planes[prim.payload], si.p);
 			n = dot(si.sn, D) > 0.f ? -si.sn : si.sn;
 			if (prim.material >= 0) {
 				const agpt_material& m = sc.mats[prim.material];
 				if (m.type == AGPT_MAT_MIRROR) alb = f3(m.mirror_r);
 				else if (m.type == AGPT_MAT_GLASS) alb = f3(m.mirror_r) + f3(m.diffuse_r);
+				else if (TEX) { const TexColors tc = HitColors(tt, prim.material, m, uv); alb = tc.diffuse + tc.spec0; }
 				else alb = f3(m.diffuse_r) + f3(m.spec_r0);
 				alb = f3(alb.x < 1.f ? alb.x : 1.f, alb.y < 1.f ? alb.y : 1.f, alb.z < 1.f ? alb.z : 1.f);
 			}
@@ -1054,6 +1068,12 @@ __global__ void __launch_bounds__(256) k_guides(DScene sc, PathState ps, int sam
 	}
 	albedo[f] = a;
 	normalDepth[f] = nd;
+}
+__global__ void __launch_bounds__(256) k_guides(DScene sc, PathState ps, int samplesInBatch, bool firstBatch, int total, float4* albedo, float4* normalDepth) {
+	Guides<false>(sc, DTexTables(), ps, samplesInBatch, firstBatch, total, albedo, normalDepth);
+}
+__global__ void __launch_bounds__(256) k_guides_tex(DScene sc, DTexTables tt, PathState ps, int samplesInBatch, bool firstBatch, int total, float4* albedo, float4* normalDepth) {
+	Guides<true>(sc, tt, ps, samplesInBatch, firstBatch, total, albedo, normalDepth);
 }
 
 #define AGPT_DENOISE_ALBEDO_EPS 0.01f

@@ -10,13 +10,16 @@
 
 #include "precomp.h"
 #include "agpt.h"
+#include "texture.h"
 
 class Material {
 public:
 	virtual ~Material() {}
 	virtual agpt_material Export() const = 0;
+	virtual const ImageTexture* BaseColorTexture() const { return nullptr; }   // extension: DisneyMaterial with an image
 };
 
+#define AGPT_HAS_IMAGE_TEXTURES 1      // extension: DisneyMaterial(ImageTexture, roughness, metallic)
 class DisneyMaterial : public Material {
 public:
 	DisneyMaterial(const float3& color, float roughness, float metallic) {
@@ -43,12 +46,21 @@ public:
 		rec.spec_r0[0] = Cspec0.x; rec.spec_r0[1] = Cspec0.y; rec.spec_r0[2] = Cspec0.z;
 		rec.lobes |= AGPT_LOBE_MICROFACET;
 	}
+	// EXTENSION: the base colour is an image (include/agpt.h agpt_upload_textures).  The record holds white's colours; the
+	// device replaces them at every hit by the texture value's, through the same arithmetic as the constructor above.
+	DisneyMaterial(std::shared_ptr<ImageTexture> texture, float roughness, float metallic)
+		: DisneyMaterial(float3(1.f), roughness, metallic) { this->texture = std::move(texture); }
 	agpt_material Export() const override { return rec; }
+	const ImageTexture* BaseColorTexture() const override { return texture.get(); }
 	static std::shared_ptr<DisneyMaterial> Make(const float3& color, float roughness, float metallic) {
 		return std::make_shared<DisneyMaterial>(color, roughness, metallic);
 	}
+	static std::shared_ptr<DisneyMaterial> Make(std::shared_ptr<ImageTexture> texture, float roughness, float metallic) {
+		return std::make_shared<DisneyMaterial>(std::move(texture), roughness, metallic);
+	}
 private:
 	agpt_material rec;
+	std::shared_ptr<ImageTexture> texture;
 };
 
 class MirrorMaterial : public Material {

@@ -65,11 +65,15 @@ struct FlatScene {
 	std::vector<FlatTriangles> meshTris;
 	std::vector<agpt_instance> instances;      // extension: placed meshes
 	agpt_envmap envmap = { 0, 0, nullptr, nullptr, nullptr, 0.f };   // borrowed from the scene's InfiniteAreaLight
+	std::vector<agpt_texture> textures;        // extension: base-colour images, texels borrowed from the materials
+	std::vector<int32_t> materialTexture;      // per material: index into textures or -1 (empty when no material has one)
 	uint64_t Bytes() const {
 		uint64_t b = prims.size() * sizeof(agpt_prim) + spheres.size() * sizeof(agpt_sphere) + planes.size() * sizeof(agpt_plane)
 			+ materials.size() * sizeof(agpt_material) + lights.size() * sizeof(agpt_light);
 		b += instances.size() * sizeof(agpt_instance);
 		for (auto& m : meshes) b += (uint64_t)m.n_nodes * 32 + (uint64_t)m.n_tris * (48 + 4 + (m.tri_normals ? 48 : 0) + (m.tri_uvs ? 24 : 0));
+		for (auto& t : textures) b += (uint64_t)t.width * t.height * 16 + 16;   // float4 texels and a descriptor on the device
+		b += materialTexture.size() * 4;
 		return b;
 	}
 };
@@ -90,6 +94,7 @@ public:
 	std::shared_ptr<FlatScene> Flatten() const {
 		auto flat = std::make_shared<FlatScene>();
 		std::map<const Material*, int> matIndex;
+		std::map<const ImageTexture*, int> texIndex;         // extension: textures de-duplicated by pointer
 		std::map<const Light*, int> lightIndex;
 		std::map<const Intersectable*, int> primIndex;
 		std::map<const TriangleMesh*, int> sharedMesh;       // meshes referenced by instances: flattened once
@@ -130,6 +135,13 @@ public:
 				if (it == matIndex.end()) {
 					it = matIndex.emplace(m, (int)flat->materials.size()).first;
 					flat->materials.push_back(m->Export());
+					int tex = -1;
+					if (const ImageTexture* t = m->BaseColorTexture()) {
+						auto ti = texIndex.find(t);
+						if (ti == texIndex.end()) { ti = texIndex.emplace(t, (int)flat->textures.size()).first; flat->textures.push_back(t->Export()); }
+						tex = ti->second;
+					}
+					flat->materialTexture.push_back(tex);
 				}
 				row.material = it->second;
 			}
@@ -160,6 +172,7 @@ public:
 			}
 			flat->prims.push_back(row);
 		}
+		if (flat->textures.empty()) flat->materialTexture.clear();
 		for (auto& l : lights) {
 			agpt_light rec;
 			memset(&rec, 0, sizeof(rec));

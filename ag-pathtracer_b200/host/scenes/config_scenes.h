@@ -44,6 +44,7 @@ inline ConfigDefaults Defaults(int config) {
 	case 9: return { 3840, 2160, 1024, 8, 0, "cfg9_ext_cfg4_with_true_instances_one_mesh_8_placements" };
 	case 10: return { 1920, 1080, 64, 16, 0, "cfg10_ext_cfg5_rough_glass_rr_by_bounce" };
 	case 11: return { 1920, 1080, 64, 16, 4, "cfg11_ext_cfg5_sampled_panel_plane_and_mesh_lights" };
+	case 12: return { 480, 270, 16, 8, 0, "cfg12_ext_procedural_image_textures" };
 	default: return { 0, 0, 0, 0, 0, "unknown" };
 	}
 }
@@ -560,6 +561,73 @@ inline void BuildConfig11(Scene* scene, int level) {
 }
 #endif
 
+#ifdef AGPT_HAS_IMAGE_TEXTURES
+// cfg 12 (EXTENSION, host mirror only -- the reference has one colour per material): procedural image textures on the base
+// colour of Disney materials, laid out so every uv rule and texture shape is used: a floor plane with a 2048 x 2048 checker
+// gradient, spheres with a 37 x 23 (non-power-of-two) image and a 64 x 1 strip, an 8 x 8 quad grid with per-vertex uvs over
+// [0, 2]^2 (repeat wrap) and normals placed once as a plain TriangleMesh and once as an Instance of a BVHTriMesh, and one
+// untextured Disney sphere.  The 37 x 23 texture is shared by two materials (flattened once).
+inline std::shared_ptr<ImageTexture> ProceduralTexture(int W, int H, int kind) {
+	std::vector<float> rgb(3 * (size_t)W * H);
+	for (int y = 0; y < H; y++)
+		for (int x = 0; x < W; x++) {
+			float* p = &rgb[3 * ((size_t)y * W + x)];
+			const float fx = (x + .5f) / W, fy = (y + .5f) / H;
+			if (kind == 0) {            // checker of 64-texel cells over a gradient
+				const bool odd = ((x >> 6) + (y >> 6)) & 1;
+				p[0] = .15f + .7f * fx; p[1] = odd ? .8f : .1f; p[2] = .15f + .7f * fy;
+			}
+			else if (kind == 1) {       // coarse colour blocks: every texel differs from its neighbours
+				p[0] = (float)((x * 7 + y * 3) % 11) / 10.f; p[1] = (float)((x * 5 + y * 13) % 7) / 6.f; p[2] = .25f + .5f * fy;
+			}
+			else {                      // stripes
+				p[0] = (x & 1) ? .9f : .2f; p[1] = .3f + .6f * fx; p[2] = (x % 3 == 0) ? .7f : .1f;
+			}
+		}
+	return ImageTexture::Make(W, H, std::move(rgb));
+}
+inline std::shared_ptr<TriangleMesh> MakeQuadGrid(int n, float size, const float3& at, std::shared_ptr<Material> mat) {
+	std::vector<float3> vertices, normals;
+	std::vector<float2> texcoords;
+	std::vector<index_type> indices;
+	for (int j = 0; j <= n; j++)
+		for (int i = 0; i <= n; i++) {
+			const float u = (float)i / n, v = (float)j / n;
+			vertices.push_back(float3(at.x + (u - .5f) * size, at.y + (v - .5f) * size, at.z + .15f * (u - .5f) * (v - .5f) * size));
+			normals.push_back(float3(-.1f * (v - .5f), -.1f * (u - .5f), -1.f));
+			texcoords.push_back(float2(2.f * u, 2.f * v));
+		}
+	for (int j = 0; j < n; j++)
+		for (int i = 0; i < n; i++) {
+			const int a = j * (n + 1) + i, b = a + 1, c = a + n + 2, d = a + n + 1;
+			for (int k : { a, b, c, a, c, d }) indices.push_back(index_type(k));
+		}
+	return std::make_shared<TriangleMesh>(indices, vertices, normals, texcoords, mat);
+}
+inline void BuildConfig12(Scene* scene) {
+	auto checker = ProceduralTexture(2048, 2048, 0);
+	auto blocks = ProceduralTexture(37, 23, 1);
+	auto strip = ProceduralTexture(64, 1, 2);
+	auto floorMat = DisneyMaterial::Make(checker, 1.f, 0.f);
+	scene->primitives.push_back(std::make_shared<Plane>(float3(0, -1, 0), float2(8, 8), floorMat));
+	scene->primitives.push_back(std::make_shared<Sphere>(float3(-2.4f, 0, 0), 1.f, DisneyMaterial::Make(blocks, .5f, 0.f)));
+	scene->primitives.push_back(std::make_shared<Sphere>(float3(0, 0, 1.f), 1.f, DisneyMaterial::Make(strip, .3f, .5f)));
+	scene->primitives.push_back(std::make_shared<Sphere>(float3(2.4f, 0, 0), 1.f, DisneyMaterial::Make(float3(.2f, .45f, .7f), .4f, 0.f)));
+	auto gridMat = DisneyMaterial::Make(blocks, .7f, .2f);
+	scene->primitives.push_back(MakeQuadGrid(8, 2.f, float3(-1.2f, 1.8f, 3.f), gridMat));
+	auto placed = std::make_shared<BVHTriMesh>(MakeQuadGrid(8, 2.f, float3(0.f), gridMat), gridMat, 1);
+	scene->primitives.push_back(std::make_shared<Instance>(placed, mat4::Translate(1.4f, 1.9f, 3.2f) * mat4::RotateY(-.4f), DisneyMaterial::Make(checker, .6f, 0.f)));
+	scene->addAreaLight(std::make_shared<Sphere>(float3(0, 8, -4), .5f, nullptr), WarmWhite(120));
+	scene->lights.push_back(std::make_shared<UniformInfiniteLight>(float3(.15f, .17f, .2f)));
+	scene->camera.lookfrom = float3(0, 2.2f, -8.5f);
+	scene->camera.lookat = float3(0, .4f, 0);
+	scene->camera.vup = float3(0, 1, 0);
+	scene->camera.aspect_ratio = 16.f / 9.f;
+	scene->camera.vfov = 40;
+	scene->camera.aperture = 0;
+}
+#endif
+
 // level <= 0 selects the BASELINE.json size of each configuration.
 inline bool BuildConfig(Scene* scene, int config, int level) {
 	switch (config) {
@@ -579,6 +647,9 @@ inline bool BuildConfig(Scene* scene, int config, int level) {
 #endif
 #ifdef AGPT_HAS_SAMPLED_AREA_LIGHTS
 	case 11: BuildConfig11(scene, level > 0 ? level : 7); return true;
+#endif
+#ifdef AGPT_HAS_IMAGE_TEXTURES
+	case 12: BuildConfig12(scene); return true;
 #endif
 	default: return false;
 	}

@@ -6,8 +6,10 @@
 #pragma once
 
 #include <cstdio>
+#include <stdexcept>
 
 #include "precomp.h"
+#include "agpt.h"
 
 class Texture {
 public:
@@ -88,3 +90,21 @@ private:
 	int width = 0, height = 0;
 	std::vector<float> rgb;
 };
+
+// EXTENSION (not a reference class: upstream has one colour per material): a linear RGB float image supplied by the
+// caller, the base colour of a DisneyMaterial.  Lookups happen on the device (include/agpt.h agpt_upload_textures).
+class ImageTexture : public Texture {
+public:
+	ImageTexture(int width, int height, std::vector<float> rgb) : width(width), height(height), rgb(std::move(rgb)) {
+		if (width < 1 || height < 1 || this->rgb.size() != 3 * (size_t)width * height) throw std::runtime_error("ImageTexture: need width, height >= 1 and width * height * 3 floats");
+	}
+	int Width() const { return width; }
+	int Height() const { return height; }
+	agpt_texture Export() const { agpt_texture t; t.width = width; t.height = height; t.rgb = rgb.data(); return t; }
+	static std::shared_ptr<ImageTexture> Make(int width, int height, std::vector<float> rgb) { return std::make_shared<ImageTexture>(width, height, std::move(rgb)); }
+
+private:
+	int width, height;
+	std::vector<float> rgb;
+};
+

@@ -257,6 +257,40 @@ int agpt_upload_instances(agpt_ctx* ctx, const agpt_instance* instances, int n);
 int agpt_upload_materials(agpt_ctx* ctx, const agpt_material* materials, int n);
 int agpt_upload_lights(agpt_ctx* ctx, const agpt_light* lights, int n);   /* refuses bad flags (see agpt_light.flags), scene unchanged */
 int agpt_upload_envmap(agpt_ctx* ctx, const agpt_envmap* env);          /* NULL clears it */
+
+/* ---- image textures on the base colour of Disney materials (EXTENSION: the reference has one colour per material) -------
+ * A texture is linear RGB float32, row-major: texel (x, y) at rgb[3 * (y * width + x) ..]; row 0 holds v in [0, 1/height).
+ * material_texture[i] is the base-colour texture of material i (an index into `textures`) or -1.  At a hit on a material with
+ * a texture, float32 with every operation rounded on its own:
+ *   1. surface uv (P = the hit point O + t * D the surface is built from):
+ *      - sphere: phi = atan2f(pHit.y, pHit.x), phi = phi < 0 ? phi + 2pi : phi; u = phi / 2pi, v = theta / pi, where pHit and
+ *        theta are those of Sphere's SurfaceInteraction (pHit = P - centre, x nudged to EPSILON * r at the poles; theta =
+ *        acos(clamp(pHit.z / r, -1, 1))) and atan2f is Sun fdlibm's e_atan2f.c in float (2pi, pi: the float constants);
+ *      - plane: u = ((P.x - o.x) / half_x + 1) * 0.5, v = ((P.z - o.z) / half_z + 1) * 0.5;
+ *      - triangle (instances: their mesh's uvs): b0 = 1 - b1 - b2, u = (b0 * uv0.u + b1 * uv1.u) + b2 * uv2.u, the same for v,
+ *        with the mesh's uvs or the default (0,0), (1,0), (1,1);
+ *   2. lookup, bilinear and repeat-wrapped, texel centres at (i + 0.5) / W:
+ *        u' = isfinite(u) ? u - floorf(u) : 0 (the same for v); s = u' * W - 0.5, x0 = (int)floorf(s), fx = s - floorf(s),
+ *        x1 = x0 + 1, each wrapped by x < 0 ? x + W : x >= W ? x - W : x (the same for t = v' * H - 0.5, y0, y1, fy);
+ *        a = T00 + fx * (T10 - T00), b = T01 + fx * (T11 - T01), c = a + fy * (b - a), Tij = texel (xi, yj)
+ *      (a constant texture returns its colour exactly; no random number is drawn: every path's draws stay where they were);
+ *   3. c replaces the colour of DisneyMaterial(color, roughness, metallic) (host/material.h) in its arithmetic:
+ *        dw = (1 - metallic) * (1 - 0); diffuse_r = dw > 0 ? dw * c : 0;  spec_r0 = Lerp(metallic, r0, c) = (1 - metallic) * r0
+ *        + metallic * c, r0 = ((eta - 1) * (eta - 1)) / ((eta + 1) * (eta + 1));
+ *      roughness, metallic, the alphas and the lobe set stay as the record has them;
+ *   4. agpt_render_guides' albedo of such a hit is that diffuse_r + spec_r0 (then clamped as for every material).
+ * Refused with AGPT_ERR_INVALID, leaving the resident textures as they were: a width or height < 1, width * height > 2^28, a
+ * NULL rgb, a texel that is not finite, an entry of material_texture outside [-1, n_textures).  (NULL, 0, NULL, 0) clears the
+ * textures.  Like every upload it makes the guides stale and drops the saved reprojection view.  At render time (with any
+ * binding >= 0) n_materials must equal the resident material count and every bound material must be AGPT_MAT_DISNEY, else
+ * AGPT_ERR_INVALID.  agpt_scene_bytes counts the texels (16 bytes each on the device) and the two small tables.
+ * statements/agpt_texture_oracle.cpp states the same on the CPU. */
+typedef struct agpt_texture {
+	int32_t width, height;
+	const float* rgb;        /* width * height * 3 floats */
+} agpt_texture;
+int agpt_upload_textures(agpt_ctx* ctx, const agpt_texture* textures, int n_textures, const int32_t* material_texture, int n_materials);
+
 int agpt_set_camera(agpt_ctx* ctx, const agpt_camera* camera);          /* Camera, camera.h:38-56 */
 int agpt_set_film(agpt_ctx* ctx, int width, int height);                /* Accumulator(w,h), myapp.h:10-13 */
 int agpt_scene_bytes(agpt_ctx* ctx, uint64_t* out);                     /* resident scene bytes in HBM */

@@ -25,6 +25,7 @@ typedef struct agpt_host_tracer agpt_host_tracer;
 const char* agpt_host_last_error(void);
 
 /* config 1..5 = BASELINE.json configs[0..4]; 6 and 8 = test-only corner-case scenes, 7 = the reference default scene;
+ * 9..12 = extension scenes of the host mirror (12: procedural image textures);
  * level <= 0 picks the configuration's own icosphere subdivision level. */
 int agpt_host_scene_create(int config, int level, agpt_host_scene** out);
 int agpt_host_scene_destroy(agpt_host_scene* scene);
@@ -47,6 +48,9 @@ typedef struct agpt_scene_tables {
 	agpt_camera camera;
 	agpt_envmap envmap;      /* width == 0: none */
 	const agpt_instance* instances; int n_instances;      /* extension: placed meshes */
+	const agpt_texture* textures;                          /* extension: base-colour images (agpt_upload_textures) */
+	const int32_t* material_texture;                       /* per material: texture index or -1; NULL when no material has one */
+	int n_textures, n_material_texture;
 } agpt_scene_tables;
 int agpt_host_scene_tables(agpt_host_scene* scene, agpt_scene_tables* out);
 
