@@ -143,6 +143,24 @@ class Texture(ctypes.Structure):      # agpt_texture
     _fields_ = [("width", c_int), ("height", c_int), ("rgb", POINTER(c_float))]
 
 
+class MaterialTextures(ctypes.Structure):      # agpt_material_textures
+    _fields_ = [("base", c_int32), ("roughness_metallic", c_int32), ("normal", c_int32), ("normal_scale", c_float), ("color", c_float * 3)]
+
+
+def material_textures(base=-1, roughness_metallic=-1, normal=-1, normal_scale=1.0, color=(0.0, 0.0, 0.0)):
+    """EXTENSION (agpt.h agpt_material_textures): one material's image bindings, indices into the images of
+    Context.upload_material_textures or -1.  `color` is the base colour used where base is -1 and roughness_metallic is not."""
+    return MaterialTextures(base, roughness_metallic, normal, normal_scale, (c_float * 3)(*color))
+
+
+def _image_rows(images, who):
+    imgs = [np.ascontiguousarray(a, np.float32) for a in images]
+    for a in imgs:
+        if a.ndim != 3 or a.shape[2] != 3:
+            raise AgptError(f"{who}: every image must be an (H, W, 3) array")
+    return imgs, (Texture * max(len(imgs), 1))(*[Texture(a.shape[1], a.shape[0], _fptr(a)) for a in imgs])
+
+
 HIT_DTYPE = np.dtype([("found", np.uint32), ("prim", np.int32), ("tri", np.int32), ("t", np.float32)])
 
 _core = None
@@ -250,14 +268,25 @@ class Context:
     def upload_textures(self, images, material_texture):
         """EXTENSION (agpt.h agpt_upload_textures): images = base-colour textures, each a numpy (H, W, 3) float32 array of linear
         RGB, row 0 at v in [0, 1/H); material_texture[i] = index into images of material i's texture, or -1.  ([], []) clears."""
-        imgs = [np.ascontiguousarray(a, np.float32) for a in images]
-        for a in imgs:
-            if a.ndim != 3 or a.shape[2] != 3:
-                raise AgptError("upload_textures: every image must be an (H, W, 3) array")
-        rows = (Texture * max(len(imgs), 1))(*[Texture(a.shape[1], a.shape[0], _fptr(a)) for a in imgs])
+        imgs, rows = _image_rows(images, "upload_textures")
         mt = np.ascontiguousarray(material_texture, np.int32)
         _check(core().agpt_upload_textures(self._h, rows if imgs else None, c_int(len(imgs)),
                                            mt.ctypes.data_as(POINTER(c_int)) if mt.size else None, c_int(mt.size)))
+
+    def upload_material_textures(self, images, bindings):
+        """EXTENSION (agpt.h agpt_upload_material_textures): images as for upload_textures (normal maps and roughness-metallic maps
+        are linear too); bindings[i] = material i's agpt.material_textures(...), a MaterialTextures row.  ([], []) clears."""
+        imgs, rows = _image_rows(images, "upload_material_textures")
+        bindings = list(bindings)
+        for b in bindings:
+            if not isinstance(b, MaterialTextures):
+                raise AgptError("upload_material_textures: every binding must be a material_textures(...) row")
+            if any(not -1 <= i < len(imgs) for i in (b.base, b.roughness_metallic, b.normal)):
+                raise AgptError("upload_material_textures: a binding points outside the images")
+            if not np.all(np.isfinite([b.normal_scale, *b.color])):
+                raise AgptError("upload_material_textures: normal_scale and color must be finite")
+        table = (MaterialTextures * max(len(bindings), 1))(*bindings)
+        _check(core().agpt_upload_material_textures(self._h, rows if imgs else None, c_int(len(imgs)), table if bindings else None, c_int(len(bindings))))
 
     def set_camera(self, cam19):
         cam19 = np.ascontiguousarray(cam19, np.float32)
@@ -477,6 +506,14 @@ class Context:
         _check(core().agpt_probe_light_sample(self._h, c_int(light), c_int(len(in8)), _fptr(in8), _fptr(out)))
         return out
 
+    def probe_material_maps(self, rays7):
+        """EXTENSION (agpt.h agpt_probe_material_maps): per ray, 32 floats: prim (-1 miss), u, v, ng, ns, ss, ts, T, B, roughness,
+        metallic, lobes, diffuse_r, spec_r0 of the closest hit as the maps shade kernel builds them."""
+        rays7 = np.ascontiguousarray(rays7, np.float32).reshape(-1, 7)
+        out = np.zeros((len(rays7), 32), np.float32)
+        _check(core().agpt_probe_material_maps(self._h, c_int(len(rays7)), _fptr(rays7), _fptr(out)))
+        return out
+
     def probe_stream(self, pixel_index, sample, k):
         out = np.empty(k, np.float32)
         _check(core().agpt_probe_stream(self._h, c_uint32(pixel_index), c_uint32(sample), c_int(k), _fptr(out)))
@@ -593,7 +630,7 @@ class HostScene:
 
     def tables(self):
         """agpt_scene_tables view (opaque bytes) of the flattened scene, valid while the scene lives."""
-        buf = ctypes.create_string_buffer(512)       # sizeof(agpt_scene_tables) = 248
+        buf = ctypes.create_string_buffer(512)       # sizeof(agpt_scene_tables) = 264
         _check(host().agpt_host_scene_tables(self._h, buf), host_side=True)
         return buf
 

@@ -101,8 +101,10 @@ struct agpt_ctx {
 	DevBuf<float4> texels;
 	DevBuf<DTexture> textures;
 	DevBuf<int> matTex;
-	std::vector<int32_t> hostMatTex;
+	DevBuf<DMatMaps> matMaps;     // roughness-metallic and normal maps (extension, agpt_upload_material_textures)
+	std::vector<agpt_material_textures> hostBindings;
 	bool hasTextures = false;     // some material has a texture: shade and guides run the textured instantiations
+	bool hasMaps = false;         // some material has a roughness-metallic or normal map: the TEX == 2 instantiations
 	DevBuf<agpt_light> lights;
 	DevBuf<float> envRgb, envFunc, envCdf;
 	float envFuncInt = 0;
@@ -374,9 +376,12 @@ static int CheckReady(agpt_ctx* c, bool needFilm) {
 	}
 	if (c->hasTextures) {
 		// textures (extension): the binding table belongs to the resident material table, and binds Disney materials only
-		NEED(c->hostMatTex.size() == (size_t)c->nMats, AGPT_ERR_INVALID, "texture bindings were uploaded for a different number of materials");
-		for (size_t i = 0; i < c->hostMatTex.size(); i++)
-			NEED(c->hostMatTex[i] < 0 || c->hostMatTypes[i] == AGPT_MAT_DISNEY, AGPT_ERR_INVALID, "a texture is bound to a material that is not AGPT_MAT_DISNEY");
+		NEED(c->hostBindings.size() == (size_t)c->nMats, AGPT_ERR_INVALID, "texture bindings were uploaded for a different number of materials");
+		for (size_t i = 0; i < c->hostBindings.size(); i++) {
+			const agpt_material_textures& b = c->hostBindings[i];
+			NEED((b.base < 0 && b.roughness_metallic < 0 && b.normal < 0) || c->hostMatTypes[i] == AGPT_MAT_DISNEY, AGPT_ERR_INVALID,
+				"a texture is bound to a material that is not AGPT_MAT_DISNEY");
+		}
 	}
 	if (c->mats.p == nullptr) {
 		// a scene of null-material (emissive) shapes only is legal upstream; shade still needs a record to point idle lanes at
@@ -498,7 +503,7 @@ int agpt_destroy(agpt_ctx* c) {
 	cudaStreamSynchronize(c->stream);
 	for (int r = 0; r < c->peerWorld; r++) if (r != c->peerRank && c->peerAccum[r]) cudaIpcCloseMemHandle(c->peerAccum[r]);
 	for (auto& m : c->meshStore) m.Free();
-	c->meshes.Free(); c->shapeLights.Free(); c->shapeCdf.Free(); c->instances.Free(); c->spheres.Free(); c->planes.Free(); c->prims.Free(); c->sphereRun.Free(); c->sphereRunBox.Free(); c->keyBoxes.Free(); c->mats.Free(); c->lights.Free(); c->texels.Free(); c->textures.Free(); c->matTex.Free();
+	c->meshes.Free(); c->shapeLights.Free(); c->shapeCdf.Free(); c->instances.Free(); c->spheres.Free(); c->planes.Free(); c->prims.Free(); c->sphereRun.Free(); c->sphereRunBox.Free(); c->keyBoxes.Free(); c->mats.Free(); c->lights.Free(); c->texels.Free(); c->textures.Free(); c->matTex.Free(); c->matMaps.Free();
 	c->accumOwn.Free(); c->resolved.Free();
 	c->moments.Free(); c->adaptiveList.Free(); c->adaptiveCount.Free();
 	c->guideAlbedo.Free(); c->guideNormal.Free(); c->denoiseE[0].Free(); c->denoiseE[1].Free(); c->denoiseG.Free(); c->denoiseOut.Free();
@@ -697,9 +702,10 @@ int agpt_upload_envmap(agpt_ctx* c, const agpt_envmap* env) {
 	return AGPT_OK;
 }
 
-// EXTENSION (agpt.h agpt_upload_textures): every argument is checked before anything resident changes.
-int agpt_upload_textures(agpt_ctx* c, const agpt_texture* textures, int n_textures, const int32_t* material_texture, int n_materials) {
-	NEED(c != nullptr && n_textures >= 0 && n_materials >= 0 && (n_textures == 0 || textures != nullptr) && (n_materials == 0 || material_texture != nullptr),
+// EXTENSION (agpt.h agpt_upload_textures, agpt_upload_material_textures): the one upload path of textures and their bindings.
+// Every argument is checked before anything resident changes.
+static int UploadMaterialTextures(agpt_ctx* c, const agpt_texture* textures, int n_textures, const agpt_material_textures* bindings, int n_materials) {
+	NEED(c != nullptr && n_textures >= 0 && n_materials >= 0 && (n_textures == 0 || textures != nullptr) && (n_materials == 0 || bindings != nullptr),
 		AGPT_ERR_INVALID, "agpt_upload_textures: bad table");
 	size_t total = 0;
 	for (int i = 0; i < n_textures; i++) {
@@ -710,8 +716,13 @@ int agpt_upload_textures(agpt_ctx* c, const agpt_texture* textures, int n_textur
 		for (size_t k = 0; k < n; k++) NEED(std::isfinite(t.rgb[k]), AGPT_ERR_INVALID, "agpt_upload_textures: texel not finite");
 		total += (size_t)t.width * t.height;
 	}
-	for (int i = 0; i < n_materials; i++)
-		NEED(material_texture[i] >= -1 && material_texture[i] < n_textures, AGPT_ERR_INVALID, "agpt_upload_textures: material points outside the texture table");
+	for (int i = 0; i < n_materials; i++) {
+		const agpt_material_textures& b = bindings[i];
+		for (int32_t t : { b.base, b.roughness_metallic, b.normal })
+			NEED(t >= -1 && t < n_textures, AGPT_ERR_INVALID, "agpt_upload_textures: material points outside the texture table");
+		NEED(std::isfinite(b.normal_scale) && std::isfinite(b.color[0]) && std::isfinite(b.color[1]) && std::isfinite(b.color[2]), AGPT_ERR_INVALID,
+			"agpt_upload_material_textures: normal_scale or color not finite");
+	}
 	CU(cudaSetDevice(c->device));
 	CU(cudaStreamSynchronize(c->stream));
 	c->stateGen++;
@@ -726,20 +737,39 @@ int agpt_upload_textures(agpt_ctx* c, const agpt_texture* textures, int n_textur
 		for (size_t k = 0; k < n; k++) texels[off + k] = make_float4(t.rgb[3 * k], t.rgb[3 * k + 1], t.rgb[3 * k + 2], 0.f);
 		off += n;
 	}
-	c->hasTextures = false;
-	c->hostMatTex.assign(material_texture, material_texture + n_materials);
-	for (int32_t t : c->hostMatTex) if (t >= 0) c->hasTextures = true;
+	c->hasTextures = false; c->hasMaps = false;
+	c->hostBindings.assign(bindings, bindings + n_materials);
+	std::vector<int32_t> matTex((size_t)n_materials);
+	std::vector<DMatMaps> maps((size_t)n_materials);
+	for (int i = 0; i < n_materials; i++) {
+		const agpt_material_textures& b = bindings[i];
+		matTex[i] = b.base;
+		maps[i] = DMatMaps{ b.base, b.roughness_metallic, b.normal, b.normal_scale, { b.color[0], b.color[1], b.color[2] }, 0.f };
+		if (b.base >= 0 || b.roughness_metallic >= 0 || b.normal >= 0) c->hasTextures = true;
+		if (b.roughness_metallic >= 0 || b.normal >= 0) c->hasMaps = true;
+	}
 	CU(c->texels.Upload(texels.data(), texels.size(), c->stream));
 	CU(c->textures.Upload(desc.data(), desc.size(), c->stream));
-	CU(c->matTex.Upload(c->hostMatTex.data(), c->hostMatTex.size(), c->stream));
+	CU(c->matTex.Upload(matTex.data(), matTex.size(), c->stream));
+	CU(c->matMaps.Upload(maps.data(), c->hasMaps ? maps.size() : 0, c->stream));     // read by the TEX == 2 kernels only
 	CU(cudaStreamSynchronize(c->stream));
 	return AGPT_OK;
+}
+int agpt_upload_textures(agpt_ctx* c, const agpt_texture* textures, int n_textures, const int32_t* material_texture, int n_materials) {
+	NEED(c != nullptr && n_materials >= 0 && (n_materials == 0 || material_texture != nullptr), AGPT_ERR_INVALID, "agpt_upload_textures: bad table");
+	std::vector<agpt_material_textures> b((size_t)n_materials);
+	for (int i = 0; i < n_materials; i++) b[i] = agpt_material_textures{ material_texture[i], -1, -1, 1.f, { 0.f, 0.f, 0.f } };
+	return UploadMaterialTextures(c, textures, n_textures, b.data(), n_materials);
+}
+int agpt_upload_material_textures(agpt_ctx* c, const agpt_texture* textures, int n_textures, const agpt_material_textures* bindings, int n_materials) {
+	return UploadMaterialTextures(c, textures, n_textures, bindings, n_materials);
 }
 
 static DTexTables MakeTexTables(const agpt_ctx* c) {
 	DTexTables t;
 	t.texels = c->texels.p; t.textures = c->textures.p; t.matTex = c->matTex.p;
 	t.nTextures = (int)c->textures.n; t.nTexels = (long long)c->texels.n;
+	t.matMaps = c->matMaps.p; t.nMatMaps = (int)c->matMaps.n;
 	return t;
 }
 
@@ -787,7 +817,7 @@ int agpt_set_film(agpt_ctx* c, int width, int height) {
 int agpt_scene_bytes(agpt_ctx* c, uint64_t* out) {
 	NEED(c != nullptr && out != nullptr, AGPT_ERR_INVALID, "null argument");
 	uint64_t b = c->envRgb.Bytes() + c->envFunc.Bytes() + c->envCdf.Bytes() + c->meshes.Bytes() + c->spheres.Bytes() + c->planes.Bytes() + c->prims.Bytes() + c->instances.Bytes() + c->mats.Bytes() + c->lights.Bytes()
-		+ c->shapeLights.Bytes() + c->shapeCdf.Bytes() + c->texels.Bytes() + c->textures.Bytes() + c->matTex.Bytes();
+		+ c->shapeLights.Bytes() + c->shapeCdf.Bytes() + c->texels.Bytes() + c->textures.Bytes() + c->matTex.Bytes() + c->matMaps.Bytes();
 	for (auto& m : c->meshStore) b += m.nodes.Bytes() + m.tris.Bytes() + m.normals.Bytes() + m.uvs.Bytes() + m.ids.Bytes();
 	*out = b;
 	return AGPT_OK;
@@ -1006,10 +1036,12 @@ static int RunWaves(agpt_ctx* c, const DScene& scIn, PathState& ps, int n, int m
 		DShapeTables st;
 		st.lights = c->shapeLights.p; st.cdf = c->shapeCdf.p;
 		const DTexTables tt = MakeTexTables(c);
-#define SHADE_B(E, G, S) k_shade_b<E, G, S, false><<<shadeBlocks, AGPT_SHADE_THREADS, 0, c->stream>>>(sc, st, ps, c->survivors.p, q[cur ^ 1], sp, c->rayCounters.p, tt)
-#define SHADE_B_TEX(E, G, S) k_shade_b<E, G, S, true><<<shadeBlocks, AGPT_SHADE_THREADS, 0, c->stream>>>(sc, st, ps, c->survivors.p, q[cur ^ 1], sp, c->rayCounters.p, tt)
+#define SHADE_B(E, G, S) k_shade_b<E, G, S, 0><<<shadeBlocks, AGPT_SHADE_THREADS, 0, c->stream>>>(sc, st, ps, c->survivors.p, q[cur ^ 1], sp, c->rayCounters.p, tt)
+#define SHADE_B_TEX(E, G, S, T) k_shade_b<E, G, S, T><<<shadeBlocks, AGPT_SHADE_THREADS, 0, c->stream>>>(sc, st, ps, c->survivors.p, q[cur ^ 1], sp, c->rayCounters.p, tt)
 		// (TEX, some material is textured: the lean textured instantiation, or the one that carries everything)
-		if (c->hasTextures) { if (c->hasShapeLights || c->envW > 0 || c->hasGlass) SHADE_B_TEX(true, true, true); else SHADE_B_TEX(false, false, false); }
+		// (TEX = 2, some material has a roughness-metallic or normal map: the per-hit material record)
+		if (c->hasMaps) { if (c->hasShapeLights || c->envW > 0 || c->hasGlass) SHADE_B_TEX(true, true, true, 2); else SHADE_B_TEX(false, false, false, 2); }
+		else if (c->hasTextures) { if (c->hasShapeLights || c->envW > 0 || c->hasGlass) SHADE_B_TEX(true, true, true, 1); else SHADE_B_TEX(false, false, false, 1); }
 		else if (c->hasShapeLights) { if (c->envW > 0 || c->hasGlass) SHADE_B(true, true, true); else SHADE_B(false, false, true); }
 		else if (c->envW > 0) { if (c->hasGlass) SHADE_B(true, true, false); else SHADE_B(true, false, false); }
 		else { if (c->hasGlass) SHADE_B(false, true, false); else SHADE_B(false, false, false); }
@@ -1312,7 +1344,8 @@ int agpt_render_guides(agpt_ctx* c, int num_samples, uint32_t flags) {
 		g.n = n; g.first_sample = done; g.sample_stride = 1; g.tiled = 1; g.samples = ns;
 		k_generate<false><<<Blocks(n, 256), 256, 0, c->stream>>>(sc, ps, q0, g);
 		LaunchClosest(count, strictBoxes, c->nInstances > 0, Blocks(n, AGPT_TRACE_THREADS), c->stream, sc, ps, q0.closest, q0.counts + 0, c->traceCounters.p, nullptr);
-		if (c->hasTextures) k_guides_tex<<<Blocks(wh, 256), 256, 0, c->stream>>>(sc, MakeTexTables(c), ps, ns, done == 0, done + ns == num_samples ? num_samples : 0, c->guideAlbedo.p, c->guideNormal.p);
+		if (c->hasMaps) k_guides_maps<<<Blocks(wh, 256), 256, 0, c->stream>>>(sc, MakeTexTables(c), ps, ns, done == 0, done + ns == num_samples ? num_samples : 0, c->guideAlbedo.p, c->guideNormal.p);
+		else if (c->hasTextures) k_guides_tex<<<Blocks(wh, 256), 256, 0, c->stream>>>(sc, MakeTexTables(c), ps, ns, done == 0, done + ns == num_samples ? num_samples : 0, c->guideAlbedo.p, c->guideNormal.p);
 		else k_guides<<<Blocks(wh, 256), 256, 0, c->stream>>>(sc, ps, ns, done == 0, done + ns == num_samples ? num_samples : 0, c->guideAlbedo.p, c->guideNormal.p);
 		CU(cudaGetLastError());
 		c->stats.kernel_launches += 3; c->stats.launches_closest++;
@@ -2054,6 +2087,39 @@ int agpt_probe_bsdf(agpt_ctx* c, int n, const agpt_material* mat, const float* i
 	return ProbeRun(c, in14, 14 * (size_t)n, out12, 12 * (size_t)n, [&](const float* din, float* dout) {
 		k_probe_bsdf<<<Blocks(n, 128), 128, 0, c->stream>>>(n, m, din, skip_specular, dout);
 	});
+}
+
+// EXTENSION (agpt.h agpt_probe_material_maps): the rays are traced as agpt_trace_rays traces them (k_generate<false>, closest hit)
+int agpt_probe_material_maps(agpt_ctx* c, int n, const float* rays7, float* out32) {
+	NEED(c != nullptr && n > 0 && rays7 && out32, AGPT_ERR_INVALID, "bad probe arguments");
+	int rcode = CheckReady(c, false);
+	if (rcode != AGPT_OK) return rcode;
+	NEED(c->hasMaps, AGPT_ERR_STATE, "agpt_probe_material_maps: no material has a roughness-metallic or normal map");
+	CU(cudaSetDevice(c->device));
+	rcode = EnsureCapacity(c, (size_t)n);
+	if (rcode != AGPT_OK) return rcode;
+	DScene sc = MakeScene(c);
+	PathState ps = MakePathState(c);
+	WaveQueues q0;
+	q0.closest = c->queues[0].p; q0.shadow = c->queues[2].p; q0.active = c->queues[4].p; q0.counts = c->counts.p; q0.keys = nullptr; q0.shadowKeys = nullptr;
+	DevBuf<float> rays, out;
+	DevBuf<uint32_t> seeds;
+	CU(rays.Upload(rays7, 7 * (size_t)n, c->stream));
+	CU(seeds.Alloc((size_t)n));
+	CU(cudaMemsetAsync(seeds.p, 0, seeds.Bytes(), c->stream));
+	CU(out.Alloc(32 * (size_t)n));
+	GenParams g;
+	memset(&g, 0, sizeof(g));
+	g.n = n; g.rays7 = rays.p; g.seeds = seeds.p;
+	k_generate<false><<<Blocks(n, 256), 256, 0, c->stream>>>(sc, ps, q0, g);
+	LaunchClosest(false, false, c->nInstances > 0, Blocks(n, AGPT_TRACE_THREADS), c->stream, sc, ps, q0.closest, q0.counts + 0, c->traceCounters.p, nullptr);
+	k_probe_material_maps<<<Blocks(n, 256), 256, 0, c->stream>>>(sc, MakeTexTables(c), ps, n, out.p);
+	CU(cudaGetLastError());
+	c->stats.kernel_launches += 3;
+	CU(cudaMemcpyAsync(out32, out.p, out.Bytes(), cudaMemcpyDeviceToHost, c->stream));
+	CU(cudaStreamSynchronize(c->stream));
+	rays.Free(); seeds.Free(); out.Free();
+	return AGPT_OK;
 }
 
 int agpt_probe_sphere_sample(agpt_ctx* c, int n, const float* in9, float* out8) {

@@ -243,8 +243,10 @@ __device__ __forceinline__ DBSDF MakeBSDF(const DSurface& s, const agpt_material
 }
 
 // Sphere hit -> interaction (intersectable.h:183-204); dpdu/dpdv are passed swapped upstream.
-// uv (extension, textured instantiations only; agpt.h agpt_upload_textures): the sphere's surface uv, or nullptr.
-__device__ __forceinline__ void SphereSurface(const agpt_sphere& sp, float3 O, float3 D, float root, DSurface& s, float2* uv = nullptr) {
+// uv (extension, textured instantiations only; agpt.h agpt_upload_textures): the sphere's surface uv, or nullptr.  dpduOut,
+// dpdvOut (extension, normal maps; agpt.h agpt_upload_material_textures): dp/du and dp/dv of that uv (before the swap), or nullptr.
+__device__ __forceinline__ void SphereSurface(const agpt_sphere& sp, float3 O, float3 D, float root, DSurface& s, float2* uv = nullptr,
+		float3* dpduOut = nullptr, float3* dpdvOut = nullptr) {
 	float3 p = O + root * D;
 	float3 pHit = p - f3(sp.center);
 	if (pHit.x == 0 && pHit.y == 0) pHit.x = AGPT_EPSILON * sp.r;
@@ -256,6 +258,7 @@ __device__ __forceinline__ void SphereSurface(const agpt_sphere& sp, float3 O, f
 	float3 dpdu = f3(-AGPT_TWOPI * pHit.y, AGPT_TWOPI * pHit.x, 0);
 	float3 dpdv = AGPT_PI * f3(pHit.z * cosPhi, pHit.z * sinPhi, -sp.r * rsin(theta));
 	SurfaceInit(s, p, dpdv, dpdu);
+	if (dpduOut) { *dpduOut = dpdu; *dpdvOut = dpdv; }
 	if (uv) {
 		float phi = ratan2T<1>(pHit.y, pHit.x);
 		if (phi < 0) phi = phi + AGPT_TWOPI;
@@ -268,9 +271,9 @@ __device__ __forceinline__ void PlaneSurface(float3 O, float3 D, float t, DSurfa
 // Triangle hit -> interaction + shading frame (trianglemesh.cpp:45-113, intersectable.h:80-89)
 // `in` (extension, agpt.h agpt_instance): the mesh is a placed one -- vertices go to world space first, the shading
 // normal through transpose(W2O); nullptr for the reference's own meshes.  uvOut (extension, textured instantiations only): the
-// interpolated uv, or nullptr.
+// interpolated uv, or nullptr.  dpduOut, dpdvOut (extension, normal maps): TriangleDerivatives' dpdu, dpdv, or nullptr.
 __device__ __forceinline__ void TriangleSurface(const DMesh& mesh, int slot, float3 O, float3 D, float t, float b1, float b2, DSurface& s, const agpt_instance* in,
-		float2* uvOut = nullptr) {
+		float2* uvOut = nullptr, float3* dpduOut = nullptr, float3* dpdvOut = nullptr) {
 	float4 a = __ldg(mesh.tris + 3 * slot), b = __ldg(mesh.tris + 3 * slot + 1), c = __ldg(mesh.tris + 3 * slot + 2);
 	float3 v0 = f3(a.x, a.y, a.z), v1 = f3(b.x, b.y, b.z), v2 = f3(c.x, c.y, c.z);
 	if (in) { v0 = XformPoint(in->object_to_world, v0); v1 = XformPoint(in->object_to_world, v1); v2 = XformPoint(in->object_to_world, v2); }
@@ -281,6 +284,7 @@ __device__ __forceinline__ void TriangleSurface(const DMesh& mesh, int slot, flo
 	float3 dpdu, dpdv;
 	TriangleDerivatives(v0, v1, v2, uv0, uv1, uv2, dpdu, dpdv);
 	SurfaceInit(s, O + t * D, dpdu, dpdv);
+	if (dpduOut) { *dpduOut = dpdu; *dpdvOut = dpdv; }
 	if (mesh.normals) {
 		float4 na = __ldg(mesh.normals + 3 * slot), nb = __ldg(mesh.normals + 3 * slot + 1), nc = __ldg(mesh.normals + 3 * slot + 2);
 		float3 ns = f3(na.x, na.y, na.z) * b0 + f3(nb.x, nb.y, nb.z) * b1 + f3(nc.x, nc.y, nc.z) * b2;
@@ -331,16 +335,72 @@ struct TexColors {
 	float3 diffuse;   // agpt_material.diffuse_r
 	float3 spec0;     // agpt_material.spec_r0
 };
+// DisneyMaterial's colour arithmetic (host/material.h) for base colour c: the one statement of it on the device
+__device__ __forceinline__ TexColors DisneyColors(float3 c, float metallic, float eta) {
+	TexColors tc;
+	const float dw = (1 - metallic) * (1 - 0.f);
+	tc.diffuse = dw > 0 ? dw * c : f3(0.f);
+	const float r0 = ((eta - 1) * (eta - 1)) / ((eta + 1) * (eta + 1));
+	tc.spec0 = Lerp(metallic, f3(r0), c);
+	return tc;
+}
 __device__ __forceinline__ TexColors HitColors(const DTexTables& tt, int material, const agpt_material& m, float2 uv) {
 	TexColors tc;
 	const int tex = tt.matTex[material];
 	if (tex < 0) { tc.diffuse = f3(m.diffuse_r); tc.spec0 = f3(m.spec_r0); return tc; }
+	return DisneyColors(TexLookup(tt, tex, uv), m.metallic, m.eta);
+}
+
+// ---------------------------------------------------------------------------------------
+// EXTENSION: roughness-metallic and normal maps on Disney materials, stated in agpt.h (agpt_upload_material_textures) and on
+// the CPU in statements/agpt_material_maps_oracle.cpp.  The TEX == 2 instantiations shade with the record this builds.
+// ---------------------------------------------------------------------------------------
+__device__ __forceinline__ float MapClamp01(float x) { return x < 0.f ? 0.f : x > 1.f ? 1.f : x; }
+// step 1: the hit's material record
+__device__ __forceinline__ agpt_material MapsMaterial(const DTexTables& tt, const DMatMaps& mm, const agpt_material& rec, float2 uv) {
+	agpt_material m = rec;
+	if (mm.roughnessMetallic < 0 && mm.base < 0) return m;
+	float r = rec.roughness, k = rec.metallic;
+	float3 C;
+	if (mm.roughnessMetallic < 0) C = TexLookup(tt, mm.base, uv);          // agpt_upload_textures step 3
+	else {
+		const float3 rm = TexLookup(tt, mm.roughnessMetallic, uv);
+		C = mm.base >= 0 ? TexLookup(tt, mm.base, uv) : f3(mm.color[0], mm.color[1], mm.color[2]);
+		r = rec.roughness * MapClamp01(rm.y); k = rec.metallic * MapClamp01(rm.z);
+		const float a = smax(.001f, smax(.001f, r * r));         // std::max, as the constructor
+		m.lobes = ((1 - k) * (1 - 0.f) > 0 ? (uint32_t)(AGPT_LOBE_DIFFUSE | AGPT_LOBE_RETRO) : 0u) | (uint32_t)AGPT_LOBE_MICROFACET;
+		m.roughness = r; m.metallic = k;
+		m.alpha_x = a; m.alpha_y = a;
+	}
+	const TexColors tc = DisneyColors(C, k, rec.eta);
+	m.diffuse_r[0] = tc.diffuse.x; m.diffuse_r[1] = tc.diffuse.y; m.diffuse_r[2] = tc.diffuse.z;
+	m.spec_r0[0] = tc.spec0.x; m.spec_r0[1] = tc.spec0.y; m.spec_r0[2] = tc.spec0.z;
+	return m;
+}
+// step 2: the normal map's shading frame; T, B = dp/du, dp/dv of the texture's uv.  Leaves s as it is in the three cases agpt.h
+// names, so a flat map reproduces the unmapped surface bit for bit.
+__device__ __forceinline__ void ApplyNormalMap(const DTexTables& tt, int tex, float scale, float2 uv, float3 T, float3 B, DSurface& s) {
 	const float3 c = TexLookup(tt, tex, uv);
-	const float dw = (1 - m.metallic) * (1 - 0.f);
-	tc.diffuse = dw > 0 ? dw * c : f3(0.f);
-	const float r0 = ((m.eta - 1) * (m.eta - 1)) / ((m.eta + 1) * (m.eta + 1));
-	tc.spec0 = Lerp(m.metallic, f3(r0), c);
-	return tc;
+	const float3 nts = f3(scale * (2 * c.x - 1), scale * (2 * c.y - 1), 2 * c.z - 1);
+	if (nts.x == 0 && nts.y == 0 && nts.z > 0) return;
+	const float3 N = s.sn;
+	float3 Tp = T - N * dot(N, T);
+	if (dot(Tp, Tp) == 0) return;
+	Tp = normalize(Tp);
+	float3 Bp = cross(N, Tp);
+	if (dot(Bp, B) < 0) Bp = -Bp;
+	float3 n = (nts.x * Tp + nts.y * Bp) + nts.z * N;
+	if (!(dot(n, N) > 0)) return;
+	n = normalize(n);
+	s.sn = n;
+	s.sdpdu = Tp - n * dot(n, Tp);
+}
+// steps 1 and 2 for a hit on material `material` (a Disney record: the render-time check binds maps to nothing else)
+__device__ __forceinline__ agpt_material HitMaps(const DTexTables& tt, int material, const agpt_material& rec, float2 uv, float3 T, float3 B, DSurface& s) {
+	AGPT_CHECK(material >= 0 && material < tt.nMatMaps, AGPT_DBG_MAPS, material);
+	const DMatMaps mm = tt.matMaps[material];
+	if (mm.normal >= 0) ApplyNormalMap(tt, mm.normal, mm.normalScale, uv, T, B, s);
+	return MapsMaterial(tt, mm, rec, uv);
 }
 
 // ---------------------------------------------------------------------------------------

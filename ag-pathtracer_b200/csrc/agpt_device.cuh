@@ -28,7 +28,8 @@
 enum { AGPT_DBG_STACK = 1, AGPT_DBG_NODE = 2, AGPT_DBG_TRI = 3, AGPT_DBG_QUEUE = 4, AGPT_DBG_PATH = 5, AGPT_DBG_PRIM = 6, AGPT_DBG_MATERIAL = 7,
        AGPT_DBG_LIST = 8 /* adaptive pixel list entry or pixel index */, AGPT_DBG_SAMPLE = 9 /* a pixel's samples past max_samples */,
        AGPT_DBG_GUIDE = 10 /* k_guides: path slot */, AGPT_DBG_TAP = 11 /* denoise, reprojection: filter or history tap outside the film */,
-       AGPT_DBG_TEXTURE = 12 /* texture index of a material */, AGPT_DBG_TEXEL = 13 /* texel index of a lookup */ };
+       AGPT_DBG_TEXTURE = 12 /* texture index of a material */, AGPT_DBG_TEXEL = 13 /* texel index of a lookup */,
+       AGPT_DBG_MAPS = 14 /* material index into the map binding table */ };
 #ifdef AGPT_DEBUG
 __device__ unsigned long long g_agptDebug[4];     // [0] failures, [1] first code, [2] first value, [3] checks executed
 #define AGPT_CHECK(cond, code, value) do { atomicAdd(&g_agptDebug[3], 1ull); if (!(cond)) { \
@@ -64,12 +65,21 @@ struct DTexture {
 	int width, height;
 	long long off;               // first texel in DTexTables::texels
 };
+// one material's bindings (agpt_material_textures): two 128-bit loads
+struct __align__(16) DMatMaps {
+	int base, roughnessMetallic, normal;   // texture indices or -1
+	float normalScale;
+	float color[3];                        // base colour when base < 0 and roughnessMetallic >= 0
+	float pad;
+};
 struct DTexTables {
 	const float4* texels;        // every texture's texels, row-major, .w unused: one bilinear lookup = four 128-bit loads
 	const DTexture* textures;
 	const int* matTex;           // per material: its base-colour texture, or -1
 	int nTextures;
 	long long nTexels;
+	const DMatMaps* matMaps;     // per material: its map bindings (agpt_upload_material_textures); read by the TEX == 2 kernels only
+	int nMatMaps;
 };
 
 struct DScene {

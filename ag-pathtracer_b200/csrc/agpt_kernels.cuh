@@ -510,10 +510,12 @@ __global__ void __launch_bounds__(256) k_shade_a(DScene sc, PathState ps, const 
 #define AGPT_SHADE_STACK_SMEM 8
 
 // SHAPES (extension): some area light samples its plane or mesh (AGPT_LIGHT_SAMPLE_SHAPE); other scenes run the
-// instantiations without that code.  TEX (extension): some Disney material has an image texture on its base colour
-// (agpt_upload_textures): two instantiations run, <false, false, false, true> and <true, true, true, true>; `tt` is read only by
-// them (the others take it last, after every parameter they had before, and their code is what it was).
-template <bool ENV, bool GLASS, bool SHAPES, bool TEX>
+// instantiations without that code.  TEX (extension): 1, some Disney material has an image texture on its base colour
+// (agpt_upload_textures): two instantiations run, <false, false, false, 1> and <true, true, true, 1>; `tt` is read only by
+// them (the others take it last, after every parameter they had before, and their code is what it was).  2, some Disney
+// material has a roughness-metallic or normal map (agpt_upload_material_textures): <false, false, false, 2> and
+// <true, true, true, 2> shade with the hit's own material record, built once per vertex before the BSDF frame.
+template <bool ENV, bool GLASS, bool SHAPES, int TEX>
 __global__ void __launch_bounds__(AGPT_SHADE_THREADS, AGPT_SHADE_MIN_BLOCKS) k_shade_b(DScene sc, DShapeTables st, PathState ps, const int* __restrict__ survivors, WaveQueues qout, ShadeParams sp,
 		RayCounters* rc, DTexTables tt) {
 	__shared__ unsigned shapeStack[SHAPES ? AGPT_SHADE_STACK_SMEM * AGPT_SHADE_THREADS : 1];
@@ -551,20 +553,23 @@ __global__ void __launch_bounds__(AGPT_SHADE_THREADS, AGPT_SHADE_MIN_BLOCKS) k_s
 		float2 uv = make_float2(0.f, 0.f);       // TEX: surface uv of the hit
 		TexColors tc;                            // TEX: the hit's diffuse reflectance and Schlick R0
 		tc.diffuse = f3(0.f); tc.spec0 = f3(0.f);
+		float3 dpdu = f3(0.f), dpdv = f3(0.f);   // TEX == 2: dp/du, dp/dv of the uv (normal maps)
+		agpt_material hm;                        // TEX == 2: the hit's material record; idle lanes keep the first record
+		if (TEX == 2) hm = sc.mats[0];
 
 		// the surface at the hit (a survivor has one); null materials pass straight through
 		if (valid) {
 			AGPT_CHECK(__float_as_int(h.w) >= 0 && __float_as_int(h.w) < sc.n_prims, AGPT_DBG_PRIM, __float_as_int(h.w));
 			agpt_prim prim = sc.prims[__float_as_int(h.w)];
 			// SurfaceInteraction of the closest hit
-			if (prim.type == AGPT_PRIM_SPHERE) SphereSurface(sc.spheres[prim.payload], O, D, h.x, si, TEX ? &uv : nullptr);
+			if (prim.type == AGPT_PRIM_SPHERE) SphereSurface(sc.spheres[prim.payload], O, D, h.x, si, TEX ? &uv : nullptr, TEX == 2 ? &dpdu : nullptr, TEX == 2 ? &dpdv : nullptr);
 			else if (prim.type == AGPT_PRIM_PLANE) PlaneSurface(O, D, h.x, si);
 			else if (prim.type == AGPT_PRIM_INSTANCE) {          // extension: a placed mesh
 				const agpt_instance& in = sc.instances[prim.payload];
-				TriangleSurface(sc.meshes[in.mesh], hitSlot, O, D, h.x, h.y, h.z, si, &in, TEX ? &uv : nullptr);
+				TriangleSurface(sc.meshes[in.mesh], hitSlot, O, D, h.x, h.y, h.z, si, &in, TEX ? &uv : nullptr, TEX == 2 ? &dpdu : nullptr, TEX == 2 ? &dpdv : nullptr);
 			}
-			else TriangleSurface(sc.meshes[prim.payload], hitSlot, O, D, h.x, h.y, h.z, si, nullptr, TEX ? &uv : nullptr);
-			if (TEX && prim.type == AGPT_PRIM_PLANE) uv = PlaneUV(sc.planes[prim.payload], si.p);
+			else TriangleSurface(sc.meshes[prim.payload], hitSlot, O, D, h.x, h.y, h.z, si, nullptr, TEX ? &uv : nullptr, TEX == 2 ? &dpdu : nullptr, TEX == 2 ? &dpdv : nullptr);
+			if (TEX && prim.type == AGPT_PRIM_PLANE) { uv = PlaneUV(sc.planes[prim.payload], si.p); dpdu = f3(1.f, 0.f, 0.f); dpdv = f3(0.f, 0.f, 1.f); }
 
 			if (prim.material < 0) {
 				// null material: pass straight through, bounce count unchanged (integrator.h:152-161)
@@ -576,9 +581,11 @@ __global__ void __launch_bounds__(AGPT_SHADE_THREADS, AGPT_SHADE_MIN_BLOCKS) k_s
 			}
 			else {
 				full = true; mat = sc.mats + prim.material;
-				if (TEX) tc = HitColors(tt, prim.material, *mat, uv);     // the one lookup of this vertex
+				if (TEX == 1) tc = HitColors(tt, prim.material, *mat, uv);     // the one lookup of this vertex
+				if (TEX == 2) hm = HitMaps(tt, prim.material, *mat, uv, dpdu, dpdv, si);   // the lookups of this vertex
 			}
 		}
+		if (TEX == 2) mat = &hm;
 
 		// ================= phase B: BSDF frame, random numbers, light sample =================
 		const float3 wo = -D;
@@ -717,7 +724,7 @@ __global__ void __launch_bounds__(AGPT_SHADE_THREADS, AGPT_SHADE_MIN_BLOCKS) k_s
 			float3 wiLoc = k == 0 ? WorldToLocal(vb.b, wiL) : sampledWi;
 			LobeEval ev;
 			ev.f = f3(0.f); ev.pdfCos = 0.f; ev.pdfMicro = 0.f; ev.fT = f3(0.f); ev.pdfT = 0.f;
-			if (need) EvalLobes<GLASS, TEX>(vb, wiLoc, ev, tc);
+			if (need) EvalLobes<GLASS, TEX == 1>(vb, wiLoc, ev, tc);
 			if (k == 0) {
 				if (need) fLight = FinishEval<GLASS>(vb, ev, wiL, &pdfLight);     // BSDF::f and BSDF::Pdf at the light direction
 			}
@@ -1012,8 +1019,9 @@ __global__ void __launch_bounds__(256) k_resolve_counts(const float4* __restrict
 // k_guides: one thread per pixel after k_generate<false> (tiled) and k_trace_closest have run the batch's camera rays.  It walks
 // the pixel's slots in sample order and adds each sample's first hit to the running sums in albedo (.xyz, .w = hits) and
 // normalDepth (.xyz, .w = t sum).  `total` > 0 on the last batch: the sums become the means of all `total` samples.
-// TEX (extension): a textured Disney material's albedo is the hit's textured diffuse_r + spec_r0 (k_guides_tex).
-template <bool TEX>
+// TEX (extension): 1, a textured Disney material's albedo is the hit's textured diffuse_r + spec_r0 (k_guides_tex); 2, the
+// hit's material record and mapped shading normal of k_shade_b<..., 2> give albedo and normal (k_guides_maps).
+template <int TEX>
 __device__ __forceinline__ void Guides(DScene sc, DTexTables tt, PathState ps, int samplesInBatch, bool firstBatch, int total, float4* albedo, float4* normalDepth) {
 	const int pixel = blockIdx.x * blockDim.x + threadIdx.x;
 	const int width = sc.width, height = sc.height;
@@ -1036,20 +1044,24 @@ __device__ __forceinline__ void Guides(DScene sc, DTexTables tt, PathState ps, i
 			const agpt_prim prim = sc.prims[hitPrim];
 			DSurface si;
 			float2 uv = make_float2(0.f, 0.f);
+			float3 dpdu = f3(0.f), dpdv = f3(0.f);
+			agpt_material hm;
 			// the surface of the closest hit as k_shade_b rebuilds it
-			if (prim.type == AGPT_PRIM_SPHERE) SphereSurface(sc.spheres[prim.payload], O, D, h.x, si, TEX ? &uv : nullptr);
+			if (prim.type == AGPT_PRIM_SPHERE) SphereSurface(sc.spheres[prim.payload], O, D, h.x, si, TEX ? &uv : nullptr, TEX == 2 ? &dpdu : nullptr, TEX == 2 ? &dpdv : nullptr);
 			else if (prim.type == AGPT_PRIM_PLANE) PlaneSurface(O, D, h.x, si);
 			else if (prim.type == AGPT_PRIM_INSTANCE) {
 				const agpt_instance& in = sc.instances[prim.payload];
-				TriangleSurface(sc.meshes[in.mesh], ps.hitSlot[slot], O, D, h.x, h.y, h.z, si, &in, TEX ? &uv : nullptr);
+				TriangleSurface(sc.meshes[in.mesh], ps.hitSlot[slot], O, D, h.x, h.y, h.z, si, &in, TEX ? &uv : nullptr, TEX == 2 ? &dpdu : nullptr, TEX == 2 ? &dpdv : nullptr);
 			}
-			else TriangleSurface(sc.meshes[prim.payload], ps.hitSlot[slot], O, D, h.x, h.y, h.z, si, nullptr, TEX ? &uv : nullptr);
-			if (TEX && prim.type == AGPT_PRIM_PLANE) uv = PlaneUV(sc.planes[prim.payload], si.p);
+			else TriangleSurface(sc.meshes[prim.payload], ps.hitSlot[slot], O, D, h.x, h.y, h.z, si, nullptr, TEX ? &uv : nullptr, TEX == 2 ? &dpdu : nullptr, TEX == 2 ? &dpdv : nullptr);
+			if (TEX && prim.type == AGPT_PRIM_PLANE) { uv = PlaneUV(sc.planes[prim.payload], si.p); dpdu = f3(1.f, 0.f, 0.f); dpdv = f3(0.f, 0.f, 1.f); }
+			if (TEX == 2 && prim.material >= 0) hm = HitMaps(tt, prim.material, sc.mats[prim.material], uv, dpdu, dpdv, si);
 			n = dot(si.sn, D) > 0.f ? -si.sn : si.sn;
 			if (prim.material >= 0) {
 				const agpt_material& m = sc.mats[prim.material];
 				if (m.type == AGPT_MAT_MIRROR) alb = f3(m.mirror_r);
 				else if (m.type == AGPT_MAT_GLASS) alb = f3(m.mirror_r) + f3(m.diffuse_r);
+				else if (TEX == 2) alb = f3(hm.diffuse_r) + f3(hm.spec_r0);
 				else if (TEX) { const TexColors tc = HitColors(tt, prim.material, m, uv); alb = tc.diffuse + tc.spec0; }
 				else alb = f3(m.diffuse_r) + f3(m.spec_r0);
 				alb = f3(alb.x < 1.f ? alb.x : 1.f, alb.y < 1.f ? alb.y : 1.f, alb.z < 1.f ? alb.z : 1.f);
@@ -1070,10 +1082,50 @@ __device__ __forceinline__ void Guides(DScene sc, DTexTables tt, PathState ps, i
 	normalDepth[f] = nd;
 }
 __global__ void __launch_bounds__(256) k_guides(DScene sc, PathState ps, int samplesInBatch, bool firstBatch, int total, float4* albedo, float4* normalDepth) {
-	Guides<false>(sc, DTexTables(), ps, samplesInBatch, firstBatch, total, albedo, normalDepth);
+	Guides<0>(sc, DTexTables(), ps, samplesInBatch, firstBatch, total, albedo, normalDepth);
 }
 __global__ void __launch_bounds__(256) k_guides_tex(DScene sc, DTexTables tt, PathState ps, int samplesInBatch, bool firstBatch, int total, float4* albedo, float4* normalDepth) {
-	Guides<true>(sc, tt, ps, samplesInBatch, firstBatch, total, albedo, normalDepth);
+	Guides<1>(sc, tt, ps, samplesInBatch, firstBatch, total, albedo, normalDepth);
+}
+__global__ void __launch_bounds__(256) k_guides_maps(DScene sc, DTexTables tt, PathState ps, int samplesInBatch, bool firstBatch, int total, float4* albedo, float4* normalDepth) {
+	Guides<2>(sc, tt, ps, samplesInBatch, firstBatch, total, albedo, normalDepth);
+}
+
+// EXTENSION probe (agpt.h agpt_probe_material_maps): for each closest hit of a ray table (k_generate<false> with rays7, then the
+// closest-hit trace), the uv, the BSDF frame and the material record of k_shade_b<..., 2>, through the calls that kernel makes.
+// out32 per ray: prim (-1: miss), u, v, ng3, ns3, ss3, ts3, T3, B3 (dp/du, dp/dv), roughness, metallic, lobes, diffuse_r3, spec_r03.
+__global__ void __launch_bounds__(256) k_probe_material_maps(DScene sc, DTexTables tt, PathState ps, int n, float* out32) {
+	const int i = blockIdx.x * blockDim.x + threadIdx.x;
+	if (i >= n) return;
+	float* o = out32 + 32 * (size_t)i;
+	for (int k = 0; k < 32; k++) o[k] = 0.f;
+	o[0] = -1.f;
+	const float4 h = ps.hitA[i];
+	const int hitPrim = __float_as_int(h.w);
+	AGPT_CHECK(hitPrim < sc.n_prims, AGPT_DBG_PRIM, hitPrim);
+	if (hitPrim < 0) return;
+	const float4 o4 = ps.rayO[i], d4 = ps.rayD[i];
+	const float3 O = f3(o4.x, o4.y, o4.z), D = f3(d4.x, d4.y, d4.z);
+	const agpt_prim prim = sc.prims[hitPrim];
+	DSurface si;
+	float2 uv = make_float2(0.f, 0.f);
+	float3 dpdu = f3(0.f), dpdv = f3(0.f);
+	if (prim.type == AGPT_PRIM_SPHERE) SphereSurface(sc.spheres[prim.payload], O, D, h.x, si, &uv, &dpdu, &dpdv);
+	else if (prim.type == AGPT_PRIM_PLANE) PlaneSurface(O, D, h.x, si);
+	else if (prim.type == AGPT_PRIM_INSTANCE) {
+		const agpt_instance& in = sc.instances[prim.payload];
+		TriangleSurface(sc.meshes[in.mesh], ps.hitSlot[i], O, D, h.x, h.y, h.z, si, &in, &uv, &dpdu, &dpdv);
+	}
+	else TriangleSurface(sc.meshes[prim.payload], ps.hitSlot[i], O, D, h.x, h.y, h.z, si, nullptr, &uv, &dpdu, &dpdv);
+	if (prim.type == AGPT_PRIM_PLANE) { uv = PlaneUV(sc.planes[prim.payload], si.p); dpdu = f3(1.f, 0.f, 0.f); dpdv = f3(0.f, 0.f, 1.f); }
+	agpt_material hm = sc.mats[0];
+	if (prim.material >= 0) hm = HitMaps(tt, prim.material, sc.mats[prim.material], uv, dpdu, dpdv, si);
+	const DBSDF b = MakeBSDF(si, &hm);
+	const float3 rows[6] = { b.ng, b.ns, b.ss, b.ts, dpdu, dpdv };
+	o[0] = (float)hitPrim; o[1] = uv.x; o[2] = uv.y;
+	for (int k = 0; k < 6; k++) { o[3 + 3 * k] = rows[k].x; o[4 + 3 * k] = rows[k].y; o[5 + 3 * k] = rows[k].z; }
+	o[21] = hm.roughness; o[22] = hm.metallic; o[23] = (float)hm.lobes;
+	for (int k = 0; k < 3; k++) { o[24 + k] = hm.diffuse_r[k]; o[27 + k] = hm.spec_r0[k]; }
 }
 
 #define AGPT_DENOISE_ALBEDO_EPS 0.01f

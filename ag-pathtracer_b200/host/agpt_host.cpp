@@ -29,7 +29,7 @@ static int UploadFlat(const FlatScene& flat, const Camera& camera, agpt_ctx* ctx
 	if ((rc = agpt_upload_envmap(ctx, flat.envmap.width > 0 ? &flat.envmap : nullptr))) return rc;
 	if ((rc = agpt_upload_instances(ctx, flat.instances.data(), (int)flat.instances.size()))) return rc;
 	if ((rc = agpt_upload_primitives(ctx, flat.prims.data(), (int)flat.prims.size()))) return rc;
-	if ((rc = agpt_upload_textures(ctx, flat.textures.data(), (int)flat.textures.size(), flat.materialTexture.data(), (int)flat.materialTexture.size()))) return rc;
+	if ((rc = agpt_upload_material_textures(ctx, flat.textures.data(), (int)flat.textures.size(), flat.materialTextures.data(), (int)flat.materialTextures.size()))) return rc;
 	agpt_camera cam = camera.Export();
 	return agpt_set_camera(ctx, &cam);
 }
@@ -99,6 +99,7 @@ int agpt_host_scene_tables(agpt_host_scene* s, agpt_scene_tables* out) {
 		out->instances = f.instances.data(); out->n_instances = (int)f.instances.size();
 		out->textures = f.textures.empty() ? nullptr : f.textures.data(); out->material_texture = f.materialTexture.empty() ? nullptr : f.materialTexture.data();
 		out->n_textures = (int)f.textures.size(); out->n_material_texture = (int)f.materialTexture.size();
+		out->material_textures = f.materialTextures.empty() ? nullptr : f.materialTextures.data(); out->n_material_textures = (int)f.materialTextures.size();
 	)
 	return AGPT_OK;
 }

@@ -58,7 +58,7 @@ public:
 			Check(agpt_upload_envmap(ctx, flat->envmap.width > 0 ? &flat->envmap : nullptr));
 			Check(agpt_upload_instances(ctx, flat->instances.data(), (int)flat->instances.size()));
 			Check(agpt_upload_primitives(ctx, flat->prims.data(), (int)flat->prims.size()));
-			Check(agpt_upload_textures(ctx, flat->textures.data(), (int)flat->textures.size(), flat->materialTexture.data(), (int)flat->materialTexture.size()));
+			Check(agpt_upload_material_textures(ctx, flat->textures.data(), (int)flat->textures.size(), flat->materialTextures.data(), (int)flat->materialTextures.size()));
 		}
 		uploaded = scene.Fingerprint();
 	}

@@ -12,17 +12,28 @@
 #include "agpt.h"
 #include "texture.h"
 
+// EXTENSION: a material's image bindings (include/agpt.h agpt_material_textures), with the images as pointers
+struct MaterialMaps {
+	const ImageTexture* base = nullptr;
+	const ImageTexture* roughnessMetallic = nullptr;   // G = roughness, B = metallic
+	const ImageTexture* normal = nullptr;              // tangent-space normal map
+	float normalScale = 1.f;
+	float3 color = float3(0.f);                        // the base colour, used when base is null and roughnessMetallic is not
+};
+
 class Material {
 public:
 	virtual ~Material() {}
 	virtual agpt_material Export() const = 0;
 	virtual const ImageTexture* BaseColorTexture() const { return nullptr; }   // extension: DisneyMaterial with an image
+	virtual MaterialMaps Maps() const { MaterialMaps m; m.base = BaseColorTexture(); return m; }   // extension: all its images
 };
 
 #define AGPT_HAS_IMAGE_TEXTURES 1      // extension: DisneyMaterial(ImageTexture, roughness, metallic)
+#define AGPT_HAS_MATERIAL_MAPS 1       // extension: DisneyMaterial::SetRoughnessMetallicMap / SetNormalMap
 class DisneyMaterial : public Material {
 public:
-	DisneyMaterial(const float3& color, float roughness, float metallic) {
+	DisneyMaterial(const float3& color, float roughness, float metallic) : color(color) {
 		memset(&rec, 0, sizeof(rec));
 		rec.type = AGPT_MAT_DISNEY;
 		rec.eta = 1.5f;
@@ -52,6 +63,17 @@ public:
 		: DisneyMaterial(float3(1.f), roughness, metallic) { this->texture = std::move(texture); }
 	agpt_material Export() const override { return rec; }
 	const ImageTexture* BaseColorTexture() const override { return texture.get(); }
+	// EXTENSION (include/agpt.h agpt_upload_material_textures): a roughness-metallic map (G scales the roughness, B the metallic
+	// of this material per hit) and a tangent-space normal map.  The colour the material was made with is kept: it is the base
+	// colour of a material with maps and without a base-colour image.
+	void SetRoughnessMetallicMap(std::shared_ptr<ImageTexture> map) { roughnessMetallic = std::move(map); }
+	void SetNormalMap(std::shared_ptr<ImageTexture> map, float scale = 1.f) { normal = std::move(map); normalScale = scale; }
+	MaterialMaps Maps() const override {
+		MaterialMaps m;
+		m.base = texture.get(); m.roughnessMetallic = roughnessMetallic.get(); m.normal = normal.get();
+		m.normalScale = normalScale; m.color = color;
+		return m;
+	}
 	static std::shared_ptr<DisneyMaterial> Make(const float3& color, float roughness, float metallic) {
 		return std::make_shared<DisneyMaterial>(color, roughness, metallic);
 	}
@@ -61,6 +83,9 @@ public:
 private:
 	agpt_material rec;
 	std::shared_ptr<ImageTexture> texture;
+	float3 color;
+	std::shared_ptr<ImageTexture> roughnessMetallic, normal;
+	float normalScale = 1.f;
 };
 
 class MirrorMaterial : public Material {

@@ -67,6 +67,8 @@ struct FlatScene {
 	agpt_envmap envmap = { 0, 0, nullptr, nullptr, nullptr, 0.f };   // borrowed from the scene's InfiniteAreaLight
 	std::vector<agpt_texture> textures;        // extension: base-colour images, texels borrowed from the materials
 	std::vector<int32_t> materialTexture;      // per material: index into textures or -1 (empty when no material has one)
+	std::vector<agpt_material_textures> materialTextures;   // extension: per material, all its image bindings (empty as above)
+	bool HasMaps() const { for (auto& b : materialTextures) if (b.roughness_metallic >= 0 || b.normal >= 0) return true; return false; }
 	uint64_t Bytes() const {
 		uint64_t b = prims.size() * sizeof(agpt_prim) + spheres.size() * sizeof(agpt_sphere) + planes.size() * sizeof(agpt_plane)
 			+ materials.size() * sizeof(agpt_material) + lights.size() * sizeof(agpt_light);
@@ -74,6 +76,7 @@ struct FlatScene {
 		for (auto& m : meshes) b += (uint64_t)m.n_nodes * 32 + (uint64_t)m.n_tris * (48 + 4 + (m.tri_normals ? 48 : 0) + (m.tri_uvs ? 24 : 0));
 		for (auto& t : textures) b += (uint64_t)t.width * t.height * 16 + 16;   // float4 texels and a descriptor on the device
 		b += materialTexture.size() * 4;
+		if (HasMaps()) b += materialTextures.size() * 32;                      // the map binding table
 		return b;
 	}
 };
@@ -135,13 +138,19 @@ public:
 				if (it == matIndex.end()) {
 					it = matIndex.emplace(m, (int)flat->materials.size()).first;
 					flat->materials.push_back(m->Export());
-					int tex = -1;
-					if (const ImageTexture* t = m->BaseColorTexture()) {
+					auto index = [&](const ImageTexture* t) {
+						if (!t) return -1;
 						auto ti = texIndex.find(t);
 						if (ti == texIndex.end()) { ti = texIndex.emplace(t, (int)flat->textures.size()).first; flat->textures.push_back(t->Export()); }
-						tex = ti->second;
-					}
-					flat->materialTexture.push_back(tex);
+						return ti->second;
+					};
+					const MaterialMaps mm = m->Maps();
+					agpt_material_textures b;
+					b.base = index(mm.base); b.roughness_metallic = index(mm.roughnessMetallic); b.normal = index(mm.normal);
+					b.normal_scale = mm.normalScale;
+					b.color[0] = mm.color.x; b.color[1] = mm.color.y; b.color[2] = mm.color.z;
+					flat->materialTexture.push_back(b.base);
+					flat->materialTextures.push_back(b);
 				}
 				row.material = it->second;
 			}
@@ -172,7 +181,7 @@ public:
 			}
 			flat->prims.push_back(row);
 		}
-		if (flat->textures.empty()) flat->materialTexture.clear();
+		if (flat->textures.empty()) { flat->materialTexture.clear(); flat->materialTextures.clear(); }
 		for (auto& l : lights) {
 			agpt_light rec;
 			memset(&rec, 0, sizeof(rec));

@@ -45,6 +45,7 @@ inline ConfigDefaults Defaults(int config) {
 	case 10: return { 1920, 1080, 64, 16, 0, "cfg10_ext_cfg5_rough_glass_rr_by_bounce" };
 	case 11: return { 1920, 1080, 64, 16, 4, "cfg11_ext_cfg5_sampled_panel_plane_and_mesh_lights" };
 	case 12: return { 480, 270, 16, 8, 0, "cfg12_ext_procedural_image_textures" };
+	case 13: return { 480, 270, 16, 8, 0, "cfg13_ext_procedural_roughness_metallic_and_normal_maps" };
 	default: return { 0, 0, 0, 0, 0, "unknown" };
 	}
 }
@@ -628,6 +629,89 @@ inline void BuildConfig12(Scene* scene) {
 }
 #endif
 
+#ifdef AGPT_HAS_MATERIAL_MAPS
+// cfg 13 (EXTENSION, host mirror only): procedural roughness-metallic and normal maps (include/agpt.h
+// agpt_upload_material_textures), laid out so every shape's tangent frame and every rule of the maps is used:
+// - a floor plane, colour-only material, with a roughness / metallic checker (metallic 0 and 1 tiles: the lobe set changes from
+//   hit to hit) and the normal map of an analytic height field;
+// - a sphere with a base-colour image, a roughness-metallic map and a bumpy normal map (its -z pole faces the camera);
+// - a sphere whose normal map mixes flat texels, tilted ones and texels with z < 0.5 (the rules that leave a surface as it is);
+// - an 8 x 8 quad grid with per-vertex uvs and interpolated normals, placed plainly, as a rotated, scaled instance and as a
+//   sheared one;
+// level 2 adds a rough glass sphere, so the instantiation that carries everything runs.
+inline std::shared_ptr<ImageTexture> HeightFieldNormals(int W, int H, float amplitude, int waves) {
+	std::vector<float> rgb(3 * (size_t)W * H);
+	for (int y = 0; y < H; y++)
+		for (int x = 0; x < W; x++) {
+			const double u = (x + .5) / W, v = (y + .5) / H, k = 2 * 3.14159265358979 * waves;
+			// h = amplitude * sin(k u) sin(k v); tangent-space normal = normalize(-dh/du, -dh/dv, 1), stored as n / 2 + 1/2
+			const double du = amplitude * k * std::cos(k * u) * std::sin(k * v), dv = amplitude * k * std::sin(k * u) * std::cos(k * v);
+			const double l = std::sqrt(du * du + dv * dv + 1);
+			float* p = &rgb[3 * ((size_t)y * W + x)];
+			p[0] = (float)(-du / l * .5 + .5); p[1] = (float)(-dv / l * .5 + .5); p[2] = (float)(1 / l * .5 + .5);
+		}
+	return ImageTexture::Make(W, H, std::move(rgb));
+}
+inline std::shared_ptr<ImageTexture> RoughnessMetallicChecker(int W, int H, int cells) {
+	std::vector<float> rgb(3 * (size_t)W * H);
+	for (int y = 0; y < H; y++)
+		for (int x = 0; x < W; x++) {
+			const int cx = x * cells / W, cy = y * cells / H;
+			float* p = &rgb[3 * ((size_t)y * W + x)];
+			p[0] = .5f;                                            // unused
+			p[1] = ((cx + 2 * cy) % 3 == 0) ? .25f : ((cx + 2 * cy) % 3 == 1) ? .6f : 1.f;   // roughness factor
+			p[2] = ((cx + cy) & 1) ? 1.f : 0.f;                   // metallic 0 / 1 tiles
+		}
+	return ImageTexture::Make(W, H, std::move(rgb));
+}
+inline std::shared_ptr<ImageTexture> MixedNormals(int W, int H) {
+	std::vector<float> rgb(3 * (size_t)W * H);
+	for (int y = 0; y < H; y++)
+		for (int x = 0; x < W; x++) {
+			float* p = &rgb[3 * ((size_t)y * W + x)];
+			const int kind = (x / 4 + y / 4) % 4;
+			if (kind == 0) { p[0] = .5f; p[1] = .5f; p[2] = 1.f; }         // flat
+			else if (kind == 1) { p[0] = .8f; p[1] = .4f; p[2] = .85f; }   // tilted
+			else if (kind == 2) { p[0] = .6f; p[1] = .9f; p[2] = .2f; }    // z < 0.5: below the surface
+			else { p[0] = .5f; p[1] = .5f; p[2] = .3f; }                   // z < 0.5 and no tilt
+		}
+	return ImageTexture::Make(W, H, std::move(rgb));
+}
+inline void BuildConfig13(Scene* scene, int level) {
+	auto floorMat = DisneyMaterial::Make(float3(.7f, .62f, .5f), .9f, 1.f);
+	floorMat->SetRoughnessMetallicMap(RoughnessMetallicChecker(64, 64, 8));
+	floorMat->SetNormalMap(HeightFieldNormals(256, 256, .02f, 6), 1.f);
+	scene->primitives.push_back(std::make_shared<Plane>(float3(0, -1, 0), float2(8, 8), floorMat));
+	auto bumps = HeightFieldNormals(64, 32, .01f, 4);
+	auto ballMat = DisneyMaterial::Make(ProceduralTexture(37, 23, 1), .6f, .8f);
+	ballMat->SetRoughnessMetallicMap(RoughnessMetallicChecker(16, 16, 4));
+	ballMat->SetNormalMap(bumps, 1.5f);
+	scene->primitives.push_back(std::make_shared<Sphere>(float3(-2.2f, 0, 0), 1.f, ballMat));
+	auto mixedMat = DisneyMaterial::Make(float3(.25f, .5f, .75f), .4f, 0.f);
+	mixedMat->SetNormalMap(MixedNormals(32, 16), .8f);
+	scene->primitives.push_back(std::make_shared<Sphere>(float3(.3f, 0, .6f), 1.f, mixedMat));
+	auto gridMat = DisneyMaterial::Make(float3(.8f, .3f, .2f), .7f, .5f);
+	gridMat->SetRoughnessMetallicMap(RoughnessMetallicChecker(8, 8, 2));
+	gridMat->SetNormalMap(bumps, 1.f);
+	scene->primitives.push_back(MakeQuadGrid(8, 2.f, float3(-1.2f, 1.8f, 3.f), gridMat));
+	auto placed = std::make_shared<BVHTriMesh>(MakeQuadGrid(8, 2.f, float3(0.f), gridMat), gridMat, 1);
+	scene->primitives.push_back(std::make_shared<Instance>(placed, mat4::Translate(1.6f, 1.7f, 3.2f) * mat4::RotateY(-.5f) * mat4::Scale(1.3f), gridMat));
+	mat4 shear;                                    // x += .35 y, z += .2 x: a sheared placement of the same grid
+	shear.cell[1] = .35f; shear.cell[8] = .2f;
+	scene->primitives.push_back(std::make_shared<Instance>(placed, mat4::Translate(-3.6f, 2.0f, 3.6f) * shear, gridMat));
+	if (level >= 2)
+		scene->primitives.push_back(std::make_shared<Sphere>(float3(2.6f, -.2f, -.4f), .8f, GlassMaterial::Make(float3(1.f), float3(.9f, .95f, 1.f), .2f)));
+	scene->addAreaLight(std::make_shared<Sphere>(float3(0, 8, -4), .5f, nullptr), WarmWhite(120));
+	scene->lights.push_back(std::make_shared<UniformInfiniteLight>(float3(.15f, .17f, .2f)));
+	scene->camera.lookfrom = float3(0, 2.2f, -8.5f);
+	scene->camera.lookat = float3(0, .4f, 0);
+	scene->camera.vup = float3(0, 1, 0);
+	scene->camera.aspect_ratio = 16.f / 9.f;
+	scene->camera.vfov = 40;
+	scene->camera.aperture = 0;
+}
+#endif
+
 // level <= 0 selects the BASELINE.json size of each configuration.
 inline bool BuildConfig(Scene* scene, int config, int level) {
 	switch (config) {
@@ -650,6 +734,9 @@ inline bool BuildConfig(Scene* scene, int config, int level) {
 #endif
 #ifdef AGPT_HAS_IMAGE_TEXTURES
 	case 12: BuildConfig12(scene); return true;
+#endif
+#ifdef AGPT_HAS_MATERIAL_MAPS
+	case 13: BuildConfig13(scene, level > 0 ? level : 1); return true;
 #endif
 	default: return false;
 	}

@@ -291,6 +291,52 @@ typedef struct agpt_texture {
 } agpt_texture;
 int agpt_upload_textures(agpt_ctx* ctx, const agpt_texture* textures, int n_textures, const int32_t* material_texture, int n_materials);
 
+/* ---- roughness-metallic and normal maps on Disney materials (EXTENSION, beside the base-colour texture above) ----------
+ * bindings[i] binds material i's maps, each an index into `textures` or -1.  agpt_upload_textures(t, n, material_texture, m)
+ * is this call with only `base` set (roughness_metallic = normal = -1, normal_scale = 1, color = 0): one upload path, the same
+ * refusals.  Every map is read with the uv and the lookup of agpt_upload_textures steps 1-2.  At a hit on material i, float32
+ * with every operation rounded on its own:
+ *   1. per-hit material.  roughness_metallic < 0: the material of agpt_upload_textures step 3 (record, or record with the base
+ *      texture's colours).  Otherwise, with c the looked-up roughness-metallic texel and C the base texture's value when
+ *      base >= 0, else `color`:
+ *        r = roughness * clamp(c.y, 0, 1), k = metallic * clamp(c.z, 0, 1)  (clamp(x, lo, hi) = x < lo ? lo : x > hi ? hi : x;
+ *        the record's roughness and metallic act as glTF factors; c.x is unused), then DisneyMaterial's constructor arithmetic
+ *        (host/material.h) on (C, r, k): dw = (1 - k) * (1 - 0); lobes = (dw > 0 ? DIFFUSE | RETRO : 0) | MICROFACET;
+ *        diffuse_r = dw > 0 ? dw * C : 0; alpha_x = alpha_y = max(.001, max(.001, r * r)); roughness = r; metallic = k;
+ *        spec_r0 = Lerp(k, r0, C), r0 = ((eta - 1) * (eta - 1)) / ((eta + 1) * (eta + 1)).  The lobe set, and with it the lobe
+ *        count and the lobe choice of Sample_f, can change from hit to hit.  A map of texels (x, 1, 1) with `color` equal to the
+ *        material's own colour gives back its record bit for bit.
+ *   2. normal map (normal >= 0), applied to the surface before the BSDF frame is built; emission, the light choice and the
+ *      geometric normal (and with it every ray offset and Pdf_Li test) are unchanged, and whatever reads shading.n after this
+ *      step (the cosine factors, UniformInfiniteLight's hemisphere) reads the mapped one.  c = the looked-up texel (linear, no sRGB decode; +y points along increasing v), s =
+ *      normal_scale: n_ts = (s * (2 * c.x - 1), s * (2 * c.y - 1), 2 * c.z - 1).  T = dp/du and B = dp/dv of the texture's uv:
+ *        - sphere: dpdu = (-2pi * pHit.y, 2pi * pHit.x, 0) and dpdv = pi * (pHit.z * cosPhi, pHit.z * sinPhi, -r * sin(theta))
+ *          of Sphere's SurfaceInteraction, before its swap (the swapped pair is what shading.dpdu holds);
+ *        - plane: T = (1, 0, 0), B = (0, 0, 1);
+ *        - triangle: dpdu, dpdv of TriangleDerivatives (trianglemesh.cpp:59-80), from world-space vertices for instances.
+ *      N = shading.n as the shape produces it (interpolated normals included).  Then
+ *        T' = T - N * dot(N, T); if dot(T', T') == 0 the surface is left as it is; T' = normalize(T');
+ *        B' = cross(N, T'), negated if dot(B', B) < 0;  n = (n_ts.x * T' + n_ts.y * B') + n_ts.z * N;
+ *        if !(dot(n, N) > 0) the surface is left as it is; n = normalize(n);
+ *        shading.n = n, shading.dpdu = T' - n * dot(n, T')   (the BSDF frame: ns = n, ss = normalize(shading.dpdu), ts = cross)
+ *      A texel with n_ts.x == 0 && n_ts.y == 0 && n_ts.z > 0 (flat; normal_scale = 0 included) leaves the surface bit for bit.
+ *   3. agpt_render_guides: the normal guide is the mapped shading.n (flipped toward the camera as for every hit), the albedo
+ *      the per-hit diffuse_r + spec_r0 (then clamped).
+ * No random number is drawn: every path's draws stay where they were.  Refused with AGPT_ERR_INVALID, leaving the resident
+ * textures as they were: everything agpt_upload_textures refuses, an index outside [-1, n_textures), a normal_scale or color
+ * that is not finite.  Like every upload it makes the guides stale and drops the saved reprojection view.  At render time
+ * (with any map bound) n_materials must equal the resident material count and every material with a map must be
+ * AGPT_MAT_DISNEY, else AGPT_ERR_INVALID.  statements/agpt_material_maps_oracle.cpp states the same on the CPU. */
+typedef struct agpt_material_textures {
+	int32_t base;                /* base-colour texture or -1 (what agpt_upload_textures binds) */
+	int32_t roughness_metallic;  /* texture or -1: G = roughness, B = metallic (glTF layout); R unused */
+	int32_t normal;              /* tangent-space normal map or -1 */
+	float normal_scale;          /* glTF normalTexture.scale; finite */
+	float color[3];              /* the material's base colour, used when base < 0 and roughness_metallic >= 0 */
+} agpt_material_textures;
+int agpt_upload_material_textures(agpt_ctx* ctx, const agpt_texture* textures, int n_textures,
+                                  const agpt_material_textures* bindings, int n_materials);
+
 int agpt_set_camera(agpt_ctx* ctx, const agpt_camera* camera);          /* Camera, camera.h:38-56 */
 int agpt_set_film(agpt_ctx* ctx, int width, int height);                /* Accumulator(w,h), myapp.h:10-13 */
 int agpt_scene_bytes(agpt_ctx* ctx, uint64_t* out);                     /* resident scene bytes in HBM */
@@ -564,6 +610,12 @@ int agpt_probe_sphere_sample(agpt_ctx* ctx, int n, const float* in9, float* out8
  * plane or mesh (agpt_light.flags): in8 = ref point3 u2 query direction3; out8 = sampled point3, its solid-angle pdf,
  * Pdf_Li(ref, query direction), light normal3 at the sampled point. */
 int agpt_probe_light_sample(agpt_ctx* ctx, int light, int n, const float* in8, float* out8);
+/* EXTENSION (agpt_upload_material_textures): the closest hit of each ray of rays7 (O, D normalised like agpt_trace_rays, tmax)
+ * on the resident scene, shaded as the roughness-metallic / normal-map shade kernel shades it.  out32 per ray: prim (-1: miss,
+ * the rest 0), u, v, ng3, ns3, ss3, ts3 (the BSDF frame after the normal map), T3, B3 (dp/du, dp/dv of the uv), roughness,
+ * metallic, lobes, diffuse_r3, spec_r03 (the hit's material record; the first record for a null material).  AGPT_ERR_STATE
+ * unless some material has a roughness-metallic or normal map. */
+int agpt_probe_material_maps(agpt_ctx* ctx, int n, const float* rays7, float* out32);
 /* First k floats of the RNG stream of (pixel_index, sample) (SURVEY 8a row 3). */
 int agpt_probe_stream(agpt_ctx* ctx, uint32_t pixel_index, uint32_t sample, int k, float* out);
 

@@ -25,7 +25,7 @@ typedef struct agpt_host_tracer agpt_host_tracer;
 const char* agpt_host_last_error(void);
 
 /* config 1..5 = BASELINE.json configs[0..4]; 6 and 8 = test-only corner-case scenes, 7 = the reference default scene;
- * 9..12 = extension scenes of the host mirror (12: procedural image textures);
+ * 9..13 = extension scenes of the host mirror (12: procedural image textures; 13: roughness-metallic and normal maps);
  * level <= 0 picks the configuration's own icosphere subdivision level. */
 int agpt_host_scene_create(int config, int level, agpt_host_scene** out);
 int agpt_host_scene_destroy(agpt_host_scene* scene);
@@ -51,6 +51,8 @@ typedef struct agpt_scene_tables {
 	const agpt_texture* textures;                          /* extension: base-colour images (agpt_upload_textures) */
 	const int32_t* material_texture;                       /* per material: texture index or -1; NULL when no material has one */
 	int n_textures, n_material_texture;
+	const agpt_material_textures* material_textures;       /* extension: per material, all its image bindings; NULL as above */
+	int n_material_textures;
 } agpt_scene_tables;
 int agpt_host_scene_tables(agpt_host_scene* scene, agpt_scene_tables* out);
 
