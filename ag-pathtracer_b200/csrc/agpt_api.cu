@@ -6,6 +6,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <memory>
 #include <string>
 #include <thread>
 #include <utility>
@@ -24,10 +25,19 @@ static int Fail(int code, const std::string& msg) { g_error = msg; return code; 
 	return Fail(AGPT_ERR_CUDA, std::string(#call) + ": " + cudaGetErrorString(e_)); } while (0)
 #define NEED(cond, code, msg) do { if (!(cond)) return Fail(code, msg); } while (0)
 
+// One device allocation and its only owner: freed when the buffer goes out of scope or is assigned another by a move.
 template <typename T>
 struct DevBuf {
 	T* p = nullptr;
 	size_t n = 0;
+	DevBuf() = default;
+	DevBuf(DevBuf&& o) noexcept : p(std::exchange(o.p, nullptr)), n(std::exchange(o.n, 0)) {}
+	DevBuf& operator=(DevBuf&& o) noexcept {
+		if (this != &o) { Free(); p = std::exchange(o.p, nullptr); n = std::exchange(o.n, 0); }
+		return *this;
+	}
+	DevBuf(const DevBuf&) = delete; DevBuf& operator=(const DevBuf&) = delete;     // one owner per allocation
+	~DevBuf() { Free(); }
 	cudaError_t Alloc(size_t count) {
 		Free();
 		if (count == 0) return cudaSuccess;
@@ -48,8 +58,20 @@ struct MeshStore {
 	DevBuf<float4> nodes, tris, normals;
 	DevBuf<float2> uvs;
 	DevBuf<int> ids;
-	void Free() { nodes.Free(); tris.Free(); normals.Free(); uvs.Free(); ids.Free(); }
 };
+
+// A stream, event or pinned block created by the context and released with it.
+template <typename H, auto Destroy>
+struct Owned {
+	H h{};
+	Owned() = default;
+	Owned(const Owned&) = delete;
+	Owned& operator=(const Owned&) = delete;
+	~Owned() { if (h) Destroy(h); }
+	operator H() const { return h; }
+};
+using OwnedStream = Owned<cudaStream_t, cudaStreamDestroy>;
+using OwnedEvent = Owned<cudaEvent_t, cudaEventDestroy>;
 
 #ifndef AGPT_BATCH_LOG2
 #define AGPT_BATCH_LOG2 27
@@ -62,15 +84,28 @@ struct MeshStore {
 static const size_t kMaxPathsPerBatch = (size_t)1 << AGPT_BATCH_LOG2;
 
 struct agpt_ctx {
+	// (declared before every buffer: members are destroyed in reverse order, so these outlive the buffers)
+	OwnedStream ownStream;
+	OwnedStream sideStream;              // any-hit trace of a wave runs here, beside the closest-hit trace
+	OwnedStream copyStream;              // agpt_write_accum_begin: the film upload runs here, beside the render that follows
+	OwnedEvent evUpload;
+	OwnedEvent evFork, evJoin;
+	OwnedEvent evA, evB, evC, evD;
+	OwnedEvent evRender0, evRender1;     // bracket of agpt_render (ms_render)
+	Owned<int*, cudaFreeHost> hostCounts;   // pinned ring of kRing x 3 ints
+	OwnedEvent ringEvents[8];
+	// Work still queued may use the buffers: it finishes before the members release them.  (Failures change nothing about what
+	// follows.)
+	~agpt_ctx() {
+		cudaSetDevice(device);
+		if (uploadPending) cudaStreamSynchronize(copyStream);
+		if (stream) cudaStreamSynchronize(stream);
+		for (int r = 0; r < peerWorld; r++) if (r != peerRank && peerAccum[r]) cudaIpcCloseMemHandle(peerAccum[r]);
+	}
+
 	int device = 0;
-	cudaStream_t ownStream = nullptr, stream = nullptr;
-	cudaStream_t sideStream = nullptr;   // any-hit trace of a wave runs here, beside the closest-hit trace
-	cudaStream_t copyStream = nullptr;   // agpt_write_accum_begin: the film upload runs here, beside the render that follows
-	cudaEvent_t evUpload = nullptr;
+	cudaStream_t stream = nullptr;       // ownStream or the caller's (agpt_set_stream)
 	bool uploadPending = false;          // a film upload is in flight: k_accumulate waits for it, every other film access joins it first
-	cudaEvent_t evFork = nullptr, evJoin = nullptr;
-	cudaEvent_t evA = nullptr, evB = nullptr, evC = nullptr, evD = nullptr;
-	cudaEvent_t evRender0 = nullptr, evRender1 = nullptr;      // bracket of agpt_render (ms_render)
 	int smCount = 0;
 
 	// scene tables
@@ -158,8 +193,6 @@ struct agpt_ctx {
 	DevBuf<int> survivors, survivorCount;   // paths k_shade_b works on this wave
 	DevBuf<unsigned long long> traceCounters;   // [2][8] totals (closest-hit, any-hit), then [2][AGPT_MAX_WAVE_ROWS][8] per wave (FlushCounters)
 	DevBuf<RayCounters> rayCounters;
-	int* hostCounts = nullptr;    // pinned ring of kRing x 3 ints
-	cudaEvent_t ringEvents[8] = {};
 
 	// multi-process sharding: the other ranks' accumulators, mapped through CUDA IPC (agpt_open_peer_accums)
 	float4* peerAccum[AGPT_MAX_PEERS] = {};
@@ -212,8 +245,8 @@ static int BuildSphereRuns(agpt_ctx* c) {
 		b[2] = make_float4(ctr[0], ctr[1], ctr[2], 1.0e4f * rmin * rmin - diag2);
 	}
 	// ray-bucket key: the root boxes of BVH mesh primitives that are small against the union of all of them
+	std::vector<float4> kb;
 	{
-		std::vector<float4> kb;
 		float lo[3] = { 1e30f, 1e30f, 1e30f }, hi[3] = { -1e30f, -1e30f, -1e30f };
 		std::vector<int> meshPrims;
 		for (int p = 0; p < n; p++)
@@ -229,11 +262,14 @@ static int BuildSphereRuns(agpt_ctx* c) {
 			for (int a = 0; a < 3; a++) v *= fmax((double)r.bmax[a] - r.bmin[a], 1e-30);
 			if (v <= 0.25 * all && kb.size() < 2 * 16) { kb.push_back(make_float4(r.bmin[0], r.bmin[1], r.bmin[2], r.bmax[0])); kb.push_back(make_float4(r.bmax[1], r.bmax[2], 0.f, 0.f)); }
 		}
-		CU(c->keyBoxes.Upload(kb.data(), kb.size(), c->stream));
 	}
-	CU(c->sphereRun.Upload(run.data(), (size_t)n, c->stream));
-	CU(c->sphereRunBox.Upload(box.data(), box.size(), c->stream));
+	DevBuf<float4> keyBoxes, runBox;
+	DevBuf<int> runs;
+	CU(keyBoxes.Upload(kb.data(), kb.size(), c->stream));
+	CU(runs.Upload(run.data(), (size_t)n, c->stream));
+	CU(runBox.Upload(box.data(), box.size(), c->stream));
 	CU(cudaStreamSynchronize(c->stream));
+	c->keyBoxes = std::move(keyBoxes); c->sphereRun = std::move(runs); c->sphereRunBox = std::move(runBox);
 	c->runsDirty = false;
 	return AGPT_OK;
 }
@@ -245,7 +281,7 @@ static int BuildShapeLights(agpt_ctx* c) {
 	const int nl = (int)c->hostLights.size();
 	std::vector<DShapeLight> table((size_t)nl);
 	std::vector<float> cdf;
-	c->hasShapeLights = false;
+	bool any = false;
 	for (int i = 0; i < nl; i++) {
 		DShapeLight& e = table[i];
 		e.cdfOff = 0; e.n = 0; e.area = 0.f; e.pad = 0.f;
@@ -254,11 +290,11 @@ static int BuildShapeLights(agpt_ctx* c) {
 		const agpt_prim& pr = c->hostPrims[l.prim];
 		if (pr.type == AGPT_PRIM_PLANE) {
 			e.area = 4.f * c->hostPlanes[pr.payload].half_x * c->hostPlanes[pr.payload].half_z;
-			c->hasShapeLights = true;
+			any = true;
 			continue;
 		}
 		if (pr.type != AGPT_PRIM_MESH && pr.type != AGPT_PRIM_BVH_MESH) continue;      // a sphere is sampled as a sphere anyway
-		c->hasShapeLights = true;
+		any = true;
 		const int n = (int)(c->meshStore[pr.payload].tris.n / 3);
 		if (n == 0) continue;
 		DevBuf<float> dev;
@@ -269,7 +305,6 @@ static int BuildShapeLights(agpt_ctx* c) {
 		c->stats.kernel_launches++;
 		CU(cudaMemcpyAsync(area.data(), dev.p, (size_t)n * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
 		CU(cudaStreamSynchronize(c->stream));
-		dev.Free();
 		Distribution1D d(area.data(), n);
 		if (d.funcInt == 0) continue;                       // nothing to sample (Distribution1D's uniform fallback is not used)
 		float total = 0;
@@ -277,12 +312,15 @@ static int BuildShapeLights(agpt_ctx* c) {
 		e.cdfOff = (int)cdf.size(); e.n = n; e.area = total;
 		cdf.insert(cdf.end(), d.cdf.begin(), d.cdf.end());
 	}
-	c->shapeLights.Free(); c->shapeCdf.Free();
-	if (c->hasShapeLights) {
-		CU(c->shapeLights.Upload(table.data(), table.size(), c->stream));
-		CU(c->shapeCdf.Upload(cdf.data(), cdf.size(), c->stream));
+	DevBuf<DShapeLight> lights;
+	DevBuf<float> lightCdf;
+	if (any) {
+		CU(lights.Upload(table.data(), table.size(), c->stream));
+		CU(lightCdf.Upload(cdf.data(), cdf.size(), c->stream));
 		CU(cudaStreamSynchronize(c->stream));
 	}
+	c->shapeLights = std::move(lights); c->shapeCdf = std::move(lightCdf);
+	c->hasShapeLights = any;
 	c->shapesDirty = false;
 	return AGPT_OK;
 }
@@ -313,6 +351,13 @@ static PathState MakePathState(agpt_ctx* c) {
 	p.rng = c->u32[0].p; p.flags = c->u32[1].p;
 	p.slots = (int)c->capacity;
 	return p;
+}
+
+// The queues k_generate fills for the first wave (queue set A, counts A; no bucket keys yet)
+static WaveQueues FirstWave(const agpt_ctx* c) {
+	WaveQueues q0;
+	q0.closest = c->queues[0].p; q0.shadow = c->queues[2].p; q0.active = c->queues[4].p; q0.counts = c->counts.p; q0.keys = nullptr; q0.shadowKeys = nullptr;
+	return q0;
 }
 
 static int EnsureCapacity(agpt_ctx* c, size_t paths) {
@@ -463,20 +508,20 @@ int agpt_create(int device, agpt_ctx** out) {
 			" (libagpt has no CPU path)");
 	NEED(device >= 0 && device < n, AGPT_ERR_INVALID, "device index out of range");
 	CU(cudaSetDevice(device));
-	agpt_ctx* c = new agpt_ctx();
+	std::unique_ptr<agpt_ctx> c(new agpt_ctx());
 	c->device = device;
 	memset(&c->stats, 0, sizeof(c->stats));
 	cudaDeviceProp prop;
 	CU(cudaGetDeviceProperties(&prop, device));
 	c->smCount = prop.multiProcessorCount;
-	CU(cudaStreamCreateWithFlags(&c->ownStream, cudaStreamNonBlocking));
+	CU(cudaStreamCreateWithFlags(&c->ownStream.h, cudaStreamNonBlocking));
 	c->stream = c->ownStream;
-	CU(cudaStreamCreateWithFlags(&c->sideStream, cudaStreamNonBlocking));
-	CU(cudaStreamCreateWithFlags(&c->copyStream, cudaStreamNonBlocking));
-	CU(cudaEventCreateWithFlags(&c->evUpload, cudaEventDisableTiming));
-	CU(cudaEventCreateWithFlags(&c->evFork, cudaEventDisableTiming)); CU(cudaEventCreateWithFlags(&c->evJoin, cudaEventDisableTiming));
-	CU(cudaEventCreate(&c->evA)); CU(cudaEventCreate(&c->evB)); CU(cudaEventCreate(&c->evC)); CU(cudaEventCreate(&c->evD));
-	CU(cudaEventCreate(&c->evRender0)); CU(cudaEventCreate(&c->evRender1));
+	CU(cudaStreamCreateWithFlags(&c->sideStream.h, cudaStreamNonBlocking));
+	CU(cudaStreamCreateWithFlags(&c->copyStream.h, cudaStreamNonBlocking));
+	CU(cudaEventCreateWithFlags(&c->evUpload.h, cudaEventDisableTiming));
+	CU(cudaEventCreateWithFlags(&c->evFork.h, cudaEventDisableTiming)); CU(cudaEventCreateWithFlags(&c->evJoin.h, cudaEventDisableTiming));
+	CU(cudaEventCreate(&c->evA.h)); CU(cudaEventCreate(&c->evB.h)); CU(cudaEventCreate(&c->evC.h)); CU(cudaEventCreate(&c->evD.h));
+	CU(cudaEventCreate(&c->evRender0.h)); CU(cudaEventCreate(&c->evRender1.h));
 	CU(c->counts.Alloc(6));
 	CU(c->survivorCount.Alloc(1));
 	CU(c->hist.Alloc(3 * AGPT_BUCKETS));
@@ -484,49 +529,20 @@ int agpt_create(int device, agpt_ctx** out) {
 	CU(c->rayCounters.Alloc(1));
 	CU(cudaMemset(c->traceCounters.p, 0, c->traceCounters.Bytes()));
 	CU(cudaMemset(c->rayCounters.p, 0, c->rayCounters.Bytes()));
-	CU(cudaMallocHost((void**)&c->hostCounts, 8 * 3 * sizeof(int)));
-	for (auto& e : c->ringEvents) CU(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+	CU(cudaMallocHost((void**)&c->hostCounts.h, 8 * 3 * sizeof(int)));
+	for (auto& e : c->ringEvents) CU(cudaEventCreateWithFlags(&e.h, cudaEventDisableTiming));
 	if (const char* e = getenv("AGPT_ASYNC_WAVES")) c->asyncWaves = atoi(e) != 0;
 	if (const char* e = getenv("AGPT_BATCH_LOG2")) { int b = atoi(e); if (b >= 10 && b <= 28) c->maxPathsPerBatch = (size_t)1 << b; }
 	if (const char* e = getenv("AGPT_BUCKET_CALIBRATE")) c->calibrateGrid = atoi(e) != 0;
 	if (const char* e = getenv("AGPT_MAX_SPHERE_RUN")) { int v = atoi(e); if (v >= 1) c->maxSphereRun = v; }
 	if (const char* e = getenv("AGPT_OVERLAP_ANY")) c->overlapAny = atoi(e) != 0;
 	if (const char* e = getenv("AGPT_BUCKET_RAYS")) c->bucketRays = atoi(e) != 0;
-	*out = c;
+	*out = c.release();
 	return AGPT_OK;
 }
 
 int agpt_destroy(agpt_ctx* c) {
-	JoinUpload(c);          // (an upload still in flight must not outlive its buffers; a failure here changes nothing about what follows)
-	if (!c) return AGPT_OK;
-	cudaSetDevice(c->device);
-	cudaStreamSynchronize(c->stream);
-	for (int r = 0; r < c->peerWorld; r++) if (r != c->peerRank && c->peerAccum[r]) cudaIpcCloseMemHandle(c->peerAccum[r]);
-	for (auto& m : c->meshStore) m.Free();
-	c->meshes.Free(); c->shapeLights.Free(); c->shapeCdf.Free(); c->instances.Free(); c->spheres.Free(); c->planes.Free(); c->prims.Free(); c->sphereRun.Free(); c->sphereRunBox.Free(); c->keyBoxes.Free(); c->mats.Free(); c->lights.Free(); c->texels.Free(); c->textures.Free(); c->matTex.Free(); c->matMaps.Free();
-	c->accumOwn.Free(); c->resolved.Free();
-	c->moments.Free(); c->adaptiveList.Free(); c->adaptiveCount.Free();
-	c->guideAlbedo.Free(); c->guideNormal.Free(); c->denoiseE[0].Free(); c->denoiseE[1].Free(); c->denoiseG.Free(); c->denoiseOut.Free();
-	c->viewG[0].Free(); c->viewG[1].Free(); c->reprojFilm.Free(); c->reprojMoments.Free();
-	c->envRgb.Free(); c->envFunc.Free(); c->envCdf.Free();
-	for (auto& b : c->f4) b.Free();
-	for (auto& b : c->i32) b.Free();
-	for (auto& b : c->u32) b.Free();
-	for (auto& b : c->queues) b.Free();
-	c->sortedClosest.Free(); c->keys[0].Free(); c->keys[1].Free(); c->hist.Free();
-	c->shadowKeys[0].Free(); c->shadowKeys[1].Free(); c->sortedShadow.Free();
-	c->survivors.Free(); c->survivorCount.Free();
-	c->counts.Free(); c->traceCounters.Free(); c->rayCounters.Free();
-	if (c->hostCounts) cudaFreeHost(c->hostCounts);
-	for (auto& e : c->ringEvents) if (e) cudaEventDestroy(e);
-	cudaEventDestroy(c->evA); cudaEventDestroy(c->evB); cudaEventDestroy(c->evC); cudaEventDestroy(c->evD);
-	cudaEventDestroy(c->evRender0); cudaEventDestroy(c->evRender1);
-	cudaEventDestroy(c->evFork); cudaEventDestroy(c->evJoin);
-	cudaStreamDestroy(c->sideStream);
-	cudaStreamDestroy(c->copyStream);
-	cudaEventDestroy(c->evUpload);
-	cudaStreamDestroy(c->ownStream);
-	delete c;
+	delete c;               // (null: nothing to do)
 	return AGPT_OK;
 }
 
@@ -596,16 +612,12 @@ int agpt_upload_meshes(agpt_ctx* c, const agpt_mesh_desc* meshes, int n) {
 	c->gridCalibrated = false;
 	c->stateGen++;
 	c->historyGen++;
-	// from here on a failure must not leave the device table pointing at freed buffers
-	for (auto& m : c->meshStore) m.Free();
-	c->meshStore.assign(n, MeshStore());
-	c->meshes.Free();
-	c->nMeshes = 0;
-	c->maxBvhDepth = 0;
+	// the new tables are built beside the resident ones, which a failure leaves in place
+	std::vector<MeshStore> store((size_t)n);
 	std::vector<DMesh> table(n);
 	for (int i = 0; i < n; i++) {
 		const agpt_mesh_desc& d = meshes[i];
-		MeshStore& st = c->meshStore[i];
+		MeshStore& st = store[i];
 		CU(st.nodes.Upload((const float4*)d.nodes, 2 * (size_t)d.n_nodes, c->stream));
 		CU(st.tris.Upload((const float4*)d.tri_verts, 3 * (size_t)d.n_tris, c->stream));
 		CU(st.ids.Upload(d.tri_ids, (size_t)d.n_tris, c->stream));
@@ -620,8 +632,10 @@ int agpt_upload_meshes(agpt_ctx* c, const agpt_mesh_desc* meshes, int n) {
 		m.nodes = st.nodes.p; m.tris = st.tris.p; m.ids = st.ids.p; m.normals = st.normals.p; m.uvs = st.uvs.p;
 		m.n_nodes = d.n_nodes; m.n_tris = d.n_tris;
 	}
-	CU(c->meshes.Upload(table.data(), (size_t)n, c->stream));
+	DevBuf<DMesh> dtable;
+	CU(dtable.Upload(table.data(), (size_t)n, c->stream));
 	CU(cudaStreamSynchronize(c->stream));
+	c->meshStore = std::move(store); c->meshes = std::move(dtable);
 	c->nMeshes = n;
 	c->maxBvhDepth = maxDepth;
 	c->hostRoots.assign((size_t)n, agpt_bvh_node());
@@ -641,6 +655,7 @@ int agpt_upload_meshes(agpt_ctx* c, const agpt_mesh_desc* meshes, int n) {
 	return AGPT_OK;
 }
 
+// The new table replaces the resident one, and `counter` describes it, only once its upload has completed.
 #define SIMPLE_UPLOAD(fn, T, member, counter) \
 	int fn(agpt_ctx* c, const T* rows, int n) { \
 		NEED(c != nullptr && n >= 0 && (n == 0 || rows != nullptr), AGPT_ERR_INVALID, "bad table"); \
@@ -648,8 +663,10 @@ int agpt_upload_meshes(agpt_ctx* c, const agpt_mesh_desc* meshes, int n) {
 		CU(cudaStreamSynchronize(c->stream)); \
 		c->stateGen++; \
 		c->historyGen++; \
-		CU(c->member.Upload(rows, (size_t)n, c->stream)); \
+		DevBuf<T> table; \
+		CU(table.Upload(rows, (size_t)n, c->stream)); \
 		CU(cudaStreamSynchronize(c->stream)); \
+		c->member = std::move(table); \
 		counter; \
 		return AGPT_OK; \
 	}
@@ -667,37 +684,29 @@ int agpt_upload_lights(agpt_ctx* c, const agpt_light* rows, int n) {
 	}
 	return UploadLights(c, rows, n);
 }
-int agpt_upload_primitives(agpt_ctx* c, const agpt_prim* rows, int n) {
-	NEED(c != nullptr && n >= 0 && (n == 0 || rows != nullptr), AGPT_ERR_INVALID, "bad table");
-	CU(cudaSetDevice(c->device));
-	CU(cudaStreamSynchronize(c->stream));
-	c->stateGen++;
-	c->historyGen++;
-	CU(c->prims.Upload(rows, (size_t)n, c->stream));
-	c->hostPrims.assign(rows, rows + n);
-	c->runsDirty = true;
-	c->shapesDirty = true;
-	CU(cudaStreamSynchronize(c->stream));
-	return AGPT_OK;
-}
-
+SIMPLE_UPLOAD(agpt_upload_primitives, agpt_prim, prims, c->hostPrims.assign(rows, rows + n); c->runsDirty = true; c->shapesDirty = true)
 SIMPLE_UPLOAD(agpt_upload_instances, agpt_instance, instances, c->nInstances = n; c->hostInstances.assign(rows, rows + n))
 
 int agpt_upload_envmap(agpt_ctx* c, const agpt_envmap* env) {
 	NEED(c != nullptr, AGPT_ERR_INVALID, "null context");
+	const bool clear = !env || env->width == 0;
+	NEED(clear || (env->width > 0 && env->height > 0 && env->rgb && env->func && env->cdf), AGPT_ERR_INVALID, "bad environment map");
 	CU(cudaSetDevice(c->device));
 	CU(cudaStreamSynchronize(c->stream));
-	c->envRgb.Free(); c->envFunc.Free(); c->envCdf.Free();
-	c->envW = c->envH = 0; c->envFuncInt = 0;
 	c->stateGen++;
 	c->historyGen++;
-	if (!env || env->width == 0) return AGPT_OK;
-	NEED(env->width > 0 && env->height > 0 && env->rgb && env->func && env->cdf, AGPT_ERR_INVALID, "bad environment map");
+	if (clear) {
+		c->envRgb.Free(); c->envFunc.Free(); c->envCdf.Free();
+		c->envW = c->envH = 0; c->envFuncInt = 0;
+		return AGPT_OK;
+	}
 	size_t n = (size_t)env->width * env->height;
-	CU(c->envRgb.Upload(env->rgb, 3 * n, c->stream));
-	CU(c->envFunc.Upload(env->func, n, c->stream));
-	CU(c->envCdf.Upload(env->cdf, n + 1, c->stream));
+	DevBuf<float> rgb, func, cdf;
+	CU(rgb.Upload(env->rgb, 3 * n, c->stream));
+	CU(func.Upload(env->func, n, c->stream));
+	CU(cdf.Upload(env->cdf, n + 1, c->stream));
 	CU(cudaStreamSynchronize(c->stream));
+	c->envRgb = std::move(rgb); c->envFunc = std::move(func); c->envCdf = std::move(cdf);
 	c->envW = env->width; c->envH = env->height; c->envFuncInt = env->func_int;
 	return AGPT_OK;
 }
@@ -737,22 +746,25 @@ static int UploadMaterialTextures(agpt_ctx* c, const agpt_texture* textures, int
 		for (size_t k = 0; k < n; k++) texels[off + k] = make_float4(t.rgb[3 * k], t.rgb[3 * k + 1], t.rgb[3 * k + 2], 0.f);
 		off += n;
 	}
-	c->hasTextures = false; c->hasMaps = false;
-	c->hostBindings.assign(bindings, bindings + n_materials);
+	bool hasTextures = false, hasMaps = false;
 	std::vector<int32_t> matTex((size_t)n_materials);
 	std::vector<DMatMaps> maps((size_t)n_materials);
 	for (int i = 0; i < n_materials; i++) {
 		const agpt_material_textures& b = bindings[i];
 		matTex[i] = b.base;
 		maps[i] = DMatMaps{ b.base, b.roughness_metallic, b.normal, b.normal_scale, { b.color[0], b.color[1], b.color[2] }, 0.f };
-		if (b.base >= 0 || b.roughness_metallic >= 0 || b.normal >= 0) c->hasTextures = true;
-		if (b.roughness_metallic >= 0 || b.normal >= 0) c->hasMaps = true;
+		if (b.base >= 0 || b.roughness_metallic >= 0 || b.normal >= 0) hasTextures = true;
+		if (b.roughness_metallic >= 0 || b.normal >= 0) hasMaps = true;
 	}
-	CU(c->texels.Upload(texels.data(), texels.size(), c->stream));
-	CU(c->textures.Upload(desc.data(), desc.size(), c->stream));
-	CU(c->matTex.Upload(matTex.data(), matTex.size(), c->stream));
-	CU(c->matMaps.Upload(maps.data(), c->hasMaps ? maps.size() : 0, c->stream));     // read by the TEX == 2 kernels only
+	DevBuf<float4> dTexels; DevBuf<DTexture> dTextures; DevBuf<int> dMatTex; DevBuf<DMatMaps> dMatMaps;
+	CU(dTexels.Upload(texels.data(), texels.size(), c->stream));
+	CU(dTextures.Upload(desc.data(), desc.size(), c->stream));
+	CU(dMatTex.Upload(matTex.data(), matTex.size(), c->stream));
+	CU(dMatMaps.Upload(maps.data(), hasMaps ? maps.size() : 0, c->stream));     // read by the TEX == 2 kernels only
 	CU(cudaStreamSynchronize(c->stream));
+	c->texels = std::move(dTexels); c->textures = std::move(dTextures); c->matTex = std::move(dMatTex); c->matMaps = std::move(dMatMaps);
+	c->hasTextures = hasTextures; c->hasMaps = hasMaps;
+	c->hostBindings.assign(bindings, bindings + n_materials);
 	return AGPT_OK;
 }
 int agpt_upload_textures(agpt_ctx* c, const agpt_texture* textures, int n_textures, const int32_t* material_texture, int n_materials) {
@@ -782,13 +794,15 @@ int agpt_set_camera(agpt_ctx* c, const agpt_camera* cam) {
 	return AGPT_OK;
 }
 
-// moments, pixel list and count for the current film, zeroed
-static int AllocMoments(agpt_ctx* c) {
-	const size_t wh = (size_t)c->width * c->height;
-	CU(c->moments.Alloc(wh));
-	CU(c->adaptiveList.Alloc(wh));
+// Zeroed moments and a pixel list for a film of wh pixels: they replace the resident ones once both exist
+static int AllocMoments(agpt_ctx* c, size_t wh) {
+	DevBuf<float4> moments;
+	DevBuf<int> list;
+	CU(moments.Alloc(wh));
+	CU(list.Alloc(wh));
 	if (!c->adaptiveCount.p) CU(c->adaptiveCount.Alloc(1));
-	CU(cudaMemsetAsync(c->moments.p, 0, c->moments.Bytes(), c->stream));
+	CU(cudaMemsetAsync(moments.p, 0, moments.Bytes(), c->stream));
+	c->moments = std::move(moments); c->adaptiveList = std::move(list);
 	return AGPT_OK;
 }
 
@@ -800,16 +814,20 @@ int agpt_set_film(agpt_ctx* c, int width, int height) {
 	if (width == c->width && height == c->height) return AGPT_OK;
 	c->historyGen++;
 	CU(cudaStreamSynchronize(c->stream));
-	bool own = c->accum == c->accumOwn.p;
+	const bool own = c->accum == c->accumOwn.p;
+	DevBuf<float4> film;
+	if (own) {
+		CU(film.Alloc((size_t)width * height));
+		CU(cudaMemsetAsync(film.p, 0, film.Bytes(), c->stream));
+	}
+	if (c->momentsOn) {                      // (the last step that can fail: it replaces the resident moments when it succeeds)
+		int rcode = AllocMoments(c, (size_t)width * height);
+		if (rcode != AGPT_OK) return rcode;
+	}
 	c->width = width; c->height = height;
 	if (own) {
-		CU(c->accumOwn.Alloc((size_t)width * height));
+		c->accumOwn = std::move(film);
 		c->accum = c->accumOwn.p;
-		CU(cudaMemsetAsync(c->accum, 0, c->accumOwn.Bytes(), c->stream));
-	}
-	if (c->momentsOn) {
-		int rcode = AllocMoments(c);
-		if (rcode != AGPT_OK) return rcode;
 	}
 	return AGPT_OK;
 }
@@ -1111,16 +1129,14 @@ int agpt_render(agpt_ctx* c, int first_sample, int num_samples, int sample_strid
 	if (rcode != AGPT_OK) return rcode;
 	DScene sc = MakeScene(c);
 	PathState ps = MakePathState(c);
-	WaveQueues q0;
-	q0.closest = c->queues[0].p; q0.shadow = c->queues[2].p; q0.active = c->queues[4].p; q0.counts = c->counts.p; q0.keys = nullptr; q0.shadowKeys = nullptr;
+	const WaveQueues q0 = FirstWave(c);
 	// evA/evC/evD are reused inside RunWaves when timing; the render bracket has its own pair
 	cudaEvent_t r0 = c->evRender0, r1 = c->evRender1;
 	CU(cudaEventRecord(r0, c->stream));
 	for (int done = 0; done < num_samples; done += perBatch) {
 		int ns = num_samples - done < perBatch ? num_samples - done : perBatch;
 		int n = (int)(wh * ns);
-		GenParams g;
-		memset(&g, 0, sizeof(g));
+		GenParams g{};
 		g.n = n; g.first_sample = first_sample + done * sample_stride; g.sample_stride = sample_stride; g.tiled = 1; g.samples = ns;
 		k_generate<false><<<Blocks(n, 256), 256, 0, c->stream>>>(sc, ps, q0, g);
 		CU(cudaGetLastError());
@@ -1158,8 +1174,8 @@ int agpt_set_moments(agpt_ctx* c, int enable) {
 	}
 	if (c->momentsOn) return AGPT_OK;
 	if (c->width > 0) {                      // (else agpt_set_film allocates them)
-		int rcode = AllocMoments(c);
-		if (rcode != AGPT_OK) { c->moments.Free(); c->adaptiveList.Free(); c->adaptiveCount.Free(); return rcode; }
+		int rcode = AllocMoments(c, (size_t)c->width * c->height);
+		if (rcode != AGPT_OK) return rcode;
 	}
 	c->momentsOn = true;
 	return AGPT_OK;
@@ -1241,14 +1257,12 @@ static int RenderListed(agpt_ctx* c, int count, int step, int maxSamples, int ma
 	if (rcode != AGPT_OK) return rcode;
 	DScene sc = MakeScene(c);
 	PathState ps = MakePathState(c);
-	WaveQueues q0;
-	q0.closest = c->queues[0].p; q0.shadow = c->queues[2].p; q0.active = c->queues[4].p; q0.counts = c->counts.p; q0.keys = nullptr; q0.shadowKeys = nullptr;
+	const WaveQueues q0 = FirstWave(c);
 	CU(cudaEventRecord(c->evRender0, c->stream));
 	for (int done = 0; done < count; done += (int)perBatch) {
 		const int np = count - done < (int)perBatch ? count - done : (int)perBatch;
 		const int n = np * step;
-		GenParams g;
-		memset(&g, 0, sizeof(g));
+		GenParams g{};
 		g.n = n; g.samples = step; g.list = c->adaptiveList.p; g.listBase = done; g.listCount = count; g.moments = c->moments.p; g.maxSamples = maxSamples;
 		k_generate<true><<<Blocks(n, 256), 256, 0, c->stream>>>(sc, ps, q0, g);
 		CU(cudaGetLastError());
@@ -1333,14 +1347,12 @@ int agpt_render_guides(agpt_ctx* c, int num_samples, uint32_t flags) {
 	if (c->guideAlbedo.n != wh) { CU(c->guideAlbedo.Alloc(wh)); CU(c->guideNormal.Alloc(wh)); }
 	DScene sc = MakeScene(c);
 	PathState ps = MakePathState(c);
-	WaveQueues q0;
-	q0.closest = c->queues[0].p; q0.shadow = c->queues[2].p; q0.active = c->queues[4].p; q0.counts = c->counts.p; q0.keys = nullptr; q0.shadowKeys = nullptr;
+	const WaveQueues q0 = FirstWave(c);
 	const bool count = flags & AGPT_FLAG_COUNTERS, strictBoxes = flags & AGPT_FLAG_STRICT_BOXES;
 	for (int done = 0; done < num_samples; done += perBatch) {
 		const int ns = num_samples - done < perBatch ? num_samples - done : perBatch;
 		const int n = (int)(wh * ns);
-		GenParams g;
-		memset(&g, 0, sizeof(g));
+		GenParams g{};
 		g.n = n; g.first_sample = done; g.sample_stride = 1; g.tiled = 1; g.samples = ns;
 		k_generate<false><<<Blocks(n, 256), 256, 0, c->stream>>>(sc, ps, q0, g);
 		LaunchClosest(count, strictBoxes, c->nInstances > 0, Blocks(n, AGPT_TRACE_THREADS), c->stream, sc, ps, q0.closest, q0.counts + 0, c->traceCounters.p, nullptr);
@@ -1478,7 +1490,19 @@ static int TraceTable(agpt_ctx* c, const DScene& sc, const float4* rayO, const f
 	c->stats.kernel_launches++;
 	CU(cudaMemcpyAsync(out_host, out.p, (size_t)n * sizeof(agpt_hit), cudaMemcpyDeviceToHost, c->stream));
 	CU(cudaStreamSynchronize(c->stream));
-	out.Free();
+	return AGPT_OK;
+}
+
+// A rays7 table (O, D, tmax per ray) on the device with an RNG seed per ray, the caller's or zeros; g names them.
+struct RayTable {
+	DevBuf<float> rays;
+	DevBuf<uint32_t> seeds;
+};
+static int UploadRays(agpt_ctx* c, RayTable& t, int n, const float* rays7, const uint32_t* seeds, uint32_t flags, GenParams& g) {
+	CU(t.rays.Upload(rays7, 7 * (size_t)n, c->stream));
+	if (seeds) CU(t.seeds.Upload(seeds, (size_t)n, c->stream));
+	else { CU(t.seeds.Alloc((size_t)n)); CU(cudaMemsetAsync(t.seeds.p, 0, t.seeds.Bytes(), c->stream)); }
+	g.n = n; g.rays7 = t.rays.p; g.seeds = t.seeds.p; g.raysFinal = (flags & AGPT_FLAG_RAYS_FINAL) ? 1 : 0;
 	return AGPT_OK;
 }
 
@@ -1492,10 +1516,8 @@ int agpt_trace_primary(agpt_ctx* c, int sample, uint32_t flags, agpt_hit* out_ho
 	if (rcode != AGPT_OK) return rcode;
 	DScene sc = MakeScene(c);
 	PathState ps = MakePathState(c);
-	WaveQueues q0;
-	q0.closest = c->queues[0].p; q0.shadow = c->queues[2].p; q0.active = c->queues[4].p; q0.counts = c->counts.p; q0.keys = nullptr; q0.shadowKeys = nullptr;
-	GenParams g;
-	memset(&g, 0, sizeof(g));
+	const WaveQueues q0 = FirstWave(c);
+	GenParams g{};
 	g.n = (int)wh; g.first_sample = sample; g.sample_stride = 1;
 	k_generate<false><<<Blocks(wh, 256), 256, 0, c->stream>>>(sc, ps, q0, g);
 	CU(cudaGetLastError());
@@ -1514,22 +1536,15 @@ int agpt_trace_rays(agpt_ctx* c, int64_t n, const float* rays7, int any_hit, uin
 	if (rcode != AGPT_OK) return rcode;
 	DScene sc = MakeScene(c);
 	PathState ps = MakePathState(c);
-	WaveQueues q0;
-	q0.closest = c->queues[0].p; q0.shadow = c->queues[2].p; q0.active = c->queues[4].p; q0.counts = c->counts.p; q0.keys = nullptr; q0.shadowKeys = nullptr;
-	DevBuf<float> rays;
-	DevBuf<uint32_t> seeds;
-	CU(rays.Upload(rays7, 7 * (size_t)n, c->stream));
-	CU(seeds.Alloc((size_t)n));
-	CU(cudaMemsetAsync(seeds.p, 0, seeds.Bytes(), c->stream));
-	GenParams g;
-	memset(&g, 0, sizeof(g));
-	g.n = (int)n; g.rays7 = rays.p; g.seeds = seeds.p; g.raysFinal = (flags & AGPT_FLAG_RAYS_FINAL) ? 1 : 0;
+	const WaveQueues q0 = FirstWave(c);
+	RayTable t;
+	GenParams g{};
+	rcode = UploadRays(c, t, (int)n, rays7, nullptr, flags, g);
+	if (rcode != AGPT_OK) return rcode;
 	k_generate<false><<<Blocks(n, 256), 256, 0, c->stream>>>(sc, ps, q0, g);
 	CU(cudaGetLastError());
 	c->stats.kernel_launches++;
-	rcode = TraceTable(c, sc, ps.rayO, ps.rayD, (int)n, any_hit, flags, out_host);
-	rays.Free(); seeds.Free();
-	return rcode;
+	return TraceTable(c, sc, ps.rayO, ps.rayD, (int)n, any_hit, flags, out_host);
 }
 
 static int LiGeneric(agpt_ctx* c, GenParams g, int max_depth, int rr_depth_arg, uint32_t flags, float* out_rgb) {
@@ -1538,8 +1553,7 @@ static int LiGeneric(agpt_ctx* c, GenParams g, int max_depth, int rr_depth_arg, 
 	if (rcode != AGPT_OK) return rcode;
 	DScene sc = MakeScene(c);
 	PathState ps = MakePathState(c);
-	WaveQueues q0;
-	q0.closest = c->queues[0].p; q0.shadow = c->queues[2].p; q0.active = c->queues[4].p; q0.counts = c->counts.p; q0.keys = nullptr; q0.shadowKeys = nullptr;
+	const WaveQueues q0 = FirstWave(c);
 	k_generate<false><<<Blocks(n, 256), 256, 0, c->stream>>>(sc, ps, q0, g);
 	CU(cudaGetLastError());
 	c->stats.kernel_launches++;
@@ -1562,12 +1576,9 @@ int agpt_li_pixels(agpt_ctx* c, int n, const int* xs, const int* ys, const int* 
 	CU(cudaSetDevice(c->device));
 	DevBuf<int> dx, dy, ds;
 	CU(dx.Upload(xs, n, c->stream)); CU(dy.Upload(ys, n, c->stream)); CU(ds.Upload(ss, n, c->stream));
-	GenParams g;
-	memset(&g, 0, sizeof(g));
+	GenParams g{};
 	g.n = n; g.xs = dx.p; g.ys = dy.p; g.ss = ds.p;
-	rcode = LiGeneric(c, g, max_depth, rr_depth_arg, flags, out_rgb);
-	dx.Free(); dy.Free(); ds.Free();
-	return rcode;
+	return LiGeneric(c, g, max_depth, rr_depth_arg, flags, out_rgb);
 }
 
 int agpt_li_rays(agpt_ctx* c, int n, const float* rays7, const uint32_t* rng_states, int max_depth, int rr_depth_arg, uint32_t flags, float* out_rgb) {
@@ -1576,16 +1587,11 @@ int agpt_li_rays(agpt_ctx* c, int n, const float* rays7, const uint32_t* rng_sta
 	NEED(n >= 0 && (n == 0 || (rays7 && rng_states && out_rgb)), AGPT_ERR_INVALID, "bad ray list");
 	if (n == 0) return AGPT_OK;
 	CU(cudaSetDevice(c->device));
-	DevBuf<float> rays;
-	DevBuf<uint32_t> seeds;
-	CU(rays.Upload(rays7, 7 * (size_t)n, c->stream));
-	CU(seeds.Upload(rng_states, (size_t)n, c->stream));
-	GenParams g;
-	memset(&g, 0, sizeof(g));
-	g.n = n; g.rays7 = rays.p; g.seeds = seeds.p; g.raysFinal = (flags & AGPT_FLAG_RAYS_FINAL) ? 1 : 0;
-	rcode = LiGeneric(c, g, max_depth, rr_depth_arg, flags, out_rgb);
-	rays.Free(); seeds.Free();
-	return rcode;
+	RayTable t;
+	GenParams g{};
+	rcode = UploadRays(c, t, n, rays7, rng_states, flags, g);
+	if (rcode != AGPT_OK) return rcode;
+	return LiGeneric(c, g, max_depth, rr_depth_arg, flags, out_rgb);
 }
 
 // ---- multi-GPU: sample-index sharding (SURVEY 8e) ---------------------------------------------
@@ -1932,7 +1938,6 @@ int agpt_probe_bandwidth(agpt_ctx* c, size_t bytes, int iters, float* gbs_out) {
 	float ms = 0;
 	cudaEventElapsedTime(&ms, c->evA, c->evB);
 	*gbs_out = ms > 0 ? (float)((double)n16 * 16 * iters / (ms * 1e-3) / 1e9) : 0.f;
-	buf.Free(); sink.Free();
 	return AGPT_OK;
 }
 
@@ -2057,7 +2062,6 @@ static int ProbeRun(agpt_ctx* c, const TIn* in, size_t nIn, TOut* out, size_t nO
 	c->stats.kernel_launches++;
 	CU(cudaMemcpyAsync(out, dout.p, nOut * sizeof(TOut), cudaMemcpyDeviceToHost, c->stream));
 	CU(cudaStreamSynchronize(c->stream));
-	din.Free(); dout.Free();
 	return AGPT_OK;
 }
 
@@ -2076,7 +2080,6 @@ int agpt_probe_bounds(agpt_ctx* c, int n, const float* boxes6, const float* rays
 	CU(cudaMemcpyAsync(out_hit, dh.p, n * sizeof(int), cudaMemcpyDeviceToHost, c->stream));
 	CU(cudaMemcpyAsync(out_t, dt.p, n * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
 	CU(cudaStreamSynchronize(c->stream));
-	db.Free(); dr.Free(); dt.Free(); dh.Free();
 	return AGPT_OK;
 }
 
@@ -2100,17 +2103,13 @@ int agpt_probe_material_maps(agpt_ctx* c, int n, const float* rays7, float* out3
 	if (rcode != AGPT_OK) return rcode;
 	DScene sc = MakeScene(c);
 	PathState ps = MakePathState(c);
-	WaveQueues q0;
-	q0.closest = c->queues[0].p; q0.shadow = c->queues[2].p; q0.active = c->queues[4].p; q0.counts = c->counts.p; q0.keys = nullptr; q0.shadowKeys = nullptr;
-	DevBuf<float> rays, out;
-	DevBuf<uint32_t> seeds;
-	CU(rays.Upload(rays7, 7 * (size_t)n, c->stream));
-	CU(seeds.Alloc((size_t)n));
-	CU(cudaMemsetAsync(seeds.p, 0, seeds.Bytes(), c->stream));
+	const WaveQueues q0 = FirstWave(c);
+	RayTable t;
+	GenParams g{};
+	rcode = UploadRays(c, t, n, rays7, nullptr, 0, g);
+	if (rcode != AGPT_OK) return rcode;
+	DevBuf<float> out;
 	CU(out.Alloc(32 * (size_t)n));
-	GenParams g;
-	memset(&g, 0, sizeof(g));
-	g.n = n; g.rays7 = rays.p; g.seeds = seeds.p;
 	k_generate<false><<<Blocks(n, 256), 256, 0, c->stream>>>(sc, ps, q0, g);
 	LaunchClosest(false, false, c->nInstances > 0, Blocks(n, AGPT_TRACE_THREADS), c->stream, sc, ps, q0.closest, q0.counts + 0, c->traceCounters.p, nullptr);
 	k_probe_material_maps<<<Blocks(n, 256), 256, 0, c->stream>>>(sc, MakeTexTables(c), ps, n, out.p);
@@ -2118,7 +2117,6 @@ int agpt_probe_material_maps(agpt_ctx* c, int n, const float* rays7, float* out3
 	c->stats.kernel_launches += 3;
 	CU(cudaMemcpyAsync(out32, out.p, out.Bytes(), cudaMemcpyDeviceToHost, c->stream));
 	CU(cudaStreamSynchronize(c->stream));
-	rays.Free(); seeds.Free(); out.Free();
 	return AGPT_OK;
 }
 
@@ -2157,7 +2155,6 @@ int agpt_probe_stream(agpt_ctx* c, uint32_t pixel_index, uint32_t sample, int k,
 	c->stats.kernel_launches++;
 	CU(cudaMemcpyAsync(out, d.p, k * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
 	CU(cudaStreamSynchronize(c->stream));
-	d.Free();
 	return AGPT_OK;
 }
 

@@ -256,7 +256,8 @@ int agpt_upload_primitives(agpt_ctx* ctx, const agpt_prim* prims, int n);
 int agpt_upload_instances(agpt_ctx* ctx, const agpt_instance* instances, int n);  /* EXTENSION; rows of AGPT_PRIM_INSTANCE point here */
 int agpt_upload_materials(agpt_ctx* ctx, const agpt_material* materials, int n);
 int agpt_upload_lights(agpt_ctx* ctx, const agpt_light* lights, int n);   /* refuses bad flags (see agpt_light.flags), scene unchanged */
-int agpt_upload_envmap(agpt_ctx* ctx, const agpt_envmap* env);          /* NULL clears it */
+int agpt_upload_envmap(agpt_ctx* ctx, const agpt_envmap* env);          /* NULL clears it;
+                                                                           a refused map (AGPT_ERR_INVALID) leaves the resident one */
 
 /* ---- image textures on the base colour of Disney materials (EXTENSION: the reference has one colour per material) -------
  * A texture is linear RGB float32, row-major: texel (x, y) at rgb[3 * (y * width + x) ..]; row 0 holds v in [0, 1/height).
