@@ -11,5 +11,6 @@ from .binding import (AgptError, Context, Group, HostScene, HostTracer, Material
                       lib_paths, make_material, pinned_film, set_build_options, get_build_options, RawMesh, MeshDesc, FLAG_RAYS_FINAL, FLAG_RR_BY_BOUNCE,
                       PRIM_DTYPE, SPHERE_DTYPE, PLANE_DTYPE, LIGHT_DTYPE, NODE_DTYPE, PRIM_SPHERE, PRIM_PLANE, PRIM_BVH_MESH, PRIM_MESH, PRIM_INSTANCE,
                       LIGHT_AREA, LIGHT_UNIFORM_INFINITE, LIGHT_INFINITE_AREA, LIGHT_SAMPLE_SHAPE, Adaptive, adaptive, DenoiseParams,
-                      denoise_params, ReprojectParams, reproject_params, MaterialTextures, material_textures)
+                      denoise_params, ReprojectParams, reproject_params, MaterialTextures, material_textures,
+                      AlphaMask, alpha_mask)
 from . import multigpu  # noqa: F401,E402

@@ -153,6 +153,16 @@ def material_textures(base=-1, roughness_metallic=-1, normal=-1, normal_scale=1.
     return MaterialTextures(base, roughness_metallic, normal, normal_scale, (c_float * 3)(*color))
 
 
+class AlphaMask(ctypes.Structure):      # agpt_alpha_mask
+    _fields_ = [("texture", c_int32), ("channel", c_int32), ("cutoff", c_float), ("pad", c_int32)]
+
+
+def alpha_mask(texture=-1, channel=0, cutoff=0.5):
+    """EXTENSION (agpt.h agpt_alpha_mask): one material's cutout mask, channel `channel` (0, 1, 2) of resident texture `texture`
+    (-1: no mask); the surface is there where that channel >= cutoff."""
+    return AlphaMask(texture, channel, cutoff, 0)
+
+
 def _image_rows(images, who):
     imgs = [np.ascontiguousarray(a, np.float32) for a in images]
     for a in imgs:
@@ -287,6 +297,18 @@ class Context:
                 raise AgptError("upload_material_textures: normal_scale and color must be finite")
         table = (MaterialTextures * max(len(bindings), 1))(*bindings)
         _check(core().agpt_upload_material_textures(self._h, rows if imgs else None, c_int(len(imgs)), table if bindings else None, c_int(len(bindings))))
+
+    def upload_alpha_masks(self, bindings):
+        """EXTENSION (agpt.h agpt_upload_alpha_masks): bindings[i] = material i's agpt.alpha_mask(...), naming a texture of the last
+        texture upload.  [] clears.  A texture upload clears the masks."""
+        bindings = list(bindings)
+        for b in bindings:
+            if not isinstance(b, AlphaMask):
+                raise AgptError("upload_alpha_masks: every binding must be an alpha_mask(...) row")
+            if b.texture < -1 or not 0 <= b.channel <= 2 or not np.isfinite(b.cutoff):
+                raise AgptError("upload_alpha_masks: need texture >= -1, channel in [0, 2] and a finite cutoff")
+        table = (AlphaMask * max(len(bindings), 1))(*bindings)
+        _check(core().agpt_upload_alpha_masks(self._h, table if bindings else None, c_int(len(bindings))))
 
     def set_camera(self, cam19):
         cam19 = np.ascontiguousarray(cam19, np.float32)
@@ -652,6 +674,12 @@ class HostScene:
         v = np.zeros((info["tris"], 9), np.float32)
         _check(host().agpt_host_mesh_export(self._h, c_int(prim), _fptr(v)), host_side=True)
         return v
+
+    def alpha_masks(self):
+        """EXTENSION: the flattened scene's alpha-mask rows (agpt_host_scene_alpha_masks), one per material, or [] without masks."""
+        p = POINTER(AlphaMask)(); n = c_int(0)
+        _check(host().agpt_host_scene_alpha_masks(self._h, byref(p), byref(n)), host_side=True)
+        return [AlphaMask(p[i].texture, p[i].channel, p[i].cutoff, 0) for i in range(n.value)]
 
     def material(self, prim):
         out = np.zeros(20, np.float32)

@@ -140,6 +140,9 @@ struct agpt_ctx {
 	std::vector<agpt_material_textures> hostBindings;
 	bool hasTextures = false;     // some material has a texture: shade and guides run the textured instantiations
 	bool hasMaps = false;         // some material has a roughness-metallic or normal map: the TEX == 2 instantiations
+	DevBuf<agpt_alpha_mask> masks;            // alpha masks (extension, agpt_upload_alpha_masks), per material
+	std::vector<agpt_alpha_mask> hostMasks;
+	bool hasMasks = false;        // some material has a mask: trace runs the MASK instantiations
 	DevBuf<agpt_light> lights;
 	DevBuf<float> envRgb, envFunc, envCdf;
 	float envFuncInt = 0;
@@ -428,6 +431,15 @@ static int CheckReady(agpt_ctx* c, bool needFilm) {
 				"a texture is bound to a material that is not AGPT_MAT_DISNEY");
 		}
 	}
+	if (c->hasMasks) {
+		// alpha masks (extension): the mask table belongs to the resident material table; masked spheres and emitters are not defined
+		NEED(c->hostMasks.size() == (size_t)c->nMats, AGPT_ERR_INVALID, "alpha masks were uploaded for a different number of materials");
+		for (const agpt_prim& p : c->hostPrims) {
+			if (p.material < 0 || c->hostMasks[p.material].texture < 0) continue;
+			NEED(p.type != AGPT_PRIM_SPHERE, AGPT_ERR_INVALID, "an alpha mask on a sphere's material");
+			NEED(p.area_light < 0, AGPT_ERR_INVALID, "an alpha mask on an emitter's material");
+		}
+	}
 	if (c->mats.p == nullptr) {
 		// a scene of null-material (emissive) shapes only is legal upstream; shade still needs a record to point idle lanes at
 		CU(cudaSetDevice(c->device));
@@ -467,20 +479,36 @@ static int JoinUpload(agpt_ctx* c) {
 	if (count) { if (fast) { if (inst) { CALL(true, true, true); } else { CALL(true, true, false); } } else { if (inst) { CALL(true, false, true); } else { CALL(true, false, false); } } } \
 	else { if (fast) { if (inst) { CALL(false, true, true); } else { CALL(false, true, false); } } else { if (inst) { CALL(false, false, true); } else { CALL(false, false, false); } } } } while (0)
 
-static void LaunchClosest(bool count, bool strictBoxes, bool inst, int blocks, cudaStream_t st, const DScene& sc, const PathState& ps, const int* queue, const int* n, unsigned long long* cnt, unsigned long long* row) {
+// mk != nullptr (some alpha mask is bound, extension): the MASK instantiations, which take INST on
+#define AGPT_DISPATCH_MASKED(count, fast, CALLM) do { \
+	if (count) { if (fast) { CALLM(true, true); } else { CALLM(true, false); } } else { if (fast) { CALLM(false, true); } else { CALLM(false, false); } } } while (0)
+
+static void LaunchClosest(bool count, bool strictBoxes, bool inst, int blocks, cudaStream_t st, const DScene& sc, const PathState& ps, const int* queue, const int* n, unsigned long long* cnt, unsigned long long* row,
+		const DMaskTables* mk) {
 #define CALL(C, F, I) k_trace_closest<C, F, I><<<blocks, AGPT_TRACE_THREADS, 0, st>>>(sc, ps, queue, n, cnt, row)
-	AGPT_DISPATCH3(count, !strictBoxes, inst, CALL);
+#define CALLM(C, F) k_trace_closest_masked<C, F><<<blocks, AGPT_TRACE_THREADS, 0, st>>>(sc, ps, queue, n, cnt, row, *mk)
+	if (mk) AGPT_DISPATCH_MASKED(count, !strictBoxes, CALLM);
+	else AGPT_DISPATCH3(count, !strictBoxes, inst, CALL);
+#undef CALLM
 #undef CALL
 }
-static void LaunchAny(bool count, bool strictBoxes, bool inst, int blocks, cudaStream_t st, const DScene& sc, const PathState& ps, const int* queue, const int* n, unsigned long long* cnt, unsigned long long* row) {
+static void LaunchAny(bool count, bool strictBoxes, bool inst, int blocks, cudaStream_t st, const DScene& sc, const PathState& ps, const int* queue, const int* n, unsigned long long* cnt, unsigned long long* row,
+		const DMaskTables* mk) {
 #define CALL(C, F, I) k_trace_any<C, F, I><<<blocks, AGPT_TRACE_THREADS, 0, st>>>(sc, ps, queue, n, cnt, row)
-	AGPT_DISPATCH3(count, !strictBoxes, inst, CALL);
+#define CALLM(C, F) k_trace_any_masked<C, F><<<blocks, AGPT_TRACE_THREADS, 0, st>>>(sc, ps, queue, n, cnt, row, *mk)
+	if (mk) AGPT_DISPATCH_MASKED(count, !strictBoxes, CALLM);
+	else AGPT_DISPATCH3(count, !strictBoxes, inst, CALL);
+#undef CALLM
 #undef CALL
 }
 template <bool ANY>
-static void LaunchTable(bool count, bool strictBoxes, bool inst, int blocks, cudaStream_t st, const DScene& sc, const float4* o, const float4* d, int n, agpt_hit* out, unsigned long long* cnt) {
+static void LaunchTable(bool count, bool strictBoxes, bool inst, int blocks, cudaStream_t st, const DScene& sc, const float4* o, const float4* d, int n, agpt_hit* out, unsigned long long* cnt,
+		const DMaskTables* mk) {
 #define CALL(C, F, I) k_trace_table<ANY, C, F, I><<<blocks, AGPT_TRACE_THREADS, 0, st>>>(sc, o, d, n, out, cnt)
-	AGPT_DISPATCH3(count, !strictBoxes, inst, CALL);
+#define CALLM(C, F) k_trace_table_masked<ANY, C, F><<<blocks, AGPT_TRACE_THREADS, 0, st>>>(sc, o, d, n, out, cnt, *mk)
+	if (mk) AGPT_DISPATCH_MASKED(count, !strictBoxes, CALLM);
+	else AGPT_DISPATCH3(count, !strictBoxes, inst, CALL);
+#undef CALLM
 #undef CALL
 }
 
@@ -765,6 +793,7 @@ static int UploadMaterialTextures(agpt_ctx* c, const agpt_texture* textures, int
 	c->texels = std::move(dTexels); c->textures = std::move(dTextures); c->matTex = std::move(dMatTex); c->matMaps = std::move(dMatMaps);
 	c->hasTextures = hasTextures; c->hasMaps = hasMaps;
 	c->hostBindings.assign(bindings, bindings + n_materials);
+	c->masks.Free(); c->hostMasks.clear(); c->hasMasks = false;     // alpha masks name textures of the old table
 	return AGPT_OK;
 }
 int agpt_upload_textures(agpt_ctx* c, const agpt_texture* textures, int n_textures, const int32_t* material_texture, int n_materials) {
@@ -783,6 +812,37 @@ static DTexTables MakeTexTables(const agpt_ctx* c) {
 	t.nTextures = (int)c->textures.n; t.nTexels = (long long)c->texels.n;
 	t.matMaps = c->matMaps.p; t.nMatMaps = (int)c->matMaps.n;
 	return t;
+}
+
+// EXTENSION (agpt.h agpt_upload_alpha_masks).  Every argument is checked before anything resident changes.
+int agpt_upload_alpha_masks(agpt_ctx* c, const agpt_alpha_mask* masks, int n_materials) {
+	NEED(c != nullptr && n_materials >= 0 && (n_materials == 0 || masks != nullptr), AGPT_ERR_INVALID, "agpt_upload_alpha_masks: bad table");
+	bool hasMasks = false;
+	for (int i = 0; i < n_materials; i++) {
+		const agpt_alpha_mask& m = masks[i];
+		NEED(m.texture >= -1 && m.texture < (int)c->textures.n, AGPT_ERR_INVALID, "agpt_upload_alpha_masks: material points outside the resident textures");
+		NEED(m.channel >= 0 && m.channel <= 2, AGPT_ERR_INVALID, "agpt_upload_alpha_masks: channel outside [0, 2]");
+		NEED(std::isfinite(m.cutoff), AGPT_ERR_INVALID, "agpt_upload_alpha_masks: cutoff not finite");
+		if (m.texture >= 0) hasMasks = true;
+	}
+	CU(cudaSetDevice(c->device));
+	CU(cudaStreamSynchronize(c->stream));
+	c->stateGen++;
+	c->historyGen++;
+	DevBuf<agpt_alpha_mask> dMasks;
+	CU(dMasks.Upload(masks, (size_t)n_materials, c->stream));
+	CU(cudaStreamSynchronize(c->stream));
+	c->masks = std::move(dMasks);
+	c->hostMasks.assign(masks, masks + n_materials);
+	c->hasMasks = hasMasks;
+	return AGPT_OK;
+}
+// the mask tables of the MASK trace instantiations in `store`, or nullptr while no mask is bound (the trace kernels without the test)
+static const DMaskTables* MaskTables(const agpt_ctx* c, DMaskTables& store) {
+	if (!c->hasMasks) return nullptr;
+	store.tt = MakeTexTables(c);
+	store.masks = c->masks.p; store.nMasks = (int)c->masks.n;
+	return &store;
 }
 
 int agpt_set_camera(agpt_ctx* c, const agpt_camera* cam) {
@@ -835,7 +895,7 @@ int agpt_set_film(agpt_ctx* c, int width, int height) {
 int agpt_scene_bytes(agpt_ctx* c, uint64_t* out) {
 	NEED(c != nullptr && out != nullptr, AGPT_ERR_INVALID, "null argument");
 	uint64_t b = c->envRgb.Bytes() + c->envFunc.Bytes() + c->envCdf.Bytes() + c->meshes.Bytes() + c->spheres.Bytes() + c->planes.Bytes() + c->prims.Bytes() + c->instances.Bytes() + c->mats.Bytes() + c->lights.Bytes()
-		+ c->shapeLights.Bytes() + c->shapeCdf.Bytes() + c->texels.Bytes() + c->textures.Bytes() + c->matTex.Bytes() + c->matMaps.Bytes();
+		+ c->shapeLights.Bytes() + c->shapeCdf.Bytes() + c->texels.Bytes() + c->textures.Bytes() + c->matTex.Bytes() + c->matMaps.Bytes() + c->masks.Bytes();
 	for (auto& m : c->meshStore) b += m.nodes.Bytes() + m.tris.Bytes() + m.normals.Bytes() + m.uvs.Bytes() + m.ids.Bytes();
 	*out = b;
 	return AGPT_OK;
@@ -1014,9 +1074,11 @@ static int RunWaves(agpt_ctx* c, const DScene& scIn, PathState& ps, int n, int m
 		const bool fork = overlap && ubClosest > 0 && ubShadow > 0;
 		if (timing) CU(cudaEventRecord(c->evA, c->stream));
 		if (fork) CU(cudaEventRecord(c->evFork, c->stream));
+		DMaskTables mkStore;
+		const DMaskTables* mk = MaskTables(c, mkStore);
 		if (ubClosest > 0) {
 			LaunchClosest(count, strictBoxes, c->nInstances > 0, Blocks(ubClosest, AGPT_TRACE_THREADS), c->stream, sc, ps, closestQueue, q[cur].counts + 0, cntClosest,
-				waveRows + (size_t)AGPT_WAVE_COUNTERS * (wave < AGPT_MAX_WAVE_ROWS ? wave : AGPT_MAX_WAVE_ROWS - 1));
+				waveRows + (size_t)AGPT_WAVE_COUNTERS * (wave < AGPT_MAX_WAVE_ROWS ? wave : AGPT_MAX_WAVE_ROWS - 1), mk);
 			c->stats.kernel_launches++; c->stats.launches_closest++;
 		}
 		if (wave == 0 && bucketing && !c->gridCalibrated && c->calibrateGrid && n >= 4096) {
@@ -1029,13 +1091,13 @@ static int RunWaves(agpt_ctx* c, const DScene& scIn, PathState& ps, int n, int m
 		if (fork) {
 			CU(cudaStreamWaitEvent(c->sideStream, c->evFork, 0));
 			LaunchAny(count, strictBoxes, c->nInstances > 0, Blocks(ubShadow, AGPT_TRACE_THREADS), c->sideStream, sc, ps, shadowQueue, q[cur].counts + 1, cntAny,
-				waveRows + (size_t)AGPT_WAVE_COUNTERS * (AGPT_MAX_WAVE_ROWS + (wave < AGPT_MAX_WAVE_ROWS ? wave : AGPT_MAX_WAVE_ROWS - 1)));
+				waveRows + (size_t)AGPT_WAVE_COUNTERS * (AGPT_MAX_WAVE_ROWS + (wave < AGPT_MAX_WAVE_ROWS ? wave : AGPT_MAX_WAVE_ROWS - 1)), mk);
 			c->stats.kernel_launches++; c->stats.launches_any++;
 			CU(cudaEventRecord(c->evJoin, c->sideStream));
 			CU(cudaStreamWaitEvent(c->stream, c->evJoin, 0));
 		} else if (ubShadow > 0) {
 			LaunchAny(count, strictBoxes, c->nInstances > 0, Blocks(ubShadow, AGPT_TRACE_THREADS), c->stream, sc, ps, shadowQueue, q[cur].counts + 1, cntAny,
-				waveRows + (size_t)AGPT_WAVE_COUNTERS * (AGPT_MAX_WAVE_ROWS + (wave < AGPT_MAX_WAVE_ROWS ? wave : AGPT_MAX_WAVE_ROWS - 1)));
+				waveRows + (size_t)AGPT_WAVE_COUNTERS * (AGPT_MAX_WAVE_ROWS + (wave < AGPT_MAX_WAVE_ROWS ? wave : AGPT_MAX_WAVE_ROWS - 1)), mk);
 			c->stats.kernel_launches++; c->stats.launches_any++;
 		}
 		CU(cudaMemsetAsync(q[cur ^ 1].counts, 0, 3 * sizeof(int), c->stream));
@@ -1355,7 +1417,8 @@ int agpt_render_guides(agpt_ctx* c, int num_samples, uint32_t flags) {
 		GenParams g{};
 		g.n = n; g.first_sample = done; g.sample_stride = 1; g.tiled = 1; g.samples = ns;
 		k_generate<false><<<Blocks(n, 256), 256, 0, c->stream>>>(sc, ps, q0, g);
-		LaunchClosest(count, strictBoxes, c->nInstances > 0, Blocks(n, AGPT_TRACE_THREADS), c->stream, sc, ps, q0.closest, q0.counts + 0, c->traceCounters.p, nullptr);
+		DMaskTables mkStore;
+		LaunchClosest(count, strictBoxes, c->nInstances > 0, Blocks(n, AGPT_TRACE_THREADS), c->stream, sc, ps, q0.closest, q0.counts + 0, c->traceCounters.p, nullptr, MaskTables(c, mkStore));
 		if (c->hasMaps) k_guides_maps<<<Blocks(wh, 256), 256, 0, c->stream>>>(sc, MakeTexTables(c), ps, ns, done == 0, done + ns == num_samples ? num_samples : 0, c->guideAlbedo.p, c->guideNormal.p);
 		else if (c->hasTextures) k_guides_tex<<<Blocks(wh, 256), 256, 0, c->stream>>>(sc, MakeTexTables(c), ps, ns, done == 0, done + ns == num_samples ? num_samples : 0, c->guideAlbedo.p, c->guideNormal.p);
 		else k_guides<<<Blocks(wh, 256), 256, 0, c->stream>>>(sc, ps, ns, done == 0, done + ns == num_samples ? num_samples : 0, c->guideAlbedo.p, c->guideNormal.p);
@@ -1484,8 +1547,10 @@ static int TraceTable(agpt_ctx* c, const DScene& sc, const float4* rayO, const f
 	CU(out.Alloc(n));
 	const bool count = flags & AGPT_FLAG_COUNTERS, strictBoxes = flags & AGPT_FLAG_STRICT_BOXES;
 	int blocks = Blocks(n, AGPT_TRACE_THREADS);
-	if (any_hit) LaunchTable<true>(count, strictBoxes, c->nInstances > 0, blocks, c->stream, sc, rayO, rayD, n, out.p, c->traceCounters.p + AGPT_WAVE_COUNTERS);
-	else LaunchTable<false>(count, strictBoxes, c->nInstances > 0, blocks, c->stream, sc, rayO, rayD, n, out.p, c->traceCounters.p);
+	DMaskTables mkStore;
+	const DMaskTables* mk = MaskTables(c, mkStore);
+	if (any_hit) LaunchTable<true>(count, strictBoxes, c->nInstances > 0, blocks, c->stream, sc, rayO, rayD, n, out.p, c->traceCounters.p + AGPT_WAVE_COUNTERS, mk);
+	else LaunchTable<false>(count, strictBoxes, c->nInstances > 0, blocks, c->stream, sc, rayO, rayD, n, out.p, c->traceCounters.p, mk);
 	CU(cudaGetLastError());
 	c->stats.kernel_launches++;
 	CU(cudaMemcpyAsync(out_host, out.p, (size_t)n * sizeof(agpt_hit), cudaMemcpyDeviceToHost, c->stream));
@@ -2111,7 +2176,8 @@ int agpt_probe_material_maps(agpt_ctx* c, int n, const float* rays7, float* out3
 	DevBuf<float> out;
 	CU(out.Alloc(32 * (size_t)n));
 	k_generate<false><<<Blocks(n, 256), 256, 0, c->stream>>>(sc, ps, q0, g);
-	LaunchClosest(false, false, c->nInstances > 0, Blocks(n, AGPT_TRACE_THREADS), c->stream, sc, ps, q0.closest, q0.counts + 0, c->traceCounters.p, nullptr);
+	DMaskTables mkStore;
+	LaunchClosest(false, false, c->nInstances > 0, Blocks(n, AGPT_TRACE_THREADS), c->stream, sc, ps, q0.closest, q0.counts + 0, c->traceCounters.p, nullptr, MaskTables(c, mkStore));
 	k_probe_material_maps<<<Blocks(n, 256), 256, 0, c->stream>>>(sc, MakeTexTables(c), ps, n, out.p);
 	CU(cudaGetLastError());
 	c->stats.kernel_launches += 3;

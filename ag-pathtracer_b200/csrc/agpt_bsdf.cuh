@@ -268,6 +268,16 @@ __device__ __forceinline__ void SphereSurface(const agpt_sphere& sp, float3 O, f
 __device__ __forceinline__ void PlaneSurface(float3 O, float3 D, float t, DSurface& s) {   // intersectable.h:128-133
 	SurfaceInit(s, O + t * D, f3(0, 0, 1), f3(1, 0, 0));
 }
+// a triangle's uvs (the mesh's, or the default (0,0), (1,0), (1,1), trianglemesh.cpp:52-56) and the uv of barycentrics b1, b2, for
+// shared by TriangleSurface and the alpha-mask test of the trace walk (agpt_upload_textures step 1).
+__device__ __forceinline__ void TriangleUVs(const DMesh& mesh, int slot, float2& uv0, float2& uv1, float2& uv2) {
+	uv0 = make_float2(0, 0); uv1 = make_float2(1, 0); uv2 = make_float2(1, 1);
+	if (mesh.uvs) { uv0 = __ldg(mesh.uvs + 3 * slot); uv1 = __ldg(mesh.uvs + 3 * slot + 1); uv2 = __ldg(mesh.uvs + 3 * slot + 2); }
+}
+__device__ __forceinline__ float2 BaryUV(float b1, float b2, float2 uv0, float2 uv1, float2 uv2) {
+	const float b0 = 1.f - b1 - b2;
+	return make_float2((b0 * uv0.x + b1 * uv1.x) + b2 * uv2.x, (b0 * uv0.y + b1 * uv1.y) + b2 * uv2.y);
+}
 // Triangle hit -> interaction + shading frame (trianglemesh.cpp:45-113, intersectable.h:80-89)
 // `in` (extension, agpt.h agpt_instance): the mesh is a placed one -- vertices go to world space first, the shading
 // normal through transpose(W2O); nullptr for the reference's own meshes.  uvOut (extension, textured instantiations only): the
@@ -278,9 +288,9 @@ __device__ __forceinline__ void TriangleSurface(const DMesh& mesh, int slot, flo
 	float3 v0 = f3(a.x, a.y, a.z), v1 = f3(b.x, b.y, b.z), v2 = f3(c.x, c.y, c.z);
 	if (in) { v0 = XformPoint(in->object_to_world, v0); v1 = XformPoint(in->object_to_world, v1); v2 = XformPoint(in->object_to_world, v2); }
 	float b0 = 1.f - b1 - b2;
-	float2 uv0 = make_float2(0, 0), uv1 = make_float2(1, 0), uv2 = make_float2(1, 1);
-	if (mesh.uvs) { uv0 = __ldg(mesh.uvs + 3 * slot); uv1 = __ldg(mesh.uvs + 3 * slot + 1); uv2 = __ldg(mesh.uvs + 3 * slot + 2); }
-	if (uvOut) *uvOut = make_float2((b0 * uv0.x + b1 * uv1.x) + b2 * uv2.x, (b0 * uv0.y + b1 * uv1.y) + b2 * uv2.y);
+	float2 uv0, uv1, uv2;
+	TriangleUVs(mesh, slot, uv0, uv1, uv2);
+	if (uvOut) *uvOut = BaryUV(b1, b2, uv0, uv1, uv2);
 	float3 dpdu, dpdv;
 	TriangleDerivatives(v0, v1, v2, uv0, uv1, uv2, dpdu, dpdv);
 	SurfaceInit(s, O + t * D, dpdu, dpdv);
@@ -329,6 +339,12 @@ __device__ __forceinline__ float3 TexLookup(const DTexTables& tt, int tex, float
 	const float3 t00 = TexelAt(tt, d, x0, y0), t10 = TexelAt(tt, d, x1, y0), t01 = TexelAt(tt, d, x0, y1), t11 = TexelAt(tt, d, x1, y1);
 	const float3 a = t00 + fx * (t10 - t00), b = t01 + fx * (t11 - t01);
 	return a + fy * (b - a);
+}
+// channel k (0, 1, 2) of the same lookup: the alpha of a mask (the three channels' arithmetic is independent, so this is the
+// one-channel lookup bit for bit)
+__device__ __forceinline__ float TexLookupChannel(const DTexTables& tt, int tex, int k, float2 uv) {
+	const float3 c = TexLookup(tt, tex, uv);
+	return k == 0 ? c.x : k == 1 ? c.y : c.z;
 }
 // The two colours a Disney material derives from its base colour (host/material.h DisneyMaterial), for one hit.
 struct TexColors {

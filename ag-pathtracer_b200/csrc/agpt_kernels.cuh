@@ -308,10 +308,10 @@ __global__ void __launch_bounds__(256) k_generate(DScene sc, PathState ps, WaveQ
 }
 
 // ---- trace kernels ---------------------------------------------------------------------
-template <bool COUNT, bool FAST, bool INST>
-__global__ void __launch_bounds__(AGPT_TRACE_THREADS, AGPT_TRACE_MIN_BLOCKS) k_trace_closest(DScene sc, PathState ps, const int* __restrict__ queue, const int* __restrict__ countPtr,
-		unsigned long long* counters, unsigned long long* waveRow) {
-	__shared__ unsigned stackMem[AGPT_STACK_SMEM * AGPT_TRACE_THREADS];
+// The bodies are shared with the MASK entry points below (extension, alpha masks: mk is read by those only).
+template <bool COUNT, bool FAST, bool INST, bool MASK>
+__device__ __forceinline__ void TraceClosest(const DScene& sc, const PathState& ps, const int* __restrict__ queue, const int* __restrict__ countPtr,
+		unsigned long long* counters, unsigned long long* waveRow, unsigned* stackMem, const DMaskTables& mk) {
 	int i = blockIdx.x * blockDim.x + threadIdx.x;
 	TraceCounters cnt = { 0, 0, 0, 0, 0, 0 };
 	// The queue length lives on the device (the host launches an upper bound of blocks).  The
@@ -329,7 +329,7 @@ __global__ void __launch_bounds__(AGPT_TRACE_THREADS, AGPT_TRACE_MIN_BLOCKS) k_t
 		d = kind ? ps.misD[path] : ps.rayD[path];
 	}
 	HitRecord hit;
-	TraceScene<false, COUNT, FAST, INST>(sc, f3(o.x, o.y, o.z), f3(d.x, d.y, d.z), o.w, hit, stackMem + threadIdx.x, AGPT_TRACE_THREADS, cnt, lane);
+	TraceScene<false, COUNT, FAST, INST, MASK>(sc, f3(o.x, o.y, o.z), f3(d.x, d.y, d.z), o.w, hit, stackMem + threadIdx.x, AGPT_TRACE_THREADS, cnt, lane, mk);
 	if (lane) {
 		if (kind == 0) {
 			ps.hitA[path] = make_float4(hit.t, hit.b1, hit.b2, __int_as_float(hit.prim));
@@ -339,11 +339,16 @@ __global__ void __launch_bounds__(AGPT_TRACE_THREADS, AGPT_TRACE_MIN_BLOCKS) k_t
 	}
 	if (COUNT) FlushCounters(cnt, lane, counters, waveRow);
 }
-
 template <bool COUNT, bool FAST, bool INST>
-__global__ void __launch_bounds__(AGPT_TRACE_THREADS, AGPT_TRACE_MIN_BLOCKS) k_trace_any(DScene sc, PathState ps, const int* __restrict__ queue, const int* __restrict__ countPtr,
+__global__ void __launch_bounds__(AGPT_TRACE_THREADS, AGPT_TRACE_MIN_BLOCKS) k_trace_closest(DScene sc, PathState ps, const int* __restrict__ queue, const int* __restrict__ countPtr,
 		unsigned long long* counters, unsigned long long* waveRow) {
 	__shared__ unsigned stackMem[AGPT_STACK_SMEM * AGPT_TRACE_THREADS];
+	TraceClosest<COUNT, FAST, INST, false>(sc, ps, queue, countPtr, counters, waveRow, stackMem, DMaskTables());
+}
+
+template <bool COUNT, bool FAST, bool INST, bool MASK>
+__device__ __forceinline__ void TraceAny(const DScene& sc, const PathState& ps, const int* __restrict__ queue, const int* __restrict__ countPtr,
+		unsigned long long* counters, unsigned long long* waveRow, unsigned* stackMem, const DMaskTables& mk) {
 	int i = blockIdx.x * blockDim.x + threadIdx.x;
 	TraceCounters cnt = { 0, 0, 0, 0, 0, 0 };
 	int path = queue[i];
@@ -354,23 +359,28 @@ __global__ void __launch_bounds__(AGPT_TRACE_THREADS, AGPT_TRACE_MIN_BLOCKS) k_t
 	float4 o = make_float4(0.f, 0.f, 0.f, 0.f), d = make_float4(1.f, 0.f, 0.f, 0.f);
 	if (lane) { o = ps.shO[path]; d = ps.shD[path]; }
 	HitRecord hit;
-	bool occluded = TraceScene<true, COUNT, FAST, INST>(sc, f3(o.x, o.y, o.z), f3(d.x, d.y, d.z), o.w, hit, stackMem + threadIdx.x, AGPT_TRACE_THREADS, cnt, lane);
+	bool occluded = TraceScene<true, COUNT, FAST, INST, MASK>(sc, f3(o.x, o.y, o.z), f3(d.x, d.y, d.z), o.w, hit, stackMem + threadIdx.x, AGPT_TRACE_THREADS, cnt, lane, mk);
 	if (lane) ps.shadowOccluded[path] = occluded ? 1 : 0;
 	if (COUNT) FlushCounters(cnt, lane, counters, waveRow);
 }
+template <bool COUNT, bool FAST, bool INST>
+__global__ void __launch_bounds__(AGPT_TRACE_THREADS, AGPT_TRACE_MIN_BLOCKS) k_trace_any(DScene sc, PathState ps, const int* __restrict__ queue, const int* __restrict__ countPtr,
+		unsigned long long* counters, unsigned long long* waveRow) {
+	__shared__ unsigned stackMem[AGPT_STACK_SMEM * AGPT_TRACE_THREADS];
+	TraceAny<COUNT, FAST, INST, false>(sc, ps, queue, countPtr, counters, waveRow, stackMem, DMaskTables());
+}
 
 // Standalone rays (agpt_trace_rays / agpt_trace_primary): hit table out.
-template <bool ANY, bool COUNT, bool FAST, bool INST>
-__global__ void __launch_bounds__(AGPT_TRACE_THREADS) k_trace_table(DScene sc, const float4* __restrict__ rayO, const float4* __restrict__ rayD,
-		int count, agpt_hit* out, unsigned long long* counters) {
-	__shared__ unsigned stackMem[AGPT_STACK_SMEM * AGPT_TRACE_THREADS];
+template <bool ANY, bool COUNT, bool FAST, bool INST, bool MASK>
+__device__ __forceinline__ void TraceTable(const DScene& sc, const float4* __restrict__ rayO, const float4* __restrict__ rayD,
+		int count, agpt_hit* out, unsigned long long* counters, unsigned* stackMem, const DMaskTables& mk) {
 	int i = blockIdx.x * blockDim.x + threadIdx.x;
 	TraceCounters cnt = { 0, 0, 0, 0, 0, 0 };
 	bool lane = i < count;
 	float4 o = make_float4(0.f, 0.f, 0.f, 0.f), d = make_float4(1.f, 0.f, 0.f, 0.f);
 	if (lane) { o = rayO[i]; d = rayD[i]; }
 	HitRecord hit;
-	bool found = TraceScene<ANY, COUNT, FAST, INST>(sc, f3(o.x, o.y, o.z), f3(d.x, d.y, d.z), o.w, hit, stackMem + threadIdx.x, AGPT_TRACE_THREADS, cnt, lane);
+	bool found = TraceScene<ANY, COUNT, FAST, INST, MASK>(sc, f3(o.x, o.y, o.z), f3(d.x, d.y, d.z), o.w, hit, stackMem + threadIdx.x, AGPT_TRACE_THREADS, cnt, lane, mk);
 	if (lane) {
 		agpt_hit h;
 		h.found = found ? 1u : 0u;
@@ -381,6 +391,36 @@ __global__ void __launch_bounds__(AGPT_TRACE_THREADS) k_trace_table(DScene sc, c
 		out[i] = h;
 	}
 	if (COUNT) FlushCounters(cnt, lane, counters, nullptr);
+}
+template <bool ANY, bool COUNT, bool FAST, bool INST>
+__global__ void __launch_bounds__(AGPT_TRACE_THREADS) k_trace_table(DScene sc, const float4* __restrict__ rayO, const float4* __restrict__ rayD,
+		int count, agpt_hit* out, unsigned long long* counters) {
+	__shared__ unsigned stackMem[AGPT_STACK_SMEM * AGPT_TRACE_THREADS];
+	TraceTable<ANY, COUNT, FAST, INST, false>(sc, rayO, rayD, count, out, counters, stackMem, DMaskTables());
+}
+
+// EXTENSION: alpha masks (agpt.h agpt_upload_alpha_masks).  The three trace kernels with the mask test, run only while some
+// mask is bound; INST is always on (its path is also right for scenes without instances), which keeps the count at 4 + 4 + 8.
+#ifndef AGPT_MASK_MIN_BLOCKS
+#define AGPT_MASK_MIN_BLOCKS AGPT_TRACE_MIN_BLOCKS   // they spill a little under it, yet 8 (fewer spills) measured 10-12 % slower (DESIGN.md section 10)
+#endif
+template <bool COUNT, bool FAST>
+__global__ void __launch_bounds__(AGPT_TRACE_THREADS, AGPT_MASK_MIN_BLOCKS) k_trace_closest_masked(DScene sc, PathState ps, const int* __restrict__ queue,
+		const int* __restrict__ countPtr, unsigned long long* counters, unsigned long long* waveRow, DMaskTables mk) {
+	__shared__ unsigned stackMem[AGPT_STACK_SMEM * AGPT_TRACE_THREADS];
+	TraceClosest<COUNT, FAST, true, true>(sc, ps, queue, countPtr, counters, waveRow, stackMem, mk);
+}
+template <bool COUNT, bool FAST>
+__global__ void __launch_bounds__(AGPT_TRACE_THREADS, AGPT_MASK_MIN_BLOCKS) k_trace_any_masked(DScene sc, PathState ps, const int* __restrict__ queue,
+		const int* __restrict__ countPtr, unsigned long long* counters, unsigned long long* waveRow, DMaskTables mk) {
+	__shared__ unsigned stackMem[AGPT_STACK_SMEM * AGPT_TRACE_THREADS];
+	TraceAny<COUNT, FAST, true, true>(sc, ps, queue, countPtr, counters, waveRow, stackMem, mk);
+}
+template <bool ANY, bool COUNT, bool FAST>
+__global__ void __launch_bounds__(AGPT_TRACE_THREADS) k_trace_table_masked(DScene sc, const float4* __restrict__ rayO, const float4* __restrict__ rayD,
+		int count, agpt_hit* out, unsigned long long* counters, DMaskTables mk) {
+	__shared__ unsigned stackMem[AGPT_STACK_SMEM * AGPT_TRACE_THREADS];
+	TraceTable<ANY, COUNT, FAST, true, true>(sc, rayO, rayD, count, out, counters, stackMem, mk);
 }
 
 // ---- shade -------------------------------------------------------------------------------

@@ -15,6 +15,7 @@
 #pragma once
 
 #include "agpt_device.cuh"
+#include "agpt_bsdf.cuh"      // the texture lookup of alpha masks
 
 #ifndef AGPT_STACK_SMEM
 #define AGPT_STACK_SMEM 24      // stack entries per thread kept in shared memory
@@ -103,6 +104,31 @@ __device__ __forceinline__ const DMesh& MeshOfPrim(const DScene& sc, const agpt_
 	return sc.meshes[(INST && pr.type == AGPT_PRIM_INSTANCE) ? sc.instances[pr.payload].mesh : pr.payload];
 }
 
+// EXTENSION: alpha masks (agpt.h agpt_upload_alpha_masks).  A candidate hit the triangle or plane test accepted on a primitive
+// of material `material` stands iff that material has no mask or the mask's channel at the hit's uv is >= its cutoff.  The
+// record is read only here, on a geometric hit: the walk keeps just the material index of the mesh it is in.
+__device__ __forceinline__ bool MaskOf(const DMaskTables& mk, int material, int& texture, int& channel, float& cutoff) {
+	if (material < 0) return false;
+	AGPT_CHECK(material < mk.nMasks, AGPT_DBG_MASK, material);
+	const agpt_alpha_mask m = mk.masks[material];
+	texture = m.texture; channel = m.channel; cutoff = m.cutoff;
+	return texture >= 0;
+}
+template <bool INST>
+__device__ __forceinline__ bool MaskTriangle(const DScene& sc, const DMaskTables& mk, int material, int primIndex, int slot, float b1, float b2) {
+	int texture, channel;
+	float cutoff;
+	if (!MaskOf(mk, material, texture, channel, cutoff)) return true;
+	float2 uv0, uv1, uv2;
+	TriangleUVs(MeshOfPrim<INST>(sc, sc.prims[primIndex]), slot, uv0, uv1, uv2);
+	return TexLookupChannel(mk.tt, texture, channel, BaryUV(b1, b2, uv0, uv1, uv2)) >= cutoff;
+}
+__device__ __forceinline__ bool MaskPlane(const DMaskTables& mk, int material, const agpt_plane& pl, float3 O, float3 D, float t) {
+	int texture, channel;
+	float cutoff;
+	if (!MaskOf(mk, material, texture, channel, cutoff)) return true;
+	return TexLookupChannel(mk.tt, texture, channel, PlaneUV(pl, O + t * D)) >= cutoff;
+}
 #ifndef AGPT_ANY_NEAR_FIRST
 #define AGPT_ANY_NEAR_FIRST 1
 #endif
@@ -130,9 +156,10 @@ __device__ __forceinline__ const DMesh& MeshOfPrim(const DScene& sc, const agpt_
 // each (a typical ray hits 1-2 of 5 roots).
 // `lane` is false for threads without a ray; they must still call (full-mask votes).
 // SMEM: stack entries per thread in shared memory (the rest of the AGPT_STACK_SMEM + AGPT_STACK_LOCAL levels in local memory).
-template <bool ANY, bool COUNT, bool FAST, bool INST, int SMEM = AGPT_STACK_SMEM>
+// MASK (extension, alpha masks): a triangle hit must also pass MaskTriangle.
+template <bool ANY, bool COUNT, bool FAST, bool INST, int SMEM = AGPT_STACK_SMEM, bool MASK = false>
 __device__ __forceinline__ bool TraceMeshRun(const DScene& sc, int p0, int p1, float3 O, float3 D, float3 rD, bool filterOk, float& rayT, HitRecord& hit,
-		unsigned* stack, int stackStride, TraceCounters& cnt, bool lane) {
+		unsigned* stack, int stackStride, TraceCounters& cnt, bool lane, const DMaskTables& mk = DMaskTables()) {
 	bool found = false;
 	unsigned local[AGPT_STACK_SMEM + AGPT_STACK_LOCAL - SMEM];
 	unsigned cand = 0;               // meshes of the run this lane still has to enter (bit m - p0)
@@ -160,6 +187,7 @@ __device__ __forceinline__ bool TraceMeshRun(const DScene& sc, int p0, int p1, f
 		if (c) cand |= 1u << (m - p0);
 	}
 	int mp = p1 - 1;                 // this lane's current mesh primitive
+	int mat = -1;                    // MASK: the material of mesh mp
 	bool inside = false;             // walking mesh mp (else: about to enter the next candidate)
 	const float4* nodes = nullptr;
 	const float4* tris = nullptr;
@@ -177,6 +205,7 @@ __device__ __forceinline__ bool TraceMeshRun(const DScene& sc, int p0, int p1, f
 				const agpt_prim pr = sc.prims[mp];
 				const DMesh& mesh = MeshOfPrim<INST>(sc, pr);
 				nodes = mesh.nodes; tris = mesh.tris;
+				if (MASK) mat = pr.material;
 				if (INST) {
 					if (pr.type == AGPT_PRIM_INSTANCE) ObjectSpaceRay<FAST>(sc.instances[pr.payload], O, D, cO, cD, crD, cFilt);
 					else { cO = O; cD = D; crD = rD; cFilt = filterOk; }
@@ -187,7 +216,14 @@ __device__ __forceinline__ bool TraceMeshRun(const DScene& sc, int p0, int p1, f
 						float4 a = LoadTable(tris + 3 * j), b = LoadTable(tris + 3 * j + 1), c = LoadTable(tris + 3 * j + 2);
 						if (COUNT) cnt.tri_tests++;
 						float t, b1, b2;
-						if ((ANY || a.w == 0.f) && TriangleTest(f3(a.x, a.y, a.z), f3(b.x, b.y, b.z), f3(c.x, c.y, c.z), cO, cD, rayT, t, b1, b2)) {
+						if constexpr (MASK) {
+							if ((ANY || a.w == 0.f) && TriangleTest(f3(a.x, a.y, a.z), f3(b.x, b.y, b.z), f3(c.x, c.y, c.z), cO, cD, rayT, t, b1, b2) && MaskTriangle<INST>(sc, mk, mat, mp, j, b1, b2)) {
+								found = true;
+								if (ANY) break;
+								rayT = t; hit.t = t; hit.b1 = b1; hit.b2 = b2; hit.prim = mp; hit.slot = j;
+							}
+						}
+						else if ((ANY || a.w == 0.f) && TriangleTest(f3(a.x, a.y, a.z), f3(b.x, b.y, b.z), f3(c.x, c.y, c.z), cO, cD, rayT, t, b1, b2)) {
 							found = true;
 							if (ANY) break;
 							rayT = t; hit.t = t; hit.b1 = b1; hit.b2 = b2; hit.prim = mp; hit.slot = j;
@@ -261,7 +297,14 @@ __device__ __forceinline__ bool TraceMeshRun(const DScene& sc, int p0, int p1, f
 						float4 a = LoadTable(tris + 3 * j), b = LoadTable(tris + 3 * j + 1), c = LoadTable(tris + 3 * j + 2);
 						if (COUNT) cnt.tri_tests++;
 						float t, b1, b2;
-						if ((ANY || a.w == 0.f) && TriangleTest(f3(a.x, a.y, a.z), f3(b.x, b.y, b.z), f3(c.x, c.y, c.z), cO, cD, rayT, t, b1, b2)) {
+						if constexpr (MASK) {
+							if ((ANY || a.w == 0.f) && TriangleTest(f3(a.x, a.y, a.z), f3(b.x, b.y, b.z), f3(c.x, c.y, c.z), cO, cD, rayT, t, b1, b2) && MaskTriangle<INST>(sc, mk, mat, mp, j, b1, b2)) {
+								found = true;
+								if (ANY) break;
+								rayT = t; hit.t = t; hit.b1 = b1; hit.b2 = b2; hit.prim = mp; hit.slot = j;
+							}
+						}
+						else if ((ANY || a.w == 0.f) && TriangleTest(f3(a.x, a.y, a.z), f3(b.x, b.y, b.z), f3(c.x, c.y, c.z), cO, cD, rayT, t, b1, b2)) {
 							found = true;
 							if (ANY) break;
 							rayT = t; hit.t = t; hit.b1 = b1; hit.b2 = b2; hit.prim = mp; hit.slot = j;
@@ -292,9 +335,10 @@ __device__ __forceinline__ bool TraceMeshRun(const DScene& sc, int p0, int p1, f
 // (Testing the spheres and planes first and the meshes afterwards, with an exact tie-aware merge,
 // was measured: closest-hit +13 % on cfg 3, +10 % in the closed room -- a second pass over the
 // primitive list for little extra pruning.  Not kept; numbers in DESIGN.md.)
-template <bool ANY, bool COUNT, bool FAST, bool INST>
+// MASK (extension, alpha masks): plane and triangle hits must also pass MaskPlane / MaskTriangle (mk: the mask tables).
+template <bool ANY, bool COUNT, bool FAST, bool INST, bool MASK = false>
 __device__ __forceinline__ bool TraceScene(const DScene& sc, float3 O, float3 D, float rayT, HitRecord& hit,
-		unsigned* stack, int stackStride, TraceCounters& cnt, bool lane) {
+		unsigned* stack, int stackStride, TraceCounters& cnt, bool lane, const DMaskTables& mk = DMaskTables()) {
 	hit.prim = -1; hit.slot = -1; hit.t = 0.f; hit.b1 = 0.f; hit.b2 = 0.f;
 	bool found = false;
 	// exact-filtered slab test (agpt_device.cuh): reciprocal direction, valid only for sane components
@@ -343,7 +387,13 @@ __device__ __forceinline__ bool TraceScene(const DScene& sc, float3 O, float3 D,
 		else if (prim.type == AGPT_PRIM_PLANE) {
 			if (COUNT && test) cnt.analytic_tests++;
 			float t;
-			if (test && PlaneTest(sc.planes[prim.payload], O, D, rayT, t)) {
+			if constexpr (MASK) {
+				if (test && PlaneTest(sc.planes[prim.payload], O, D, rayT, t) && MaskPlane(mk, prim.material, sc.planes[prim.payload], O, D, t)) {
+					if (!ANY) { rayT = t; hit.t = t; hit.prim = p; hit.slot = -1; }
+					found = true;
+				}
+			}
+			else if (test && PlaneTest(sc.planes[prim.payload], O, D, rayT, t)) {
 				if (!ANY) { rayT = t; hit.t = t; hit.prim = p; hit.slot = -1; }
 				found = true;
 			}
@@ -352,7 +402,7 @@ __device__ __forceinline__ bool TraceScene(const DScene& sc, float3 O, float3 D,
 		else {
 			int q = p + 1;                                     // run of consecutive mesh primitives (<= 32 per call)
 			while (q < sc.n_prims && q < p + 32 && sc.prims[q].type >= AGPT_PRIM_BVH_MESH) q++;
-			if (TraceMeshRun<ANY, COUNT, FAST, INST>(sc, p, q, O, D, rD, filterOk, rayT, hit, stack, stackStride, cnt, test)) found = true;
+			if (TraceMeshRun<ANY, COUNT, FAST, INST, AGPT_STACK_SMEM, MASK>(sc, p, q, O, D, rD, filterOk, rayT, hit, stack, stackStride, cnt, test, mk)) found = true;
 			p = q;
 		}
 	}

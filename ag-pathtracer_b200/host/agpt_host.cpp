@@ -30,6 +30,7 @@ static int UploadFlat(const FlatScene& flat, const Camera& camera, agpt_ctx* ctx
 	if ((rc = agpt_upload_instances(ctx, flat.instances.data(), (int)flat.instances.size()))) return rc;
 	if ((rc = agpt_upload_primitives(ctx, flat.prims.data(), (int)flat.prims.size()))) return rc;
 	if ((rc = agpt_upload_material_textures(ctx, flat.textures.data(), (int)flat.textures.size(), flat.materialTextures.data(), (int)flat.materialTextures.size()))) return rc;
+	if ((rc = agpt_upload_alpha_masks(ctx, flat.alphaMasks.data(), (int)flat.alphaMasks.size()))) return rc;   // after the textures it names
 	agpt_camera cam = camera.Export();
 	return agpt_set_camera(ctx, &cam);
 }
@@ -100,6 +101,16 @@ int agpt_host_scene_tables(agpt_host_scene* s, agpt_scene_tables* out) {
 		out->textures = f.textures.empty() ? nullptr : f.textures.data(); out->material_texture = f.materialTexture.empty() ? nullptr : f.materialTexture.data();
 		out->n_textures = (int)f.textures.size(); out->n_material_texture = (int)f.materialTexture.size();
 		out->material_textures = f.materialTextures.empty() ? nullptr : f.materialTextures.data(); out->n_material_textures = (int)f.materialTextures.size();
+	)
+	return AGPT_OK;
+}
+
+int agpt_host_scene_alpha_masks(agpt_host_scene* s, const agpt_alpha_mask** out, int* n) {
+	if (!s || !out || !n) return HostFail("null argument");
+	HOST_TRY(
+		FlatScene& f = Flat(s);
+		*out = f.alphaMasks.empty() ? nullptr : f.alphaMasks.data();
+		*n = (int)f.alphaMasks.size();
 	)
 	return AGPT_OK;
 }

@@ -21,12 +21,32 @@ struct MaterialMaps {
 	float3 color = float3(0.f);                        // the base colour, used when base is null and roughnessMetallic is not
 };
 
+// EXTENSION: a material's alpha mask (include/agpt.h agpt_alpha_mask), with the image as a pointer
+struct MaterialAlphaMask {
+	const ImageTexture* image = nullptr;   // null: no mask
+	int channel = 0;                       // 0, 1, 2
+	float cutoff = 0.5f;                   // the surface is there where the channel >= cutoff
+};
+
+#define AGPT_HAS_ALPHA_MASKS 1         // extension: Material::SetAlphaMask
 class Material {
 public:
 	virtual ~Material() {}
 	virtual agpt_material Export() const = 0;
 	virtual const ImageTexture* BaseColorTexture() const { return nullptr; }   // extension: DisneyMaterial with an image
 	virtual MaterialMaps Maps() const { MaterialMaps m; m.base = BaseColorTexture(); return m; }   // extension: all its images
+	// EXTENSION (include/agpt.h agpt_upload_alpha_masks): cutout geometry on a material of any type -- channel `channel` of
+	// `image` at the hit's uv decides whether a ray hits the surface (glTF alphaMode MASK with alphaCutoff `cutoff`).  Set it before
+	// the scene's first render: CudaPathTracer re-uploads a scene when its primitive or light list changes (Scene::Fingerprint,
+	// which takes materials as immutable), so a mask set later needs an explicit CudaPathTracer::Upload.
+	void SetAlphaMask(std::shared_ptr<ImageTexture> image, int channel = 0, float cutoff = 0.5f) {
+		if (channel < 0 || channel > 2 || !std::isfinite(cutoff)) throw std::runtime_error("SetAlphaMask: need a channel in [0, 2] and a finite cutoff");
+		maskImage = std::move(image); mask.image = maskImage.get(); mask.channel = channel; mask.cutoff = cutoff;
+	}
+	MaterialAlphaMask AlphaMask() const { return mask; }
+private:
+	std::shared_ptr<ImageTexture> maskImage;
+	MaterialAlphaMask mask;
 };
 
 #define AGPT_HAS_IMAGE_TEXTURES 1      // extension: DisneyMaterial(ImageTexture, roughness, metallic)

@@ -68,6 +68,7 @@ struct FlatScene {
 	std::vector<agpt_texture> textures;        // extension: base-colour images, texels borrowed from the materials
 	std::vector<int32_t> materialTexture;      // per material: index into textures or -1 (empty when no material has one)
 	std::vector<agpt_material_textures> materialTextures;   // extension: per material, all its image bindings (empty as above)
+	std::vector<agpt_alpha_mask> alphaMasks;   // extension: per material, its alpha mask (empty when no material has one)
 	bool HasMaps() const { for (auto& b : materialTextures) if (b.roughness_metallic >= 0 || b.normal >= 0) return true; return false; }
 	uint64_t Bytes() const {
 		uint64_t b = prims.size() * sizeof(agpt_prim) + spheres.size() * sizeof(agpt_sphere) + planes.size() * sizeof(agpt_plane)
@@ -77,6 +78,7 @@ struct FlatScene {
 		for (auto& t : textures) b += (uint64_t)t.width * t.height * 16 + 16;   // float4 texels and a descriptor on the device
 		b += materialTexture.size() * 4;
 		if (HasMaps()) b += materialTextures.size() * 32;                      // the map binding table
+		b += alphaMasks.size() * sizeof(agpt_alpha_mask);
 		return b;
 	}
 };
@@ -151,6 +153,8 @@ public:
 					b.color[0] = mm.color.x; b.color[1] = mm.color.y; b.color[2] = mm.color.z;
 					flat->materialTexture.push_back(b.base);
 					flat->materialTextures.push_back(b);
+					const MaterialAlphaMask am = m->AlphaMask();
+					flat->alphaMasks.push_back(agpt_alpha_mask{ index(am.image), am.channel, am.cutoff, 0 });
 				}
 				row.material = it->second;
 			}
@@ -182,6 +186,9 @@ public:
 			flat->prims.push_back(row);
 		}
 		if (flat->textures.empty()) { flat->materialTexture.clear(); flat->materialTextures.clear(); }
+		bool masked = false;
+		for (auto& am : flat->alphaMasks) masked = masked || am.texture >= 0;
+		if (!masked) flat->alphaMasks.clear();
 		for (auto& l : lights) {
 			agpt_light rec;
 			memset(&rec, 0, sizeof(rec));

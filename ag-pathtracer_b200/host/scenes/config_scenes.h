@@ -46,6 +46,7 @@ inline ConfigDefaults Defaults(int config) {
 	case 11: return { 1920, 1080, 64, 16, 4, "cfg11_ext_cfg5_sampled_panel_plane_and_mesh_lights" };
 	case 12: return { 480, 270, 16, 8, 0, "cfg12_ext_procedural_image_textures" };
 	case 13: return { 480, 270, 16, 8, 0, "cfg13_ext_procedural_roughness_metallic_and_normal_maps" };
+	case 14: return { 480, 270, 16, 8, 0, "cfg14_ext_alpha_masked_cutouts" };
 	default: return { 0, 0, 0, 0, 0, "unknown" };
 	}
 }
@@ -712,6 +713,105 @@ inline void BuildConfig13(Scene* scene, int level) {
 }
 #endif
 
+#if defined(AGPT_HAS_ALPHA_MASKS) && defined(AGPT_HAS_MATERIAL_MAPS)
+// cfg 14 (EXTENSION, host mirror only -- the reference's surfaces are solid): alpha-masked cutout geometry (include/agpt.h
+// agpt_upload_alpha_masks), laid out so every masked path of the trace walk is used:
+// - a BVHTriMesh of 1,536 leaf quads with per-vertex uvs over an elliptical leaf; the leaf image is the leaves' base colour and,
+//   through its green channel, their mask; a ring of its texels equals the cutoff exactly;
+// - the same leaf mesh as two rotated, scaled Instances with a second material masked by the red channel of another image;
+// - a plain TriangleMesh quad with the default uvs and a checker mask;
+// - a horizontal masked Plane (a grate) between the sphere area light and the floor: shadow rays go through its holes;
+// - a masked mirror quad, and the sky (UniformInfiniteLight) behind every hole.
+// Level 2 adds roughness-metallic and normal maps on the leaves, so masked trace runs beside the mapped shade.
+inline std::shared_ptr<ImageTexture> LeafImage(int W, int H) {
+	std::vector<float> rgb(3 * (size_t)W * H);
+	for (int y = 0; y < H; y++)
+		for (int x = 0; x < W; x++) {
+			const float u = (x + .5f) / W - .5f, v = (y + .5f) / H - .5f;
+			const float e = (u * u) / (.45f * .45f) + (v * v) / (.3f * .3f);      // elliptical leaf
+			float* p = &rgb[3 * ((size_t)y * W + x)];
+			p[0] = .15f + .3f * (v + .5f);
+			p[1] = e < .8f ? 1.f : e < 1.f ? .5f : 0.f;                             // the alpha; .5 = the cutoff, on a ring
+			p[2] = .1f + .2f * (u + .5f);
+		}
+	return ImageTexture::Make(W, H, std::move(rgb));
+}
+inline std::shared_ptr<ImageTexture> MaskPattern(int W, int H, int kind) {
+	std::vector<float> rgb(3 * (size_t)W * H);
+	for (int y = 0; y < H; y++)
+		for (int x = 0; x < W; x++) {
+			float* p = &rgb[3 * ((size_t)y * W + x)];
+			float a;
+			if (kind == 0) a = ((x + y) & 1) ? 1.f : 0.f;                                  // checker
+			else if (kind == 1) a = (x % 4 == 0 || y % 4 == 0) ? 1.f : .25f;               // grate bars
+			else { const float u = (x + .5f) / W - .5f, v = (y + .5f) / H - .5f; a = u * u + v * v < .2f ? .9f : .1f; }   // disc
+			p[0] = a; p[1] = .5f * a; p[2] = a;
+		}
+	return ImageTexture::Make(W, H, std::move(rgb));
+}
+inline std::shared_ptr<TriangleMesh> MakeLeaves(int n, std::shared_ptr<Material> mat) {
+	std::vector<float3> vertices, normals;
+	std::vector<float2> texcoords;
+	std::vector<index_type> indices;
+	uint32_t s = 12345u;
+	auto rnd = [&]() { s = s * 1664525u + 1013904223u; return (float)(s >> 8) / 16777216.f; };
+	for (int i = 0; i < n; i++) {
+		const float3 c(-2.5f + 2.f * rnd(), 1.f + 2.2f * rnd(), -1.f + 2.f * rnd());
+		const float a = 6.2831853f * rnd(), b = 1.2f * (rnd() - .5f), size = .25f + .2f * rnd();
+		const float3 t(std::cos(a) * size, b * size, std::sin(a) * size), w(-std::sin(a) * .6f * size * b, .6f * size, std::cos(a) * .6f * size * b);
+		const int base = (int)vertices.size();
+		const float3 corner[4] = { c - t - w, c + t - w, c + t + w, c - t + w };
+		const float2 uv[4] = { float2(0, 0), float2(1, 0), float2(1, 1), float2(0, 1) };
+		for (int k = 0; k < 4; k++) { vertices.push_back(corner[k]); texcoords.push_back(uv[k]); }
+		for (int k : { 0, 1, 2, 0, 2, 3 }) indices.push_back(index_type(base + k));
+	}
+	return std::make_shared<TriangleMesh>(indices, vertices, normals, texcoords, mat);
+}
+inline std::shared_ptr<TriangleMesh> MakeQuad(const float3& o, const float3& e1, const float3& e2, bool uvs, std::shared_ptr<Material> mat) {
+	std::vector<float3> vertices = { o, o + e1, o + e1 + e2, o + e2 }, normals;
+	std::vector<float2> texcoords;
+	if (uvs) texcoords = { float2(0, 0), float2(1, 0), float2(1, 1), float2(0, 1) };
+	std::vector<index_type> indices;
+	for (int v : { 0, 1, 2, 0, 2, 3 }) indices.push_back(index_type(v));
+	return std::make_shared<TriangleMesh>(indices, vertices, normals, texcoords, mat);
+}
+inline void BuildConfig14(Scene* scene, int level) {
+	scene->primitives.push_back(std::make_shared<Plane>(float3(0, -1, 0), float2(8, 8), DisneyMaterial::Make(float3(.6f, .58f, .55f), .9f, 0.f)));
+	auto leaf = LeafImage(64, 64);
+	auto leafMat = DisneyMaterial::Make(leaf, .6f, 0.f);
+	leafMat->SetAlphaMask(leaf, 1, .5f);
+	if (level >= 2) {
+		leafMat->SetRoughnessMetallicMap(RoughnessMetallicChecker(16, 16, 4));
+		leafMat->SetNormalMap(HeightFieldNormals(32, 32, .01f, 2), 1.f);
+	}
+	auto leaves = MakeLeaves(1536, leafMat);
+	auto bvh = std::make_shared<BVHTriMesh>(leaves, leafMat, 1);
+	scene->primitives.push_back(bvh);
+	auto discs = MaskPattern(32, 32, 2);
+	auto otherLeaf = DisneyMaterial::Make(float3(.55f, .35f, .15f), .5f, 0.f);
+	otherLeaf->SetAlphaMask(discs, 0, .5f);
+	scene->primitives.push_back(std::make_shared<Instance>(bvh, mat4::Translate(3.8f, -.4f, 1.5f) * mat4::RotateY(.7f) * mat4::Scale(.7f), otherLeaf));
+	scene->primitives.push_back(std::make_shared<Instance>(bvh, mat4::Translate(-1.f, -.9f, 4.f) * mat4::RotateY(-.4f) * mat4::Scale(1.2f), leafMat));
+	auto checkerMat = DisneyMaterial::Make(float3(.2f, .45f, .7f), .4f, 0.f);
+	checkerMat->SetAlphaMask(MaskPattern(8, 8, 0), 0, .5f);
+	scene->primitives.push_back(MakeQuad(float3(1.f, -1.f, -1.5f), float3(2.f, 0, .3f), float3(0, 2.f, 0), false, checkerMat));
+	auto grateMat = DisneyMaterial::Make(float3(.5f, .5f, .52f), .7f, 1.f);
+	grateMat->SetAlphaMask(MaskPattern(16, 16, 1), 2, .5f);
+	scene->primitives.push_back(std::make_shared<Plane>(float3(0, 4.f, 0), float2(3.f, 3.f), grateMat));
+	auto mirror = MirrorMaterial::Make(float3(.9f, .9f, .9f));
+	mirror->SetAlphaMask(discs, 0, .5f);
+	scene->primitives.push_back(MakeQuad(float3(-4.2f, -1.f, 2.f), float3(1.8f, 0, -.6f), float3(0, 2.5f, 0), true, mirror));
+	scene->addAreaLight(std::make_shared<Sphere>(float3(0, 6.f, .5f), .5f, nullptr), WarmWhite(150));
+	scene->lights.push_back(std::make_shared<UniformInfiniteLight>(float3(.3f, .35f, .45f)));
+	scene->camera.lookfrom = float3(0, 2.f, -8.5f);
+	scene->camera.lookat = float3(0, 1.f, 0);
+	scene->camera.vup = float3(0, 1, 0);
+	scene->camera.aspect_ratio = 16.f / 9.f;
+	scene->camera.vfov = 45;
+	scene->camera.aperture = 0;
+}
+#endif
+
 // level <= 0 selects the BASELINE.json size of each configuration.
 inline bool BuildConfig(Scene* scene, int config, int level) {
 	switch (config) {
@@ -737,6 +837,9 @@ inline bool BuildConfig(Scene* scene, int config, int level) {
 #endif
 #ifdef AGPT_HAS_MATERIAL_MAPS
 	case 13: BuildConfig13(scene, level > 0 ? level : 1); return true;
+#endif
+#if defined(AGPT_HAS_ALPHA_MASKS) && defined(AGPT_HAS_MATERIAL_MAPS)
+	case 14: BuildConfig14(scene, level > 0 ? level : 1); return true;
 #endif
 	default: return false;
 	}

@@ -338,6 +338,36 @@ typedef struct agpt_material_textures {
 int agpt_upload_material_textures(agpt_ctx* ctx, const agpt_texture* textures, int n_textures,
                                   const agpt_material_textures* bindings, int n_materials);
 
+/* ---- alpha masks: cutout geometry (EXTENSION: glTF alphaMode MASK; the reference's surfaces are solid everywhere) --------
+ * masks[i] applies to material i of any type (Disney, mirror, glass): the mask is geometry, not BSDF.  Its alpha is channel
+ * `channel` (0, 1, 2) of resident texture `texture` (agpt_upload_textures / agpt_upload_material_textures), which needs no
+ * base or map binding of its own; -1: no mask.  A candidate hit on a primitive whose material has a mask -- one the test of
+ * its ray accepts (closest-hit: the triangle or plane test and the degenerate-triangle test; any-hit: the triangle or plane
+ * test) -- is then, in float32 with every operation rounded on its own:
+ *   1. given a uv by agpt_upload_textures step 1: triangle b0 = 1 - b1 - b2, (b0 * uv0 + b1 * uv1) + b2 * uv2 with the mesh's
+ *      uvs or the default ones (instances: their mesh's uvs and the object-space barycentrics); plane ((P - o) / half + 1) * 0.5
+ *      with P = O + t * D;
+ *   2. looked up by agpt_upload_textures step 2 (bilinear, repeat-wrapped, nested lerp), keeping channel `channel`: alpha;
+ *   3. kept iff alpha >= cutoff.  Otherwise it is as if the triangle or plane test had returned false: ray.t is unchanged and
+ *      the walk goes on, in the reference's order and with its tie rules.
+ * The rule holds for every ray through Scene::Intersect / IntersectP: path, MIS and shadow rays, agpt_trace_primary,
+ * agpt_trace_rays, agpt_li_*, and the rays of agpt_render_guides.  No random number is drawn: every path's draws stay where
+ * they were.  Refused with AGPT_ERR_INVALID, leaving the resident masks as they were: a texture outside [-1, resident
+ * textures), a channel outside [0, 2], a cutoff that is not finite.  (NULL, 0) clears the masks, and so does every successful
+ * texture upload (the indices name the old table).  Like every upload it makes the guides stale and drops the saved
+ * reprojection view.  At render time (with any mask bound) n_materials must equal the resident material count, and no
+ * primitive whose material has a mask may be a sphere or have area_light >= 0 (masked spheres and emitters are not defined),
+ * else AGPT_ERR_INVALID.  agpt_scene_bytes counts the mask table (16 bytes per material).  Scenes without a mask run the trace
+ * kernels they ran before; with one, trace runs instantiations that add the test.  statements/agpt_alpha_oracle.cpp states
+ * the same on the CPU. */
+typedef struct agpt_alpha_mask {
+	int32_t texture;   /* index into the resident textures, or -1: no mask */
+	int32_t channel;   /* 0, 1, 2: which channel of that texture is the alpha */
+	float cutoff;      /* glTF alphaCutoff: the surface is there where alpha >= cutoff; finite */
+	int32_t pad;
+} agpt_alpha_mask;
+int agpt_upload_alpha_masks(agpt_ctx* ctx, const agpt_alpha_mask* masks, int n_materials);
+
 int agpt_set_camera(agpt_ctx* ctx, const agpt_camera* camera);          /* Camera, camera.h:38-56 */
 int agpt_set_film(agpt_ctx* ctx, int width, int height);                /* Accumulator(w,h), myapp.h:10-13 */
 int agpt_scene_bytes(agpt_ctx* ctx, uint64_t* out);                     /* resident scene bytes in HBM */

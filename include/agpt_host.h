@@ -25,7 +25,7 @@ typedef struct agpt_host_tracer agpt_host_tracer;
 const char* agpt_host_last_error(void);
 
 /* config 1..5 = BASELINE.json configs[0..4]; 6 and 8 = test-only corner-case scenes, 7 = the reference default scene;
- * 9..13 = extension scenes of the host mirror (12: procedural image textures; 13: roughness-metallic and normal maps);
+ * 9..14 = extension scenes of the host mirror (12: procedural image textures; 13: roughness-metallic and normal maps; 14: alpha masks);
  * level <= 0 picks the configuration's own icosphere subdivision level. */
 int agpt_host_scene_create(int config, int level, agpt_host_scene** out);
 int agpt_host_scene_destroy(agpt_host_scene* scene);
@@ -55,6 +55,9 @@ typedef struct agpt_scene_tables {
 	int n_material_textures;
 } agpt_scene_tables;
 int agpt_host_scene_tables(agpt_host_scene* scene, agpt_scene_tables* out);
+/* extension: the flattened scene's alpha masks (agpt_upload_alpha_masks), one row per material, or (NULL, 0) when no material
+ * has one; the texture indices name agpt_scene_tables.textures.  Valid while the scene lives. */
+int agpt_host_scene_alpha_masks(agpt_host_scene* scene, const agpt_alpha_mask** out, int* n);
 
 /* exports for comparison with the oracle's view of the same scene (oracle/ref_harness.cpp) */
 int agpt_host_camera_export(agpt_host_scene* scene, float* out19);
