@@ -2,13 +2,16 @@
 // wavefront kernels.  Host code here only moves tables into HBM, sizes launches and drives
 // the wave loop; every ray is traced and shaded on the device.  There is no CPU path: if no
 // CUDA device can be opened agpt_create() fails and the caller gets the CUDA error text.
+#include <algorithm>
 #include <cmath>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
 #include <memory>
+#include <optional>
 #include <string>
 #include <thread>
+#include <type_traits>
 #include <utility>
 #include <vector>
 
@@ -345,22 +348,53 @@ static DScene MakeScene(const agpt_ctx* c) {
 	return s;
 }
 
-static PathState MakePathState(agpt_ctx* c) {
-	PathState p;
+// ---- launch plan: which instantiation of each kernel family runs for the resident scene ------------------------------------
+// Built once per call, after CheckReady has built the lazy tables.  It is the only code that turns the scene's feature flags into
+// kernel choices: the launch dispatchers take it instead of flags of their own.
+struct LaunchPlan {
+	bool inst;                      // some primitive row is an instance: the INST trace instantiations
+	bool env;                       // an environment map (InfiniteAreaLight)
+	bool glass;                     // some material is a rough dielectric
+	bool shapes;                    // some area light samples its plane or mesh
+	int tex;                        // 1: some material is textured; 2: some material has a roughness-metallic or normal map
+	DShapeTables st;
+	DTexTables tt;
+	std::optional<DMaskTables> mk;  // some alpha mask is bound: the *_masked trace kernels
+};
+
+static LaunchPlan PlanLaunches(const agpt_ctx* c) {
+	LaunchPlan p;
+	p.inst = c->nInstances > 0; p.env = c->envW > 0; p.glass = c->hasGlass; p.shapes = c->hasShapeLights;
+	p.tex = c->hasMaps ? 2 : c->hasTextures ? 1 : 0;
+	p.st.lights = c->shapeLights.p; p.st.cdf = c->shapeCdf.p;
+	p.tt.texels = c->texels.p; p.tt.textures = c->textures.p; p.tt.matTex = c->matTex.p;
+	p.tt.nTextures = (int)c->textures.n; p.tt.nTexels = (long long)c->texels.n;
+	p.tt.matMaps = c->matMaps.p; p.tt.nMatMaps = (int)c->matMaps.n;
+	if (c->hasMasks) p.mk = DMaskTables{ p.tt, c->masks.p, (int)c->masks.n };
+	return p;
+}
+
+// What every call that generates paths or rays starts from: the scene, the path slots, the queues k_generate fills for the first
+// wave (queue set A, counts A; no bucket keys yet) and the launch plan
+struct Frame {
+	DScene sc;
+	PathState ps;
+	WaveQueues q0;
+	LaunchPlan plan;
+};
+
+static Frame MakeFrame(agpt_ctx* c) {
+	Frame f{ MakeScene(c), PathState(), WaveQueues(), PlanLaunches(c) };
+	PathState& p = f.ps;
 	p.rayO = c->f4[0].p; p.rayD = c->f4[1].p; p.hitA = c->f4[2].p; p.beta = c->f4[3].p; p.L = c->f4[4].p;
 	p.neeLight = c->f4[5].p; p.neeMis = c->f4[6].p; p.neeBeta = c->f4[7].p;
 	p.shO = c->f4[8].p; p.shD = c->f4[9].p; p.misO = c->f4[10].p; p.misD = c->f4[11].p; p.Lout = c->f4[12].p;
 	p.hitSlot = c->i32[0].p; p.shadowOccluded = c->i32[1].p; p.misPrim = c->i32[2].p;
 	p.rng = c->u32[0].p; p.flags = c->u32[1].p;
 	p.slots = (int)c->capacity;
-	return p;
-}
-
-// The queues k_generate fills for the first wave (queue set A, counts A; no bucket keys yet)
-static WaveQueues FirstWave(const agpt_ctx* c) {
-	WaveQueues q0;
+	WaveQueues& q0 = f.q0;
 	q0.closest = c->queues[0].p; q0.shadow = c->queues[2].p; q0.active = c->queues[4].p; q0.counts = c->counts.p; q0.keys = nullptr; q0.shadowKeys = nullptr;
-	return q0;
+	return f;
 }
 
 static int EnsureCapacity(agpt_ctx* c, size_t paths) {
@@ -378,8 +412,6 @@ static int EnsureCapacity(agpt_ctx* c, size_t paths) {
 	c->capacity = paths;
 	return AGPT_OK;
 }
-
-static int BuildSphereRuns(agpt_ctx* c);
 
 // agpt_light.flags (extension): only AGPT_LIGHT_SAMPLE_SHAPE, and only on area lights
 static int CheckLightFlags(const agpt_light& l) {
@@ -473,43 +505,80 @@ static int JoinUpload(agpt_ctx* c) {
 }
 #define JOIN(c) do { int j_ = JoinUpload(c); if (j_ != AGPT_OK) return j_; } while (0)
 
-// ---- launch helpers: template flags from run-time flags --------------------------------------
-// (COUNT, FAST = !strictBoxes, INST = the scene has instances) -> one of eight instantiations
-#define AGPT_DISPATCH3(count, fast, inst, CALL) do { \
-	if (count) { if (fast) { if (inst) { CALL(true, true, true); } else { CALL(true, true, false); } } else { if (inst) { CALL(true, false, true); } else { CALL(true, false, false); } } } \
-	else { if (fast) { if (inst) { CALL(false, true, true); } else { CALL(false, true, false); } } else { if (inst) { CALL(false, false, true); } else { CALL(false, false, false); } } } } while (0)
-
-// mk != nullptr (some alpha mask is bound, extension): the MASK instantiations, which take INST on
-#define AGPT_DISPATCH_MASKED(count, fast, CALLM) do { \
-	if (count) { if (fast) { CALLM(true, true); } else { CALLM(true, false); } } else { if (fast) { CALLM(false, true); } else { CALLM(false, false); } } } while (0)
-
-static void LaunchClosest(bool count, bool strictBoxes, bool inst, int blocks, cudaStream_t st, const DScene& sc, const PathState& ps, const int* queue, const int* n, unsigned long long* cnt, unsigned long long* row,
-		const DMaskTables* mk) {
-#define CALL(C, F, I) k_trace_closest<C, F, I><<<blocks, AGPT_TRACE_THREADS, 0, st>>>(sc, ps, queue, n, cnt, row)
-#define CALLM(C, F) k_trace_closest_masked<C, F><<<blocks, AGPT_TRACE_THREADS, 0, st>>>(sc, ps, queue, n, cnt, row, *mk)
-	if (mk) AGPT_DISPATCH_MASKED(count, !strictBoxes, CALLM);
-	else AGPT_DISPATCH3(count, !strictBoxes, inst, CALL);
-#undef CALLM
-#undef CALL
+// ---- launches ---------------------------------------------------------------------------
+// f(std::bool_constant<b>...) for the run-time flags b...: one instantiation per combination of the flags given
+template <typename F>
+static void WithBools(F&& f) { f(); }
+template <typename F, typename... B>
+static void WithBools(F&& f, bool b, B... rest) {
+	if (b) WithBools([&](auto... t) { f(std::true_type(), t...); }, rest...);
+	else WithBools([&](auto... t) { f(std::false_type(), t...); }, rest...);
 }
-static void LaunchAny(bool count, bool strictBoxes, bool inst, int blocks, cudaStream_t st, const DScene& sc, const PathState& ps, const int* queue, const int* n, unsigned long long* cnt, unsigned long long* row,
-		const DMaskTables* mk) {
-#define CALL(C, F, I) k_trace_any<C, F, I><<<blocks, AGPT_TRACE_THREADS, 0, st>>>(sc, ps, queue, n, cnt, row)
-#define CALLM(C, F) k_trace_any_masked<C, F><<<blocks, AGPT_TRACE_THREADS, 0, st>>>(sc, ps, queue, n, cnt, row, *mk)
-	if (mk) AGPT_DISPATCH_MASKED(count, !strictBoxes, CALLM);
-	else AGPT_DISPATCH3(count, !strictBoxes, inst, CALL);
-#undef CALLM
-#undef CALL
+
+// k_generate for g.n paths into the frame's slots and first-wave queues; LIST, the adaptive rounds' mode, when g names a pixel list
+static int Generate(agpt_ctx* c, const Frame& f, const GenParams& g) {
+	WithBools([&](auto LIST) { k_generate<LIST><<<Blocks(g.n, 256), 256, 0, c->stream>>>(f.sc, f.ps, f.q0, g); }, g.list != nullptr);
+	CU(cudaGetLastError());
+	c->stats.kernel_launches++;
+	return AGPT_OK;
 }
-template <bool ANY>
-static void LaunchTable(bool count, bool strictBoxes, bool inst, int blocks, cudaStream_t st, const DScene& sc, const float4* o, const float4* d, int n, agpt_hit* out, unsigned long long* cnt,
-		const DMaskTables* mk) {
-#define CALL(C, F, I) k_trace_table<ANY, C, F, I><<<blocks, AGPT_TRACE_THREADS, 0, st>>>(sc, o, d, n, out, cnt)
-#define CALLM(C, F) k_trace_table_masked<ANY, C, F><<<blocks, AGPT_TRACE_THREADS, 0, st>>>(sc, o, d, n, out, cnt, *mk)
-	if (mk) AGPT_DISPATCH_MASKED(count, !strictBoxes, CALLM);
-	else AGPT_DISPATCH3(count, !strictBoxes, inst, CALL);
-#undef CALLM
-#undef CALL
+
+// Trace kernels take <lead..., COUNT = AGPT_FLAG_COUNTERS, FAST = !AGPT_FLAG_STRICT_BOXES, INST>; while a mask is bound the
+// *_masked ones run instead, which always take the instance path and so have no INST.
+template <typename Plain, typename Masked, typename... Lead>
+static void LaunchTrace(const LaunchPlan& p, uint32_t flags, Plain plain, Masked masked, Lead... lead) {
+	const bool count = flags & AGPT_FLAG_COUNTERS, fast = !(flags & AGPT_FLAG_STRICT_BOXES);
+	if (p.mk) WithBools(masked, lead..., count, fast);
+	else WithBools(plain, lead..., count, fast, p.inst);
+}
+
+static void LaunchClosest(const LaunchPlan& p, uint32_t flags, int rays, cudaStream_t st, const DScene& sc, const PathState& ps, const int* queue, const int* n,
+		unsigned long long* cnt, unsigned long long* row) {
+	const int b = Blocks(rays, AGPT_TRACE_THREADS);
+	LaunchTrace(p, flags, [&](auto C, auto F, auto I) { k_trace_closest<C, F, I><<<b, AGPT_TRACE_THREADS, 0, st>>>(sc, ps, queue, n, cnt, row); },
+		[&](auto C, auto F) { k_trace_closest_masked<C, F><<<b, AGPT_TRACE_THREADS, 0, st>>>(sc, ps, queue, n, cnt, row, *p.mk); });
+}
+static void LaunchAny(const LaunchPlan& p, uint32_t flags, int rays, cudaStream_t st, const DScene& sc, const PathState& ps, const int* queue, const int* n,
+		unsigned long long* cnt, unsigned long long* row) {
+	const int b = Blocks(rays, AGPT_TRACE_THREADS);
+	LaunchTrace(p, flags, [&](auto C, auto F, auto I) { k_trace_any<C, F, I><<<b, AGPT_TRACE_THREADS, 0, st>>>(sc, ps, queue, n, cnt, row); },
+		[&](auto C, auto F) { k_trace_any_masked<C, F><<<b, AGPT_TRACE_THREADS, 0, st>>>(sc, ps, queue, n, cnt, row, *p.mk); });
+}
+static void LaunchTable(const LaunchPlan& p, uint32_t flags, bool any, cudaStream_t st, const DScene& sc, const float4* o, const float4* d, int n, agpt_hit* out,
+		unsigned long long* cnt) {
+	const int b = Blocks(n, AGPT_TRACE_THREADS);
+	LaunchTrace(p, flags, [&](auto A, auto C, auto F, auto I) { k_trace_table<A, C, F, I><<<b, AGPT_TRACE_THREADS, 0, st>>>(sc, o, d, n, out, cnt); },
+		[&](auto A, auto C, auto F) { k_trace_table_masked<A, C, F><<<b, AGPT_TRACE_THREADS, 0, st>>>(sc, o, d, n, out, cnt, *p.mk); }, any);
+}
+
+// k_shade_a<ENV>: ENV, the scene has an environment map
+static void LaunchShadeA(const LaunchPlan& p, int active, cudaStream_t st, const DScene& sc, const PathState& ps, const int* queue, const int* n, int* survivors,
+		int* survivorCount, int max_depth) {
+	WithBools([&](auto E) { k_shade_a<E><<<Blocks(active, 256), 256, 0, st>>>(sc, ps, queue, n, survivors, survivorCount, max_depth); }, p.env);
+}
+
+// k_shade_b<ENV, GLASS, SHAPES, TEX> has ten instantiations; each carries only what it needs, or everything.
+//   a plain scene:                  <ENV, GLASS, false, 0>  (four)
+//   a sampled shape light:          <false, false, true, 0>, or <true, true, true, 0> with an environment map or glass
+//   textures (TEX 1), maps (TEX 2): <false, false, false, TEX>, or <true, true, true, TEX> with a shape light, an
+//                                   environment map or glass
+static void LaunchShadeB(const LaunchPlan& p, int blocks, cudaStream_t st, const DScene& sc, const PathState& ps, const int* survivors, const WaveQueues& qout,
+		const ShadeParams& sp, RayCounters* rc) {
+	auto launch = [&](auto E, auto G, auto S, auto T) { k_shade_b<E, G, S, T><<<blocks, AGPT_SHADE_THREADS, 0, st>>>(sc, p.st, ps, survivors, qout, sp, rc, p.tt); };
+	const bool envOrGlass = p.env || p.glass;
+	if (p.tex == 2) WithBools([&](auto all) { launch(all, all, all, std::integral_constant<int, 2>()); }, envOrGlass || p.shapes);
+	else if (p.tex == 1) WithBools([&](auto all) { launch(all, all, all, std::integral_constant<int, 1>()); }, envOrGlass || p.shapes);
+	else if (p.shapes) WithBools([&](auto all) { launch(all, all, std::true_type(), std::integral_constant<int, 0>()); }, envOrGlass);
+	else WithBools([&](auto E, auto G) { launch(E, G, std::false_type(), std::integral_constant<int, 0>()); }, p.env, p.glass);
+}
+
+// k_guides; a textured material's albedo needs the texture tables (k_guides_tex), a mapped one also its material record (k_guides_maps)
+static void LaunchGuides(const LaunchPlan& p, int pixels, cudaStream_t st, const DScene& sc, const PathState& ps, int ns, bool first, int total, float4* albedo,
+		float4* normalDepth) {
+	const int blocks = Blocks(pixels, 256);
+	if (p.tex == 2) k_guides_maps<<<blocks, 256, 0, st>>>(sc, p.tt, ps, ns, first, total, albedo, normalDepth);
+	else if (p.tex == 1) k_guides_tex<<<blocks, 256, 0, st>>>(sc, p.tt, ps, ns, first, total, albedo, normalDepth);
+	else k_guides<<<blocks, 256, 0, st>>>(sc, ps, ns, first, total, albedo, normalDepth);
 }
 
 
@@ -622,6 +691,16 @@ static int ValidateBvh(const agpt_mesh_desc& d, int meshIndex, int* depthOut) {
 	return AGPT_OK;
 }
 
+// Every agpt_upload_* once its arguments have passed their checks: the work still queued on the old tables finishes, and the
+// guides and the saved reprojection view of the old scene become stale.
+static int BeginSceneChange(agpt_ctx* c) {
+	CU(cudaSetDevice(c->device));
+	CU(cudaStreamSynchronize(c->stream));
+	c->stateGen++;
+	c->historyGen++;
+	return AGPT_OK;
+}
+
 int agpt_upload_meshes(agpt_ctx* c, const agpt_mesh_desc* meshes, int n) {
 	NEED(c != nullptr && n >= 0 && (n == 0 || meshes != nullptr), AGPT_ERR_INVALID, "bad mesh table");
 	// validate every descriptor before touching what is resident: a refused upload leaves the old scene intact
@@ -635,11 +714,9 @@ int agpt_upload_meshes(agpt_ctx* c, const agpt_mesh_desc* meshes, int n) {
 		if (rcode != AGPT_OK) return rcode;
 		if (depth > maxDepth) maxDepth = depth;
 	}
-	CU(cudaSetDevice(c->device));
-	CU(cudaStreamSynchronize(c->stream));
+	int rcode = BeginSceneChange(c);
+	if (rcode != AGPT_OK) return rcode;
 	c->gridCalibrated = false;
-	c->stateGen++;
-	c->historyGen++;
 	// the new tables are built beside the resident ones, which a failure leaves in place
 	std::vector<MeshStore> store((size_t)n);
 	std::vector<DMesh> table(n);
@@ -687,10 +764,8 @@ int agpt_upload_meshes(agpt_ctx* c, const agpt_mesh_desc* meshes, int n) {
 #define SIMPLE_UPLOAD(fn, T, member, counter) \
 	int fn(agpt_ctx* c, const T* rows, int n) { \
 		NEED(c != nullptr && n >= 0 && (n == 0 || rows != nullptr), AGPT_ERR_INVALID, "bad table"); \
-		CU(cudaSetDevice(c->device)); \
-		CU(cudaStreamSynchronize(c->stream)); \
-		c->stateGen++; \
-		c->historyGen++; \
+		int rcode = BeginSceneChange(c); \
+		if (rcode != AGPT_OK) return rcode; \
 		DevBuf<T> table; \
 		CU(table.Upload(rows, (size_t)n, c->stream)); \
 		CU(cudaStreamSynchronize(c->stream)); \
@@ -719,10 +794,8 @@ int agpt_upload_envmap(agpt_ctx* c, const agpt_envmap* env) {
 	NEED(c != nullptr, AGPT_ERR_INVALID, "null context");
 	const bool clear = !env || env->width == 0;
 	NEED(clear || (env->width > 0 && env->height > 0 && env->rgb && env->func && env->cdf), AGPT_ERR_INVALID, "bad environment map");
-	CU(cudaSetDevice(c->device));
-	CU(cudaStreamSynchronize(c->stream));
-	c->stateGen++;
-	c->historyGen++;
+	int rcode = BeginSceneChange(c);
+	if (rcode != AGPT_OK) return rcode;
 	if (clear) {
 		c->envRgb.Free(); c->envFunc.Free(); c->envCdf.Free();
 		c->envW = c->envH = 0; c->envFuncInt = 0;
@@ -760,10 +833,8 @@ static int UploadMaterialTextures(agpt_ctx* c, const agpt_texture* textures, int
 		NEED(std::isfinite(b.normal_scale) && std::isfinite(b.color[0]) && std::isfinite(b.color[1]) && std::isfinite(b.color[2]), AGPT_ERR_INVALID,
 			"agpt_upload_material_textures: normal_scale or color not finite");
 	}
-	CU(cudaSetDevice(c->device));
-	CU(cudaStreamSynchronize(c->stream));
-	c->stateGen++;
-	c->historyGen++;
+	int rcode = BeginSceneChange(c);
+	if (rcode != AGPT_OK) return rcode;
 	std::vector<float4> texels(total);
 	std::vector<DTexture> desc((size_t)n_textures);
 	size_t off = 0;
@@ -806,14 +877,6 @@ int agpt_upload_material_textures(agpt_ctx* c, const agpt_texture* textures, int
 	return UploadMaterialTextures(c, textures, n_textures, bindings, n_materials);
 }
 
-static DTexTables MakeTexTables(const agpt_ctx* c) {
-	DTexTables t;
-	t.texels = c->texels.p; t.textures = c->textures.p; t.matTex = c->matTex.p;
-	t.nTextures = (int)c->textures.n; t.nTexels = (long long)c->texels.n;
-	t.matMaps = c->matMaps.p; t.nMatMaps = (int)c->matMaps.n;
-	return t;
-}
-
 // EXTENSION (agpt.h agpt_upload_alpha_masks).  Every argument is checked before anything resident changes.
 int agpt_upload_alpha_masks(agpt_ctx* c, const agpt_alpha_mask* masks, int n_materials) {
 	NEED(c != nullptr && n_materials >= 0 && (n_materials == 0 || masks != nullptr), AGPT_ERR_INVALID, "agpt_upload_alpha_masks: bad table");
@@ -825,10 +888,8 @@ int agpt_upload_alpha_masks(agpt_ctx* c, const agpt_alpha_mask* masks, int n_mat
 		NEED(std::isfinite(m.cutoff), AGPT_ERR_INVALID, "agpt_upload_alpha_masks: cutoff not finite");
 		if (m.texture >= 0) hasMasks = true;
 	}
-	CU(cudaSetDevice(c->device));
-	CU(cudaStreamSynchronize(c->stream));
-	c->stateGen++;
-	c->historyGen++;
+	int rcode = BeginSceneChange(c);
+	if (rcode != AGPT_OK) return rcode;
 	DevBuf<agpt_alpha_mask> dMasks;
 	CU(dMasks.Upload(masks, (size_t)n_materials, c->stream));
 	CU(cudaStreamSynchronize(c->stream));
@@ -836,13 +897,6 @@ int agpt_upload_alpha_masks(agpt_ctx* c, const agpt_alpha_mask* masks, int n_mat
 	c->hostMasks.assign(masks, masks + n_materials);
 	c->hasMasks = hasMasks;
 	return AGPT_OK;
-}
-// the mask tables of the MASK trace instantiations in `store`, or nullptr while no mask is bound (the trace kernels without the test)
-static const DMaskTables* MaskTables(const agpt_ctx* c, DMaskTables& store) {
-	if (!c->hasMasks) return nullptr;
-	store.tt = MakeTexTables(c);
-	store.masks = c->masks.p; store.nMasks = (int)c->masks.n;
-	return &store;
 }
 
 int agpt_set_camera(agpt_ctx* c, const agpt_camera* cam) {
@@ -972,7 +1026,7 @@ int agpt_resolve(agpt_ctx* c, int samples, uint32_t* host) {
 }
 
 // ---- the wave loop -------------------------------------------------------------------------
-// Runs `n` already-generated paths (slots 0..n-1, queues A and counts A filled by k_generate) to
+// Generates the g.n paths of g (k_generate: slots 0..n-1, queues A and counts A) and runs them to
 // completion.  Queue lengths stay on the device (kernels read them); the host sizes grids from
 // upper bounds.  Default: after every wave the host waits for that wave's three counts (one
 // 12-byte copy to pinned memory), so the bounds are exact and the loop ends with the wave that
@@ -1019,9 +1073,15 @@ static int CalibrateBucketGrid(agpt_ctx* c, const PathState& ps, int n) {
 	return AGPT_OK;
 }
 
-static int RunWaves(agpt_ctx* c, const DScene& scIn, PathState& ps, int n, int max_depth, int rr_depth_arg, uint32_t flags) {
-	const bool count = flags & AGPT_FLAG_COUNTERS, timing = flags & AGPT_FLAG_TIMING, strictBoxes = flags & AGPT_FLAG_STRICT_BOXES;
-	DScene sc = scIn;
+static int RunWaves(agpt_ctx* c, const Frame& f, const GenParams& g, int max_depth, int rr_depth_arg, uint32_t flags) {
+	const bool count = flags & AGPT_FLAG_COUNTERS, timing = flags & AGPT_FLAG_TIMING;
+	const int n = g.n;
+	int rcode = Generate(c, f, g);
+	if (rcode != AGPT_OK) return rcode;
+	const PathState& ps = f.ps;
+	DScene sc = f.sc;
+	c->stats.paths += (uint64_t)n;
+	c->stats.rays_closest += (uint64_t)n;     // camera rays; the rest is counted on the device
 	WaveQueues q[2];
 	for (int k = 0; k < 2; k++) {
 		q[k].closest = c->queues[0 + k].p; q[k].shadow = c->queues[2 + k].p; q[k].active = c->queues[4 + k].p;
@@ -1046,7 +1106,6 @@ static int RunWaves(agpt_ctx* c, const DScene& scIn, PathState& ps, int n, int m
 		// ---- one wave on q[cur] -> q[cur ^ 1] ----
 		const int* closestQueue = q[cur].closest;
 		const int* shadowQueue = q[cur].shadow;
-		WaveQueues qin = q[cur];
 		if (wave > 0 && bucketing) {
 			// bucket pass: rays that start in the same cell going the same way end up adjacent
 			// (not worth its six launches for the last few thousand rays of a batch)
@@ -1072,33 +1131,29 @@ static int RunWaves(agpt_ctx* c, const DScene& scIn, PathState& ps, int n, int m
 		// unless per-kernel timing is on, the any-hit trace runs on the side stream so that each
 		// fills the SMs the other's tail leaves idle.
 		const bool fork = overlap && ubClosest > 0 && ubShadow > 0;
+		const int row = wave < AGPT_MAX_WAVE_ROWS ? wave : AGPT_MAX_WAVE_ROWS - 1;
 		if (timing) CU(cudaEventRecord(c->evA, c->stream));
 		if (fork) CU(cudaEventRecord(c->evFork, c->stream));
-		DMaskTables mkStore;
-		const DMaskTables* mk = MaskTables(c, mkStore);
 		if (ubClosest > 0) {
-			LaunchClosest(count, strictBoxes, c->nInstances > 0, Blocks(ubClosest, AGPT_TRACE_THREADS), c->stream, sc, ps, closestQueue, q[cur].counts + 0, cntClosest,
-				waveRows + (size_t)AGPT_WAVE_COUNTERS * (wave < AGPT_MAX_WAVE_ROWS ? wave : AGPT_MAX_WAVE_ROWS - 1), mk);
+			LaunchClosest(f.plan, flags, ubClosest, c->stream, sc, ps, closestQueue, q[cur].counts + 0, cntClosest, waveRows + (size_t)AGPT_WAVE_COUNTERS * row);
 			c->stats.kernel_launches++; c->stats.launches_closest++;
 		}
 		if (wave == 0 && bucketing && !c->gridCalibrated && c->calibrateGrid && n >= 4096) {
 			// first camera rays of this scene and camera: lay the bucket grid where they land
-			int rcode = CalibrateBucketGrid(c, ps, n);
+			rcode = CalibrateBucketGrid(c, ps, n);
 			if (rcode != AGPT_OK) return rcode;
 			SetBucketGrid(sc, c->gridLo, c->gridHi);
 		}
 		if (timing) CU(cudaEventRecord(c->evB, c->stream));
-		if (fork) {
-			CU(cudaStreamWaitEvent(c->sideStream, c->evFork, 0));
-			LaunchAny(count, strictBoxes, c->nInstances > 0, Blocks(ubShadow, AGPT_TRACE_THREADS), c->sideStream, sc, ps, shadowQueue, q[cur].counts + 1, cntAny,
-				waveRows + (size_t)AGPT_WAVE_COUNTERS * (AGPT_MAX_WAVE_ROWS + (wave < AGPT_MAX_WAVE_ROWS ? wave : AGPT_MAX_WAVE_ROWS - 1)), mk);
+		if (ubShadow > 0) {
+			if (fork) CU(cudaStreamWaitEvent(c->sideStream, c->evFork, 0));
+			LaunchAny(f.plan, flags, ubShadow, fork ? c->sideStream : c->stream, sc, ps, shadowQueue, q[cur].counts + 1, cntAny,
+				waveRows + (size_t)AGPT_WAVE_COUNTERS * (AGPT_MAX_WAVE_ROWS + row));
 			c->stats.kernel_launches++; c->stats.launches_any++;
-			CU(cudaEventRecord(c->evJoin, c->sideStream));
-			CU(cudaStreamWaitEvent(c->stream, c->evJoin, 0));
-		} else if (ubShadow > 0) {
-			LaunchAny(count, strictBoxes, c->nInstances > 0, Blocks(ubShadow, AGPT_TRACE_THREADS), c->stream, sc, ps, shadowQueue, q[cur].counts + 1, cntAny,
-				waveRows + (size_t)AGPT_WAVE_COUNTERS * (AGPT_MAX_WAVE_ROWS + (wave < AGPT_MAX_WAVE_ROWS ? wave : AGPT_MAX_WAVE_ROWS - 1)), mk);
-			c->stats.kernel_launches++; c->stats.launches_any++;
+			if (fork) {
+				CU(cudaEventRecord(c->evJoin, c->sideStream));
+				CU(cudaStreamWaitEvent(c->stream, c->evJoin, 0));
+			}
 		}
 		CU(cudaMemsetAsync(q[cur ^ 1].counts, 0, 3 * sizeof(int), c->stream));
 		if (timing) CU(cudaEventRecord(c->evC, c->stream));
@@ -1108,27 +1163,10 @@ static int RunWaves(agpt_ctx* c, const DScene& scIn, PathState& ps, int n, int m
 		// then k_shade_b (per survivor: the BSDF work), blocks striding over the list
 		CU(cudaMemsetAsync(c->survivorCount.p, 0, sizeof(int), c->stream));
 		sp.count = c->survivorCount.p;
-		const int shadeBlocks = Blocks(ubActive, AGPT_SHADE_THREADS);      // upper bound: blocks past the survivor count return at once
-		if (c->envW > 0) k_shade_a<true><<<Blocks(ubActive, 256), 256, 0, c->stream>>>(sc, ps, qin.active, q[cur].counts + 2, c->survivors.p, c->survivorCount.p, max_depth);
-		else k_shade_a<false><<<Blocks(ubActive, 256), 256, 0, c->stream>>>(sc, ps, qin.active, q[cur].counts + 2, c->survivors.p, c->survivorCount.p, max_depth);
-		// (ENV: the scene has an InfiniteAreaLight, GLASS: a rough-dielectric material -- each instantiation carries only what it needs;
-		// SHAPES, an area light that samples its plane or mesh: the lean one, or the one that carries everything)
-		DShapeTables st;
-		st.lights = c->shapeLights.p; st.cdf = c->shapeCdf.p;
-		const DTexTables tt = MakeTexTables(c);
-#define SHADE_B(E, G, S) k_shade_b<E, G, S, 0><<<shadeBlocks, AGPT_SHADE_THREADS, 0, c->stream>>>(sc, st, ps, c->survivors.p, q[cur ^ 1], sp, c->rayCounters.p, tt)
-#define SHADE_B_TEX(E, G, S, T) k_shade_b<E, G, S, T><<<shadeBlocks, AGPT_SHADE_THREADS, 0, c->stream>>>(sc, st, ps, c->survivors.p, q[cur ^ 1], sp, c->rayCounters.p, tt)
-		// (TEX, some material is textured: the lean textured instantiation, or the one that carries everything)
-		// (TEX = 2, some material has a roughness-metallic or normal map: the per-hit material record)
-		if (c->hasMaps) { if (c->hasShapeLights || c->envW > 0 || c->hasGlass) SHADE_B_TEX(true, true, true, 2); else SHADE_B_TEX(false, false, false, 2); }
-		else if (c->hasTextures) { if (c->hasShapeLights || c->envW > 0 || c->hasGlass) SHADE_B_TEX(true, true, true, 1); else SHADE_B_TEX(false, false, false, 1); }
-		else if (c->hasShapeLights) { if (c->envW > 0 || c->hasGlass) SHADE_B(true, true, true); else SHADE_B(false, false, true); }
-		else if (c->envW > 0) { if (c->hasGlass) SHADE_B(true, true, false); else SHADE_B(true, false, false); }
-		else { if (c->hasGlass) SHADE_B(false, true, false); else SHADE_B(false, false, false); }
-#undef SHADE_B
-#undef SHADE_B_TEX
-		c->stats.kernel_launches++;
-		c->stats.kernel_launches++; c->stats.launches_shade++;
+		LaunchShadeA(f.plan, ubActive, c->stream, sc, ps, q[cur].active, q[cur].counts + 2, c->survivors.p, c->survivorCount.p, max_depth);
+		// upper bound: blocks past the survivor count return at once
+		LaunchShadeB(f.plan, Blocks(ubActive, AGPT_SHADE_THREADS), c->stream, sc, ps, c->survivors.p, q[cur ^ 1], sp, c->rayCounters.p);
+		c->stats.kernel_launches += 2; c->stats.launches_shade++;
 		CU(cudaGetLastError());
 		if (timing) CU(cudaEventRecord(c->evD, c->stream));
 		// counts of the NEXT wave -> pinned ring slot, marked by an event
@@ -1176,40 +1214,36 @@ static int RunWaves(agpt_ctx* c, const DScene& scIn, PathState& ps, int n, int m
 	return AGPT_OK;
 }
 
+// Samples per pixel in one batch of a whole-film call: as many as maxPathsPerBatch holds, at least one, at most num_samples (>= 1)
+static int SamplesPerBatch(const agpt_ctx* c, int num_samples) {
+	const int fit = (int)(c->maxPathsPerBatch / ((size_t)c->width * c->height));
+	return std::min(std::max(fit, 1), num_samples);
+}
+
 int agpt_render(agpt_ctx* c, int first_sample, int num_samples, int sample_stride, int max_depth, int rr_depth_arg, uint32_t flags) {
 	int rcode = CheckReady(c, true);
 	if (rcode != AGPT_OK) return rcode;
 	NEED(num_samples >= 0 && sample_stride >= 1 && max_depth >= 0, AGPT_ERR_INVALID, "bad sample range or depth");
 	NEED(c->accum != nullptr, AGPT_ERR_STATE, "no accumulator");
 	CU(cudaSetDevice(c->device));
-	const size_t wh = (size_t)c->width * c->height;
-	int perBatch = (int)(c->maxPathsPerBatch / wh);
-	if (perBatch < 1) perBatch = 1;
-	if (perBatch > num_samples) perBatch = num_samples;
 	if (num_samples == 0) return AGPT_OK;
+	const size_t wh = (size_t)c->width * c->height;
+	const int perBatch = SamplesPerBatch(c, num_samples);
 	rcode = EnsureCapacity(c, wh * perBatch);
 	if (rcode != AGPT_OK) return rcode;
-	DScene sc = MakeScene(c);
-	PathState ps = MakePathState(c);
-	const WaveQueues q0 = FirstWave(c);
+	const Frame f = MakeFrame(c);
 	// evA/evC/evD are reused inside RunWaves when timing; the render bracket has its own pair
 	cudaEvent_t r0 = c->evRender0, r1 = c->evRender1;
 	CU(cudaEventRecord(r0, c->stream));
 	for (int done = 0; done < num_samples; done += perBatch) {
 		int ns = num_samples - done < perBatch ? num_samples - done : perBatch;
-		int n = (int)(wh * ns);
 		GenParams g{};
-		g.n = n; g.first_sample = first_sample + done * sample_stride; g.sample_stride = sample_stride; g.tiled = 1; g.samples = ns;
-		k_generate<false><<<Blocks(n, 256), 256, 0, c->stream>>>(sc, ps, q0, g);
-		CU(cudaGetLastError());
-		c->stats.kernel_launches++;
-		c->stats.paths += (uint64_t)n;
-		c->stats.rays_closest += (uint64_t)n;     // camera rays; the rest is counted on the device
-		rcode = RunWaves(c, sc, ps, n, max_depth, rr_depth_arg, flags);
+		g.n = (int)(wh * ns); g.first_sample = first_sample + done * sample_stride; g.sample_stride = sample_stride; g.tiled = 1; g.samples = ns;
+		rcode = RunWaves(c, f, g, max_depth, rr_depth_arg, flags);
 		if (rcode != AGPT_OK) return rcode;
 		if (c->uploadPending) CU(cudaStreamWaitEvent(c->stream, c->evUpload, 0));      // the film this batch adds to may still be on its way (agpt_write_accum_begin)
-		if (c->momentsOn) k_accumulate<true, false><<<Blocks(wh, 256), 256, 0, c->stream>>>(ps.Lout, c->accum, c->width, c->height, ns, c->moments.p);
-		else k_accumulate<false, false><<<Blocks(wh, 256), 256, 0, c->stream>>>(ps.Lout, c->accum, c->width, c->height, ns);
+		if (c->momentsOn) k_accumulate<true, false><<<Blocks(wh, 256), 256, 0, c->stream>>>(f.ps.Lout, c->accum, c->width, c->height, ns, c->moments.p);
+		else k_accumulate<false, false><<<Blocks(wh, 256), 256, 0, c->stream>>>(f.ps.Lout, c->accum, c->width, c->height, ns);
 		CU(cudaGetLastError());
 		c->stats.kernel_launches++;
 	}
@@ -1317,23 +1351,15 @@ static int RenderListed(agpt_ctx* c, int count, int step, int maxSamples, int ma
 	if (perBatch > (size_t)count) perBatch = (size_t)count;
 	int rcode = EnsureCapacity(c, perBatch * step);
 	if (rcode != AGPT_OK) return rcode;
-	DScene sc = MakeScene(c);
-	PathState ps = MakePathState(c);
-	const WaveQueues q0 = FirstWave(c);
+	const Frame f = MakeFrame(c);
 	CU(cudaEventRecord(c->evRender0, c->stream));
 	for (int done = 0; done < count; done += (int)perBatch) {
 		const int np = count - done < (int)perBatch ? count - done : (int)perBatch;
-		const int n = np * step;
 		GenParams g{};
-		g.n = n; g.samples = step; g.list = c->adaptiveList.p; g.listBase = done; g.listCount = count; g.moments = c->moments.p; g.maxSamples = maxSamples;
-		k_generate<true><<<Blocks(n, 256), 256, 0, c->stream>>>(sc, ps, q0, g);
-		CU(cudaGetLastError());
-		c->stats.kernel_launches++;
-		c->stats.paths += (uint64_t)n;
-		c->stats.rays_closest += (uint64_t)n;
-		rcode = RunWaves(c, sc, ps, n, max_depth, rr_depth_arg, flags);
+		g.n = np * step; g.samples = step; g.list = c->adaptiveList.p; g.listBase = done; g.listCount = count; g.moments = c->moments.p; g.maxSamples = maxSamples;
+		rcode = RunWaves(c, f, g, max_depth, rr_depth_arg, flags);
 		if (rcode != AGPT_OK) return rcode;
-		k_accumulate<true, true><<<Blocks(np, 256), 256, 0, c->stream>>>(ps.Lout, c->accum, c->width, c->height, step, c->moments.p, c->adaptiveList.p + done, np, maxSamples);
+		k_accumulate<true, true><<<Blocks(np, 256), 256, 0, c->stream>>>(f.ps.Lout, c->accum, c->width, c->height, step, c->moments.p, c->adaptiveList.p + done, np, maxSamples);
 		CU(cudaGetLastError());
 		c->stats.kernel_launches++;
 	}
@@ -1400,30 +1426,23 @@ int agpt_render_guides(agpt_ctx* c, int num_samples, uint32_t flags) {
 	NEED(num_samples >= 1 && num_samples <= (1 << 24), AGPT_ERR_INVALID, "agpt_render_guides: need 1 <= num_samples <= 1<<24");
 	CU(cudaSetDevice(c->device));
 	const size_t wh = (size_t)c->width * c->height;
-	int perBatch = (int)(c->maxPathsPerBatch / wh);
-	if (perBatch < 1) perBatch = 1;
-	if (perBatch > num_samples) perBatch = num_samples;
+	const int perBatch = SamplesPerBatch(c, num_samples);
 	rcode = EnsureCapacity(c, wh * perBatch);
 	if (rcode != AGPT_OK) return rcode;
 	c->guidesGen = 0;                                    // valid again only once this call has completed
 	if (c->guideAlbedo.n != wh) { CU(c->guideAlbedo.Alloc(wh)); CU(c->guideNormal.Alloc(wh)); }
-	DScene sc = MakeScene(c);
-	PathState ps = MakePathState(c);
-	const WaveQueues q0 = FirstWave(c);
-	const bool count = flags & AGPT_FLAG_COUNTERS, strictBoxes = flags & AGPT_FLAG_STRICT_BOXES;
+	const Frame f = MakeFrame(c);
 	for (int done = 0; done < num_samples; done += perBatch) {
 		const int ns = num_samples - done < perBatch ? num_samples - done : perBatch;
 		const int n = (int)(wh * ns);
 		GenParams g{};
 		g.n = n; g.first_sample = done; g.sample_stride = 1; g.tiled = 1; g.samples = ns;
-		k_generate<false><<<Blocks(n, 256), 256, 0, c->stream>>>(sc, ps, q0, g);
-		DMaskTables mkStore;
-		LaunchClosest(count, strictBoxes, c->nInstances > 0, Blocks(n, AGPT_TRACE_THREADS), c->stream, sc, ps, q0.closest, q0.counts + 0, c->traceCounters.p, nullptr, MaskTables(c, mkStore));
-		if (c->hasMaps) k_guides_maps<<<Blocks(wh, 256), 256, 0, c->stream>>>(sc, MakeTexTables(c), ps, ns, done == 0, done + ns == num_samples ? num_samples : 0, c->guideAlbedo.p, c->guideNormal.p);
-		else if (c->hasTextures) k_guides_tex<<<Blocks(wh, 256), 256, 0, c->stream>>>(sc, MakeTexTables(c), ps, ns, done == 0, done + ns == num_samples ? num_samples : 0, c->guideAlbedo.p, c->guideNormal.p);
-		else k_guides<<<Blocks(wh, 256), 256, 0, c->stream>>>(sc, ps, ns, done == 0, done + ns == num_samples ? num_samples : 0, c->guideAlbedo.p, c->guideNormal.p);
+		rcode = Generate(c, f, g);
+		if (rcode != AGPT_OK) return rcode;
+		LaunchClosest(f.plan, flags, n, c->stream, f.sc, f.ps, f.q0.closest, f.q0.counts + 0, c->traceCounters.p, nullptr);
+		LaunchGuides(f.plan, (int)wh, c->stream, f.sc, f.ps, ns, done == 0, done + ns == num_samples ? num_samples : 0, c->guideAlbedo.p, c->guideNormal.p);
 		CU(cudaGetLastError());
-		c->stats.kernel_launches += 3; c->stats.launches_closest++;
+		c->stats.kernel_launches += 2; c->stats.launches_closest++;
 	}
 	CU(cudaStreamSynchronize(c->stream));
 	c->guidesGen = c->stateGen;
@@ -1542,15 +1561,14 @@ int agpt_reproject_film(agpt_ctx* c, const agpt_reproject* params) {
 	return AGPT_OK;
 }
 
-static int TraceTable(agpt_ctx* c, const DScene& sc, const float4* rayO, const float4* rayD, int n, int any_hit, uint32_t flags, agpt_hit* out_host) {
+// The g.n rays k_generate makes from g, traced into a hit table on the host
+static int TraceTable(agpt_ctx* c, const Frame& f, const GenParams& g, int any_hit, uint32_t flags, agpt_hit* out_host) {
+	const int n = g.n;
+	int rcode = Generate(c, f, g);
+	if (rcode != AGPT_OK) return rcode;
 	DevBuf<agpt_hit> out;
 	CU(out.Alloc(n));
-	const bool count = flags & AGPT_FLAG_COUNTERS, strictBoxes = flags & AGPT_FLAG_STRICT_BOXES;
-	int blocks = Blocks(n, AGPT_TRACE_THREADS);
-	DMaskTables mkStore;
-	const DMaskTables* mk = MaskTables(c, mkStore);
-	if (any_hit) LaunchTable<true>(count, strictBoxes, c->nInstances > 0, blocks, c->stream, sc, rayO, rayD, n, out.p, c->traceCounters.p + AGPT_WAVE_COUNTERS, mk);
-	else LaunchTable<false>(count, strictBoxes, c->nInstances > 0, blocks, c->stream, sc, rayO, rayD, n, out.p, c->traceCounters.p, mk);
+	LaunchTable(f.plan, flags, any_hit != 0, c->stream, f.sc, f.ps.rayO, f.ps.rayD, n, out.p, c->traceCounters.p + (any_hit ? AGPT_WAVE_COUNTERS : 0));
 	CU(cudaGetLastError());
 	c->stats.kernel_launches++;
 	CU(cudaMemcpyAsync(out_host, out.p, (size_t)n * sizeof(agpt_hit), cudaMemcpyDeviceToHost, c->stream));
@@ -1579,15 +1597,9 @@ int agpt_trace_primary(agpt_ctx* c, int sample, uint32_t flags, agpt_hit* out_ho
 	const size_t wh = (size_t)c->width * c->height;
 	rcode = EnsureCapacity(c, wh);
 	if (rcode != AGPT_OK) return rcode;
-	DScene sc = MakeScene(c);
-	PathState ps = MakePathState(c);
-	const WaveQueues q0 = FirstWave(c);
 	GenParams g{};
 	g.n = (int)wh; g.first_sample = sample; g.sample_stride = 1;
-	k_generate<false><<<Blocks(wh, 256), 256, 0, c->stream>>>(sc, ps, q0, g);
-	CU(cudaGetLastError());
-	c->stats.kernel_launches++;
-	return TraceTable(c, sc, ps.rayO, ps.rayD, (int)wh, 0, flags, out_host);
+	return TraceTable(c, MakeFrame(c), g, 0, flags, out_host);
 }
 
 int agpt_trace_rays(agpt_ctx* c, int64_t n, const float* rays7, int any_hit, uint32_t flags, agpt_hit* out_host) {
@@ -1599,35 +1611,22 @@ int agpt_trace_rays(agpt_ctx* c, int64_t n, const float* rays7, int any_hit, uin
 	// same normalisation as the Ray constructor, done on the device by k_generate
 	rcode = EnsureCapacity(c, (size_t)n);
 	if (rcode != AGPT_OK) return rcode;
-	DScene sc = MakeScene(c);
-	PathState ps = MakePathState(c);
-	const WaveQueues q0 = FirstWave(c);
 	RayTable t;
 	GenParams g{};
 	rcode = UploadRays(c, t, (int)n, rays7, nullptr, flags, g);
 	if (rcode != AGPT_OK) return rcode;
-	k_generate<false><<<Blocks(n, 256), 256, 0, c->stream>>>(sc, ps, q0, g);
-	CU(cudaGetLastError());
-	c->stats.kernel_launches++;
-	return TraceTable(c, sc, ps.rayO, ps.rayD, (int)n, any_hit, flags, out_host);
+	return TraceTable(c, MakeFrame(c), g, any_hit, flags, out_host);
 }
 
 static int LiGeneric(agpt_ctx* c, GenParams g, int max_depth, int rr_depth_arg, uint32_t flags, float* out_rgb) {
 	int n = g.n;
 	int rcode = EnsureCapacity(c, (size_t)n);
 	if (rcode != AGPT_OK) return rcode;
-	DScene sc = MakeScene(c);
-	PathState ps = MakePathState(c);
-	const WaveQueues q0 = FirstWave(c);
-	k_generate<false><<<Blocks(n, 256), 256, 0, c->stream>>>(sc, ps, q0, g);
-	CU(cudaGetLastError());
-	c->stats.kernel_launches++;
-	c->stats.paths += (uint64_t)n;
-	c->stats.rays_closest += (uint64_t)n;
-	rcode = RunWaves(c, sc, ps, n, max_depth, rr_depth_arg, flags & AGPT_FLAG_RR_BY_BOUNCE);
+	const Frame f = MakeFrame(c);
+	rcode = RunWaves(c, f, g, max_depth, rr_depth_arg, flags & AGPT_FLAG_RR_BY_BOUNCE);
 	if (rcode != AGPT_OK) return rcode;
 	std::vector<float4> host(n);
-	CU(cudaMemcpyAsync(host.data(), ps.Lout, (size_t)n * sizeof(float4), cudaMemcpyDeviceToHost, c->stream));
+	CU(cudaMemcpyAsync(host.data(), f.ps.Lout, (size_t)n * sizeof(float4), cudaMemcpyDeviceToHost, c->stream));
 	CU(cudaStreamSynchronize(c->stream));
 	for (int i = 0; i < n; i++) { out_rgb[3 * i] = host[i].x; out_rgb[3 * i + 1] = host[i].y; out_rgb[3 * i + 2] = host[i].z; }
 	return AGPT_OK;
@@ -2166,21 +2165,19 @@ int agpt_probe_material_maps(agpt_ctx* c, int n, const float* rays7, float* out3
 	CU(cudaSetDevice(c->device));
 	rcode = EnsureCapacity(c, (size_t)n);
 	if (rcode != AGPT_OK) return rcode;
-	DScene sc = MakeScene(c);
-	PathState ps = MakePathState(c);
-	const WaveQueues q0 = FirstWave(c);
+	const Frame f = MakeFrame(c);
 	RayTable t;
 	GenParams g{};
 	rcode = UploadRays(c, t, n, rays7, nullptr, 0, g);
 	if (rcode != AGPT_OK) return rcode;
 	DevBuf<float> out;
 	CU(out.Alloc(32 * (size_t)n));
-	k_generate<false><<<Blocks(n, 256), 256, 0, c->stream>>>(sc, ps, q0, g);
-	DMaskTables mkStore;
-	LaunchClosest(false, false, c->nInstances > 0, Blocks(n, AGPT_TRACE_THREADS), c->stream, sc, ps, q0.closest, q0.counts + 0, c->traceCounters.p, nullptr, MaskTables(c, mkStore));
-	k_probe_material_maps<<<Blocks(n, 256), 256, 0, c->stream>>>(sc, MakeTexTables(c), ps, n, out.p);
+	rcode = Generate(c, f, g);
+	if (rcode != AGPT_OK) return rcode;
+	LaunchClosest(f.plan, 0, n, c->stream, f.sc, f.ps, f.q0.closest, f.q0.counts + 0, c->traceCounters.p, nullptr);
+	k_probe_material_maps<<<Blocks(n, 256), 256, 0, c->stream>>>(f.sc, f.plan.tt, f.ps, n, out.p);
 	CU(cudaGetLastError());
-	c->stats.kernel_launches += 3;
+	c->stats.kernel_launches += 2;
 	CU(cudaMemcpyAsync(out32, out.p, out.Bytes(), cudaMemcpyDeviceToHost, c->stream));
 	CU(cudaStreamSynchronize(c->stream));
 	return AGPT_OK;
@@ -2204,8 +2201,7 @@ int agpt_probe_light_sample(agpt_ctx* c, int light, int n, const float* in8, flo
 		"not an area light that samples its plane or mesh (AGPT_LIGHT_SAMPLE_SHAPE)");
 	CU(cudaSetDevice(c->device));
 	const DScene sc = MakeScene(c);
-	DShapeTables st;
-	st.lights = c->shapeLights.p; st.cdf = c->shapeCdf.p;
+	const DShapeTables st = PlanLaunches(c).st;
 	return ProbeRun(c, in8, 8 * (size_t)n, out8, 8 * (size_t)n, [&](const float* din, float* dout) {
 		k_probe_light_sample<<<Blocks(n, 128), 128, 0, c->stream>>>(sc, st, light, n, din, dout);
 	});
