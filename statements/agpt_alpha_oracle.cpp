@@ -312,6 +312,13 @@ void SetMasks(AlphaScene& as, const agpt_alpha_mask* masks, int n) {
 	if (masks) as.masks.assign(masks, masks + n);
 }
 
+// the six counters of agpt_alpha_oracle_render (closest, any, interior, boxes, tris, analytic) into counters_out, unless NULL
+void PutCounters(const Counters& c, unsigned long long* counters_out) {
+	if (!counters_out) return;
+	const uint64_t v[6] = { c.raysClosest, c.raysAny, c.interior, c.boxes, c.tris, c.analytic };
+	for (int i = 0; i < 6; i++) counters_out[i] = v[i];
+}
+
 } // namespace
 
 extern "C" {
@@ -357,10 +364,7 @@ void agpt_alpha_oracle_render(void* h, int W, int H, int s0, int ns, int max_dep
 		std::lock_guard<std::mutex> g(lock);
 		total.Add(c);
 	});
-	if (counters_out) {
-		const uint64_t v[6] = { total.raysClosest, total.raysAny, total.interior, total.boxes, total.tris, total.analytic };
-		for (int i = 0; i < 6; i++) counters_out[i] = v[i];
-	}
+	PutCounters(total, counters_out);
 }
 
 // agpt_li_pixels: radiance of single camera paths
@@ -376,8 +380,8 @@ void agpt_alpha_oracle_li_pixels(void* h, int W, int H, int n, const int* xs, co
 	}
 }
 
-// agpt_trace_rays: closest or any hit of caller rays (rays7 = O, D normalised like the Ray ctor, tmax)
-void agpt_alpha_oracle_trace_rays(void* h, long long n, const float* rays7, int any_hit, agpt_hit* out) {
+// agpt_trace_rays: closest or any hit of caller rays (rays7 = O, D normalised like the Ray ctor, tmax); counters_out (6, or NULL) as for agpt_alpha_oracle_render
+void agpt_alpha_oracle_trace_rays(void* h, long long n, const float* rays7, int any_hit, agpt_hit* out, unsigned long long* counters_out) {
 	const AlphaScene& as = *(AlphaScene*)h;
 	const OScene& sc = *as.ms.ts.sc;
 	Counters c;
@@ -395,10 +399,12 @@ void agpt_alpha_oracle_trace_rays(void* h, long long n, const float* rays7, int 
 			o.tri = hit.slot >= 0 ? MeshOfPrim(sc, sc.prims[hit.prim]).ids[hit.slot] : -1;
 		}
 	}
+	PutCounters(c, counters_out);
 }
 
-// agpt_trace_primary: the closest hit of every camera ray of sample `sample`, row-major from the top row
-void agpt_alpha_oracle_primary_hits(void* h, int W, int H, int sample, agpt_hit* out) {
+// agpt_trace_primary: the closest hit of every camera ray of sample `sample`, row-major from the top row; counters_out (6, or NULL) as for
+// agpt_alpha_oracle_render
+void agpt_alpha_oracle_primary_hits(void* h, int W, int H, int sample, agpt_hit* out, unsigned long long* counters_out) {
 	const AlphaScene& as = *(AlphaScene*)h;
 	const OScene& sc = *as.ms.ts.sc;
 	Counters c;
@@ -415,6 +421,7 @@ void agpt_alpha_oracle_primary_hits(void* h, int W, int H, int sample, agpt_hit*
 			o.tri = (found && hit.slot >= 0) ? MeshOfPrim(sc, sc.prims[hit.prim]).ids[hit.slot] : -1;
 			o.t = found ? hit.t : 0.f;
 		}
+	PutCounters(c, counters_out);
 }
 
 // agpt_render_guides: the maps statement's guide record over the masked first hit

@@ -27,40 +27,85 @@ def _host(agpt):
         pytest.skip("libagpt_host.so not built")
 
 
-@pytest.mark.parametrize("cfg,level", [(1, 0), (5, 2), (13, 1)])
+@pytest.mark.parametrize("cfg,level", [(1, 0), (5, 2), (7, 0), (9, 2), (10, 2), (12, 0), (13, 1)])
 def test_without_masks_the_statement_is_the_oracle(agpt, cfg, level):
+    """Film, counters, guides and hit tables.  cfg 7: environment map, 9: instances, 10: glass, 12 and 13: textures and maps (whose
+    oracle is the maps statement)."""
     _host(agpt)
     from oracle import port_binding as port
     hs = agpt.HostScene(cfg, level)
     d = agpt.config_defaults(cfg)
     got, cnt = ab.AlphaScene(hs).render(32, 18, 0, 2, d["max_depth"], d["depth_arg"], counters=True)
-    if cfg == 13:       # mapped materials: the oracle with the maps is the maps statement
+    if cfg in (12, 13):       # bound images: the oracle with textures and maps is the maps statement
         want, wcnt = mb.MapsScene(hs).render(32, 18, 0, 2, d["max_depth"], d["depth_arg"], counters=True)
     else:
         want, wcnt = port.PortScene(hs).render(32, 18, 0, 2, d["max_depth"], d["depth_arg"])
     assert np.array_equal(bits(got), bits(want))
     for k in ("rays_closest", "rays_any", "interior", "boxes", "tris", "analytic"):
         assert cnt[k] == wcnt[k], k
-    # the restated guide record and the any-hit and closest-hit tables
+    # the restated guide record and the any-hit and closest-hit tables, with the closest-hit walk's counters
     for g, w in zip(ab.AlphaScene(hs).guides(32, 18, 2), mb.MapsScene(hs).guides(32, 18, 2)):
         assert np.array_equal(bits(g), bits(w))
-    if cfg != 13:
-        ps = port.PortScene(hs)
-        cam = hs.camera()
-        rng = np.random.default_rng(cfg)
-        D = rng.normal(size=(2000, 3)).astype(np.float32)
-        O = np.broadcast_to(np.float32(cam[0:3]), D.shape)
-        rays7 = np.concatenate([O, D, np.full((len(D), 1), 1e30, np.float32)], 1).astype(np.float32)
-        for any_hit in (False, True):
-            got_t, want_t = ab.AlphaScene(hs).trace_rays(rays7, any_hit), ps.trace_rays(rays7, any_hit)[0]
-            for f in ("found", "prim", "tri"):
-                assert np.array_equal(got_t[f], want_t[f]), (any_hit, f)
-            assert np.array_equal(bits(got_t["t"]), bits(want_t["t"]))
-        hits = ab.AlphaScene(hs).primary_hits(32, 18, 1).reshape(-1)
-        want_hits = ps.primary_hits(32, 18, 1)
+    ps = port.PortScene(hs)
+    cam = hs.camera()
+    rng = np.random.default_rng(cfg)
+    D = rng.normal(size=(2000, 3)).astype(np.float32)
+    O = np.broadcast_to(np.float32(cam[0:3]), D.shape)
+    rays7 = np.concatenate([O, D, np.full((len(D), 1), 1e30, np.float32)], 1).astype(np.float32)
+    for any_hit in (False, True):
+        got_t, tcnt = ab.AlphaScene(hs).trace_rays(rays7, any_hit, counters=True)
+        want_t, wtcnt = ps.trace_rays(rays7, any_hit)
         for f in ("found", "prim", "tri"):
-            assert np.array_equal(hits[f], want_hits[f])
-        assert np.array_equal(bits(hits["t"]), bits(want_hits["t"]))
+            assert np.array_equal(got_t[f], want_t[f]), (any_hit, f)
+        assert np.array_equal(bits(got_t["t"]), bits(want_t["t"]))
+        assert tcnt["rays_any" if any_hit else "rays_closest"] == len(rays7)
+        if not any_hit:
+            assert (tcnt["interior"], tcnt["boxes"], tcnt["tris"]) == (wtcnt["interior"], wtcnt["boxes"], wtcnt["tris"])
+            assert tcnt["tris"] + tcnt["analytic"] > 0
+    hits, hcnt = ab.AlphaScene(hs).primary_hits(32, 18, 1, counters=True)
+    want_hits, whcnt = ps.primary_hits(32, 18, 1, want_counts=True)
+    for f in ("found", "prim", "tri"):
+        assert np.array_equal(hits.reshape(-1)[f], want_hits[f])
+    assert np.array_equal(bits(hits.reshape(-1)["t"]), bits(want_hits["t"]))
+    assert hcnt["rays_closest"] == 32 * 18
+    assert (hcnt["interior"], hcnt["boxes"], hcnt["tris"]) == (whcnt["interior"], whcnt["boxes"], whcnt["tris"])
+
+
+def test_a_rejected_tie_goes_to_the_next_triangle(agpt):
+    """Two coincident triangles of one plain TriangleMesh at the same t, in tables built by hand: the walk keeps the first it tests,
+    so masking the first leaves the second's hit, masking the second changes nothing and masking both leaves a miss.  The first
+    triangle's uvs sit on texel 0 of a 2 x 1 mask, the second's on texel 1."""
+    verts = np.zeros((2, 3, 4), np.float32)
+    verts[:, 0, :3] = (-1, 0, -1); verts[:, 1, :3] = (1, 0, -1); verts[:, 2, :3] = (0, 0, 1)
+    uvs = np.zeros((2, 3, 2), np.float32)
+    uvs[0] = (.25, .5); uvs[1] = (.75, .5)
+    mesh = agpt.RawMesh(verts, tri_ids=[7, 9], uvs=uvs)
+    prims = np.zeros(1, agpt.PRIM_DTYPE)
+    prims[0] = (agpt.PRIM_MESH, 0, 0, -1)
+    mat = agpt.make_material(agpt.MAT_DISNEY, (.7, .7, .7), .5, 0.)
+    xz = np.array([[0, 0], [.25, -.5], [-.3, .1], [.5, -.9]], np.float32)
+    rays7 = np.concatenate([xz[:, :1], np.full((len(xz), 1), 5), xz[:, 1:], np.tile([0, -1, 0, 1e30], (len(xz), 1))], 1).astype(np.float32)
+
+    def trace(texels):
+        img = np.repeat(np.float32([1, 1] if texels is None else texels)[None, :, None], 3, 2)
+        st = ab.AlphaScene.from_tables(prims, [mesh], materials=[mat], images=[img], bindings=[agpt.material_textures()],
+                                       masks=[agpt.alpha_mask(0, 0, .5)] if texels is not None else [])
+        return st.trace_rays(rays7), st.trace_rays(rays7, any_hit=True)
+
+    both, both_any = trace(None)
+    first, _ = trace([1, 0])
+    second, second_any = trace([0, 1])
+    none, none_any = trace([0, 0])
+    # the tie: each triangle alone is hit at the same t
+    assert both["found"].all() and first["found"].all() and second["found"].all()
+    assert np.array_equal(bits(first["t"]), bits(second["t"]))
+    assert (first["tri"] == 7).all() and (second["tri"] == 9).all()
+    for h in (first, trace([1, 1])[0]):
+        for f in ("found", "prim", "tri"):
+            assert np.array_equal(h[f], both[f]), f
+        assert np.array_equal(bits(h["t"]), bits(both["t"]))
+    assert (none["found"] == 0).all() and (none["prim"] == -1).all() and (none_any["found"] == 0).all()
+    assert both_any["found"].all() and second_any["found"].all()
 
 
 @pytest.mark.parametrize("channel", [0, 1, 2])

@@ -69,7 +69,10 @@ def outputs(agpt, ctx, d, flags):
     ctx.render(0, 2, d["max_depth"], d["depth_arg"], flags | agpt.FLAG_COUNTERS)
     film = ctx.read_accum().copy()
     st = ctx.stats()
-    rays = (st.rays_closest, st.rays_shadow, st.rays_mis, st.rays_mis_culled, st.rays_tail_culled)
+    # walk counters of both kernel kinds; not the analytic records, which sphere runs read where any lane of a warp may hit the
+    # run's box, so that past the camera rays their count depends on the order of queue appends
+    rays = (st.rays_closest, st.rays_shadow, st.rays_mis, st.rays_mis_culled, st.rays_tail_culled,
+            *[tuple(getattr(st, f)) for f in ("node_visits", "box_tests", "tri_tests")])
     hits = ctx.trace_primary(1).copy()
     ctx.render_guides(2)
     guides = ctx.read_guides()
@@ -88,13 +91,59 @@ def test_all_ones_masks_leave_every_output_unchanged(agpt, actx, cfg, level):
     assert bind_ones(agpt, actx, hs) > 0
     got = outputs(agpt, actx, d, flags)
     assert np.array_equal(bits(got[0]), bits(want[0])), "film"
-    assert got[1] == want[1], "ray counts"
+    assert got[1] == want[1], "ray counts and walk counters"
     for f in ("found", "prim", "tri"):
         assert np.array_equal(got[2][f], want[2][f]), f
     assert np.array_equal(bits(got[2]["t"]), bits(want[2]["t"]))
     for g, w in zip(got[3], want[3]):
         assert np.array_equal(bits(g), bits(w)), "guides"
     assert np.array_equal(bits(got[4]), bits(want[4])), "denoised"
+
+
+CHECKER = np.kron(np.indices((4, 4)).sum(0) % 2, np.ones((2, 2)))[..., None].repeat(3, 2).astype(np.float32)     # 8 x 8 of 0 and 1
+
+
+@pytest.mark.parametrize("cfg,level,h", [(7, 0, 54), (9, 2, 54), (10, 2, 54), (12, 0, 54), (13, 1, 54), (13, 2, 54), (13, 1, 56)])
+def test_checker_masks_beside_every_shade_variant_equal_the_statement(agpt, actx, cfg, level, h):
+    """A checker mask on every material that may carry one, appended to the scene's own images: the masked trace beside the
+    environment map (cfg 7), instances (9), glass with roulette by bounce (10), textures (12) and maps (13).  Film, ray accounting,
+    single paths, primary hits and guides equal the statement's, and the mask does remove primary hits."""
+    hs = agpt.HostScene(cfg, level)
+    d = agpt.config_defaults(cfg)
+    rr = cfg == 10
+    flags = agpt.FLAG_RR_BY_BOUNCE if rr else 0
+    images, binds, prims, n_mat = scene_textures(agpt, hs)
+    binds = binds or [agpt.material_textures() for _ in range(n_mat)]
+    excluded = {int(p[2]) for p in prims if p[0] == agpt.PRIM_SPHERE or p[3] >= 0}
+    masks = [agpt.alpha_mask(len(images), 0, .5) if i not in excluded else agpt.alpha_mask() for i in range(n_mat)]
+    assert sum(m.texture >= 0 for m in masks) > 0
+    hs.upload(actx)
+    actx.upload_material_textures(images + [CHECKER], binds)
+    actx.upload_alpha_masks(masks)
+    st = ab.AlphaScene(hs, masks=[], rr_by_bounce=rr)
+    st.set_textures(images + [CHECKER], binds)
+    st.set_masks(masks)
+    actx.set_film(W, h); actx.clear(); actx.reset_stats()
+    actx.render(0, 2, d["max_depth"], d["depth_arg"], flags | agpt.FLAG_COUNTERS)
+    s = actx.stats()
+    want, cnt = st.render(W, h, 0, 2, d["max_depth"], d["depth_arg"], counters=True)
+    assert np.array_equal(bits(actx.read_accum()[..., :3]), bits(want[..., :3])), "film"
+    assert s.rays_shadow == cnt["rays_any"]
+    assert s.rays_closest + s.rays_mis + s.rays_mis_culled + s.rays_tail_culled == cnt["rays_closest"]
+    rng = np.random.default_rng(cfg + level)
+    xs, ys, ss = rng.integers(0, W, 200), rng.integers(0, h, 200), rng.integers(0, 64, 200)
+    got = actx.li_pixels(xs, ys, ss, d["max_depth"], d["depth_arg"], flags)
+    assert np.array_equal(bits(got), bits(st.li_pixels(W, h, xs, ys, ss, d["max_depth"], d["depth_arg"]))), "paths"
+    got = actx.trace_primary(1)
+    want = st.primary_hits(W, h, 1).reshape(-1)
+    for f in ("found", "prim", "tri"):
+        assert np.array_equal(got[f], want[f]), f
+    assert np.array_equal(bits(got["t"]), bits(want["t"]))
+    bare = ab.AlphaScene(hs, masks=[]).primary_hits(W, h, 1).reshape(-1)
+    assert np.count_nonzero((bare["prim"] != want["prim"]) | (bits(bare["t"]) != bits(want["t"]))) > 50, "the mask removes primary hits"
+    actx.render_guides(2)
+    for g, w in zip(actx.read_guides(), st.guides(W, h, 2)):
+        assert np.array_equal(bits(g), bits(w)), "guides"
 
 
 @pytest.fixture(scope="module")
@@ -104,7 +153,7 @@ def cfg14(agpt):
 
 @pytest.mark.parametrize("level", [1, 2])
 @pytest.mark.parametrize("h", [54, 56])
-@pytest.mark.parametrize("depth,flags", [(1, 0), (None, 0), (None, 16)])
+@pytest.mark.parametrize("depth,flags", [(1, 0), (None, 0), (None, 16), (None, 4), (None, 4 | 16)])
 def test_cfg14_film_and_ray_accounting_equal_the_statement(agpt, actx, cfg14, level, h, depth, flags):
     hs = cfg14[level]
     d = agpt.config_defaults(14)
@@ -113,7 +162,7 @@ def test_cfg14_film_and_ray_accounting_equal_the_statement(agpt, actx, cfg14, le
     actx.render(0, 2, depth, 0, flags | agpt.FLAG_COUNTERS)
     got = actx.read_accum()
     st = actx.stats()
-    want, cnt = ab.AlphaScene(hs, rr_by_bounce=bool(flags)).render(W, h, 0, 2, depth, 0, counters=True)
+    want, cnt = ab.AlphaScene(hs, rr_by_bounce=bool(flags & agpt.FLAG_RR_BY_BOUNCE)).render(W, h, 0, 2, depth, 0, counters=True)
     assert np.array_equal(bits(got[..., :3]), bits(want[..., :3]))
     assert st.rays_shadow == cnt["rays_any"]
     assert st.rays_closest + st.rays_mis + st.rays_mis_culled + st.rays_tail_culled == cnt["rays_closest"]
@@ -147,12 +196,17 @@ def test_cfg14_paths_hits_and_guides_equal_the_statement(agpt, actx, cfg14, leve
     dirs = targets - origins
     dirs /= np.linalg.norm(dirs, axis=1, keepdims=True)
     rays7 = np.concatenate([origins, dirs, np.full((len(dirs), 1), 1e30)], 1).astype(np.float32)
-    for any_hit in (False, True):
-        got = actx.trace_rays(rays7, any_hit)
-        want = st.trace_rays(rays7, any_hit)
-        for f in ("found", "prim", "tri"):
-            assert np.array_equal(got[f], want[f]), (any_hit, f)
-        assert np.array_equal(bits(got["t"]), bits(want["t"]))
+    for flags in (0, agpt.FLAG_COUNTERS | agpt.FLAG_STRICT_BOXES):
+        for any_hit in (False, True):
+            actx.reset_stats()
+            got = actx.trace_rays(rays7, any_hit, flags)
+            want, cnt = st.trace_rays(rays7, any_hit, counters=True)
+            for f in ("found", "prim", "tri"):
+                assert np.array_equal(got[f], want[f]), (flags, any_hit, f)
+            assert np.array_equal(bits(got["t"]), bits(want["t"]))
+            if flags and not any_hit:       # the any-hit kernels count two boxes per visit: not the statement's count
+                s = actx.stats()
+                assert (s.node_visits[0], s.box_tests[0], s.tri_tests[0]) == (cnt["interior"], cnt["boxes"], cnt["tris"])
     # some of those rays pass through holes: without the masks they would all stop at the first geometric hit
     nomask = ab.AlphaScene(hs, masks=[]).trace_rays(rays7)
     assert np.count_nonzero(nomask["prim"] != actx.trace_rays(rays7)["prim"]) > 100
@@ -289,19 +343,24 @@ ZERO = np.zeros((1, 1, 3), np.float32)
 QUARTER = np.full((1, 1, 3), .25, np.float32)
 
 
-@pytest.mark.parametrize("kind", ["mesh", "instance", "plane"])
+@pytest.mark.parametrize("kind", ["mesh", "instance", "plane", "shape_lights"])
 def test_all_zero_mask_equals_the_scene_without_that_primitive(agpt, actx, cfg14, kind):
-    """A mask that keeps no hit (a constant 0, or a constant 0.25 at cutoff 0.5 on the plane) on the material of one primitive of
-    cfg 14, whose other masks stay bound: film,
-    ray counts, guides and hit tables equal those of the scene with that primitive deleted (later primitives and the lights'
-    primitive indices renumbered).  That scene runs the kernels without the mask test, so the reference here is not the statement.
-    cfg 14 level 1: the mirror quad (a plain TriangleMesh), the instance with its own material, and the grate plane."""
-    hs = cfg14[1]
-    d = agpt.config_defaults(14)
+    """A mask that keeps no hit (a constant 0, or a constant 0.25 at cutoff 0.5 on the plane) on the material of one primitive,
+    whose scene's other masks stay bound: film, ray counts, guides and hit tables equal those of the scene with that primitive
+    deleted (later primitives and the lights' primitive indices renumbered).  That scene runs the kernels without the mask test,
+    so the reference here is not the statement.  cfg 14 level 1: the mirror quad (a plain TriangleMesh), the instance with its
+    own material, and the grate plane.  cfg 11 level 2 (shape_lights): a non-emitting BVH mesh of the room lit by sampled plane
+    and mesh lights, which have no CPU statement with masks; this puts the masked trace beside the shade kernels that sample
+    shape lights."""
+    cfg = 11 if kind == "shape_lights" else 14
+    hs = agpt.HostScene(11, 2) if cfg == 11 else cfg14[1]
+    d = agpt.config_defaults(cfg)
     images, binds, _, n_mat = scene_textures(agpt, hs)
+    binds = binds or [agpt.material_textures() for _ in range(n_mat)]
     prims, lights = table_rows(agpt, hs)
-    want_type = {"mesh": agpt.PRIM_MESH, "instance": agpt.PRIM_INSTANCE, "plane": agpt.PRIM_PLANE}[kind]
-    k = int([i for i in np.nonzero(prims["type"] == want_type)[0] if np.count_nonzero(prims["material"] == prims["material"][i]) == 1][-1])
+    want_type = {"mesh": agpt.PRIM_MESH, "instance": agpt.PRIM_INSTANCE, "plane": agpt.PRIM_PLANE, "shape_lights": agpt.PRIM_BVH_MESH}[kind]
+    k = int([i for i in np.nonzero(prims["type"] == want_type)[0]
+             if prims["area_light"][i] < 0 and np.count_nonzero(prims["material"] == prims["material"][i]) == 1][-1])
     rng = np.random.default_rng(7)
     targets = np.concatenate([rng.uniform([-4, -1, -2], [4, 4.2, 5], (3000, 3)), rng.uniform([-3, 3.9, -3], [3, 4.1, 3], (1000, 3))])
     origins = np.where(targets[:, 1:2] > 3.8, np.array([.2, 5.3, .4]), np.array([.3, 2.0, -8.5]))
@@ -321,7 +380,7 @@ def test_all_zero_mask_equals_the_scene_without_that_primitive(agpt, actx, cfg14
     # masked: the scene's own masks, that primitive's replaced by one that keeps nothing (the texture indices stay as they were)
     hs.upload(actx)
     actx.upload_material_textures(images + [ZERO, QUARTER], binds)
-    masks = hs.alpha_masks()
+    masks = hs.alpha_masks() or [agpt.alpha_mask() for _ in range(n_mat)]
     masks[int(prims["material"][k])] = agpt.alpha_mask(len(images) + (1 if kind == "plane" else 0), 2, .5)
     actx.upload_alpha_masks(masks)
     got = run()

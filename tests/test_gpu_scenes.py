@@ -125,26 +125,28 @@ def test_filtered_slab_test_equals_strict(agpt, gpu_ctx, cfg, level):
 
 def test_bucketing_does_not_change_results(agpt):
     """Queue order and batching are free: without the ray-bucket pass, without the side stream,
-    with the run-ahead wave loop and with one sample per batch the film is bit-identical."""
+    with the run-ahead wave loop and with one sample per batch the film is bit-identical.  cfg 3, and
+    cfg 14 level 1, whose alpha masks put the masked any-hit kernel on the side stream."""
     import os
-    cfg, level, W, H = 3, 3, 160, 90
-    d = agpt.config_defaults(cfg)
-    hs = agpt.HostScene(cfg, level)
-    films = []
-    for env in ({"AGPT_BUCKET_RAYS": "0"}, {"AGPT_BUCKET_RAYS": "1", "AGPT_OVERLAP_ANY": "0"}, {"AGPT_ASYNC_WAVES": "1"}, {"AGPT_BATCH_LOG2": "14"}):
-        old = {k: os.environ.get(k) for k in env}
-        os.environ.update(env)
-        try:
-            ctx = agpt.Context(0)
-        finally:
-            for k, v in old.items():
-                if v is None:
-                    os.environ.pop(k, None)
-                else:
-                    os.environ[k] = v
-        hs.upload(ctx); ctx.set_film(W, H)
-        ctx.render(0, 4, d["max_depth"], d["depth_arg"])
-        films.append(ctx.read_accum())
-        ctx.close()
-    for f in films[1:]:
-        assert np.array_equal(bits(films[0]), bits(f))
+    W, H = 160, 90
+    for cfg, level in ((3, 3), (14, 1)):
+        d = agpt.config_defaults(cfg)
+        hs = agpt.HostScene(cfg, level)
+        films = []
+        for env in ({"AGPT_BUCKET_RAYS": "0"}, {"AGPT_BUCKET_RAYS": "1", "AGPT_OVERLAP_ANY": "0"}, {"AGPT_ASYNC_WAVES": "1"}, {"AGPT_BATCH_LOG2": "14"}):
+            old = {k: os.environ.get(k) for k in env}
+            os.environ.update(env)
+            try:
+                ctx = agpt.Context(0)
+            finally:
+                for k, v in old.items():
+                    if v is None:
+                        os.environ.pop(k, None)
+                    else:
+                        os.environ[k] = v
+            hs.upload(ctx); ctx.set_film(W, H)
+            ctx.render(0, 4, d["max_depth"], d["depth_arg"])
+            films.append(ctx.read_accum())
+            ctx.close()
+        for f in films[1:]:
+            assert np.array_equal(bits(films[0]), bits(f)), cfg
