@@ -12,5 +12,5 @@ from .binding import (AgptError, Context, Group, HostScene, HostTracer, Material
                       PRIM_DTYPE, SPHERE_DTYPE, PLANE_DTYPE, LIGHT_DTYPE, NODE_DTYPE, PRIM_SPHERE, PRIM_PLANE, PRIM_BVH_MESH, PRIM_MESH, PRIM_INSTANCE,
                       LIGHT_AREA, LIGHT_UNIFORM_INFINITE, LIGHT_INFINITE_AREA, LIGHT_SAMPLE_SHAPE, Adaptive, adaptive, DenoiseParams,
                       denoise_params, ReprojectParams, reproject_params, MaterialTextures, material_textures,
-                      AlphaMask, alpha_mask)
+                      AlphaMask, alpha_mask, Emission, emission)
 from . import multigpu  # noqa: F401,E402

@@ -163,6 +163,16 @@ def alpha_mask(texture=-1, channel=0, cutoff=0.5):
     return AlphaMask(texture, channel, cutoff, 0)
 
 
+class Emission(ctypes.Structure):       # agpt_emission
+    _fields_ = [("texture", c_int32), ("factor", c_float * 3)]
+
+
+def emission(texture=-1, factor=(0.0, 0.0, 0.0)):
+    """EXTENSION (agpt.h agpt_emission): one material's emission, `factor` (linear RGB, finite, >= 0) times resident texture
+    `texture` at the hit's uv, or `factor` alone for texture -1.  The material emits iff some factor component is > 0."""
+    return Emission(texture, (c_float * 3)(*factor))
+
+
 def _image_rows(images, who):
     imgs = [np.ascontiguousarray(a, np.float32) for a in images]
     for a in imgs:
@@ -309,6 +319,18 @@ class Context:
                 raise AgptError("upload_alpha_masks: need texture >= -1, channel in [0, 2] and a finite cutoff")
         table = (AlphaMask * max(len(bindings), 1))(*bindings)
         _check(core().agpt_upload_alpha_masks(self._h, table if bindings else None, c_int(len(bindings))))
+
+    def upload_emission(self, rows):
+        """EXTENSION (agpt.h agpt_upload_emission): rows[i] = material i's agpt.emission(...), naming a texture of the last
+        texture upload.  [] clears.  A texture upload clears the table."""
+        rows = list(rows)
+        for r in rows:
+            if not isinstance(r, Emission):
+                raise AgptError("upload_emission: every row must be an emission(...) row")
+            if r.texture < -1 or not all(np.isfinite(f) and f >= 0 for f in r.factor):
+                raise AgptError("upload_emission: need texture >= -1 and a finite factor >= 0")
+        table = (Emission * max(len(rows), 1))(*rows)
+        _check(core().agpt_upload_emission(self._h, table if rows else None, c_int(len(rows))))
 
     def set_camera(self, cam19):
         cam19 = np.ascontiguousarray(cam19, np.float32)
@@ -680,6 +702,12 @@ class HostScene:
         p = POINTER(AlphaMask)(); n = c_int(0)
         _check(host().agpt_host_scene_alpha_masks(self._h, byref(p), byref(n)), host_side=True)
         return [AlphaMask(p[i].texture, p[i].channel, p[i].cutoff, 0) for i in range(n.value)]
+
+    def emission(self):
+        """EXTENSION: the flattened scene's emission rows (agpt_host_scene_emission), one per material, or [] when none emits."""
+        p = POINTER(Emission)(); n = c_int(0)
+        _check(host().agpt_host_scene_emission(self._h, byref(p), byref(n)), host_side=True)
+        return [Emission(p[i].texture, (c_float * 3)(*p[i].factor)) for i in range(n.value)]
 
     def material(self, prim):
         out = np.zeros(20, np.float32)

@@ -3,6 +3,7 @@
 // the wave loop; every ray is traced and shaded on the device.  There is no CPU path: if no
 // CUDA device can be opened agpt_create() fails and the caller gets the CUDA error text.
 #include <algorithm>
+#include <climits>
 #include <cmath>
 #include <cstdio>
 #include <cstdlib>
@@ -146,6 +147,9 @@ struct agpt_ctx {
 	DevBuf<agpt_alpha_mask> masks;            // alpha masks (extension, agpt_upload_alpha_masks), per material
 	std::vector<agpt_alpha_mask> hostMasks;
 	bool hasMasks = false;        // some material has a mask: trace runs the MASK instantiations
+	DevBuf<agpt_emission> emission;           // emissive materials (extension, agpt_upload_emission), per material
+	std::vector<agpt_emission> hostEmission;
+	bool hasEmission = false;     // some row emits: k_shade_a_emit runs and tail rays are traced
 	DevBuf<agpt_light> lights;
 	DevBuf<float> envRgb, envFunc, envCdf;
 	float envFuncInt = 0;
@@ -360,6 +364,7 @@ struct LaunchPlan {
 	DShapeTables st;
 	DTexTables tt;
 	std::optional<DMaskTables> mk;  // some alpha mask is bound: the *_masked trace kernels
+	std::optional<DEmitTables> em;  // some emission row emits: k_shade_a_emit, and the path ray at max_depth is traced
 };
 
 static LaunchPlan PlanLaunches(const agpt_ctx* c) {
@@ -371,6 +376,7 @@ static LaunchPlan PlanLaunches(const agpt_ctx* c) {
 	p.tt.nTextures = (int)c->textures.n; p.tt.nTexels = (long long)c->texels.n;
 	p.tt.matMaps = c->matMaps.p; p.tt.nMatMaps = (int)c->matMaps.n;
 	if (c->hasMasks) p.mk = DMaskTables{ p.tt, c->masks.p, (int)c->masks.n };
+	if (c->hasEmission) p.em = DEmitTables{ p.tt, c->emission.p, (int)c->emission.n };
 	return p;
 }
 
@@ -412,6 +418,9 @@ static int EnsureCapacity(agpt_ctx* c, size_t paths) {
 	c->capacity = paths;
 	return AGPT_OK;
 }
+
+// agpt_upload_emission (extension): a row emits iff some factor component is > 0
+static bool Emits(const agpt_emission& e) { return e.factor[0] > 0.f || e.factor[1] > 0.f || e.factor[2] > 0.f; }
 
 // agpt_light.flags (extension): only AGPT_LIGHT_SAMPLE_SHAPE, and only on area lights
 static int CheckLightFlags(const agpt_light& l) {
@@ -471,6 +480,14 @@ static int CheckReady(agpt_ctx* c, bool needFilm) {
 			NEED(p.type != AGPT_PRIM_SPHERE, AGPT_ERR_INVALID, "an alpha mask on a sphere's material");
 			NEED(p.area_light < 0, AGPT_ERR_INVALID, "an alpha mask on an emitter's material");
 		}
+	}
+	if (c->hasEmission) {
+		// emissive materials (extension): the table belongs to the resident material table; an area light's Le and a material's
+		// emission on one shape are not defined
+		NEED(c->hostEmission.size() == (size_t)c->nMats, AGPT_ERR_INVALID, "emission rows were uploaded for a different number of materials");
+		for (const agpt_prim& p : c->hostPrims)
+			NEED(p.material < 0 || p.area_light < 0 || !Emits(c->hostEmission[p.material]), AGPT_ERR_INVALID,
+				"an emissive material on a primitive that is an area light");
 	}
 	if (c->mats.p == nullptr) {
 		// a scene of null-material (emissive) shapes only is legal upstream; shade still needs a record to point idle lanes at
@@ -551,10 +568,11 @@ static void LaunchTable(const LaunchPlan& p, uint32_t flags, bool any, cudaStrea
 		[&](auto A, auto C, auto F) { k_trace_table_masked<A, C, F><<<b, AGPT_TRACE_THREADS, 0, st>>>(sc, o, d, n, out, cnt, *p.mk); }, any);
 }
 
-// k_shade_a<ENV>: ENV, the scene has an environment map
+// k_shade_a<ENV>: ENV, the scene has an environment map; k_shade_a_emit<ENV> while an emission row emits
 static void LaunchShadeA(const LaunchPlan& p, int active, cudaStream_t st, const DScene& sc, const PathState& ps, const int* queue, const int* n, int* survivors,
 		int* survivorCount, int max_depth) {
-	WithBools([&](auto E) { k_shade_a<E><<<Blocks(active, 256), 256, 0, st>>>(sc, ps, queue, n, survivors, survivorCount, max_depth); }, p.env);
+	if (p.em) WithBools([&](auto E) { k_shade_a_emit<E><<<Blocks(active, 256), 256, 0, st>>>(sc, ps, queue, n, survivors, survivorCount, max_depth, *p.em); }, p.env);
+	else WithBools([&](auto E) { k_shade_a<E><<<Blocks(active, 256), 256, 0, st>>>(sc, ps, queue, n, survivors, survivorCount, max_depth); }, p.env);
 }
 
 // k_shade_b<ENV, GLASS, SHAPES, TEX> has ten instantiations; each carries only what it needs, or everything.
@@ -865,6 +883,7 @@ static int UploadMaterialTextures(agpt_ctx* c, const agpt_texture* textures, int
 	c->hasTextures = hasTextures; c->hasMaps = hasMaps;
 	c->hostBindings.assign(bindings, bindings + n_materials);
 	c->masks.Free(); c->hostMasks.clear(); c->hasMasks = false;     // alpha masks name textures of the old table
+	c->emission.Free(); c->hostEmission.clear(); c->hasEmission = false;     // ... and so do emission rows
 	return AGPT_OK;
 }
 int agpt_upload_textures(agpt_ctx* c, const agpt_texture* textures, int n_textures, const int32_t* material_texture, int n_materials) {
@@ -896,6 +915,27 @@ int agpt_upload_alpha_masks(agpt_ctx* c, const agpt_alpha_mask* masks, int n_mat
 	c->masks = std::move(dMasks);
 	c->hostMasks.assign(masks, masks + n_materials);
 	c->hasMasks = hasMasks;
+	return AGPT_OK;
+}
+
+// EXTENSION (agpt.h agpt_upload_emission).  Every argument is checked before anything resident changes.
+int agpt_upload_emission(agpt_ctx* c, const agpt_emission* rows, int n_materials) {
+	NEED(c != nullptr && n_materials >= 0 && (n_materials == 0 || rows != nullptr), AGPT_ERR_INVALID, "agpt_upload_emission: bad table");
+	bool hasEmission = false;
+	for (int i = 0; i < n_materials; i++) {
+		const agpt_emission& e = rows[i];
+		NEED(e.texture >= -1 && e.texture < (int)c->textures.n, AGPT_ERR_INVALID, "agpt_upload_emission: material points outside the resident textures");
+		for (float f : e.factor) NEED(std::isfinite(f) && f >= 0.f, AGPT_ERR_INVALID, "agpt_upload_emission: factor not finite or negative");
+		if (Emits(e)) hasEmission = true;
+	}
+	int rcode = BeginSceneChange(c);
+	if (rcode != AGPT_OK) return rcode;
+	DevBuf<agpt_emission> dRows;
+	CU(dRows.Upload(rows, (size_t)n_materials, c->stream));
+	CU(cudaStreamSynchronize(c->stream));
+	c->emission = std::move(dRows);
+	c->hostEmission.assign(rows, rows + n_materials);
+	c->hasEmission = hasEmission;
 	return AGPT_OK;
 }
 
@@ -949,7 +989,8 @@ int agpt_set_film(agpt_ctx* c, int width, int height) {
 int agpt_scene_bytes(agpt_ctx* c, uint64_t* out) {
 	NEED(c != nullptr && out != nullptr, AGPT_ERR_INVALID, "null argument");
 	uint64_t b = c->envRgb.Bytes() + c->envFunc.Bytes() + c->envCdf.Bytes() + c->meshes.Bytes() + c->spheres.Bytes() + c->planes.Bytes() + c->prims.Bytes() + c->instances.Bytes() + c->mats.Bytes() + c->lights.Bytes()
-		+ c->shapeLights.Bytes() + c->shapeCdf.Bytes() + c->texels.Bytes() + c->textures.Bytes() + c->matTex.Bytes() + c->matMaps.Bytes() + c->masks.Bytes();
+		+ c->shapeLights.Bytes() + c->shapeCdf.Bytes() + c->texels.Bytes() + c->textures.Bytes() + c->matTex.Bytes() + c->matMaps.Bytes() + c->masks.Bytes()
+		+ c->emission.Bytes();
 	for (auto& m : c->meshStore) b += m.nodes.Bytes() + m.tris.Bytes() + m.normals.Bytes() + m.uvs.Bytes() + m.ids.Bytes();
 	*out = b;
 	return AGPT_OK;
@@ -1158,7 +1199,11 @@ static int RunWaves(agpt_ctx* c, const Frame& f, const GenParams& g, int max_dep
 		CU(cudaMemsetAsync(q[cur ^ 1].counts, 0, 3 * sizeof(int), c->stream));
 		if (timing) CU(cudaEventRecord(c->evC, c->stream));
 		ShadeParams sp;
-		sp.count = q[cur].counts + 2; sp.max_depth = max_depth; sp.rr_depth_arg = rr_depth_arg; sp.rr_by_bounce = (flags & AGPT_FLAG_RR_BY_BOUNCE) ? 1 : 0; sp.exact_counts = count ? 1 : 0;
+		// with an emitting row bound the path ray at bounces == max_depth may hit an emitter, so k_shade_b must not cull it: it sees
+		// a depth one larger (sp.max_depth is read by that cull only), while k_shade_a still ends every path at max_depth, after its
+		// emission.  k_shade_b's code stays as it is.
+		const int shadeDepth = f.plan.em ? (max_depth == INT_MAX ? INT_MAX : max_depth + 1) : max_depth;
+		sp.count = q[cur].counts + 2; sp.max_depth = shadeDepth; sp.rr_depth_arg = rr_depth_arg; sp.rr_by_bounce = (flags & AGPT_FLAG_RR_BY_BOUNCE) ? 1 : 0; sp.exact_counts = count ? 1 : 0;
 		// shade: k_shade_a (per active entry: NEE fold, emission, termination -> survivor list),
 		// then k_shade_b (per survivor: the BSDF work), blocks striding over the list
 		CU(cudaMemsetAsync(c->survivorCount.p, 0, sizeof(int), c->stream));

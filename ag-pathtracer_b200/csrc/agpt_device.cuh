@@ -29,7 +29,8 @@ enum { AGPT_DBG_STACK = 1, AGPT_DBG_NODE = 2, AGPT_DBG_TRI = 3, AGPT_DBG_QUEUE =
        AGPT_DBG_LIST = 8 /* adaptive pixel list entry or pixel index */, AGPT_DBG_SAMPLE = 9 /* a pixel's samples past max_samples */,
        AGPT_DBG_GUIDE = 10 /* k_guides: path slot */, AGPT_DBG_TAP = 11 /* denoise, reprojection: filter or history tap outside the film */,
        AGPT_DBG_TEXTURE = 12 /* texture index of a material */, AGPT_DBG_TEXEL = 13 /* texel index of a lookup */,
-       AGPT_DBG_MAPS = 14 /* material index into the map binding table */, AGPT_DBG_MASK = 15 /* material index into the mask table */ };
+       AGPT_DBG_MAPS = 14 /* material index into the map binding table */, AGPT_DBG_MASK = 15 /* material index into the mask table */,
+       AGPT_DBG_EMIT = 16 /* material index into the emission table */ };
 #ifdef AGPT_DEBUG
 __device__ unsigned long long g_agptDebug[4];     // [0] failures, [1] first code, [2] first value, [3] checks executed
 #define AGPT_CHECK(cond, code, value) do { atomicAdd(&g_agptDebug[3], 1ull); if (!(cond)) { \
@@ -87,6 +88,12 @@ struct DMaskTables {
 	DTexTables tt;                   // the resident texels and textures (the bindings are not read)
 	const agpt_alpha_mask* masks;    // per material: {texture or -1, channel, cutoff}
 	int nMasks;
+};
+// EXTENSION: emissive materials (agpt.h agpt_upload_emission), passed to k_shade_a_emit only, beside DScene.
+struct DEmitTables {
+	DTexTables tt;                   // the resident texels and textures (the bindings are not read)
+	const agpt_emission* rows;       // per material: {texture or -1, factor}
+	int nRows;
 };
 
 struct DScene {

@@ -432,6 +432,36 @@ struct ShadeParams {
 	int exact_counts;     // AGPT_FLAG_COUNTERS: rays_mis_culled must be exact, so no MIS sample is dropped before its BSDF value is known
 };
 
+// EXTENSION: emissive materials (agpt.h agpt_upload_emission).  E of the closest hit of `path` on primitive `prim`, or false
+// when its material does not emit (null materials never do).  The uv is the one k_shade_b's surface helpers give: SphereSurface;
+// PlaneUV at O + t * D, the point PlaneSurface builds; a triangle's TriangleUVs and BaryUV, as in TriangleSurface (instances: their
+// mesh's uvs and the object-space barycentrics).  The 16-byte row is read only here, at a hit.
+__device__ __forceinline__ bool EmissionAt(const DScene& sc, const PathState& ps, const DEmitTables& em, int path, const agpt_prim& prim, float4 h,
+		float3& E) {
+	if (prim.material < 0) return false;
+	AGPT_CHECK(prim.material < em.nRows, AGPT_DBG_EMIT, prim.material);
+	const float4 r = __ldg(reinterpret_cast<const float4*>(em.rows + prim.material));
+	E = f3(r.y, r.z, r.w);
+	if (!(E.x > 0.f || E.y > 0.f || E.z > 0.f)) return false;
+	const int tex = __float_as_int(r.x);
+	if (tex < 0) return true;
+	float2 uv;
+	if (prim.type == AGPT_PRIM_SPHERE || prim.type == AGPT_PRIM_PLANE) {
+		const float4 o4 = ps.rayO[path], d4 = ps.rayD[path];
+		const float3 O = f3(o4.x, o4.y, o4.z), D = f3(d4.x, d4.y, d4.z);
+		if (prim.type == AGPT_PRIM_SPHERE) { DSurface si; SphereSurface(sc.spheres[prim.payload], O, D, h.x, si, &uv); }
+		else uv = PlaneUV(sc.planes[prim.payload], O + h.x * D);
+	}
+	else {
+		const DMesh& mesh = sc.meshes[prim.type == AGPT_PRIM_INSTANCE ? sc.instances[prim.payload].mesh : prim.payload];
+		float2 uv0, uv1, uv2;
+		TriangleUVs(mesh, ps.hitSlot[path], uv0, uv1, uv2);
+		uv = BaryUV(h.y, h.z, uv0, uv1, uv2);
+	}
+	E = E * TexLookup(em.tt, tex, uv);
+	return true;
+}
+
 // ENV: the scene has an InfiniteAreaLight; scenes without one run the leaner instantiation.
 //
 // Shade is two kernels.  Most entries of the active list need almost no work: their path left
@@ -445,10 +475,15 @@ struct ShadeParams {
 // (A single kernel with the survivors compacted through a shared-memory ring was measured too:
 // per-block rings with two barriers per round -22 % shade on cfg 3 but +10 % in closed rooms;
 // per-warp rings without barriers desynchronise the warps and stall on instruction fetch.)
-template <bool ENV>
-__global__ void __launch_bounds__(256) k_shade_a(DScene sc, PathState ps, const int* __restrict__ active, const int* __restrict__ activeCount,
-		int* __restrict__ survivors, int* survivorCount, int max_depth) {
-	const int i = blockIdx.x * blockDim.x + threadIdx.x;
+//
+// EMIT (extension, emissive materials): the body also adds the emission of the hit's material at every vertex (EmissionAt).
+// k_shade_a is <ENV, false>; k_shade_a_emit, run only while an emitting row is bound, is <ENV, true>.  tid is threadIdx.x as
+// the entry points read it: there the compiler knows its range from their launch bound, and the survivor append's shared-memory
+// indexing stays what it was.
+template <bool ENV, bool EMIT>
+__device__ __forceinline__ void ShadeA(const DScene& sc, const PathState& ps, const int* __restrict__ active, const int* __restrict__ activeCount,
+		int* __restrict__ survivors, int* survivorCount, int max_depth, const DEmitTables& em, unsigned tid) {
+	const int i = blockIdx.x * blockDim.x + tid;
 	int path = active[i];              // unconditional (allocation slack), overlaps with the count load
 	const bool valid = i < *activeCount;
 	if (!valid) path = 0;
@@ -509,6 +544,14 @@ __global__ void __launch_bounds__(256) k_shade_a(DScene sc, PathState ps, const 
 					}
 				}
 			}
+			// (2b) emissive materials (extension): at every hit, after the area-light / sky term, before the max-depth end
+			if (EMIT && found) {
+				float3 E;
+				if (EmissionAt(sc, ps, em, path, sc.prims[hitPrim], h, E)) {
+					float4 b4 = ps.beta[path];
+					L += f3(b4.x, b4.y, b4.z) * E;
+				}
+			}
 			survive = found && bounces < max_depth;     // integrator.h:150
 		}
 		if (!survive) ps.Lout[path] = make_float4(L.x, L.y, L.z, 0.f);      // the path is complete
@@ -521,17 +564,27 @@ __global__ void __launch_bounds__(256) k_shade_a(DScene sc, PathState ps, const 
 	// per warp, are what the kernel would otherwise wait for), order inside the block kept
 	__shared__ int warpBase[8];
 	__shared__ int blockBase;
-	const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+	const int lane = tid & 31, warp = tid >> 5;
 	const unsigned m = __ballot_sync(0xffffffffu, survive);
 	if (lane == 0) warpBase[warp] = __popc(m);
 	__syncthreads();
-	if (threadIdx.x == 0) {
+	if (tid == 0) {
 		int total = 0;
 		for (int w = 0; w < 8; w++) { int c = warpBase[w]; warpBase[w] = total; total += c; }
 		blockBase = total ? atomicAdd(survivorCount, total) : 0;
 	}
 	__syncthreads();
 	if (survive) survivors[blockBase + warpBase[warp] + __popc(m & ((1u << lane) - 1u))] = path;
+}
+template <bool ENV>
+__global__ void __launch_bounds__(256) k_shade_a(DScene sc, PathState ps, const int* __restrict__ active, const int* __restrict__ activeCount,
+		int* __restrict__ survivors, int* survivorCount, int max_depth) {
+	ShadeA<ENV, false>(sc, ps, active, activeCount, survivors, survivorCount, max_depth, DEmitTables(), threadIdx.x);
+}
+template <bool ENV>
+__global__ void __launch_bounds__(256) k_shade_a_emit(DScene sc, PathState ps, const int* __restrict__ active, const int* __restrict__ activeCount,
+		int* __restrict__ survivors, int* survivorCount, int max_depth, DEmitTables em) {
+	ShadeA<ENV, true>(sc, ps, active, activeCount, survivors, survivorCount, max_depth, em, threadIdx.x);
 }
 
 // The kernel is ~100 KB of SASS (IEEE division / sqrt sequences, double-precision sincos), far

@@ -31,6 +31,7 @@ static int UploadFlat(const FlatScene& flat, const Camera& camera, agpt_ctx* ctx
 	if ((rc = agpt_upload_primitives(ctx, flat.prims.data(), (int)flat.prims.size()))) return rc;
 	if ((rc = agpt_upload_material_textures(ctx, flat.textures.data(), (int)flat.textures.size(), flat.materialTextures.data(), (int)flat.materialTextures.size()))) return rc;
 	if ((rc = agpt_upload_alpha_masks(ctx, flat.alphaMasks.data(), (int)flat.alphaMasks.size()))) return rc;   // after the textures it names
+	if ((rc = agpt_upload_emission(ctx, flat.emission.data(), (int)flat.emission.size()))) return rc;          // likewise
 	agpt_camera cam = camera.Export();
 	return agpt_set_camera(ctx, &cam);
 }
@@ -111,6 +112,16 @@ int agpt_host_scene_alpha_masks(agpt_host_scene* s, const agpt_alpha_mask** out,
 		FlatScene& f = Flat(s);
 		*out = f.alphaMasks.empty() ? nullptr : f.alphaMasks.data();
 		*n = (int)f.alphaMasks.size();
+	)
+	return AGPT_OK;
+}
+
+int agpt_host_scene_emission(agpt_host_scene* s, const agpt_emission** out, int* n) {
+	if (!s || !out || !n) return HostFail("null argument");
+	HOST_TRY(
+		FlatScene& f = Flat(s);
+		*out = f.emission.empty() ? nullptr : f.emission.data();
+		*n = (int)f.emission.size();
 	)
 	return AGPT_OK;
 }

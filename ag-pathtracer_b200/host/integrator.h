@@ -60,6 +60,7 @@ public:
 			Check(agpt_upload_primitives(ctx, flat->prims.data(), (int)flat->prims.size()));
 			Check(agpt_upload_material_textures(ctx, flat->textures.data(), (int)flat->textures.size(), flat->materialTextures.data(), (int)flat->materialTextures.size()));
 			Check(agpt_upload_alpha_masks(ctx, flat->alphaMasks.data(), (int)flat->alphaMasks.size()));   // after the textures it names
+			Check(agpt_upload_emission(ctx, flat->emission.data(), (int)flat->emission.size()));          // likewise
 		}
 		uploaded = scene.Fingerprint();
 	}

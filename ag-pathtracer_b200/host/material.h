@@ -28,7 +28,14 @@ struct MaterialAlphaMask {
 	float cutoff = 0.5f;                   // the surface is there where the channel >= cutoff
 };
 
+// EXTENSION: a material's emission (include/agpt.h agpt_emission), with the image as a pointer
+struct MaterialEmission {
+	const ImageTexture* image = nullptr;   // null: constant emission
+	float3 factor = float3(0.f);           // linear RGB radiance scale; the material emits iff some component is > 0
+};
+
 #define AGPT_HAS_ALPHA_MASKS 1         // extension: Material::SetAlphaMask
+#define AGPT_HAS_EMISSION 1            // extension: Material::SetEmission
 class Material {
 public:
 	virtual ~Material() {}
@@ -44,9 +51,21 @@ public:
 		maskImage = std::move(image); mask.image = maskImage.get(); mask.channel = channel; mask.cutoff = cutoff;
 	}
 	MaterialAlphaMask AlphaMask() const { return mask; }
+	// EXTENSION (include/agpt.h agpt_upload_emission): the material emits factor, or factor * image at the hit's uv (glTF
+	// emissiveFactor x emissive strength, emissiveTexture; linear texels), wherever a path ray hits it, on a material of any type
+	// that keeps its BSDF.  Emissive materials are not lights: they are not sampled by next-event estimation.  Set it before the
+	// scene's first render, for the reason SetAlphaMask gives.
+	void SetEmission(float3 factor, std::shared_ptr<ImageTexture> image = nullptr) {
+		for (float f : { factor.x, factor.y, factor.z })
+			if (!std::isfinite(f) || f < 0.f) throw std::runtime_error("SetEmission: need a finite factor >= 0");
+		emissionImage = std::move(image); emission.image = emissionImage.get(); emission.factor = factor;
+	}
+	MaterialEmission Emission() const { return emission; }
 private:
 	std::shared_ptr<ImageTexture> maskImage;
 	MaterialAlphaMask mask;
+	std::shared_ptr<ImageTexture> emissionImage;
+	MaterialEmission emission;
 };
 
 #define AGPT_HAS_IMAGE_TEXTURES 1      // extension: DisneyMaterial(ImageTexture, roughness, metallic)

@@ -69,6 +69,7 @@ struct FlatScene {
 	std::vector<int32_t> materialTexture;      // per material: index into textures or -1 (empty when no material has one)
 	std::vector<agpt_material_textures> materialTextures;   // extension: per material, all its image bindings (empty as above)
 	std::vector<agpt_alpha_mask> alphaMasks;   // extension: per material, its alpha mask (empty when no material has one)
+	std::vector<agpt_emission> emission;       // extension: per material, its emission (empty when no material emits)
 	bool HasMaps() const { for (auto& b : materialTextures) if (b.roughness_metallic >= 0 || b.normal >= 0) return true; return false; }
 	uint64_t Bytes() const {
 		uint64_t b = prims.size() * sizeof(agpt_prim) + spheres.size() * sizeof(agpt_sphere) + planes.size() * sizeof(agpt_plane)
@@ -79,6 +80,7 @@ struct FlatScene {
 		b += materialTexture.size() * 4;
 		if (HasMaps()) b += materialTextures.size() * 32;                      // the map binding table
 		b += alphaMasks.size() * sizeof(agpt_alpha_mask);
+		b += emission.size() * sizeof(agpt_emission);
 		return b;
 	}
 };
@@ -155,6 +157,8 @@ public:
 					flat->materialTextures.push_back(b);
 					const MaterialAlphaMask am = m->AlphaMask();
 					flat->alphaMasks.push_back(agpt_alpha_mask{ index(am.image), am.channel, am.cutoff, 0 });
+					const MaterialEmission me = m->Emission();
+					flat->emission.push_back(agpt_emission{ index(me.image), { me.factor.x, me.factor.y, me.factor.z } });
 				}
 				row.material = it->second;
 			}
@@ -189,6 +193,9 @@ public:
 		bool masked = false;
 		for (auto& am : flat->alphaMasks) masked = masked || am.texture >= 0;
 		if (!masked) flat->alphaMasks.clear();
+		bool emits = false;
+		for (auto& e : flat->emission) emits = emits || e.factor[0] > 0.f || e.factor[1] > 0.f || e.factor[2] > 0.f;
+		if (!emits) flat->emission.clear();
 		for (auto& l : lights) {
 			agpt_light rec;
 			memset(&rec, 0, sizeof(rec));

@@ -47,6 +47,7 @@ inline ConfigDefaults Defaults(int config) {
 	case 12: return { 480, 270, 16, 8, 0, "cfg12_ext_procedural_image_textures" };
 	case 13: return { 480, 270, 16, 8, 0, "cfg13_ext_procedural_roughness_metallic_and_normal_maps" };
 	case 14: return { 480, 270, 16, 8, 0, "cfg14_ext_alpha_masked_cutouts" };
+	case 15: return { 480, 270, 16, 8, 0, "cfg15_ext_emissive_materials" };
 	default: return { 0, 0, 0, 0, 0, "unknown" };
 	}
 }
@@ -812,6 +813,79 @@ inline void BuildConfig14(Scene* scene, int level) {
 }
 #endif
 
+#if defined(AGPT_HAS_EMISSION) && defined(AGPT_HAS_ALPHA_MASKS) && defined(AGPT_HAS_MATERIAL_MAPS)
+// cfg 15 (EXTENSION, host mirror only -- the reference's only emitters are AreaLights around null-material shapes): emissive
+// materials (include/agpt.h agpt_upload_emission) in a closed room, laid out so every uv rule of the emission lookup is used:
+// - a screen: a BVHTriMesh of 2 x 2 quads with uvs over [0, 2]^2 (repeat wrap), a colour-bar / checker image as its emission
+//   and as the base colour of the glossy Disney material under it (a BVHTriMesh of only two triangles flattens to a two-entry
+//   node table, which agpt_upload_meshes refuses);
+// - a constant-emission Disney sphere, and a factor-only emissive Plane strip under the ceiling;
+// - a small icosphere (default uvs) placed twice as Instances, its emission a striped image;
+// - a mirror on the side wall that sees the screen (specular chains).
+// Level 1 lights the room with one sphere AreaLight as well, so next-event estimation and emission combine.  Level 2 has no
+// light at all (every path runs with n_lights == 0) and adds an emissive sign whose letters are cut out by an alpha mask (the
+// mask image is also its emission image).
+inline std::shared_ptr<ImageTexture> ColourBars(int W, int H) {
+	static const float bars[7][3] = { { .75f, .75f, .75f }, { .75f, .75f, 0 }, { 0, .75f, .75f }, { 0, .75f, 0 }, { .75f, 0, .75f }, { .75f, 0, 0 }, { 0, 0, .75f } };
+	std::vector<float> rgb(3 * (size_t)W * H);
+	for (int y = 0; y < H; y++)
+		for (int x = 0; x < W; x++) {
+			float* p = &rgb[3 * ((size_t)y * W + x)];
+			if (y < H / 3) { const float c = ((x / 4 + y / 4) & 1) ? 1.f : .05f; p[0] = c; p[1] = c; p[2] = c; }   // checker (row 0: v near 0)
+			else { const float* b = bars[(x * 7) / W]; p[0] = b[0]; p[1] = b[1]; p[2] = b[2]; }
+		}
+	return ImageTexture::Make(W, H, std::move(rgb));
+}
+inline std::shared_ptr<ImageTexture> SignLetters(int W, int H) {
+	std::vector<float> rgb(3 * (size_t)W * H);
+	for (int y = 0; y < H; y++)
+		for (int x = 0; x < W; x++) {
+			const int cx = x % 8, cy = y % 16, letter = x / 8;
+			// blocky strokes: a left bar, and a top, middle or bottom bar that changes from letter to letter
+			const bool on = cx == 1 || cx == 2 || ((cy == 2 || cy == 3) && letter % 2 == 0) || ((cy == 7 || cy == 8) && letter % 3 != 1) ||
+				((cy == 12 || cy == 13) && cx < 6) || (cx == 5 && letter % 2 == 1 && cy > 2 && cy < 13);
+			float* p = &rgb[3 * ((size_t)y * W + x)];
+			p[0] = on ? 1.f : 0.f; p[1] = on ? .5f + .5f * (float)letter / (W / 8) : 0.f; p[2] = on ? .25f : 0.f;
+		}
+	return ImageTexture::Make(W, H, std::move(rgb));
+}
+inline void BuildConfig15(Scene* scene, int level) {
+	auto wallMat = DisneyMaterial::Make(float3(.7f, .68f, .65f), .9f, 0.f);
+	scene->primitives.push_back(MakeRoom(float3(-5.f, -1.f, -6.f), float3(5.f, 5.f, 6.f), wallMat));
+	auto bars = ColourBars(64, 48);
+	auto screenMat = DisneyMaterial::Make(bars, .25f, 0.f);
+	screenMat->SetEmission(float3(2.f, 2.f, 2.f), bars);
+	scene->primitives.push_back(std::make_shared<BVHTriMesh>(MakeQuadGrid(2, 2.5f, float3(0, 1.35f, 5.5f), screenMat), screenMat, 1));
+	auto ballMat = DisneyMaterial::Make(float3(.8f, .3f, .2f), .5f, 0.f);
+	ballMat->SetEmission(float3(1.5f, .6f, .2f));
+	scene->primitives.push_back(std::make_shared<Sphere>(float3(2.6f, -.2f, 2.f), .8f, ballMat));
+	auto stripMat = DisneyMaterial::Make(float3(.9f, .9f, .9f), .8f, 0.f);
+	stripMat->SetEmission(float3(4.f, 4.f, 4.5f));
+	scene->primitives.push_back(std::make_shared<Plane>(float3(0, 4.9f, 1.f), float2(3.f, .2f), stripMat));
+	auto icoMat = DisneyMaterial::Make(float3(.2f, .5f, .8f), .4f, 0.f);
+	icoMat->SetEmission(float3(1.f, 1.f, 1.f), ProceduralTexture(64, 1, 2));
+	auto unit = std::make_shared<BVHTriMesh>(MakeIcosphere(2, float3(0, 0, 0), 1.f, icoMat), icoMat, 1);
+	scene->primitives.push_back(std::make_shared<Instance>(unit, mat4::Translate(-2.6f, -.5f, 1.5f) * mat4::Scale(.5f), icoMat));
+	scene->primitives.push_back(std::make_shared<Instance>(unit, mat4::Translate(-.9f, -.6f, -.5f) * mat4::RotateY(.6f) * mat4::Scale(.4f), icoMat));
+	auto mirror = MirrorMaterial::Make(float3(.9f, .9f, .9f));
+	scene->primitives.push_back(MakeQuad(float3(-4.8f, -.5f, -1.f), float3(0, 0, 4.5f), float3(0, 3.5f, 0), true, mirror));
+	if (level >= 2) {
+		auto letters = SignLetters(48, 16);
+		auto signMat = DisneyMaterial::Make(float3(.1f, .1f, .12f), .6f, 0.f);
+		signMat->SetAlphaMask(letters, 0, .5f);
+		signMat->SetEmission(float3(3.f, 1.2f, .4f), letters);
+		scene->primitives.push_back(MakeQuad(float3(-1.5f, 3.1f, 4.f), float3(3.f, 0, 0), float3(0, 1.f, 0), true, signMat));
+	}
+	else scene->addAreaLight(std::make_shared<Sphere>(float3(0, 4.2f, 0), .35f, nullptr), WarmWhite(60));
+	scene->camera.lookfrom = float3(.5f, 1.6f, -5.5f);
+	scene->camera.lookat = float3(-.3f, 1.2f, 3.f);
+	scene->camera.vup = float3(0, 1, 0);
+	scene->camera.aspect_ratio = 16.f / 9.f;
+	scene->camera.vfov = 60;
+	scene->camera.aperture = 0;
+}
+#endif
+
 // level <= 0 selects the BASELINE.json size of each configuration.
 inline bool BuildConfig(Scene* scene, int config, int level) {
 	switch (config) {
@@ -840,6 +914,9 @@ inline bool BuildConfig(Scene* scene, int config, int level) {
 #endif
 #if defined(AGPT_HAS_ALPHA_MASKS) && defined(AGPT_HAS_MATERIAL_MAPS)
 	case 14: BuildConfig14(scene, level > 0 ? level : 1); return true;
+#endif
+#if defined(AGPT_HAS_EMISSION) && defined(AGPT_HAS_ALPHA_MASKS) && defined(AGPT_HAS_MATERIAL_MAPS)
+	case 15: BuildConfig15(scene, level > 0 ? level : 1); return true;
 #endif
 	default: return false;
 	}

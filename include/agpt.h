@@ -202,7 +202,9 @@ typedef struct agpt_stats {
 	uint64_t rays_mis_culled;  /* MIS rays the reference traces but that provably cannot reach their light: not traced, not counted above.
 	                            * Exact in renders made with AGPT_FLAG_COUNTERS; otherwise an upper bound (such samples are dropped before their BSDF
 	                            * value is known, and the reference does not trace a sample whose value is black) */
-	uint64_t rays_tail_culled; /* path rays the reference traces at bounces == MaxDepth and then discards (integrator.h:139,150): not traced, not counted above */
+	uint64_t rays_tail_culled; /* path rays the reference traces at bounces == MaxDepth and then discards (integrator.h:139,150): not traced, not counted above.
+	                            * 0 while an emitting row is bound (agpt_upload_emission): those rays may hit an emitter, so they are traced and
+	                            * counted in rays_closest */
 	/* traversal work, only counted with AGPT_FLAG_COUNTERS; [0] closest-hit kernel, [1] any-hit kernel */
 	uint64_t node_visits[2];   /* interior sibling pairs fetched (64 B each) */
 	uint64_t box_tests[2];
@@ -367,6 +369,38 @@ typedef struct agpt_alpha_mask {
 	int32_t pad;
 } agpt_alpha_mask;
 int agpt_upload_alpha_masks(agpt_ctx* ctx, const agpt_alpha_mask* masks, int n_materials);
+
+/* ---- emissive materials (EXTENSION: glTF emissiveFactor / emissiveTexture, KHR_materials_emissive_strength folded into the
+ * factor; the reference's only emitters are AreaLights around null-material shapes) ---------------------------------------
+ * rows[i] belongs to material i of any type (Disney, mirror, glass); the material keeps its BSDF.  A row EMITS iff some factor
+ * component is > 0.  Its emitted radiance at a hit, in float32 with every operation rounded on its own:
+ *   texture < 0:  E = factor;
+ *   otherwise:    E_c = factor_c * T_c, T = the lookup (agpt_upload_textures step 2: bilinear, repeat-wrapped, nested lerp) of
+ *                 resident texture `texture` at the hit's uv (agpt_upload_textures step 1: sphere, plane, triangle; instances
+ *                 through their mesh's uvs).  Texels are linear (no sRGB decode).  Emission is two-sided.
+ * The one new term of Li: at every vertex where the path ray has a closest hit, at bounce indices 0 .. max_depth whatever
+ * specularBounce says, on a primitive whose material >= 0 emits, L = L + beta * E -- after that vertex's area-light / sky term
+ * and before the bounces >= maxDepth break.  Skip-through (null-material) hits never emit, and candidates an alpha mask
+ * rejects are not hits.  No random number is drawn: every path's draws stay where they were.
+ * Emissive materials are not lights: they are not in the light list, UniformSampleOneLight never picks them, and a shadow or
+ * MIS ray that hits one sees an occluder as before.  Their light reaches other surfaces only through BSDF-sampled
+ * continuations: unbiased, but noisier than next-event estimation for small bright emitters.  Because the path ray at
+ * bounces == max_depth may now hit an emitter, it is traced while an emitting row is bound (it counts in rays_closest, and
+ * rays_tail_culled stays 0).
+ * Refused with AGPT_ERR_INVALID, leaving the resident table as it was: n_materials < 0, rows == NULL with n_materials > 0, a
+ * texture outside [-1, resident textures), a factor component that is not finite or is < 0.  (NULL, 0) clears the table, and
+ * so does every successful texture upload (the indices name the old table).  Like every upload it makes the guides stale and
+ * drops the saved reprojection view.  At render time (with an emitting row bound) n_materials must equal the resident
+ * material count, and no primitive whose material emits may have area_light >= 0 (an area light's Le and a material's
+ * emission on one shape are not defined), else AGPT_ERR_INVALID.  agpt_scene_bytes counts the table (16 bytes per material).
+ * agpt_render_guides ignores emission: the albedo guide stays the reflectance.  agpt_render, agpt_li_pixels, agpt_li_rays,
+ * adaptive rendering and agpt_render_multi all include the term.  Scenes without an emitting row run the shade kernels they ran
+ * before.  statements/agpt_emission_oracle.cpp states the same on the CPU. */
+typedef struct agpt_emission {
+	int32_t texture;   /* index into the resident textures, or -1: constant emission */
+	float factor[3];   /* linear RGB radiance scale (glTF emissiveFactor x emissive strength); finite, >= 0 */
+} agpt_emission;     /* 16 bytes */
+int agpt_upload_emission(agpt_ctx* ctx, const agpt_emission* rows, int n_materials);
 
 int agpt_set_camera(agpt_ctx* ctx, const agpt_camera* camera);          /* Camera, camera.h:38-56 */
 int agpt_set_film(agpt_ctx* ctx, int width, int height);                /* Accumulator(w,h), myapp.h:10-13 */

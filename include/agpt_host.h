@@ -25,7 +25,8 @@ typedef struct agpt_host_tracer agpt_host_tracer;
 const char* agpt_host_last_error(void);
 
 /* config 1..5 = BASELINE.json configs[0..4]; 6 and 8 = test-only corner-case scenes, 7 = the reference default scene;
- * 9..14 = extension scenes of the host mirror (12: procedural image textures; 13: roughness-metallic and normal maps; 14: alpha masks);
+ * 9..15 = extension scenes of the host mirror (12: procedural image textures; 13: roughness-metallic and normal maps; 14: alpha masks;
+ * 15: emissive materials);
  * level <= 0 picks the configuration's own icosphere subdivision level. */
 int agpt_host_scene_create(int config, int level, agpt_host_scene** out);
 int agpt_host_scene_destroy(agpt_host_scene* scene);
@@ -58,6 +59,9 @@ int agpt_host_scene_tables(agpt_host_scene* scene, agpt_scene_tables* out);
 /* extension: the flattened scene's alpha masks (agpt_upload_alpha_masks), one row per material, or (NULL, 0) when no material
  * has one; the texture indices name agpt_scene_tables.textures.  Valid while the scene lives. */
 int agpt_host_scene_alpha_masks(agpt_host_scene* scene, const agpt_alpha_mask** out, int* n);
+/* extension: the flattened scene's emission rows (agpt_upload_emission), one per material, or (NULL, 0) when no material
+ * emits; the texture indices name agpt_scene_tables.textures.  Valid while the scene lives. */
+int agpt_host_scene_emission(agpt_host_scene* scene, const agpt_emission** out, int* n);
 
 /* exports for comparison with the oracle's view of the same scene (oracle/ref_harness.cpp) */
 int agpt_host_camera_export(agpt_host_scene* scene, float* out19);
